@@ -25,6 +25,8 @@ One "step" = one pass of the hot path (waveguide -> resampler -> PCM) over the w
   cpu_baseline : the CPU oracle (a C restatement of the reference, kind "port"), one utterance per thread on all host
               cores, on a bounded sample of the same workload.
 --impl reference runs only that CPU arm, sized to finish in minutes, and prints its own JSON line.
+--dump-outputs DIR writes what the headline's resident path computed in its last timed step (see dump_outputs) as .npy
+files, so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import ctypes as C
@@ -140,6 +142,34 @@ class ClockSampler(object):
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 60 * 10 ** 6          # a dump stays below 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir, res, maxima, seed=0):
+    """Writes what a caller of the resident path receives after its last step: every utterance's maximum sample value
+    (maxima.npy) and, for whole utterances drawn in a fixed seeded order while the files stay within DUMP_BYTES, their
+    output-rate samples (samples.npy, in the precision mode's type) and PCM16 values (pcm.npy, as float32), back to back;
+    utterances.npy and number_samples.npy say which utterances and how many samples each."""
+    os.makedirs(out_dir, exist_ok=True)
+    picks, lengths, samples, pcm = [], [], [], []
+    size = maxima.nbytes
+    for u in np.random.default_rng(seed).permutation(res.batch.n):
+        smp, p, _ = res.fetch_utterance(int(u))
+        cost = smp.nbytes + 4 * p.size + 16
+        if size + cost > DUMP_BYTES:
+            break
+        size += cost
+        picks.append(int(u))
+        lengths.append(smp.shape[0])
+        samples.append(smp)
+        pcm.append(p.astype(np.float32))
+    arrays = {"maxima": maxima, "utterances": np.array(picks, np.float64), "number_samples": np.array(lengths, np.float64),
+              "samples": np.concatenate(samples) if samples else np.zeros(0, res.batch.sample_dtype),
+              "pcm": np.concatenate(pcm) if pcm else np.zeros(0, np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def oracle_throughput(ip, n_frames, n_utt, threads, seed, first_index):
     """Times the CPU oracle (one utterance per thread) on n_utt utterances of the workload; returns
     (audio_s_per_s, seconds)."""
@@ -246,7 +276,13 @@ def main():
     ap.add_argument("--no-fast-mode", action="store_true", help="skip the FP32 fast-mode measurement of the headline")
     ap.add_argument("--no-configs", action="store_true", help="skip the all-configs section (N = 1)")
     ap.add_argument("--also-fp32", action="store_true", help=argparse.SUPPRESS)      # (round-1 flag; fast_mode is the default now)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's outputs of its last timed step to DIR/*.npy "
+                                                          "(rank 0; configs 0-3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == 4):
+        ap.error("--dump-outputs writes the outputs of the batched GPU path (configs 0-3)")
 
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -400,8 +436,9 @@ def main():
             out["tolerance"] = ">= 80 dB SNR, +-1 LSB"
         return out
 
-    def measure_batch(precision, ips, n_frames, frames, steps, warmup, e2e_mode, with_clocks=True):
-        """e2e_mode: None, "blocking" (one TRMBatchSynthesize per step) or "pipelined" (async, 3 in flight, + blocking)"""
+    def measure_batch(precision, ips, n_frames, frames, steps, warmup, e2e_mode, with_clocks=True, dump_dir=None):
+        """e2e_mode: None, "blocking" (one TRMBatchSynthesize per step) or "pipelined" (async, 3 in flight, + blocking).
+        dump_dir: where dump_outputs writes the resident path's outputs of the last timed step (None: nowhere)."""
         prec = g.TRM_PRECISION_FP64 if precision == "fp64" else g.TRM_PRECISION_FP32
         n_utt = len(n_frames)
         batch = g.TRMBatch(ips, n_frames, precision=prec)
@@ -440,6 +477,8 @@ def main():
         value = audio_all / (ms_per_step * 1e-3)
         maxima = np.zeros(n_utt, np.float64)
         res.fetch(None, None, maxima, None)
+        if dump_dir:
+            dump_outputs(dump_dir, res, maxima)
         fetched = {u: res.fetch_utterance(u) for u in picks}          # the timed batch's own results
         res.free()
         parity = check_against_oracle(precision, ips, frames.array, n_frames, picks, lambda u: fetched[u][0],
@@ -538,9 +577,10 @@ def main():
         return dict(value=value, ms_per_step=ms_per_step, stage_ms=stage_ms, clocks=clocks, e2e=e2e, lay=lay,
                     audio_all=audio_all, parity=parity, launches=3 * steps)
 
-    def measure_sweep(precision, n_total):
+    def measure_sweep(precision, n_total, steps=1):
         """configs[4]: ONE fixed set of n_total x 2 s utterances (walk2 tracks generated on the device, audio reduced to
-        checksums on the device), sharded over the ranks by contiguous index ranges: strong scaling."""
+        checksums on the device), sharded over the ranks by contiguous index ranges: strong scaling.  One step = one sweep
+        over the whole set; `ms_total` is the time of one sweep, averaged over the `steps` timed sweeps."""
         prec = g.TRM_PRECISION_FP64 if precision == "fp64" else g.TRM_PRECISION_FP32
         ip = g.TRMInputParameters(44100.0)
         nf = 501
@@ -554,13 +594,16 @@ def main():
         torch.cuda.synchronize()
         sampler.start()
         t0 = time.perf_counter()
-        r = g.sweep_synthesize(ip, nf, n_local, seed=args.seed, first_index=lo, precision=prec, device=local_rank, probes=probes)
+        kern = 0.0
+        for _ in range(steps):
+            r = g.sweep_synthesize(ip, nf, n_local, seed=args.seed, first_index=lo, precision=prec, device=local_rank, probes=probes)
+            kern += r["kernel_ms"] * 1e-3
         torch.cuda.synchronize()
-        wall = time.perf_counter() - t0
+        wall = (time.perf_counter() - t0) / steps
         barrier()
         clocks = sampler.stop()
         wall = max_over_ranks(wall)
-        kern = max_over_ranks(r["kernel_ms"] * 1e-3)
+        kern = max_over_ranks(kern / steps)
         audio = float(n_total) * (nf - 1) / 250.0
         with np.errstate(over="ignore"):
             cs = int(r["checksums"].sum(dtype=np.uint64))
@@ -586,7 +629,7 @@ def main():
                 "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 16 * n_total,
                 "api": "TRMSweepSynthesize (include/trm.h): tracks generated on the device from (seed, index), per-utterance PCM checksum "
                        "and maximum back; wall clock around the call, all chunks"},
-                "utterances": n_total, "utterances_this_rank": n_local, "audio_seconds": audio, "launches": r["launches"],
+                "utterances": n_total, "utterances_this_rank": n_local, "audio_seconds": audio, "launches": r["launches"] * steps,
                 "checksum_of_checksums": "0x%016x" % cs, "clocks": clocks,
                 "parity": {"checked_utterances": [lo + int(u) for u in r["probes"]], "max_pcm_lsb": worst,
                            "against": "CPU oracle on TRMWorkloadWalk2 (the host twin of the device generator)", "tolerance": "+-1 LSB, maxima"},
@@ -598,11 +641,11 @@ def main():
     headline_cfg = args.config
     fast = None
     if headline_cfg == 4:
-        r4 = measure_sweep(args.precision, args.sweep_utterances)
-        f4 = None if args.no_fast_mode or args.precision == "fp32" else measure_sweep("fp32", args.sweep_utterances)
+        r4 = measure_sweep(args.precision, args.sweep_utterances, args.steps)
+        f4 = None if args.no_fast_mode or args.precision == "fp32" else measure_sweep("fp32", args.sweep_utterances, args.steps)
         if rank == 0:
             line = {
-                "metric": METRIC, "value": r4["value"], "unit": UNIT, "n_gpus": world, "steps": 1, "warmup": 1,
+                "metric": METRIC, "value": r4["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": 1,
                 "ms_per_step": r4["ms_total"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": "f64" if args.precision == "fp64" else "f32", "data": "synthetic",
                 "config": {"workload": "configs[4]: %d synthetic 2 s utterances (walk2 random-walk tracks generated on the device, male voice, "
@@ -629,7 +672,8 @@ def main():
 
     name, ips, n_frames, frames = build_workload(g, W, headline_cfg, rank, args)
     e2e_mode = None if args.no_e2e else "pipelined"
-    r = measure_batch(args.precision, ips, n_frames, frames, args.steps, args.warmup, e2e_mode)
+    r = measure_batch(args.precision, ips, n_frames, frames, args.steps, args.warmup, e2e_mode,
+                      dump_dir=args.dump_outputs if rank == 0 else None)
     lay = r["lay"]
     roofline, roofline_src, roofline_pcm = rooflines(args.precision, lay, r["stage_ms"])
     if not args.no_fast_mode and args.precision == "fp64":

@@ -4,8 +4,13 @@ Run in the build container (where /root/reference is mounted):   python tests/go
 
 Every vector is produced by the CPU oracle (oracle/trm_oracle.c) AND, for the tube-rate signal, checked here
 against the REFERENCE'S OWN compiled C (Applications/TRAcT/tube.c via oracle/_ref/tube_ref) before it is
-written; the agreement (max relative difference) is stored next to each vector.  The reference ships no
+written; the agreement (max relative difference) is stored next to each vector, together with the reference's FIR
+coefficients (ref_fir) and its controlPeriod, sampleRate, numberTaps and padSize (ref_derived).  The reference ships no
 golden audio of its own (SURVEY.md section 4), so these files are the pinned contract.
+
+ref_fir and ref_derived of static_aa_44k, walk_44k, walk_short_tube_down and walk_sine_nomod were added to the file after
+it was first written, from the oracle: tests/test_oracle.py had found the compiled reference equal to the oracle in exactly
+these values for these four cases, and the oracle code that computes them has not changed since.
 """
 import os
 import sys
@@ -59,6 +64,10 @@ def main():
         out[name + "/max"] = np.array([r.maximumSampleValue])
         out[name + "/pcm"] = O.pcm16(ip, r.samples, r.maximumSampleValue)
         out[name + "/ref_agreement"] = np.array([agree, src_agree])
+        derived = [ref["controlPeriod"], ref["sampleRate"], ref["numberTaps"], ref["padSize"]]
+        assert derived == [r.info.controlPeriod, r.info.sampleRate, r.info.numberTaps, r.info.padSize], name
+        out[name + "/ref_fir"] = ref["fir"]
+        out[name + "/ref_derived"] = np.array(derived, np.int32)
         print("%-22s frames %3d tube %6d out %6d  oracle-vs-compiled-reference: tube %.2e  src(float) %.2e" % (
             name, frames.shape[0], r.tube.size, r.numberSamples, agree, src_agree))
     np.savez_compressed(os.path.join(HERE, "trm_golden.npz"), **out)

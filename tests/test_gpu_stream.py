@@ -100,19 +100,21 @@ def test_down_sampling_voice_streams_too(precision):
 import oracle_lib as O  # noqa: E402
 
 
-@pytest.mark.skipif(not O.have_reference_binary(), reason="oracle/_ref/tube_ref not built (needs /root/reference)")
 @pytest.mark.parametrize("case", ["walk_44k", "walk_short_tube_down"])
 def test_stream_against_the_reference_float_stream(case):
-    """TRAcT's mode of use, checked against the reference itself: oracle/_ref/tube_ref is Applications/TRAcT/tube.c
-    compiled unmodified; its converter (dataFill / dataEmpty, tube.c:2348-2521) emits the un-normalised FLOAT stream TRAcT
-    plays (tube.c:1096-1191).  TRMStream, fed the same frames in small pushes, must return that stream -- to the float
-    precision tube.c emits (2e-7 of peak, as tests/test_oracle.py uses for the same comparison)."""
+    """TRAcT's mode of use, checked against the reference itself: Applications/TRAcT/tube.c's converter (dataFill /
+    dataEmpty, tube.c:2348-2521) emits the un-normalised FLOAT stream TRAcT plays (tube.c:1096-1191).  The golden vectors
+    hold that stream: tests/golden/make_golden.py ran the compiled tube.c on these frames and recorded that the stored
+    samples, rounded to float, were identical to its output (ref_agreement[1] == 0).  TRMStream, fed the same frames in
+    small pushes, must return that stream -- to the float precision tube.c emits (2e-7 of peak, as tests/test_oracle.py
+    uses for the same comparison)."""
     import os
     g = _g()
     z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "trm_golden.npz"))
     oip = O.OracleInputParameters.from_buffer_copy(bytes(z[case + "/ip"]))
     frames = z[case + "/frames"]
-    ref = O.run_reference(oip, frames)
+    assert z[case + "/ref_agreement"][1] == 0.0
+    ref_out = z[case + "/samples"].astype(np.float32)
     ip = g.TRMInputParameters(float(oip.outputRate))
     for name, _ in oip._fields_:
         if hasattr(ip, name):
@@ -128,6 +130,6 @@ def test_stream_against_the_reference_float_stream(case):
         at += m
     st.free()
     y = np.concatenate(parts)
-    assert y.shape[0] == ref["out"].shape[0]
-    peak = float(np.abs(ref["out"]).max())
-    assert np.abs(y.astype(np.float32) - ref["out"]).max() <= 2e-7 * peak
+    assert y.shape[0] == ref_out.shape[0]
+    peak = float(np.abs(ref_out).max())
+    assert np.abs(y.astype(np.float32) - ref_out).max() <= 2e-7 * peak
