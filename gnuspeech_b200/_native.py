@@ -135,6 +135,12 @@ def lib():
     sig("TRMStreamCapacity", i64, vp)
     sig("TRMStreamPush", C.c_int, vp, vp, C.c_int, C.c_int, vp, vp)
     sig("TRMStreamFree", None, vp)
+    sig("TRMStreamPoolCreate", vp, C.c_int, C.c_int, C.c_int, C.c_int, P(C.c_int))
+    sig("TRMStreamPoolOpen", C.c_int, vp, vp)
+    sig("TRMStreamPoolClose", C.c_int, vp, C.c_int)
+    sig("TRMStreamPoolSlotCapacity", i64, vp)
+    sig("TRMStreamPoolPush", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp)
+    sig("TRMStreamPoolFree", None, vp)
     sig("TRMBatchSynthesizeAsync", vp, vp, vp, vp, vp, vp, C.c_int, vp)
     sig("TRMBatchWait", C.c_int, vp)
     sig("TRMBatchMakeResident", vp, vp, vp, C.c_int, P(C.c_int))

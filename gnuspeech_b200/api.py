@@ -535,6 +535,61 @@ class TRMStream(object):
         self.free()
 
 
+class TRMStreamPool(object):
+    """Streaming slots that open, advance and end independently, each with its own voice (TRMStreamPoolCreate / Open /
+    Push / Close): a server's requests arrive at different times with different voices, and one push advances any subset
+    of them, each by its own number of frames, with one waveguide and one resampler launch.  Each slot's pushes,
+    concatenated, equal the one-shot synthesis of its utterance bit for bit.  Used by one thread at a time."""
+
+    def __init__(self, capacity, precision=N.TRM_PRECISION_FP64, max_frames_per_push=64, device=0):
+        err = C.c_int(0)
+        self.capacity = capacity
+        self.max_frames_per_push = max_frames_per_push
+        self.dtype = np.float64 if precision != N.TRM_PRECISION_FP32 else np.float32
+        self._h = N.lib().TRMStreamPoolCreate(capacity, precision, max_frames_per_push, device, C.byref(err))
+        if not self._h:
+            check(err.value or N.TRM_ERR_CUDA, "TRMStreamPoolCreate")
+
+    def open(self, ip):
+        """Opens a free slot with voice `ip` (a TRMInputParameters); returns the slot number."""
+        slot = N.lib().TRMStreamPoolOpen(self._h, C.byref(ip))
+        if slot < 0:
+            check(slot, "TRMStreamPoolOpen")
+        return slot
+
+    def close(self, slot):
+        """Abandons an open slot without its tail; the slot becomes free."""
+        check(N.lib().TRMStreamPoolClose(self._h, slot), "TRMStreamPoolClose")
+
+    def slot_capacity(self):
+        return int(N.lib().TRMStreamPoolSlotCapacity(self._h))
+
+    def push(self, frames, flush=()):
+        """frames: {slot: (m, 16) float64} (m may be 0); flush: slots that end with this push.  Returns {slot: samples}
+        for every slot named in `frames` or `flush`."""
+        slots = list(frames.keys()) + [s for s in flush if s not in frames]
+        parts = [np.ascontiguousarray(frames.get(s, np.zeros((0, 16))), dtype=np.float64).reshape(-1, 16) for s in slots]
+        n = len(slots)
+        slot_a = np.array(slots, dtype=np.int32)
+        nf_a = np.array([p.shape[0] for p in parts], dtype=np.int32)
+        fl = set(flush)
+        flush_a = np.array([1 if s in fl else 0 for s in slots], dtype=np.uint8)
+        allf = np.concatenate(parts) if parts else np.zeros((0, 16))
+        out = np.zeros(max(1, n * self.slot_capacity()), self.dtype)
+        off = np.zeros(n + 1, np.int64)
+        check(N.lib().TRMStreamPoolPush(self._h, n, _ptr(slot_a), _ptr(nf_a), _ptr(allf) if allf.shape[0] else None,
+                                        _ptr(flush_a), _ptr(out), _ptr(off)), "TRMStreamPoolPush")
+        return {s: out[off[i]:off[i + 1]].copy() for i, s in enumerate(slots)}
+
+    def free(self):
+        if self._h:
+            N.lib().TRMStreamPoolFree(self._h)
+            self._h = None
+
+    def __del__(self):
+        self.free()
+
+
 class TRMBatchTicket(object):
     """Handle of an asynchronous TRMBatch call; keeps the call's buffers alive until wait() returns."""
 

@@ -42,7 +42,8 @@ constexpr int STATE_HE = 0, STATE_HO = 24, STATE_XM = 48, STATE_SER = 50;
 inline size_t tube_state_bytes(size_t esz) { return STATE_HDR * 8 + STATE_R * esz; }
 
 struct TubeArgs {
-    void *state;                 // streaming: [n_utt] carried states (loaded at start, stored at the end), else null
+    void *state;                 // streaming: carried states indexed like desc (loaded at the start, stored after each
+                                 // utterance's last block), else null
     const trm_cuda_utterance *desc;
     const int *order;            // slot -> utterance (longest first), may be null
     int n_utt;
@@ -72,6 +73,38 @@ struct SrcArgs {
     int n_tiles;
     long long total_items;
     long long item_begin, item_end;  // work items this launch processes ([0, total_items) when item_end == 0)
+};
+
+// Resampler of a stream pool (src_pool_kernel): entries are slots at independent positions.  desc[e] is the resampler view
+// of entry e: outputs [out_start, n_out) of its stream are produced and written to out[out_offset + (n - out_start)]
+// (packed, entry after entry); input sample q of the stream is tube[tube_offset + q], valid for q in [in_start, n_tube).
+struct SrcPoolArgs {
+    const trm_cuda_utterance *desc;
+    int n;
+    const long long *item_base;      // [n+1] prefix sum of work items (runs of 32 consecutive outputs of one entry)
+    long long total_items;
+    const void *tube;                // Real[]
+    void *out;                       // Real[]
+    const void *table;               // HD<Real>[256][13] (down-sampling phase walk)
+    const void *ctab;                // Real[65536][SRC_CLD] (up-sampling coefficient rows)
+};
+
+// Per-push bookkeeping kernels of a stream pool (kernels_aux.cu)
+struct PoolPrepArgs {
+    const trm_cuda_utterance *src;   // [n] waveguide descriptors of this push
+    const int *slot;                 // [n] slot of each
+    const int *reset;                // [n] != 0: the slot was opened since its last launch, its carried state starts fresh
+    trm_cuda_utterance *dst;         // [capacity] descriptor array the waveguide indexes by slot
+    void *state;                     // [capacity] carried states
+    unsigned long long state_bytes;
+    unsigned long long noise_k0;
+    int n;
+};
+struct PoolMoveArgs {
+    const long long *moves;          // [n][3]: source element, destination element, length (elements)
+    void *buf;                       // history buffers of all slots
+    int esz;                         // bytes per element
+    int n;
 };
 
 struct PcmArgs {

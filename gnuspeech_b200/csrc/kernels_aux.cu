@@ -94,3 +94,44 @@ extern "C" int trm_k_pcm_checksum(const trm_cuda_utterance *desc, int n_utt, con
     pcm_checksum_kernel<<<n_utt, 256, 0, s>>>(desc, n_utt, pcm, sums);
     return (int)cudaGetLastError();
 }
+
+// ---- stream pool bookkeeping (trm_cuda_pool_push) ---------------------------------------------------------------------
+// One CTA per entry: its waveguide descriptor goes to the slot's place in the array the waveguide kernel indexes, and a
+// slot opened since its last launch gets a fresh carried state -- everything zero, the noise generator at its start, the
+// "no sample yet" flag set (what trm_cuda_stream_create writes on the host).
+__global__ void pool_prepare_kernel(trm::PoolPrepArgs a)
+{
+    const int e = blockIdx.x, slot = a.slot[e];
+    const unsigned *src = reinterpret_cast<const unsigned *>(a.src + e);
+    unsigned *dst = reinterpret_cast<unsigned *>(a.dst + slot);
+    for (int i = threadIdx.x; i < (int)(sizeof(trm_cuda_utterance) / 4); i += blockDim.x) dst[i] = src[i];
+    if (a.reset[e]) {
+        unsigned long long *st = reinterpret_cast<unsigned long long *>(reinterpret_cast<unsigned char *>(a.state) + (size_t)slot * a.state_bytes);
+        for (int i = threadIdx.x; i < (int)(a.state_bytes / 8); i += blockDim.x) st[i] = i == 2 ? a.noise_k0 : (i == 3 ? 1ull : 0ull);
+    }
+}
+
+// One CTA per entry: the kept tube-rate history of a slot moves to the front of its other buffer (ragged lengths).
+__global__ void pool_move_kernel(trm::PoolMoveArgs a)
+{
+    const long long *m = a.moves + 3 * (size_t)blockIdx.x;
+    const int w = a.esz / 4;                                            // 4-byte words per element
+    const unsigned *src = reinterpret_cast<const unsigned *>(a.buf) + m[0] * w;
+    unsigned *dst = reinterpret_cast<unsigned *>(a.buf) + m[1] * w;
+    const long long words = m[2] * w;
+    for (long long i = threadIdx.x; i < words; i += blockDim.x) dst[i] = src[i];
+}
+
+extern "C" int trm_k_pool_prepare(const trm::PoolPrepArgs *a, cudaStream_t s)
+{
+    if (a->n <= 0) return 0;
+    pool_prepare_kernel<<<a->n, 128, 0, s>>>(*a);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int trm_k_pool_move(const trm::PoolMoveArgs *a, cudaStream_t s)
+{
+    if (a->n <= 0) return 0;
+    pool_move_kernel<<<a->n, 128, 0, s>>>(*a);
+    return (int)cudaGetLastError();
+}

@@ -49,16 +49,18 @@ template <typename R> static int configure_kernels(KernelInfo *info)
         if (info) info->n_src_shapes = SrcShapes<R>::N;
     }
     const int wide_smem = (int)sizeof(WideSmem<R>);
-    e = cudaFuncSetAttribute(tube_wide_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, wide_smem);
-    if (e != cudaSuccess) return (int)e;
-    e = cudaFuncSetAttribute(tube_wide_kernel<R>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return (int)e;
+    for (auto k : {tube_wide_kernel<R, false>, tube_wide_kernel<R, true>}) {
+        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, wide_smem);
+        if (e != cudaSuccess) return (int)e;
+        e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return (int)e;
+    }
     if (info) {
         info->wide_smem_bytes = wide_smem;
         info->wide_threads = Wide<R>::THREADS;
         info->wide_max_utt = 2 * Wide<R>::MAX_PAIRS;
         cudaFuncAttributes fa;
-        if (cudaFuncGetAttributes(&fa, tube_wide_kernel<R>) == cudaSuccess) info->wide_regs = fa.numRegs;
+        if (cudaFuncGetAttributes(&fa, tube_wide_kernel<R, false>) == cudaSuccess) info->wide_regs = fa.numRegs;
         if (cudaFuncGetAttributes(&fa, pcm_kernel<R>) == cudaSuccess) info->pcm_regs = fa.numRegs;
     }
     return 0;
@@ -77,13 +79,14 @@ static int upload_constants(const double *fir, int taps, const unsigned long lon
     return (int)e;
 }
 
-// waveguide: one CTA per group of <= 2*MAX_PAIRS utterances (tube_wide.cuh)
-template <typename R> static int launch_tube_wide(const TubeArgs &a, int n_groups, cudaStream_t s)
+// waveguide: one CTA per group of <= 2*MAX_PAIRS utterances (tube_wide.cuh); per_utt: state stored per utterance (pools)
+template <typename R> static int launch_tube_wide(const TubeArgs &a, int n_groups, cudaStream_t s, bool per_utt = false)
 {
     if (a.n_utt <= 0 || n_groups <= 0) return 0;
     if ((a.n_utt + n_groups - 1) / n_groups > 2 * Wide<R>::MAX_PAIRS) return (int)cudaErrorInvalidConfiguration;
     WideArgs w{a, n_groups};
-    tube_wide_kernel<R><<<n_groups, Wide<R>::THREADS, sizeof(WideSmem<R>), s>>>(w);
+    if (per_utt) tube_wide_kernel<R, true><<<n_groups, Wide<R>::THREADS, sizeof(WideSmem<R>), s>>>(w);
+    else tube_wide_kernel<R, false><<<n_groups, Wide<R>::THREADS, sizeof(WideSmem<R>), s>>>(w);
     return (int)cudaGetLastError();
 }
 
@@ -99,6 +102,15 @@ template <typename R> static int launch_src(const SrcArgs &a, int grid, int shap
     } else {
         return (int)cudaErrorInvalidValue;
     }
+    return (int)cudaGetLastError();
+}
+
+template <typename R> static int launch_src_pool(const SrcPoolArgs &a, int grid, cudaStream_t s)
+{
+    if (a.total_items <= 0 || a.n <= 0) return 0;
+    const long long need = (a.total_items + 7) / 8;                      // 8 warps per CTA, one work item per warp
+    if ((long long)grid > need) grid = (int)need;
+    src_pool_kernel<R><<<grid, 256, 0, s>>>(a);
     return (int)cudaGetLastError();
 }
 
@@ -132,9 +144,17 @@ template <typename R> static int launch_pcm(const PcmArgs &a, long long max_n_ou
     {                                                                                                             \
         return TRM_KERNEL_NS::launch_tube_wide<R>(*a, n_groups, s);                                                         \
     }                                                                                                             \
+    extern "C" int trm_k_tube_wide_pool_##SUF(const trm::TubeArgs *a, int n_groups, cudaStream_t s)               \
+    {                                                                                                             \
+        return TRM_KERNEL_NS::launch_tube_wide<R>(*a, n_groups, s, true);                                                   \
+    }                                                                                                             \
     extern "C" int trm_k_src_##SUF(const trm::SrcArgs *a, int grid, int shape, cudaStream_t s)                    \
     {                                                                                                             \
         return TRM_KERNEL_NS::launch_src<R>(*a, grid, shape, s);                                                            \
+    }                                                                                                             \
+    extern "C" int trm_k_src_pool_##SUF(const trm::SrcPoolArgs *a, int grid, cudaStream_t s)                       \
+    {                                                                                                             \
+        return TRM_KERNEL_NS::launch_src_pool<R>(*a, grid, s);                                                              \
     }                                                                                                             \
     extern "C" int trm_k_src_ctab_##SUF(const void *tab, void *ctab, cudaStream_t s)                              \
     {                                                                                                             \

@@ -488,6 +488,84 @@ __global__ void __launch_bounds__(SrcCfg<R, SHAPE>::THREADS, SrcCfg<R, SHAPE>::M
     if (item_hi > item_lo) flush_max();
 }
 
+// Resampler of a stream pool (trm_cuda_pool_push): the entries are streams at unrelated positions with their own voices,
+// so src_kernel's tiles (lane = utterance, one output index per warp) do not apply -- a tile spans from the earliest
+// missing output of its utterances to the latest, and the coefficients are not warp-uniform across signatures.  Here a
+// work item is a run of 32 consecutive outputs of ONE entry and lane = output.  Each lane reads its coefficient row
+// ctab[F] (the context's table, L2-resident) and its inputs directly.  The values and their order are src_kernel's: the
+// same coefficients, the taps left wing newest -> oldest from 0.0 then right wing, the same `acc += x * c` expression in
+// the same translation unit (so FMA contraction treats both kernels alike), and the same phase walk when
+// down-sampling -- the pool's output is bit-identical to the batch path's.
+template <typename R>
+__global__ void __launch_bounds__(256) src_pool_kernel(SrcPoolArgs args)
+{
+    constexpr int A = 16 / (int)sizeof(R);
+    const int lane = threadIdx.x & 31;
+    const long long n_warps = (long long)gridDim.x * (blockDim.x >> 5);
+    const R *__restrict__ X = reinterpret_cast<const R *>(args.tube);
+    const HD<R> *__restrict__ tab = reinterpret_cast<const HD<R> *>(args.table);
+    const R *__restrict__ ct = reinterpret_cast<const R *>(args.ctab);
+    for (long long item = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); item < args.total_items; item += n_warps) {
+        int lo = 0, hi = args.n;                                         // entry: largest e with item_base[e] <= item
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (args.item_base[mid] <= item) lo = mid; else hi = mid;
+        }
+        const trm_cuda_utterance *__restrict__ D = args.desc + lo;
+        const long long n = D->out_start + (item - args.item_base[lo]) * 32 + lane;   // output index in the stream
+        if (n >= D->n_out) continue;
+        const long long base = D->tube_offset, q_lo = D->in_start, q_hi = D->n_tube;
+        const int pad = D->padSize;
+        // xb[p] = x[p - pad]; zero before the first sample and after the last one (a flush: the converter's tail)
+        auto x = [&](long long q) -> R { return (q >= q_lo && q < q_hi) ? X[base + q] : (R)0; };
+        const unsigned long long T = (unsigned long long)n * D->tri;
+        const long long P = (long long)(T >> 16);
+        const unsigned F = (unsigned)(T & 0xFFFFull);
+        R acc = (R)0;
+        if (D->upsample) {
+            R xv[SRC_TAPS];
+#pragma unroll
+            for (int t = 0; t < SRC_ZC; ++t) {
+                xv[t] = x(P - t - pad);                                  // left wing xb[P - t]
+                xv[SRC_ZC + t] = x(P + 1 + t - pad);                     // right wing xb[P + 1 + t]
+            }
+            const R *crow = ct + (size_t)F * SRC_CLD;
+#pragma unroll
+            for (int q = 0; q < (SRC_TAPS + A - 1) / A; ++q) {
+                Vec16<R> cq;
+                cq.load(crow + A * q);
+#pragma unroll
+                for (int e = 0; e < A; ++e) {
+                    const int t = A * q + e;
+                    if (t < SRC_TAPS) acc += xv[t] * cq.e[e];
+                }
+            }
+        } else {
+            const double ratio = D->sampleRateRatio;
+            const unsigned phaseIncrement = D->phaseIncrement;
+            unsigned ph = (unsigned)rint((double)F * ratio), ii;
+            long long q = P - pad;
+            while ((ii = (ph >> 8)) < (unsigned)TRM_SRC_FILTER_LEN) {
+                const HD<R> c = tab[(ii & 255u) * SRC_ZC + (ii >> 8)];
+                const R impulse = c.h + (c.dh * ((R)(ph & 255u) / (R)256));
+                acc += (x(q) * impulse);
+                q -= 1;
+                ph += phaseIncrement;
+            }
+            ph = (unsigned)rint((double)((~F) & 0xFFFFu) * ratio);
+            q = P + 1 - pad;
+            while ((ii = (ph >> 8)) < (unsigned)TRM_SRC_FILTER_LEN) {
+                const HD<R> c = tab[(ii & 255u) * SRC_ZC + (ii >> 8)];
+                const R impulse = c.h + (c.dh * ((R)(ph & 255u) / (R)256));
+                acc += (x(q) * impulse);
+                q += 1;
+                ph += phaseIncrement;
+            }
+        }
+        reinterpret_cast<R *>(args.out)[D->out_offset + (n - D->out_start)] = acc;
+    }
+}
+
 // All interpolated filter coefficients of the up-sampling converter: row F (the 16-bit fraction of the time register)
 // holds the 13 left-wing and 13 right-wing coefficients of an output with that fraction, computed with the reference's two
 // operations per coefficient (TRMSampleRateConverter.m:179-203).  Built once per context.

@@ -21,8 +21,10 @@
     int trm_k_configure_##SUF(trm::KernelInfo *);                               \
     int trm_k_upload_##SUF(const double *, int, const unsigned long long *);    \
     int trm_k_tube_wide_##SUF(const trm::TubeArgs *, int, cudaStream_t);        \
+    int trm_k_tube_wide_pool_##SUF(const trm::TubeArgs *, int, cudaStream_t);   \
     int trm_k_src_##SUF(const trm::SrcArgs *, int, int, cudaStream_t);          \
     int trm_k_src_ctab_##SUF(const void *, void *, cudaStream_t);               \
+    int trm_k_src_pool_##SUF(const trm::SrcPoolArgs *, int, cudaStream_t);     \
     int trm_k_pcm_##SUF(const trm::PcmArgs *, long long, cudaStream_t);
 extern "C" {
 TRM_DECLARE_LAUNCHERS(f64)
@@ -31,6 +33,8 @@ TRM_DECLARE_LAUNCHERS(f64s)
 int trm_k_framegen(const trm::FrameGenArgs *, cudaStream_t);
 int trm_k_workload_walk2(unsigned long long, unsigned long long, long long, int, double *, cudaStream_t);
 int trm_k_pcm_checksum(const trm_cuda_utterance *, int, const int16_t *, unsigned long long *, cudaStream_t);
+int trm_k_pool_prepare(const trm::PoolPrepArgs *, cudaStream_t);
+int trm_k_pool_move(const trm::PoolMoveArgs *, cudaStream_t);
 }
 
 // precision codes of include/trm.h: 0 = FP64 conformance, 1 = FP32 fast, 2 = FP64 strict
@@ -40,11 +44,13 @@ struct KernelSet {
     int (*tube_wide)(const trm::TubeArgs *, int, cudaStream_t);
     int (*src)(const trm::SrcArgs *, int, int, cudaStream_t);
     int (*pcm)(const trm::PcmArgs *, long long, cudaStream_t);
+    int (*src_pool)(const trm::SrcPoolArgs *, int, cudaStream_t);
+    int (*tube_wide_pool)(const trm::TubeArgs *, int, cudaStream_t);   // state stored per utterance (tube_wide.cuh)
 };
 static const KernelSet g_kernels[3] = {
-    {trm_k_tube_wide_f64, trm_k_src_f64, trm_k_pcm_f64},
-    {trm_k_tube_wide_f32, trm_k_src_f32, trm_k_pcm_f32},
-    {trm_k_tube_wide_f64s, trm_k_src_f64s, trm_k_pcm_f64s},
+    {trm_k_tube_wide_f64, trm_k_src_f64, trm_k_pcm_f64, trm_k_src_pool_f64, trm_k_tube_wide_pool_f64},
+    {trm_k_tube_wide_f32, trm_k_src_f32, trm_k_pcm_f32, trm_k_src_pool_f32, trm_k_tube_wide_pool_f32},
+    {trm_k_tube_wide_f64s, trm_k_src_f64s, trm_k_pcm_f64s, trm_k_src_pool_f64s, trm_k_tube_wide_pool_f64s},
 };
 
 // FMA-chain kernels used to MEASURE the FP32 / FP64 CUDA-core peak of the device the bench runs on
@@ -388,8 +394,7 @@ int plan_chunk(const trm_cuda_utterance *desc, int u0, int u1, const trm::Kernel
     std::stable_sort(p.order.begin(), p.order.end(),
                      [&](int a, int b) { return p.desc[a].n_tube > p.desc[b].n_tube; });
     // time split candidates: dense frames, the same frame count everywhere (so that a frame range is one strided copy) and
-    // one control period (so that every utterance of a CTA reaches the split after the same number of 16-sample blocks:
-    // the kernels save an utterance's state when its CTA's loop ends)
+    // one control period (so that the split falls on the same tube sample for every utterance)
     p.split_frame = 0;
     p.uniform_frames = 0;
     if (n > 0 && p.frames_dense) {
@@ -1316,6 +1321,337 @@ int trm_cuda_stream_push(trm_cuda_stream *s, const double *frames_host, int m, i
     }
     if (flush) s->flushed = true;
     if (n_samples) *n_samples = n_ret > 0 ? n_ret : 0;
+    return 0;
+}
+
+/* ------------------------------------------------------------------------------------------------------------
+ * stream pool: slots at independent positions, each with its own voice (the per-slot form of trm_cuda_stream_push)
+ * ---------------------------------------------------------------------------------------------------------- */
+struct trm_cuda_pool {
+    struct Slot {
+        bool open = false;
+        bool fresh = false;             // opened since its last waveguide launch: the carried state starts from zero there
+        trm_cuda_utterance voice{};     // descriptor template (voice = the slot's wavetable row)
+        int cur = 0;                    // history buffer that holds the slot's tube-rate samples
+        long long frames_seen = 0, s_done = 0, out_done = 0, in_start = 0;   // as trm_cuda_stream, per slot
+        std::vector<double> pending;    // [pend_frames][16]: frames from the control interval in progress on
+        long long pend_first = 0;
+        int pend_frames = 0;
+    };
+    trm_cuda_ctx *ctx = nullptr;
+    int precision = 0, cap = 0, max_m = 0;
+    size_t esz = 8;
+    std::vector<Slot> slots;
+    long long stride = 0;               // history elements per slot and buffer
+    long long cap_out = 0;              // output samples one slot can return from one push
+    unsigned char *d_tube = nullptr;    // [2][cap][stride] tube-rate history, two buffers per slot
+    unsigned char *d_out = nullptr;     // [cap * cap_out] outputs of a push, packed entry after entry
+    unsigned char *d_state = nullptr;   // [cap] carried waveguide states
+    trm_cuda_utterance *d_desc = nullptr;   // [cap] waveguide descriptors, indexed by slot like the states
+    double *d_wavetables = nullptr;     // [cap][512]: row s is slot s's glottal table
+    Arena scratch;                      // per-push tables and frames (one upload)
+    HostStage stage;
+    cudaStream_t st = nullptr;
+    long long tube_at(int slot, int buf) const { return ((long long)buf * cap + slot) * stride; }
+};
+
+static int pool_err(int code, const char *what)
+{
+    g_err = what;
+    return code;
+}
+
+int trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max_frames_per_push, trm_cuda_pool **out)
+{
+    *out = nullptr;
+    if (capacity <= 0 || max_frames_per_push <= 0 || precision < 0 || precision > 2) return pool_err(-4, "trm_cuda_pool_create: bad sizes");
+    CK(cudaSetDevice(ctx->device));
+    trm_cuda_pool *p = new trm_cuda_pool();
+    p->ctx = ctx; p->precision = precision; p->cap = capacity; p->max_m = max_frames_per_push;
+    p->esz = prec_esz(precision);
+    p->slots.resize(capacity);
+    cudaError_t e = cudaMalloc((void **)&p->d_state, (size_t)capacity * trm::tube_state_bytes(p->esz));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&p->d_desc, (size_t)capacity * sizeof(trm_cuda_utterance));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&p->d_wavetables, (size_t)capacity * TRM_TABLE_LENGTH * sizeof(double));
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->st, cudaStreamNonBlocking);
+    if (e != cudaSuccess) { trm_cuda_pool_destroy(p); return fail("trm_cuda_pool_create", e); }
+    *out = p;
+    return 0;
+}
+
+int trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *v)
+{
+    if (v->controlPeriod <= 0 || v->tri == 0) return pool_err(-4, "trm_cuda_pool: voice without rates");
+    // the sizes trm_cuda_stream_create gives one stream of this voice
+    const long long max_new = (long long)(p->max_m + 1) * v->controlPeriod + 32;
+    const long long stride = (long long)align_up((size_t)(max_new + 128), 32);
+    const long long cap_out = (long long)align_up((size_t)(src_safe_outputs(max_new + 64, v->tri) + 64), 32);
+    CK(cudaSetDevice(p->ctx->device));
+    if (stride > p->stride) {
+        unsigned char *t = nullptr;
+        CK(cudaMalloc((void **)&t, (size_t)2 * p->cap * stride * p->esz));
+        if (p->d_tube) {
+            // the open slots' histories move to the wider rows (row r = buffer * cap + slot in both layouts)
+            cudaError_t e = cudaMemcpy2D(t, (size_t)stride * p->esz, p->d_tube, (size_t)p->stride * p->esz, (size_t)p->stride * p->esz,
+                                         (size_t)2 * p->cap, cudaMemcpyDeviceToDevice);
+            if (e != cudaSuccess) { cudaFree(t); return fail("trm_cuda_pool_reserve", e); }
+            cudaFree(p->d_tube);
+        }
+        p->d_tube = t;
+        p->stride = stride;
+    }
+    if (cap_out > p->cap_out) {
+        if (p->d_out) cudaFree(p->d_out);
+        p->d_out = nullptr;
+        p->cap_out = 0;
+        CK(cudaMalloc((void **)&p->d_out, (size_t)p->cap * cap_out * p->esz));
+        p->cap_out = cap_out;
+    }
+    return 0;
+}
+
+int trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, int *slot)
+{
+    *slot = -1;
+    int s = 0;
+    while (s < p->cap && p->slots[s].open) ++s;
+    if (s == p->cap) return pool_err(-7, "trm_cuda_pool_open: every slot is open");
+    int rc = trm_cuda_pool_reserve(p, voice);
+    if (rc != 0) return rc;
+    CK(cudaMemcpy(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH, wavetable, TRM_TABLE_LENGTH * sizeof(double), cudaMemcpyHostToDevice));
+    trm_cuda_pool::Slot &sl = p->slots[s];
+    sl = trm_cuda_pool::Slot();
+    sl.open = true;
+    sl.fresh = true;
+    sl.voice = *voice;
+    sl.voice.voice = s;
+    *slot = s;
+    return 0;
+}
+
+int trm_cuda_pool_close(trm_cuda_pool *p, int slot)
+{
+    if (slot < 0 || slot >= p->cap) return pool_err(-4, "trm_cuda_pool_close: no such slot");
+    if (!p->slots[slot].open) return pool_err(-7, "trm_cuda_pool_close: the slot is not open");
+    p->slots[slot] = trm_cuda_pool::Slot();
+    return 0;
+}
+
+int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p) { return p->cap_out; }
+
+void trm_cuda_pool_destroy(trm_cuda_pool *p)
+{
+    if (!p) return;
+    cudaSetDevice(p->ctx->device);
+    if (p->st) { cudaStreamSynchronize(p->st); cudaStreamDestroy(p->st); }
+    if (p->d_tube) cudaFree(p->d_tube);
+    if (p->d_out) cudaFree(p->d_out);
+    if (p->d_state) cudaFree(p->d_state);
+    if (p->d_desc) cudaFree(p->d_desc);
+    if (p->d_wavetables) cudaFree(p->d_wavetables);
+    p->scratch.release();
+    p->stage.release();
+    delete p;
+}
+
+int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                       const uint8_t *flush, void *samples_host, int64_t *out_offset)
+{
+    // ---- arguments: everything is checked before the pool changes -----------------------------------------------
+    if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_push: bad entry count");
+    if (!out_offset || (n > 0 && (!slot || !n_frames))) return pool_err(-4, "trm_cuda_pool_push: null argument");
+    long long total_in = 0;
+    {
+        std::vector<unsigned char> named((size_t)p->cap, 0);
+        for (int i = 0; i < n; ++i) {
+            const int s = slot[i];
+            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_push: no such slot");
+            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_push: the slot is not open");
+            if (named[s]) return pool_err(-4, "trm_cuda_pool_push: a slot is named twice");
+            named[s] = 1;
+            if (n_frames[i] < 0 || n_frames[i] > p->max_m) return pool_err(-4, "trm_cuda_pool_push: more frames than the pool was created for");
+            total_in += n_frames[i];
+        }
+    }
+    if (total_in > 0 && !frames_host) return pool_err(-4, "trm_cuda_pool_push: null frames");
+    out_offset[0] = 0;
+    if (n == 0) return 0;
+    trm_cuda_ctx *ctx = p->ctx;
+    CK(cudaSetDevice(ctx->device));
+
+    // ---- per entry: what trm_cuda_stream_push computes for one stream ------------------------------------------------
+    struct Entry {
+        int slot = 0;
+        bool flush = false, run = false;
+        long long target = 0, n_new = 0, out_total = 0, next_in = 0;
+        int skip = 0, nf_call = 0;
+    };
+    std::vector<Entry> E((size_t)n);
+    const double *fp = frames_host;
+    long long wg_frames = 0, total_out = 0;
+    int n_wg = 0;
+    for (int i = 0; i < n; ++i) {
+        Entry &e = E[i];
+        e.slot = slot[i];
+        e.flush = flush && flush[i];
+        trm_cuda_pool::Slot &sl = p->slots[e.slot];
+        const int m = n_frames[i];
+        if (m) {
+            sl.pending.insert(sl.pending.end(), fp, fp + (size_t)m * 16);
+            fp += (size_t)m * 16;
+            sl.pend_frames += m;
+            sl.frames_seen += m;
+        }
+        const long long cp = sl.voice.controlPeriod;
+        const unsigned tri = sl.voice.tri;
+        const int pad = sl.voice.padSize;
+        const long long avail = sl.frames_seen >= 2 ? (sl.frames_seen - 1) * cp : 0;
+        e.target = e.flush ? avail : avail / trm::TB * trm::TB;
+        e.n_new = e.target - sl.s_done;
+        e.out_total = e.flush ? (long long)(((unsigned long long)(e.target + 2 * pad) * 65536ull + tri - 1) / tri) : src_safe_outputs(e.target, tri);
+        e.run = !(e.flush && sl.frames_seen < 1) && (e.n_new > 0 || (e.flush && e.out_total > sl.out_done));
+        long long n_ret = 0;
+        if (e.run) {
+            const long long f0 = sl.s_done / cp;
+            e.skip = (int)(f0 - sl.pend_first);
+            e.nf_call = sl.pend_frames - e.skip;
+            if (e.n_new > 0) { ++n_wg; wg_frames += e.nf_call; }
+            n_ret = e.out_total - sl.out_done;
+            long long next_in = e.flush ? e.target : (long long)(((unsigned long long)e.out_total * tri) >> 16) - 2 * pad - 4;
+            if (next_in < 0) next_in = 0;
+            next_in = next_in / 4 * 4;
+            if (next_in < sl.in_start) next_in = sl.in_start;
+            e.next_in = next_in;
+            if (e.target - sl.in_start > p->stride || n_ret > p->cap_out) return fail_msg("trm_cuda_pool_push: internal capacity");
+        }
+        total_out += n_ret > 0 ? n_ret : 0;
+        out_offset[i + 1] = total_out;
+    }
+
+    // ---- host tables of the push, laid out as in the device scratch: one upload ------------------------------------
+    std::vector<int> wg;                                  // entries that run the waveguide, longest first
+    std::vector<trm_cuda_utterance> rd;                   // resampler views of the entries that return samples
+    std::vector<long long> ib(1, 0), mv;                  // work-item prefix; history moves {src, dst, len}
+    for (int i = 0; i < n; ++i) {
+        const Entry &e = E[i];
+        if (!e.run) continue;
+        const trm_cuda_pool::Slot &sl = p->slots[e.slot];
+        if (e.n_new > 0) wg.push_back(i);
+        const long long n_ret = e.out_total - sl.out_done;
+        if (n_ret > 0) {
+            trm_cuda_utterance r = sl.voice;              // global sample indices of the stream
+            r.n_tube = e.target;
+            r.tube_offset = p->tube_at(e.slot, sl.cur) - sl.in_start;
+            r.n_out = e.out_total;
+            r.out_start = sl.out_done;
+            r.in_start = sl.in_start;
+            r.out_offset = out_offset[i];
+            r.pcm_offset = 0;
+            rd.push_back(r);
+            ib.push_back(ib.back() + (n_ret + 31) / 32);
+        }
+        const long long keep = e.target - e.next_in;
+        if (!e.flush && keep > 0) {
+            mv.push_back(p->tube_at(e.slot, sl.cur) + (e.next_in - sl.in_start));
+            mv.push_back(p->tube_at(e.slot, sl.cur ^ 1));
+            mv.push_back(keep);
+        }
+    }
+    std::stable_sort(wg.begin(), wg.end(), [&](int a, int b) { return E[a].n_new > E[b].n_new; });
+    const size_t n_rd = rd.size(), n_mv = mv.size() / 3;
+    const size_t o_dt = 0;
+    const size_t o_ord = o_dt + align_up(wg.size() * sizeof(trm_cuda_utterance), 256);
+    const size_t o_rst = o_ord + align_up(wg.size() * sizeof(int), 256);
+    const size_t o_rd = o_rst + align_up(wg.size() * sizeof(int), 256);
+    const size_t o_ib = o_rd + align_up(n_rd * sizeof(trm_cuda_utterance), 256);
+    const size_t o_mv = o_ib + align_up(ib.size() * sizeof(long long), 256);
+    const size_t o_fr = o_mv + align_up(mv.size() * sizeof(long long), 256);
+    const size_t bytes = o_fr + (size_t)wg_frames * 128;
+    int rc;
+    if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
+    if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
+    unsigned char *h = p->stage.base;
+    {
+        trm_cuda_utterance *dt = (trm_cuda_utterance *)(h + o_dt);
+        int *ord = (int *)(h + o_ord), *rst = (int *)(h + o_rst);
+        double *fr = (double *)(h + o_fr);
+        long long f_at = 0;
+        for (size_t k = 0; k < wg.size(); ++k) {
+            const Entry &e = E[wg[k]];
+            const trm_cuda_pool::Slot &sl = p->slots[e.slot];
+            trm_cuda_utterance d = sl.voice;
+            d.frame_offset = f_at;
+            d.n_frames = e.nf_call;
+            d.n_tube = e.n_new;
+            d.tube_offset = p->tube_at(e.slot, sl.cur) + (sl.s_done - sl.in_start);
+            d.jc0 = (int)(sl.s_done % sl.voice.controlPeriod);
+            d.out_start = 0; d.in_start = 0;
+            dt[k] = d;
+            ord[k] = e.slot;
+            rst[k] = sl.fresh ? 1 : 0;
+            memcpy(fr + (size_t)f_at * 16, &sl.pending[(size_t)e.skip * 16], (size_t)e.nf_call * 128);
+            f_at += e.nf_call;
+        }
+        if (n_rd) memcpy(h + o_rd, rd.data(), n_rd * sizeof(trm_cuda_utterance));
+        memcpy(h + o_ib, ib.data(), ib.size() * sizeof(long long));
+        if (n_mv) memcpy(h + o_mv, mv.data(), mv.size() * sizeof(long long));
+    }
+    unsigned char *d = p->scratch.base;
+    cudaStream_t st = p->st;
+    CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, st));
+    const KernelSet &K = g_kernels[p->precision];
+    const trm::KernelInfo &ki = ctx->ki(p->precision);
+    const int n_w = (int)wg.size();
+    if (n_w > 0) {
+        trm::PoolPrepArgs pa{};
+        pa.src = (const trm_cuda_utterance *)(d + o_dt); pa.slot = (const int *)(d + o_ord); pa.reset = (const int *)(d + o_rst);
+        pa.dst = p->d_desc; pa.state = p->d_state; pa.state_bytes = trm::tube_state_bytes(p->esz); pa.noise_k0 = ctx->noise_k0; pa.n = n_w;
+        if ((rc = trm_k_pool_prepare(&pa, st)) != 0) return fail("pool prepare launch", (cudaError_t)rc);
+        // one waveguide launch over the slots with new samples; the kernel maps CTA positions to slots through `order`
+        trm::TubeArgs a{};
+        a.state = p->d_state; a.desc = p->d_desc; a.order = (const int *)(d + o_ord); a.n_utt = n_w;
+        a.frames = d + o_fr; a.frames_f32 = 0; a.tube = p->d_tube; a.wavetables = p->d_wavetables; a.noise_k0 = ctx->noise_k0;
+        const int gmax = ki.wide_max_utt;
+        const int groups = std::max(1, std::min(ctx->sm_count, (n_w + 1) / 2));
+        const int g2 = (n_w + groups - 1) / groups > gmax ? (n_w + gmax - 1) / gmax : groups;
+        if ((rc = K.tube_wide_pool(&a, g2, st)) != 0) return fail("pool waveguide launch", (cudaError_t)rc);
+    }
+    if (n_rd > 0) {
+        trm::SrcPoolArgs a{};
+        a.desc = (const trm_cuda_utterance *)(d + o_rd); a.n = (int)n_rd; a.item_base = (const long long *)(d + o_ib);
+        a.total_items = ib.back(); a.tube = p->d_tube; a.out = p->d_out;
+        a.table = prec_is_f64(p->precision) ? ctx->d_tab_f64 : ctx->d_tab_f32;
+        a.ctab = prec_is_f64(p->precision) ? ctx->d_ctab_f64 : ctx->d_ctab_f32;
+        if ((rc = K.src_pool(&a, ctx->sm_count * 8, st)) != 0) return fail("pool resampler launch", (cudaError_t)rc);
+    }
+    if (n_mv > 0) {
+        trm::PoolMoveArgs a{};
+        a.moves = (const long long *)(d + o_mv); a.buf = p->d_tube; a.esz = (int)p->esz; a.n = (int)n_mv;
+        if ((rc = trm_k_pool_move(&a, st)) != 0) return fail("pool history move launch", (cudaError_t)rc);
+    }
+    if (samples_host && total_out > 0) CK(cudaMemcpyAsync(samples_host, p->d_out, (size_t)total_out * p->esz, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+
+    // ---- bookkeeping -------------------------------------------------------------------------------------------
+    for (int i = 0; i < n; ++i) {
+        const Entry &e = E[i];
+        trm_cuda_pool::Slot &sl = p->slots[e.slot];
+        if (e.flush) { sl = trm_cuda_pool::Slot(); continue; }     // ended: the slot is free again
+        if (!e.run) continue;
+        if (e.n_new > 0) sl.fresh = false;
+        sl.in_start = e.next_in;
+        sl.s_done = e.target;
+        sl.out_done = e.out_total;
+        sl.cur ^= 1;
+        // frames before the interval the next push starts in are done with
+        const long long nf0 = sl.s_done / sl.voice.controlPeriod;
+        const int drop = (int)(nf0 - sl.pend_first);
+        if (drop > 0) {
+            sl.pending.erase(sl.pending.begin(), sl.pending.begin() + (size_t)drop * 16);
+            sl.pend_frames -= drop;
+            sl.pend_first = nf0;
+        }
+    }
     return 0;
 }
 

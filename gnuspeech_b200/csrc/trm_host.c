@@ -1145,6 +1145,91 @@ void TRMStreamFree(TRMStream *t)
     free(t);
 }
 
+/* ---- stream pool: independent streaming slots, each with its own voice ---- */
+struct TRMStreamPool {
+    trm_cuda_pool *p;
+};
+
+/* shim codes: -4 / -7 are argument / call-order refusals (message set by the shim), anything else is CUDA */
+static int pool_rc(int rc)
+{
+    if (rc == TRM_ERR_PARAM || rc == TRM_ERR_STATE) return set_err(rc, "%s", trm_cuda_last_error());
+    return cuda_err();
+}
+
+TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_per_push, int device, int *err)
+{
+    int dummy;
+    if (!err) err = &dummy;
+    if (capacity <= 0 || max_frames_per_push <= 0 || !precision_ok(precision)) {
+        *err = set_err(TRM_ERR_PARAM, "bad stream pool arguments%s", "");
+        return NULL;
+    }
+    TRMStreamPool *t = calloc(1, sizeof *t);
+    if (!t) { *err = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); return NULL; }
+    trm_cuda_ctx *ctx;
+    int lane;
+    if ((*err = acquire_ctx(device, &ctx, &lane)) != TRM_OK) { free(t); return NULL; }
+    int rc = trm_cuda_pool_create(ctx, precision, capacity, max_frames_per_push, &t->p);
+    release_ctx(device, lane);      /* the pool owns its buffers, wavetables, stream and scratch: no lane is held */
+    if (rc == 0) {
+        /* initial sizes: the default voice (TRMInputParametersSetDefaults at 44.1 kHz) */
+        TRMInputParameters ip;
+        voice_set vs;
+        trm_cuda_utterance d;
+        memset(&vs, 0, sizeof vs);
+        TRMInputParametersSetDefaults(&ip, 44100.0f);
+        if (describe(&ip, 2, &vs, &d, NULL) == TRM_OK) rc = trm_cuda_pool_reserve(t->p, &d);
+        voice_set_free(&vs);
+    }
+    if (rc != 0) {
+        *err = pool_rc(rc);
+        trm_cuda_pool_destroy(t->p);
+        free(t);
+        return NULL;
+    }
+    *err = TRM_OK;
+    return t;
+}
+
+int TRMStreamPoolOpen(TRMStreamPool *t, const TRMInputParameters *voice)
+{
+    if (!t || !voice) return set_err(TRM_ERR_PARAM, "null stream pool or voice%s", "");
+    voice_set vs;
+    trm_cuda_utterance d;
+    memset(&vs, 0, sizeof vs);
+    int rc = describe(voice, 2, &vs, &d, NULL);
+    if (rc != TRM_OK) { voice_set_free(&vs); return rc; }
+    int slot = -1;
+    rc = trm_cuda_pool_open(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, &slot);
+    voice_set_free(&vs);
+    return rc != 0 ? pool_rc(rc) : slot;
+}
+
+int TRMStreamPoolClose(TRMStreamPool *t, int slot)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    const int rc = trm_cuda_pool_close(t->p, slot);
+    return rc != 0 ? pool_rc(rc) : TRM_OK;
+}
+
+int64_t TRMStreamPoolSlotCapacity(const TRMStreamPool *t) { return t ? trm_cuda_pool_slot_capacity(t->p) : 0; }
+
+int TRMStreamPoolPush(TRMStreamPool *t, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
+                      const uint8_t *flush, void *samples_out, int64_t *out_offset)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    const int rc = trm_cuda_pool_push(t->p, n, slot, n_frames, (const double *)frames, flush, samples_out, out_offset);
+    return rc != 0 ? pool_rc(rc) : TRM_OK;
+}
+
+void TRMStreamPoolFree(TRMStreamPool *t)
+{
+    if (!t) return;
+    trm_cuda_pool_destroy(t->p);
+    free(t);
+}
+
 /* ---- asynchronous calls: one host thread per ticket; two tickets per device overlap (context lanes) ---- */
 struct TRMBatchTicket {
     pthread_t th;

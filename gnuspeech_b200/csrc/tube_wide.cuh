@@ -174,6 +174,17 @@ template <typename R> __device__ __forceinline__ R *state_vals(void *state, int 
     return reinterpret_cast<R *>(state_hdr<R>(state, u) + STATE_HDR);
 }
 
+// Streaming state capture.  PER_UTT = false (batch, time split, TRMStream: every utterance of a CTA gets the same number
+// of samples, or there is no state): the state is stored when the CTA's loop ends.  PER_UTT = true (stream pool,
+// trm_cuda_pool_push: the utterances of one CTA may have different sample counts, and the warps keep running past an
+// utterance's end until the longest one of the CTA is done): each utterance's state is stored at the end of the block
+// that holds its last sample.  Two instantiations, so that the paths without per-utterance capture keep their code.
+__device__ __forceinline__ bool ends_in_block(long long n_tube, int blk)
+{
+    const long long left = n_tube - (long long)blk * TB;
+    return left > 0 && left <= TB;
+}
+
 struct WideArgs {
     TubeArgs t;
     int n_groups;      // CTAs; group g holds utterances order[start(g) .. start(g+1))
@@ -194,7 +205,7 @@ __device__ __forceinline__ void wide_group(int n, int n_groups, int g, int &star
 // =========================================================================================================
 // recurrence warp (warp 0 of the CTA): lane = utterance
 // =========================================================================================================
-template <typename R>
+template <typename R, bool PER_UTT>
 __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideArgs &wargs, int g_start, int g_count, int n_blocks, int lane)
 {
     constexpr bool FAST = sizeof(R) == 4;                  // FP32 fast mode
@@ -342,8 +353,16 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                     }
                 }
                 __syncwarp(FULL);
+                if (PER_UTT && sv && ends_in_block(W.n_tube[lane], blk)) {
+#pragma unroll
+                    for (int q = 0; q < 10; ++q) { sv[q] = t[q]; sv[10 + q] = bt[q]; }
+#pragma unroll
+                    for (int q = 0; q < 6; ++q) { sv[20 + q] = nt[q]; sv[26 + q] = nb[q]; }
+                    sv[32] = m_ry; sv[33] = m_rx; sv[34] = m_rY; sv[35] = n_ry; sv[36] = n_rx; sv[37] = n_rY;
+                    sv[38] = y1; sv[39] = y2; sv[40] = thy;
+                }
             }
-            if (sv) {
+            if (!PER_UTT && sv) {
 #pragma unroll
                 for (int q = 0; q < 10; ++q) { sv[q] = t[q]; sv[10 + q] = bt[q]; }
 #pragma unroll
@@ -480,8 +499,16 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                     }
                 }
                 __syncwarp(FULL);
+                if (PER_UTT && sv && ends_in_block(W.n_tube[lane], blk)) {
+                    sv[0] = t0; sv[1] = t1; sv[2] = t2; sv[3] = t3; sv[4] = t4; sv[5] = t5; sv[6] = t6; sv[7] = t7; sv[8] = t8; sv[9] = t9;
+                    sv[10] = b0; sv[11] = b1; sv[12] = b2; sv[13] = b3; sv[14] = b4; sv[15] = b5; sv[16] = b6; sv[17] = b7; sv[18] = b8; sv[19] = b9;
+                    sv[20] = nt0; sv[21] = nt1; sv[22] = nt2; sv[23] = nt3; sv[24] = nt4; sv[25] = nt5;
+                    sv[26] = nb0; sv[27] = nb1; sv[28] = nb2; sv[29] = nb3; sv[30] = nb4; sv[31] = nb5;
+                    sv[32] = m_ry; sv[33] = m_rx; sv[34] = m_rY; sv[35] = n_ry; sv[36] = n_rx; sv[37] = n_rY;
+                    sv[38] = y1; sv[39] = y2; sv[40] = thy;
+                }
             }
-            if (sv) {
+            if (!PER_UTT && sv) {
                 sv[0] = t0; sv[1] = t1; sv[2] = t2; sv[3] = t3; sv[4] = t4; sv[5] = t5; sv[6] = t6; sv[7] = t7; sv[8] = t8; sv[9] = t9;
                 sv[10] = b0; sv[11] = b1; sv[12] = b2; sv[13] = b3; sv[14] = b4; sv[15] = b5; sv[16] = b6; sv[17] = b7; sv[18] = b8; sv[19] = b9;
                 sv[20] = nt0; sv[21] = nt1; sv[22] = nt2; sv[23] = nt3; sv[24] = nt4; sv[25] = nt5;
@@ -620,8 +647,16 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                     }
                 }
                 __syncwarp(FULL);
+                if (PER_UTT && sv && ends_in_block(W.n_tube[lane], blk)) {
+#pragma unroll
+                    for (int q = 0; q < 10; ++q) { sv[q] = t[q]; sv[10 + q] = bt[q]; }
+#pragma unroll
+                    for (int q = 0; q < 6; ++q) { sv[20 + q] = nt[q]; sv[26 + q] = nb[q]; }
+                    sv[32] = m_ry; sv[33] = m_rx; sv[34] = m_rY; sv[35] = n_ry; sv[36] = n_rx; sv[37] = n_rY;
+                    sv[38] = y1; sv[39] = y2; sv[40] = thy;
+                }
             }
-            if (sv) {
+            if (!PER_UTT && sv) {
 #pragma unroll
                 for (int q = 0; q < 10; ++q) { sv[q] = t[q]; sv[10 + q] = bt[q]; }
 #pragma unroll
@@ -636,7 +671,7 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
 // feed-forward warp: utterances 2*pair and 2*pair+1 of the group, lane = sample of a 16-sample block
 // (phases S0 / A1 / S1 / A2; the results go to the ring)
 // =========================================================================================================
-template <typename R>
+template <typename R, bool PER_UTT>
 __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const WideArgs &wargs, int g_start, int g_count, int n_blocks, int pair, int lane)
 {
     constexpr bool FAST = sizeof(R) == 4;                  // FP32 fast mode
@@ -1297,6 +1332,17 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             if (hl < FIR_HIST - TB) { S.HE[TB + hl] = e1; S.HO[TB + hl] = o1; }
         }
         __syncwarp(FULL);
+        if (PER_UTT && st_h && ends_in_block(n_tube, blk)) {
+            // the utterance's last sample is in this block (a whole block except at the end of a stream): the state after it
+            if (hl == 0) {
+                st_h[0] = (unsigned long long)__double_as_longlong(pos);
+                st_h[1] = pos_fx;
+                st_h[2] = kb;
+                st_h[3] = 0ull;
+                st_v[STATE_XM] = xm1; st_v[STATE_XM + 1] = xm2;
+            }
+            for (int i = hl; i < FIR_HIST; i += TB) { st_v[STATE_HE + i] = S.HE[i]; st_v[STATE_HO + i] = S.HO[i]; }
+        }
         TPH(8);
     }
 #if TRM_PROFILE_PHASES
@@ -1306,8 +1352,8 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
                tph[2] / n_blocks, tph[3] / n_blocks, tph[4] / n_blocks,
                tph[5] / n_blocks, tph[6] / n_blocks, tph[7] / n_blocks, tph[8] / n_blocks, n_blocks);
 #endif
-    if (st_h) {
-        // streaming calls cover whole 16-sample blocks, so everything here is the state after the last sample
+    if (!PER_UTT && st_h) {
+        // lockstep calls cover whole 16-sample blocks of equally long utterances: the state after the last sample
         if (hl == 0) {
             st_h[0] = (unsigned long long)__double_as_longlong(pos);
             st_h[1] = pos_fx;
@@ -1319,7 +1365,7 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
     }
 }
 
-template <typename R>
+template <typename R, bool PER_UTT>
 __global__ void __launch_bounds__(Wide<R>::THREADS, 1) tube_wide_kernel(WideArgs wargs)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1368,16 +1414,16 @@ __global__ void __launch_bounds__(Wide<R>::THREADS, 1) tube_wide_kernel(WideArgs
         if (warp < 4) {
             asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(Wide<R>::REGS_HI));
             if (n_cta <= 0 || pair >= n_pairs) return;
-            if (warp == 0) wide_recurrence_warp<R>(W, wargs, g_start, g_count, n_blocks, lane);
-            else wide_feed_forward_warp<R>(W, wargs, g_start, g_count, n_blocks, pair, lane);
+            if (warp == 0) wide_recurrence_warp<R, PER_UTT>(W, wargs, g_start, g_count, n_blocks, lane);
+            else wide_feed_forward_warp<R, PER_UTT>(W, wargs, g_start, g_count, n_blocks, pair, lane);
         } else {
             if (n_cta <= 0 || warp == WIDE_IDLE_WARP || pair >= n_pairs) return;
-            wide_feed_forward_warp<R>(W, wargs, g_start, g_count, n_blocks, pair, lane);
+            wide_feed_forward_warp<R, PER_UTT>(W, wargs, g_start, g_count, n_blocks, pair, lane);
         }
     } else {
         if (n_cta <= 0 || warp == WIDE_IDLE_WARP || pair >= n_pairs) return;
-        if (warp == 0) wide_recurrence_warp<R>(W, wargs, g_start, g_count, n_blocks, lane);
-        else wide_feed_forward_warp<R>(W, wargs, g_start, g_count, n_blocks, pair, lane);
+        if (warp == 0) wide_recurrence_warp<R, PER_UTT>(W, wargs, g_start, g_count, n_blocks, lane);
+        else wide_feed_forward_warp<R, PER_UTT>(W, wargs, g_start, g_count, n_blocks, pair, lane);
     }
 }
 

@@ -312,6 +312,38 @@ int TRMStreamPush(TRMStream *stream, const TRMParameters *frames, int m, int flu
 void TRMStreamFree(TRMStream *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Stream pool: serving many streams that start, advance and end independently, each with its own voice (tract length,
+ * so control period, tube rate and converter signature; glottal pulse; output rate).  A slot is opened with a voice;
+ * each push advances any subset of the open slots, each by its own number of frames, and all of them are synthesized by
+ * one waveguide launch and one resampler launch.  A slot ends with its own flush (or is abandoned with Close) and can
+ * then be opened again.  The contract of TRMStream holds per slot: its pushes, concatenated, are bit-identical to the
+ * one-shot TRMBatch synthesis of that utterance with that voice, whatever the other slots do.
+ * A pool owns its device buffers and one 512-entry wavetable row per slot (written when the slot opens); it holds no
+ * context lane between calls.  A pool is used by one thread at a time.  No CPU fallback: without a device
+ * TRMStreamPoolCreate fails with TRM_ERR_CUDA.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct TRMStreamPool TRMStreamPool;
+/* capacity slots on one device, one arithmetic mode for all of them. */
+TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_per_push, int device, int *err);
+/* Opens a free slot with this voice (validated exactly as TRMBatchCreate validates a voice); returns the slot >= 0 or a
+ * negative TRM_ERR_*.  Pool full: TRM_ERR_STATE. */
+int TRMStreamPoolOpen(TRMStreamPool *pool, const TRMInputParameters *voice);
+/* Abandons an open slot without its tail (client went away); the slot becomes free. */
+int TRMStreamPoolClose(TRMStreamPool *pool, int slot);
+/* Samples one slot can return from one push (row bound for samples_out).  Sized at creation for the default voice; it
+ * grows when a slot opens with a voice that produces more samples per control frame than any before, so read it after
+ * opening slots. */
+int64_t TRMStreamPoolSlotCapacity(const TRMStreamPool *pool);
+/* Advances n distinct open slots: slot[i] gets n_frames[i] (0..max) frames, taken back to back from `frames`; flush[i] != 0
+ * (flush may be NULL: no flush) ends slot[i] (converter tail, as at the end of -synthesize) and frees it.  Samples (double,
+ * or float in FP32 mode) are packed: entry i's are samples_out[out_offset[i] .. out_offset[i+1]); samples_out holds
+ * n * SlotCapacity elements.  An unopened slot (TRM_ERR_STATE), a slot named twice or too many frames (TRM_ERR_PARAM)
+ * fail the whole push before any work: the pool is left exactly as it was. */
+int TRMStreamPoolPush(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
+                      const uint8_t *flush, void *samples_out, int64_t *out_offset /* [n + 1] */);
+void TRMStreamPoolFree(TRMStreamPool *pool);
+
+/* ---------------------------------------------------------------------------------------------
  * Sweeps (BASELINE configs[4]: 10^6 synthetic 2 s utterances): n utterances of one voice whose control tracks are the walk2
  * workload of include/trm_workload.h, generated on the device (utterance k = index first_index + k of stream `seed`) --
  * 64 GB of frames per million utterances never cross PCIe.  The audio stays on the device as well: per utterance an

@@ -185,6 +185,27 @@ int  trm_cuda_stream_push(trm_cuda_stream *s, const double *frames_host, int m, 
                           int64_t *n_samples);
 void trm_cuda_stream_destroy(trm_cuda_stream *s);
 /*
+ * Stream pool: `capacity` streaming slots that open, advance and end independently, each with its own voice (its own
+ * template: control period, converter signature, glottal table).  A push advances any subset of open slots, each by its
+ * own number of frames; all of them are synthesized by one waveguide launch and one resampler launch.  Each slot's pushes,
+ * concatenated, are bit-identical to synthesizing its utterance at once.  Used by one thread at a time.
+ * Return codes: 0, -4 (bad argument), -7 (call order: slot not open, pool full), -5 (CUDA error; trm_cuda_last_error()).
+ * Arguments are checked before any device work: a call that returns -4 or -7 leaves the pool as it was.
+ */
+typedef struct trm_cuda_pool trm_cuda_pool;
+int  trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max_frames_per_push, trm_cuda_pool **out);
+/* sizes the per-slot buffers for this voice (grows them if needed; SlotCapacity may grow) without opening a slot */
+int  trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *voice);
+/* voice.voice is ignored: `wavetable` (512 doubles) becomes the slot's own glottal table.  *slot receives the slot. */
+int  trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, int *slot);
+int  trm_cuda_pool_close(trm_cuda_pool *p, int slot);
+int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one slot can return from one push */
+/* entry i: slot[i] gets n_frames[i] frames (taken back to back from frames_host, rows of 16 doubles); flush[i] != 0 ends
+ * the slot and frees it.  samples_host receives the samples packed (entry i: [out_offset[i], out_offset[i+1])). */
+int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                        const uint8_t *flush, void *samples_host, int64_t *out_offset);
+void trm_cuda_pool_destroy(trm_cuda_pool *p);
+/*
  * Control frames on the device (replaces -[EventList generateOutputInTimeRange:...], EventList.m:883-1061): uploads
  * the event lists of the n utterances (utterance u: events[ev_offset[u] .. +ev_count[u]); fg: one entry per
  * utterance, or one for all if shared_fg), runs the generator kernel and leaves the frames -- desc[u].n_frames of
