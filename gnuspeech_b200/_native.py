@@ -140,6 +140,7 @@ def lib():
     sig("TRMStreamPoolClose", C.c_int, vp, C.c_int)
     sig("TRMStreamPoolSlotCapacity", i64, vp)
     sig("TRMStreamPoolPush", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp)
+    sig("TRMStreamPoolPushPCM16", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("TRMStreamPoolFree", None, vp)
     sig("TRMBatchSynthesizeAsync", vp, vp, vp, vp, vp, vp, C.c_int, vp)
     sig("TRMBatchWait", C.c_int, vp)

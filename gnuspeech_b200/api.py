@@ -564,22 +564,43 @@ class TRMStreamPool(object):
     def slot_capacity(self):
         return int(N.lib().TRMStreamPoolSlotCapacity(self._h))
 
-    def push(self, frames, flush=()):
-        """frames: {slot: (m, 16) float64} (m may be 0); flush: slots that end with this push.  Returns {slot: samples}
-        for every slot named in `frames` or `flush`."""
+    @staticmethod
+    def _entries(frames, flush):
+        """The push's entries as the C call takes them: slots, frame counts, frames back to back, flush flags."""
         slots = list(frames.keys()) + [s for s in flush if s not in frames]
         parts = [np.ascontiguousarray(frames.get(s, np.zeros((0, 16))), dtype=np.float64).reshape(-1, 16) for s in slots]
-        n = len(slots)
         slot_a = np.array(slots, dtype=np.int32)
         nf_a = np.array([p.shape[0] for p in parts], dtype=np.int32)
         fl = set(flush)
         flush_a = np.array([1 if s in fl else 0 for s in slots], dtype=np.uint8)
         allf = np.concatenate(parts) if parts else np.zeros((0, 16))
+        return slots, slot_a, nf_a, (allf if allf.shape[0] else None), flush_a
+
+    def push(self, frames, flush=()):
+        """frames: {slot: (m, 16) float64} (m may be 0); flush: slots that end with this push.  Returns {slot: samples}
+        for every slot named in `frames` or `flush`."""
+        slots, slot_a, nf_a, fr, flush_a = self._entries(frames, flush)
+        n = len(slots)
         out = np.zeros(max(1, n * self.slot_capacity()), self.dtype)
         off = np.zeros(n + 1, np.int64)
-        check(N.lib().TRMStreamPoolPush(self._h, n, _ptr(slot_a), _ptr(nf_a), _ptr(allf) if allf.shape[0] else None,
-                                        _ptr(flush_a), _ptr(out), _ptr(off)), "TRMStreamPoolPush")
+        check(N.lib().TRMStreamPoolPush(self._h, n, _ptr(slot_a), _ptr(nf_a), _ptr(fr), _ptr(flush_a), _ptr(out), _ptr(off)),
+              "TRMStreamPoolPush")
         return {s: out[off[i]:off[i + 1]].copy() for i, s in enumerate(slots)}
+
+    def push_pcm16(self, frames, peak, flush=()):
+        """As push, but each slot's new output comes back as 16-bit PCM scaled against `peak` (a float for every slot,
+        or {slot: float}): rint(y * (32767 / peak) * amplitude(volume)), times the stereo gains for a 2-channel voice,
+        saturated to the int16 range (TRMStreamPoolPushPCM16).  Returns {slot: (pcm, max)}: pcm is flat interleaved
+        int16 as TRMTubeModel.pcm16 returns it, max is max |y| over the samples this push produced (0.0 if none)."""
+        slots, slot_a, nf_a, fr, flush_a = self._entries(frames, flush)
+        n = len(slots)
+        peak_a = np.array([peak[s] if isinstance(peak, dict) else peak for s in slots], dtype=np.float64)
+        pcm = np.zeros(max(1, 2 * n * self.slot_capacity()), np.int16)
+        off = np.zeros(n + 1, np.int64)
+        mx = np.zeros(max(1, n), np.float64)
+        check(N.lib().TRMStreamPoolPushPCM16(self._h, n, _ptr(slot_a), _ptr(nf_a), _ptr(fr), _ptr(flush_a), _ptr(peak_a),
+                                             _ptr(pcm), _ptr(off), _ptr(mx)), "TRMStreamPoolPushPCM16")
+        return {s: (pcm[off[i]:off[i + 1]].copy(), float(mx[i])) for i, s in enumerate(slots)}
 
     def free(self):
         if self._h:

@@ -89,6 +89,20 @@ struct SrcPoolArgs {
     const void *ctab;                // Real[65536][SRC_CLD] (up-sampling coefficient rows)
 };
 
+// PCM16 of a stream pool push (pcm_pool_kernel): the same entries and work items as SrcPoolArgs, read from the packed
+// outputs.  Entry e's PCM goes to pcm[desc[e].pcm_offset + channels * (n - out_start)] (packed, entry after entry),
+// scaled against peak[e]; maxbits[e] (zero on entry) receives the bit pattern of max |y| over its outputs, as double.
+struct PcmPoolArgs {
+    const trm_cuda_utterance *desc;
+    int n;
+    const long long *item_base;      // [n+1] prefix sum of work items (runs of 32 consecutive outputs of one entry)
+    long long total_items;
+    const void *out;                 // Real[]
+    const double *peak;              // [n]
+    int16_t *pcm;
+    unsigned long long *maxbits;     // [n]
+};
+
 // Per-push bookkeeping kernels of a stream pool (kernels_aux.cu)
 struct PoolPrepArgs {
     const trm_cuda_utterance *src;   // [n] waveguide descriptors of this push

@@ -114,6 +114,15 @@ template <typename R> static int launch_src_pool(const SrcPoolArgs &a, int grid,
     return (int)cudaGetLastError();
 }
 
+template <typename R> static int launch_pcm_pool(const PcmPoolArgs &a, int grid, cudaStream_t s)
+{
+    if (a.total_items <= 0 || a.n <= 0) return 0;
+    const long long need = (a.total_items + 7) / 8;                      // 8 warps per CTA, one work item per warp
+    if ((long long)grid > need) grid = (int)need;
+    pcm_pool_kernel<R><<<grid, 256, 0, s>>>(a);
+    return (int)cudaGetLastError();
+}
+
 template <typename R> static int launch_src_ctab(const void *tab, void *ctab, cudaStream_t s)
 {
     const unsigned n = 65536u * SRC_CLD;
@@ -155,6 +164,10 @@ template <typename R> static int launch_pcm(const PcmArgs &a, long long max_n_ou
     extern "C" int trm_k_src_pool_##SUF(const trm::SrcPoolArgs *a, int grid, cudaStream_t s)                       \
     {                                                                                                             \
         return TRM_KERNEL_NS::launch_src_pool<R>(*a, grid, s);                                                              \
+    }                                                                                                             \
+    extern "C" int trm_k_pcm_pool_##SUF(const trm::PcmPoolArgs *a, int grid, cudaStream_t s)                       \
+    {                                                                                                             \
+        return TRM_KERNEL_NS::launch_pcm_pool<R>(*a, grid, s);                                                              \
     }                                                                                                             \
     extern "C" int trm_k_src_ctab_##SUF(const void *tab, void *ctab, cudaStream_t s)                              \
     {                                                                                                             \

@@ -566,6 +566,58 @@ __global__ void __launch_bounds__(256) src_pool_kernel(SrcPoolArgs args)
     }
 }
 
+// PCM16 of a stream pool push (trm_cuda_pool_push_pcm16), run after src_pool_kernel on its packed outputs with the same
+// work items (32 consecutive outputs of one entry, lane = output).  The scaling is pcm_kernel's, expression for
+// expression, with the caller's peak in place of the utterance's maximum; the result is then saturated to the int16
+// range, which never triggers when the peak is the true maximum (|y * scale| <= 32767 * amplitude <= 32767).  Entry
+// offsets are not 16-byte aligned (packed), so loads and stores are scalar; a stereo entry's PCM may start at an odd
+// element (after a mono entry with an odd count), so its two channels are two int16 stores.  max |y| per warp, then
+// one integer atomicMax on the double's bit pattern per work item (order independent for non-negative doubles); NaN
+// never wins, as in src_kernel.
+__device__ __forceinline__ int16_t pcm_sat(double v)
+{
+    const int q = __double2int_rn(v);
+    return (int16_t)(q < -32768 ? -32768 : (q > 32767 ? 32767 : q));
+}
+
+template <typename R>
+__global__ void __launch_bounds__(256) pcm_pool_kernel(PcmPoolArgs args)
+{
+    const int lane = threadIdx.x & 31;
+    const long long n_warps = (long long)gridDim.x * (blockDim.x >> 5);
+    const R *__restrict__ Y = reinterpret_cast<const R *>(args.out);
+    for (long long item = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); item < args.total_items; item += n_warps) {
+        int lo = 0, hi = args.n;                                         // entry: largest e with item_base[e] <= item
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (args.item_base[mid] <= item) lo = mid; else hi = mid;
+        }
+        const trm_cuda_utterance *__restrict__ D = args.desc + lo;
+        const long long k = (item - args.item_base[lo]) * 32 + lane;   // output of this push, relative to out_start
+        double m = 0.0;
+        if (D->out_start + k < D->n_out) {
+            const R v = Y[D->out_offset + k];
+            const double scale = (32767.0 / args.peak[lo]) * D->volumeAmp;          // TRMTubeModel.m:515
+            if (D->channels == 2) {
+                const double ls = D->leftGain * scale, rs = D->rightGain * scale;  // TRMTubeModel.m:532-533
+                int16_t *p = args.pcm + D->pcm_offset + 2 * k;
+                p[0] = pcm_sat((double)v * ls);
+                p[1] = pcm_sat((double)v * rs);
+            } else {
+                args.pcm[D->pcm_offset + k] = pcm_sat((double)v * scale);
+            }
+            const double av = fabs((double)v);
+            m = av > m ? av : m;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const double t = __shfl_xor_sync(0xffffffffu, m, o);
+            m = t > m ? t : m;
+        }
+        if (lane == 0 && m > 0.0) atomicMax(args.maxbits + lo, (unsigned long long)__double_as_longlong(m));
+    }
+}
+
 // All interpolated filter coefficients of the up-sampling converter: row F (the 16-bit fraction of the time register)
 // holds the 13 left-wing and 13 right-wing coefficients of an output with that fraction, computed with the reference's two
 // operations per coefficient (TRMSampleRateConverter.m:179-203).  Built once per context.

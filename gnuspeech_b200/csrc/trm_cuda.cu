@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -25,6 +26,7 @@
     int trm_k_src_##SUF(const trm::SrcArgs *, int, int, cudaStream_t);          \
     int trm_k_src_ctab_##SUF(const void *, void *, cudaStream_t);               \
     int trm_k_src_pool_##SUF(const trm::SrcPoolArgs *, int, cudaStream_t);     \
+    int trm_k_pcm_pool_##SUF(const trm::PcmPoolArgs *, int, cudaStream_t);     \
     int trm_k_pcm_##SUF(const trm::PcmArgs *, long long, cudaStream_t);
 extern "C" {
 TRM_DECLARE_LAUNCHERS(f64)
@@ -46,11 +48,12 @@ struct KernelSet {
     int (*pcm)(const trm::PcmArgs *, long long, cudaStream_t);
     int (*src_pool)(const trm::SrcPoolArgs *, int, cudaStream_t);
     int (*tube_wide_pool)(const trm::TubeArgs *, int, cudaStream_t);   // state stored per utterance (tube_wide.cuh)
+    int (*pcm_pool)(const trm::PcmPoolArgs *, int, cudaStream_t);
 };
 static const KernelSet g_kernels[3] = {
-    {trm_k_tube_wide_f64, trm_k_src_f64, trm_k_pcm_f64, trm_k_src_pool_f64, trm_k_tube_wide_pool_f64},
-    {trm_k_tube_wide_f32, trm_k_src_f32, trm_k_pcm_f32, trm_k_src_pool_f32, trm_k_tube_wide_pool_f32},
-    {trm_k_tube_wide_f64s, trm_k_src_f64s, trm_k_pcm_f64s, trm_k_src_pool_f64s, trm_k_tube_wide_pool_f64s},
+    {trm_k_tube_wide_f64, trm_k_src_f64, trm_k_pcm_f64, trm_k_src_pool_f64, trm_k_tube_wide_pool_f64, trm_k_pcm_pool_f64},
+    {trm_k_tube_wide_f32, trm_k_src_f32, trm_k_pcm_f32, trm_k_src_pool_f32, trm_k_tube_wide_pool_f32, trm_k_pcm_pool_f32},
+    {trm_k_tube_wide_f64s, trm_k_src_f64s, trm_k_pcm_f64s, trm_k_src_pool_f64s, trm_k_tube_wide_pool_f64s, trm_k_pcm_pool_f64s},
 };
 
 // FMA-chain kernels used to MEASURE the FP32 / FP64 CUDA-core peak of the device the bench runs on
@@ -1346,6 +1349,8 @@ struct trm_cuda_pool {
     long long cap_out = 0;              // output samples one slot can return from one push
     unsigned char *d_tube = nullptr;    // [2][cap][stride] tube-rate history, two buffers per slot
     unsigned char *d_out = nullptr;     // [cap * cap_out] outputs of a push, packed entry after entry
+    int16_t *d_pcm = nullptr;           // [pcm_cap] PCM16 of a push, packed entry after entry (allocated by the first PCM push)
+    long long pcm_cap = 0;
     unsigned char *d_state = nullptr;   // [cap] carried waveguide states
     trm_cuda_utterance *d_desc = nullptr;   // [cap] waveguide descriptors, indexed by slot like the states
     double *d_wavetables = nullptr;     // [cap][512]: row s is slot s's glottal table
@@ -1446,6 +1451,7 @@ void trm_cuda_pool_destroy(trm_cuda_pool *p)
     if (p->st) { cudaStreamSynchronize(p->st); cudaStreamDestroy(p->st); }
     if (p->d_tube) cudaFree(p->d_tube);
     if (p->d_out) cudaFree(p->d_out);
+    if (p->d_pcm) cudaFree(p->d_pcm);
     if (p->d_state) cudaFree(p->d_state);
     if (p->d_desc) cudaFree(p->d_desc);
     if (p->d_wavetables) cudaFree(p->d_wavetables);
@@ -1454,12 +1460,23 @@ void trm_cuda_pool_destroy(trm_cuda_pool *p)
     delete p;
 }
 
-int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
-                       const uint8_t *flush, void *samples_host, int64_t *out_offset)
+// What a PCM push returns instead of samples (trm_cuda_pool_push_pcm16)
+struct PoolPcm {
+    const double *peak;     // [n]
+    int16_t *out;           // packed PCM16, or NULL
+    int64_t *offset;        // [n+1]
+    double *max;            // [n], or NULL
+};
+
+// One push: samples (pcm == nullptr) into samples_host, or PCM16 as `pcm` says.  out_offset receives the packed sample
+// offsets either way (the layout of d_out).
+static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                     const uint8_t *flush, void *samples_host, int64_t *out_offset, const PoolPcm *pcm)
 {
     // ---- arguments: everything is checked before the pool changes -----------------------------------------------
     if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_push: bad entry count");
     if (!out_offset || (n > 0 && (!slot || !n_frames))) return pool_err(-4, "trm_cuda_pool_push: null argument");
+    if (pcm && (!pcm->offset || (n > 0 && !pcm->peak))) return pool_err(-4, "trm_cuda_pool_push_pcm16: null argument");
     long long total_in = 0;
     {
         std::vector<unsigned char> named((size_t)p->cap, 0);
@@ -1470,14 +1487,23 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
             if (named[s]) return pool_err(-4, "trm_cuda_pool_push: a slot is named twice");
             named[s] = 1;
             if (n_frames[i] < 0 || n_frames[i] > p->max_m) return pool_err(-4, "trm_cuda_pool_push: more frames than the pool was created for");
+            if (pcm && !(std::isfinite(pcm->peak[i]) && pcm->peak[i] > 0.0)) return pool_err(-4, "trm_cuda_pool_push_pcm16: a peak is not finite and > 0");
             total_in += n_frames[i];
         }
     }
     if (total_in > 0 && !frames_host) return pool_err(-4, "trm_cuda_pool_push: null frames");
     out_offset[0] = 0;
+    if (pcm) pcm->offset[0] = 0;
     if (n == 0) return 0;
     trm_cuda_ctx *ctx = p->ctx;
     CK(cudaSetDevice(ctx->device));
+    if (pcm && p->pcm_cap < 2 * p->cap * p->cap_out) {   // stereo: two int16 per sample
+        if (p->d_pcm) cudaFree(p->d_pcm);
+        p->d_pcm = nullptr;
+        p->pcm_cap = 0;
+        CK(cudaMalloc((void **)&p->d_pcm, (size_t)2 * p->cap * p->cap_out * sizeof(int16_t)));
+        p->pcm_cap = 2 * (long long)p->cap * p->cap_out;
+    }
 
     // ---- per entry: what trm_cuda_stream_push computes for one stream ------------------------------------------------
     struct Entry {
@@ -1526,12 +1552,14 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
         }
         total_out += n_ret > 0 ? n_ret : 0;
         out_offset[i + 1] = total_out;
+        if (pcm) pcm->offset[i + 1] = pcm->offset[i] + (n_ret > 0 ? n_ret * sl.voice.channels : 0);
     }
 
     // ---- host tables of the push, laid out as in the device scratch: one upload ------------------------------------
     std::vector<int> wg;                                  // entries that run the waveguide, longest first
     std::vector<trm_cuda_utterance> rd;                   // resampler views of the entries that return samples
     std::vector<long long> ib(1, 0), mv;                  // work-item prefix; history moves {src, dst, len}
+    std::vector<int> rd_entry;                            // entry of each resampler view
     for (int i = 0; i < n; ++i) {
         const Entry &e = E[i];
         if (!e.run) continue;
@@ -1546,8 +1574,9 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
             r.out_start = sl.out_done;
             r.in_start = sl.in_start;
             r.out_offset = out_offset[i];
-            r.pcm_offset = 0;
+            r.pcm_offset = pcm ? pcm->offset[i] : 0;
             rd.push_back(r);
+            rd_entry.push_back(i);
             ib.push_back(ib.back() + (n_ret + 31) / 32);
         }
         const long long keep = e.target - e.next_in;
@@ -1565,7 +1594,10 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
     const size_t o_rd = o_rst + align_up(wg.size() * sizeof(int), 256);
     const size_t o_ib = o_rd + align_up(n_rd * sizeof(trm_cuda_utterance), 256);
     const size_t o_mv = o_ib + align_up(ib.size() * sizeof(long long), 256);
-    const size_t o_fr = o_mv + align_up(mv.size() * sizeof(long long), 256);
+    const size_t n_pk = pcm ? n_rd : 0;                   // PCM: peak and max |y| of each resampler view
+    const size_t o_pk = o_mv + align_up(mv.size() * sizeof(long long), 256);
+    const size_t o_mx = o_pk + align_up(n_pk * sizeof(double), 256);
+    const size_t o_fr = o_mx + align_up(n_pk * sizeof(unsigned long long), 256);
     const size_t bytes = o_fr + (size_t)wg_frames * 128;
     int rc;
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
@@ -1595,6 +1627,8 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
         if (n_rd) memcpy(h + o_rd, rd.data(), n_rd * sizeof(trm_cuda_utterance));
         memcpy(h + o_ib, ib.data(), ib.size() * sizeof(long long));
         if (n_mv) memcpy(h + o_mv, mv.data(), mv.size() * sizeof(long long));
+        for (size_t j = 0; j < n_pk; ++j) ((double *)(h + o_pk))[j] = pcm->peak[rd_entry[j]];
+        if (n_pk) memset(h + o_mx, 0, n_pk * sizeof(unsigned long long));
     }
     unsigned char *d = p->scratch.base;
     cudaStream_t st = p->st;
@@ -1624,13 +1658,31 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
         a.ctab = prec_is_f64(p->precision) ? ctx->d_ctab_f64 : ctx->d_ctab_f32;
         if ((rc = K.src_pool(&a, ctx->sm_count * 8, st)) != 0) return fail("pool resampler launch", (cudaError_t)rc);
     }
+    if (n_pk > 0) {
+        trm::PcmPoolArgs a{};
+        a.desc = (const trm_cuda_utterance *)(d + o_rd); a.n = (int)n_rd; a.item_base = (const long long *)(d + o_ib);
+        a.total_items = ib.back(); a.out = p->d_out; a.peak = (const double *)(d + o_pk); a.pcm = p->d_pcm;
+        a.maxbits = (unsigned long long *)(d + o_mx);
+        if ((rc = K.pcm_pool(&a, ctx->sm_count * 8, st)) != 0) return fail("pool PCM launch", (cudaError_t)rc);
+    }
     if (n_mv > 0) {
         trm::PoolMoveArgs a{};
         a.moves = (const long long *)(d + o_mv); a.buf = p->d_tube; a.esz = (int)p->esz; a.n = (int)n_mv;
         if ((rc = trm_k_pool_move(&a, st)) != 0) return fail("pool history move launch", (cudaError_t)rc);
     }
-    if (samples_host && total_out > 0) CK(cudaMemcpyAsync(samples_host, p->d_out, (size_t)total_out * p->esz, cudaMemcpyDeviceToHost, st));
+    if (pcm) {
+        if (pcm->out && pcm->offset[n] > 0)
+            CK(cudaMemcpyAsync(pcm->out, p->d_pcm, (size_t)pcm->offset[n] * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
+        // the maxima come back into the staging buffer (its upload precedes this copy on the stream)
+        if (pcm->max && n_pk) CK(cudaMemcpyAsync(h + o_mx, d + o_mx, n_pk * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    } else if (samples_host && total_out > 0) {
+        CK(cudaMemcpyAsync(samples_host, p->d_out, (size_t)total_out * p->esz, cudaMemcpyDeviceToHost, st));
+    }
     CK(cudaStreamSynchronize(st));
+    if (pcm && pcm->max) {
+        for (int i = 0; i < n; ++i) pcm->max[i] = 0.0;
+        for (size_t j = 0; j < n_pk; ++j) memcpy(&pcm->max[rd_entry[j]], h + o_mx + j * sizeof(unsigned long long), sizeof(double));
+    }
 
     // ---- bookkeeping -------------------------------------------------------------------------------------------
     for (int i = 0; i < n; ++i) {
@@ -1653,6 +1705,21 @@ int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32
         }
     }
     return 0;
+}
+
+int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                       const uint8_t *flush, void *samples_host, int64_t *out_offset)
+{
+    return pool_push(p, n, slot, n_frames, frames_host, flush, samples_host, out_offset, nullptr);
+}
+
+int trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                             const uint8_t *flush, const double *peak, int16_t *pcm_host, int64_t *pcm_offset, double *max_host)
+{
+    if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_push: bad entry count");
+    std::vector<int64_t> out_offset((size_t)n + 1);
+    const PoolPcm pcm{peak, pcm_host, pcm_offset, max_host};
+    return pool_push(p, n, slot, n_frames, frames_host, flush, nullptr, out_offset.data(), &pcm);
 }
 
 int trm_cuda_resident_create(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,

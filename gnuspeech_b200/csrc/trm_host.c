@@ -1223,6 +1223,15 @@ int TRMStreamPoolPush(TRMStreamPool *t, int n, const int32_t *slot, const int32_
     return rc != 0 ? pool_rc(rc) : TRM_OK;
 }
 
+int TRMStreamPoolPushPCM16(TRMStreamPool *t, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
+                           const uint8_t *flush, const double *peak, int16_t *pcm_out, int64_t *pcm_offset, double *max_out)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    const int rc = trm_cuda_pool_push_pcm16(t->p, n, slot, n_frames, (const double *)frames, flush, peak, pcm_out, pcm_offset,
+                                            max_out);
+    return rc != 0 ? pool_rc(rc) : TRM_OK;
+}
+
 void TRMStreamPoolFree(TRMStreamPool *t)
 {
     if (!t) return;

@@ -341,6 +341,21 @@ int64_t TRMStreamPoolSlotCapacity(const TRMStreamPool *pool);
  * fail the whole push before any work: the pool is left exactly as it was. */
 int TRMStreamPoolPush(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
                       const uint8_t *flush, void *samples_out, int64_t *out_offset /* [n + 1] */);
+/* As TRMStreamPoolPush, but entry i's new output comes back as 16-bit PCM, host endian, channels interleaved as the
+ * slot's voice says (1 or 2):
+ *   scale = (32767 / peak[i]) * amplitude(volume);  mono: rint(y * scale);
+ *   stereo: rint(y * leftGain * scale), rint(y * rightGain * scale)   (the WAV variant, TRMTubeModel.m:515-559),
+ *   saturated to [-32768, 32767].
+ * With peak[i] equal to the utterance's maximumSampleValue, a slot's PCM pushes, concatenated, equal TRMBatch's pcm_out
+ * for that utterance bit for bit.  Entry i's PCM is pcm_out[pcm_offset[i] .. pcm_offset[i+1]) (int16 elements; frames =
+ * elements / channels); pcm_out holds 2 * n * TRMStreamPoolSlotCapacity elements.  max_out[i] (may be NULL): max |y| over
+ * the samples entry i produced in this push, 0.0 if none (NaN never wins, as in maximumSampleValue); the maximum over a
+ * slot's pushes equals TRMBatch's maximumSampleValue.  peak[i] must be finite and > 0 (TRM_ERR_PARAM).  All refusals of
+ * TRMStreamPoolPush apply, and are checked, with peak, before any device work: a refused push leaves the pool unchanged.
+ * A slot may be advanced by TRMStreamPoolPush and TRMStreamPoolPushPCM16 in any order. */
+int TRMStreamPoolPushPCM16(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames,
+                           const TRMParameters *frames, const uint8_t *flush, const double *peak,
+                           int16_t *pcm_out, int64_t *pcm_offset /* [n + 1] */, double *max_out);
 void TRMStreamPoolFree(TRMStreamPool *pool);
 
 /* ---------------------------------------------------------------------------------------------

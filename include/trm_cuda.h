@@ -204,6 +204,11 @@ int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one 
  * the slot and frees it.  samples_host receives the samples packed (entry i: [out_offset[i], out_offset[i+1])). */
 int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
                         const uint8_t *flush, void *samples_host, int64_t *out_offset);
+/* the same push, returning PCM16 scaled against peak[i] (finite, > 0), saturated: entry i's int16 elements are
+ * pcm_host[pcm_offset[i], pcm_offset[i+1]), channels interleaved; max_host[i] (may be NULL) receives max |y| over the
+ * samples entry i produced (0.0 if none).  pcm_kernel's arithmetic (TRMTubeModel.m:515-559) and include/trm.h's contract. */
+int  trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
+                              const uint8_t *flush, const double *peak, int16_t *pcm_host, int64_t *pcm_offset, double *max_host);
 void trm_cuda_pool_destroy(trm_cuda_pool *p);
 /*
  * Control frames on the device (replaces -[EventList generateOutputInTimeRange:...], EventList.m:883-1061): uploads

@@ -2,6 +2,7 @@
 
 Rows: n active slots x pushes of m frames (4 ms each), FP64 and FP32:
   pool     -- n slots of the default male voice, every slot pushed with m frames (the lockstep shape through the pool)
+  pool pcm -- the same slots and frames through TRMStreamPoolPushPCM16 (mono PCM16 instead of samples; also for mixed)
   stream   -- the same through one TRMStream of n streams
   mixed    -- n slots at random positions with three voices (male 44.1 kHz, female, 10 cm tract at 22.05 kHz),
               random frame counts 0..m per slot and push, 10 % of the slots flushing or opening per push
@@ -28,12 +29,35 @@ def vp(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
-def pool_lockstep(prec, n, m, frames, warm, reps):
+class Push(object):
+    """One pool push into pageable numpy buffers: samples (TRMStreamPoolPush), or PCM16 scaled against a fixed peak
+    with the per-entry maxima (TRMStreamPoolPushPCM16)."""
+
+    def __init__(self, pool, n, prec, pcm):
+        self.pool, self.pcm = pool, pcm
+        cap = pool.slot_capacity()
+        self.off = np.zeros(n + 1, np.int64)
+        if pcm:
+            self.out = np.zeros(2 * n * cap, np.int16)
+            self.peak = np.ones(n, np.float64)
+            self.mx = np.zeros(n, np.float64)
+        else:
+            self.out = np.zeros(n * cap, np.float64 if prec != 1 else np.float32)
+
+    def __call__(self, slots, nf, fr, fl):
+        L, h, n = N.lib(), self.pool._h, len(slots)
+        if self.pcm:
+            N.check(L.TRMStreamPoolPushPCM16(h, n, vp(slots), vp(nf), vp(fr), vp(fl), vp(self.peak), vp(self.out), vp(self.off),
+                                             vp(self.mx)), "push pcm16")
+        else:
+            N.check(L.TRMStreamPoolPush(h, n, vp(slots), vp(nf), vp(fr), vp(fl), vp(self.out), vp(self.off)), "push")
+
+
+def pool_lockstep(prec, n, m, frames, warm, reps, pcm=False):
     ip = g.TRMInputParameters(44100.0)
     pool = g.TRMStreamPool(n, precision=prec, max_frames_per_push=m + 1)
     slots = np.array([pool.open(ip) for _ in range(n)], np.int32)
-    out = np.zeros(n * pool.slot_capacity(), np.float64 if prec != 1 else np.float32)
-    off = np.zeros(n + 1, np.int64)
+    push = Push(pool, n, prec, pcm)
     fl = np.zeros(n, np.uint8)
     t = []
     for k in range(warm + reps):
@@ -41,7 +65,7 @@ def pool_lockstep(prec, n, m, frames, warm, reps):
         fr = np.ascontiguousarray(frames[:n, a:b])
         nf = np.full(n, b - a, np.int32)
         t0 = time.perf_counter()
-        N.check(N.lib().TRMStreamPoolPush(pool._h, n, vp(slots), vp(nf), vp(fr), vp(fl), vp(out), vp(off)), "push")
+        push(slots, nf, fr, fl)
         if k >= warm:
             t.append(time.perf_counter() - t0)
     pool.free()
@@ -64,7 +88,7 @@ def stream_lockstep(prec, n, m, frames, warm, reps):
     return float(np.median(t))
 
 
-def pool_mixed(prec, n, m, frames, warm, reps, seed=5):
+def pool_mixed(prec, n, m, frames, warm, reps, pcm=False, seed=5):
     rng = np.random.default_rng(seed)
     female = g.MMSynthesisParameters("Female").inputParameters()
     female.channels = 1
@@ -73,9 +97,7 @@ def pool_mixed(prec, n, m, frames, warm, reps, seed=5):
     pos = {}                                             # slot -> frames sent (row into `frames`)
     for i in range(n):
         pos[pool.open(voices[i % 3])] = int(rng.integers(0, 40))     # random positions in the frame tracks
-    cap = pool.slot_capacity()
-    out = np.zeros(n * cap, np.float64 if prec != 1 else np.float32)
-    off = np.zeros(n + 1, np.int64)
+    push = Push(pool, n, prec, pcm)
     t, audio = [], []
     # every slot's first push: bring it to its position
     for k in range(warm + reps):
@@ -86,7 +108,7 @@ def pool_mixed(prec, n, m, frames, warm, reps, seed=5):
         nf = np.array([r.shape[0] for r in rows], np.int32)
         fr = np.ascontiguousarray(np.concatenate(rows))
         t0 = time.perf_counter()
-        N.check(N.lib().TRMStreamPoolPush(pool._h, len(slots), vp(slots), vp(nf), vp(fr), vp(fl), vp(out), vp(off)), "push")
+        push(slots, nf, fr, fl)
         dt = time.perf_counter() - t0
         if k >= warm:
             t.append(dt)
@@ -117,20 +139,22 @@ def main():
     reps, warm = args.pushes, args.warmup
     m_max = 25
     frames = W.random_walk(max(sizes), 1 + (warm + reps + 1) * m_max, seed=3).reshape(max(sizes), -1, 16)
-    print("%-5s %-6s %6s %6s %11s %11s %7s %12s" % ("prec", "shape", "slots", "push", "pool ms", "stream ms", "ratio",
-                                                   "audio-s/s"), flush=True)
+    print("%-5s %-6s %6s %6s %11s %11s %11s %7s %9s %12s" % ("prec", "shape", "slots", "push", "pool ms", "pool pcm ms",
+                                                            "stream ms", "ratio", "pcm/pool", "audio-s/s"), flush=True)
     for prec, name in ((0, "fp64"), (1, "fp32")):
         for n in sizes:
             for m in (5, 25):
                 tp = pool_lockstep(prec, n, m, frames, warm, reps)
+                tq = pool_lockstep(prec, n, m, frames, warm, reps, pcm=True)
                 ts = stream_lockstep(prec, n, m, frames, warm, reps)
-                print("%-5s %-6s %6d %4dms %11.3f %11.3f %7.2f %12.0f" % (name, "lock", n, m * 4, tp * 1e3, ts * 1e3, tp / ts,
-                                                                          n * m * 0.004 / tp), flush=True)
+                print("%-5s %-6s %6d %4dms %11.3f %11.3f %11.3f %7.2f %9.2f %12.0f" % (
+                    name, "lock", n, m * 4, tp * 1e3, tq * 1e3, ts * 1e3, tp / ts, tq / tp, n * m * 0.004 / tp), flush=True)
         for n in sizes[-2:]:
             for m in (5, 25):
                 tm, audio = pool_mixed(prec, n, m, frames, warm, reps)
-                print("%-5s %-6s %6d %4dms %11.3f %11s %7s %12.0f" % (name, "mixed", n, m * 4, tm * 1e3, "-", "-", audio / tm),
-                      flush=True)
+                tq, _ = pool_mixed(prec, n, m, frames, warm, reps, pcm=True)
+                print("%-5s %-6s %6d %4dms %11.3f %11.3f %11s %7s %9.2f %12.0f" % (
+                    name, "mixed", n, m * 4, tm * 1e3, tq * 1e3, "-", "-", tq / tm, audio / tm), flush=True)
 
 
 if __name__ == "__main__":
