@@ -179,12 +179,17 @@ __device__ __forceinline__ double blend(unsigned m, double x, double y)
     return __hiloint2double((int)hi, (int)lo);
 }
 
-// fast-mode amplitude(): 10^((dB-60)/20) as 2^(..), FP32 (relative error ~5e-7, i.e. -126 dB on a linear gain)
-__device__ __forceinline__ float amplitude_f(float dB)
+// amplitude()'s lower clamp (TRMUtility.m:26-41) as the reference decides it: `dB -= 60; if (dB <= -60) return 0` in double
+// holds for every dB <= 2^-48 (half an ulp of 60 rounds to even, to -60), not only for dB <= 0
+constexpr double AMP_ZERO_DB = 0x1p-48;
+
+// fast-mode amplitude(): 10^((dB-60)/20) as 2^(..), FP32 (relative error ~5e-7, i.e. -126 dB on a linear gain).  The clamp
+// to 0 is decided on the double parameter: (float)dB - 60 already rounds to -60 below 2^-19, where the reference gives 1e-3.
+__device__ __forceinline__ float amplitude_f(double dB)
 {
-    const float x = dB - 60.0f;
+    const float x = (float)dB - 60.0f;
     const float v = exp2f(fminf(x, 0.0f) * 0.16609640474436813f);    // x >= 0 -> exactly 1
-    return (x <= -60.0f) ? 0.0f : v;
+    return (dB <= AMP_ZERO_DB) ? 0.0f : v;
 }
 
 // fast-mode glottal table: rise 3x^2 - 2x^3 (x = i/div1), fall 1 - (j*j)/L^2, closed 0 -- evaluated, never loaded

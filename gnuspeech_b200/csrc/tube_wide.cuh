@@ -957,19 +957,20 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
         R ax, ah1;
         R bp_alpha2;
         if constexpr (F64C) {
-            // amplitude() (TRMUtility.m:26-41): clamps decided on the exact parameter, value from the geometric sequence
+            // amplitude() (TRMUtility.m:26-41): clamps decided on the interpolated parameter (the reference's adds) with the
+            // reference's bounds, 0 for dB <= 2^-48 and 1 for dB >= 60; value from the geometric sequence
             const double p1 = prm[0], p2 = prm[1], p3 = prm[2], fpos = prm[3];
-            ax_d = (p1 <= 0.0) ? 0.0 : ((p1 >= 60.0) ? 1.0 : prm[15]);
+            ax_d = (p1 <= AMP_ZERO_DB) ? 0.0 : ((p1 >= 60.0) ? 1.0 : prm[15]);
             {
                 // glottal closure point rint(ax * tnDelta) (TRMWavetable.m:122): when the product is within 1e-6 of a
                 // rounding boundary, decide with the amplitude computed directly from the parameter
                 const double tq = ax_d * S.CST[C_TNDELTA];
-                if (fabs(fabs(tq - rint(tq)) - 0.5) < 1e-6 && p1 > 0.0 && p1 < 60.0)
+                if (fabs(fabs(tq - rint(tq)) - 0.5) < 1e-6 && p1 > AMP_ZERO_DB && p1 < 60.0)
                     ax_d = exp2_inline((p1 - 60.0) * 0.16609640474436813);
             }
             ax = ax_d;
-            ah1 = (p2 <= 0.0) ? 0.0 : ((p2 >= 60.0) ? 1.0 : prm[16]);
-            const double fa = (p3 <= 0.0) ? 0.0 : ((p3 >= 60.0) ? 1.0 : prm[17]);
+            ah1 = (p2 <= AMP_ZERO_DB) ? 0.0 : ((p2 >= 60.0) ? 1.0 : prm[16]);
+            const double fa = (p3 <= AMP_ZERO_DB) ? 0.0 : ((p3 >= 60.0) ? 1.0 : prm[17]);
             const double dd = S.CST[C_DAMP];
             double r2[8];
 #pragma unroll
@@ -1010,7 +1011,7 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             W.ring[slot][9][hl][ucol] = make_double2(tap[7], gamma2);
             reinterpret_cast<double *>(&W.ring[slot][10][hl][ucol])[0] = beta2;
         } else if constexpr (FAST) {
-            const float axf = amplitude_f((float)prm[1]);
+            const float axf = amplitude_f(prm[1]);
             ax_d = (double)axf;
             {
                 const float tq = axf * (float)S.CST[C_TNDELTA];
@@ -1018,8 +1019,8 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
                 if (fabsf(fr - 0.5f) < 2e-3f) ax_d = amplitude_db(prm[1]);
             }
             ax = axf;
-            ah1 = amplitude_f((float)prm[2]);
-            const float fa = amplitude_f((float)prm[3]);
+            ah1 = amplitude_f(prm[2]);
+            const float fa = amplitude_f(prm[3]);
             const float dd = (float)S.CST[C_DAMP];
             float r2[8];
 #pragma unroll
