@@ -58,6 +58,11 @@ class TRMBatchLayoutStruct(C.Structure):
                 ("audio_seconds", C.c_double), ("tube_samples", C.c_int64), ("out_samples", C.c_int64)]
 
 
+class TRMStreamSnapshotInfoStruct(C.Structure):
+    _fields_ = [("precision", C.c_int32), ("channels", C.c_int32), ("voice", TRMInputParametersStruct),
+                ("frames_pushed", C.c_int64), ("samples_returned", C.c_int64), ("bytes", C.c_int64)]
+
+
 _lib = None
 
 
@@ -142,6 +147,9 @@ def lib():
     sig("TRMStreamPoolPush", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp)
     sig("TRMStreamPoolPushPCM16", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("TRMStreamPoolFree", None, vp)
+    sig("TRMStreamPoolSave", C.c_int, vp, C.c_int, vp, vp, i64, vp)
+    sig("TRMStreamPoolRestore", C.c_int, vp, C.c_int, vp, vp, vp)
+    sig("TRMStreamPoolSnapshotInfo", C.c_int, vp, i64, P(TRMStreamSnapshotInfoStruct))
     sig("TRMBatchSynthesizeAsync", vp, vp, vp, vp, vp, vp, C.c_int, vp)
     sig("TRMBatchWait", C.c_int, vp)
     sig("TRMBatchMakeResident", vp, vp, vp, C.c_int, P(C.c_int))

@@ -602,6 +602,29 @@ class TRMStreamPool(object):
                                              _ptr(pcm), _ptr(off), _ptr(mx)), "TRMStreamPoolPushPCM16")
         return {s: (pcm[off[i]:off[i + 1]].copy(), float(mx[i])) for i, s in enumerate(slots)}
 
+    def save(self, slots):
+        """Snapshots of open slots (TRMStreamPoolSave): {slot: bytes}.  Each restores into any pool of this precision
+        and continues the stream bit for bit; the saved slots are not changed."""
+        slots = [int(s) for s in slots]
+        slot_a = np.array(slots, dtype=np.int32)
+        off = np.zeros(len(slots) + 1, np.int64)
+        check(N.lib().TRMStreamPoolSave(self._h, len(slots), _ptr(slot_a), None, 0, _ptr(off)), "TRMStreamPoolSave")
+        blob = np.zeros(max(1, int(off[-1])), np.uint8)
+        check(N.lib().TRMStreamPoolSave(self._h, len(slots), _ptr(slot_a), _ptr(blob), blob.size, _ptr(off)),
+              "TRMStreamPoolSave")
+        return {s: blob[off[i]:off[i + 1]].tobytes() for i, s in enumerate(slots)}
+
+    def restore(self, snapshots):
+        """Opens one free slot per snapshot (bytes from save, in this or any other pool of the same precision); returns
+        the slots in order.  All or nothing (TRMStreamPoolRestore)."""
+        snapshots = [bytes(b) for b in snapshots]
+        off = np.zeros(len(snapshots) + 1, np.int64)
+        off[1:] = np.cumsum([len(b) for b in snapshots])
+        blob = np.frombuffer(b"".join(snapshots) or b"\0", np.uint8)
+        out = np.zeros(max(1, len(snapshots)), np.int32)
+        check(N.lib().TRMStreamPoolRestore(self._h, len(snapshots), _ptr(blob), _ptr(off), _ptr(out)), "TRMStreamPoolRestore")
+        return [int(s) for s in out[:len(snapshots)]]
+
     def free(self):
         if self._h:
             N.lib().TRMStreamPoolFree(self._h)
@@ -609,6 +632,20 @@ class TRMStreamPool(object):
 
     def __del__(self):
         self.free()
+
+
+def snapshot_info(snapshot):
+    """What a stream pool snapshot holds, after the checks a restore makes apart from the destination pool
+    (TRMStreamPoolSnapshotInfo; needs no device): {precision, channels, voice (TRMInputParameters), frames_pushed,
+    samples_returned, bytes}.  Raises TRMError for a snapshot a restore would refuse on its own."""
+    b = bytes(snapshot)
+    buf = C.create_string_buffer(b, max(1, len(b)))
+    info = N.TRMStreamSnapshotInfoStruct()
+    check(N.lib().TRMStreamPoolSnapshotInfo(buf, len(b), C.byref(info)), "TRMStreamPoolSnapshotInfo")
+    voice = TRMInputParameters()
+    C.memmove(C.byref(voice), C.byref(info.voice), C.sizeof(voice))
+    return {"precision": info.precision, "channels": info.channels, "voice": voice, "frames_pushed": info.frames_pushed,
+            "samples_returned": info.samples_returned, "bytes": info.bytes}
 
 
 class TRMBatchTicket(object):

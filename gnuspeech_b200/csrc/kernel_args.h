@@ -114,10 +114,13 @@ struct PoolPrepArgs {
     unsigned long long noise_k0;
     int n;
 };
-struct PoolMoveArgs {
-    const long long *moves;          // [n][3]: source element, destination element, length (elements)
-    void *buf;                       // history buffers of all slots
-    int esz;                         // bytes per element
+// Ragged device-to-device copies (segment_copy_kernel): a push's history moves, a snapshot's gather and scatter
+struct CopySeg {
+    unsigned long long src, dst;     // device addresses
+    unsigned long long bytes;        // a multiple of 4
+};
+struct SegCopyArgs {
+    const CopySeg *seg;              // [n], no two overlapping
     int n;
 };
 

@@ -111,15 +111,23 @@ __global__ void pool_prepare_kernel(trm::PoolPrepArgs a)
     }
 }
 
-// One CTA per entry: the kept tube-rate history of a slot moves to the front of its other buffer (ragged lengths).
-__global__ void pool_move_kernel(trm::PoolMoveArgs a)
+// One CTA per segment {src, dst, bytes} (ragged lengths): 16-byte accesses when both addresses and the length are
+// multiples of 16, 4-byte words otherwise.  A push's history moves and a snapshot's state and history always take the
+// 16-byte path (rows start on 32 elements, histories hold a multiple of 4 elements, states are 416 or 800 bytes).
+__global__ void segment_copy_kernel(trm::SegCopyArgs a)
 {
-    const long long *m = a.moves + 3 * (size_t)blockIdx.x;
-    const int w = a.esz / 4;                                            // 4-byte words per element
-    const unsigned *src = reinterpret_cast<const unsigned *>(a.buf) + m[0] * w;
-    unsigned *dst = reinterpret_cast<unsigned *>(a.buf) + m[1] * w;
-    const long long words = m[2] * w;
-    for (long long i = threadIdx.x; i < words; i += blockDim.x) dst[i] = src[i];
+    const trm::CopySeg g = a.seg[blockIdx.x];
+    if (((g.src | g.dst | g.bytes) & 15ull) == 0) {
+        const uint4 *src = reinterpret_cast<const uint4 *>(g.src);
+        uint4 *dst = reinterpret_cast<uint4 *>(g.dst);
+        const long long n = (long long)(g.bytes >> 4);
+        for (long long i = threadIdx.x; i < n; i += blockDim.x) dst[i] = src[i];
+    } else {
+        const unsigned *src = reinterpret_cast<const unsigned *>(g.src);
+        unsigned *dst = reinterpret_cast<unsigned *>(g.dst);
+        const long long n = (long long)(g.bytes >> 2);
+        for (long long i = threadIdx.x; i < n; i += blockDim.x) dst[i] = src[i];
+    }
 }
 
 extern "C" int trm_k_pool_prepare(const trm::PoolPrepArgs *a, cudaStream_t s)
@@ -129,9 +137,9 @@ extern "C" int trm_k_pool_prepare(const trm::PoolPrepArgs *a, cudaStream_t s)
     return (int)cudaGetLastError();
 }
 
-extern "C" int trm_k_pool_move(const trm::PoolMoveArgs *a, cudaStream_t s)
+extern "C" int trm_k_segment_copy(const trm::SegCopyArgs *a, cudaStream_t s)
 {
     if (a->n <= 0) return 0;
-    pool_move_kernel<<<a->n, 128, 0, s>>>(*a);
+    segment_copy_kernel<<<a->n, 128, 0, s>>>(*a);
     return (int)cudaGetLastError();
 }

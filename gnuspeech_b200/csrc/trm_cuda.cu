@@ -36,7 +36,7 @@ int trm_k_framegen(const trm::FrameGenArgs *, cudaStream_t);
 int trm_k_workload_walk2(unsigned long long, unsigned long long, long long, int, double *, cudaStream_t);
 int trm_k_pcm_checksum(const trm_cuda_utterance *, int, const int16_t *, unsigned long long *, cudaStream_t);
 int trm_k_pool_prepare(const trm::PoolPrepArgs *, cudaStream_t);
-int trm_k_pool_move(const trm::PoolMoveArgs *, cudaStream_t);
+int trm_k_segment_copy(const trm::SegCopyArgs *, cudaStream_t);
 }
 
 // precision codes of include/trm.h: 0 = FP64 conformance, 1 = FP32 fast, 2 = FP64 strict
@@ -1358,6 +1358,7 @@ struct trm_cuda_pool {
     HostStage stage;
     cudaStream_t st = nullptr;
     long long tube_at(int slot, int buf) const { return ((long long)buf * cap + slot) * stride; }
+    unsigned long long tube_addr(long long elem) const { return (unsigned long long)(uintptr_t)(d_tube + (size_t)elem * esz); }
 };
 
 static int pool_err(int code, const char *what)
@@ -1384,13 +1385,27 @@ int trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max
     return 0;
 }
 
+// the sizes trm_cuda_stream_create gives one stream of this voice: history elements per slot and buffer, samples per push
+static void pool_sizes(const trm_cuda_pool *p, const trm_cuda_utterance *v, long long *stride, long long *cap_out)
+{
+    const long long max_new = (long long)(p->max_m + 1) * v->controlPeriod + 32;
+    *stride = (long long)align_up((size_t)(max_new + 128), 32);
+    *cap_out = (long long)align_up((size_t)(src_safe_outputs(max_new + 64, v->tri) + 64), 32);
+}
+
+// first tube-rate sample the converter still needs once out_total outputs exist (multiple of 4, >= 0)
+static long long pool_keep_from(long long out_total, unsigned tri, int pad)
+{
+    long long next_in = (long long)(((unsigned long long)out_total * tri) >> 16) - 2 * pad - 4;
+    if (next_in < 0) next_in = 0;
+    return next_in / 4 * 4;
+}
+
 int trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *v)
 {
     if (v->controlPeriod <= 0 || v->tri == 0) return pool_err(-4, "trm_cuda_pool: voice without rates");
-    // the sizes trm_cuda_stream_create gives one stream of this voice
-    const long long max_new = (long long)(p->max_m + 1) * v->controlPeriod + 32;
-    const long long stride = (long long)align_up((size_t)(max_new + 128), 32);
-    const long long cap_out = (long long)align_up((size_t)(src_safe_outputs(max_new + 64, v->tri) + 64), 32);
+    long long stride, cap_out;
+    pool_sizes(p, v, &stride, &cap_out);
     CK(cudaSetDevice(p->ctx->device));
     if (stride > p->stride) {
         unsigned char *t = nullptr;
@@ -1543,9 +1558,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             e.nf_call = sl.pend_frames - e.skip;
             if (e.n_new > 0) { ++n_wg; wg_frames += e.nf_call; }
             n_ret = e.out_total - sl.out_done;
-            long long next_in = e.flush ? e.target : (long long)(((unsigned long long)e.out_total * tri) >> 16) - 2 * pad - 4;
-            if (next_in < 0) next_in = 0;
-            next_in = next_in / 4 * 4;
+            long long next_in = e.flush ? e.target / 4 * 4 : pool_keep_from(e.out_total, tri, pad);
             if (next_in < sl.in_start) next_in = sl.in_start;
             e.next_in = next_in;
             if (e.target - sl.in_start > p->stride || n_ret > p->cap_out) return fail_msg("trm_cuda_pool_push: internal capacity");
@@ -1558,7 +1571,8 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     // ---- host tables of the push, laid out as in the device scratch: one upload ------------------------------------
     std::vector<int> wg;                                  // entries that run the waveguide, longest first
     std::vector<trm_cuda_utterance> rd;                   // resampler views of the entries that return samples
-    std::vector<long long> ib(1, 0), mv;                  // work-item prefix; history moves {src, dst, len}
+    std::vector<long long> ib(1, 0);                      // work-item prefix
+    std::vector<trm::CopySeg> mv;                         // history moves
     std::vector<int> rd_entry;                            // entry of each resampler view
     for (int i = 0; i < n; ++i) {
         const Entry &e = E[i];
@@ -1580,14 +1594,12 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             ib.push_back(ib.back() + (n_ret + 31) / 32);
         }
         const long long keep = e.target - e.next_in;
-        if (!e.flush && keep > 0) {
-            mv.push_back(p->tube_at(e.slot, sl.cur) + (e.next_in - sl.in_start));
-            mv.push_back(p->tube_at(e.slot, sl.cur ^ 1));
-            mv.push_back(keep);
-        }
+        if (!e.flush && keep > 0)
+            mv.push_back({p->tube_addr(p->tube_at(e.slot, sl.cur) + (e.next_in - sl.in_start)), p->tube_addr(p->tube_at(e.slot, sl.cur ^ 1)),
+                          (unsigned long long)keep * p->esz});
     }
     std::stable_sort(wg.begin(), wg.end(), [&](int a, int b) { return E[a].n_new > E[b].n_new; });
-    const size_t n_rd = rd.size(), n_mv = mv.size() / 3;
+    const size_t n_rd = rd.size(), n_mv = mv.size();
     const size_t o_dt = 0;
     const size_t o_ord = o_dt + align_up(wg.size() * sizeof(trm_cuda_utterance), 256);
     const size_t o_rst = o_ord + align_up(wg.size() * sizeof(int), 256);
@@ -1595,7 +1607,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     const size_t o_ib = o_rd + align_up(n_rd * sizeof(trm_cuda_utterance), 256);
     const size_t o_mv = o_ib + align_up(ib.size() * sizeof(long long), 256);
     const size_t n_pk = pcm ? n_rd : 0;                   // PCM: peak and max |y| of each resampler view
-    const size_t o_pk = o_mv + align_up(mv.size() * sizeof(long long), 256);
+    const size_t o_pk = o_mv + align_up(n_mv * sizeof(trm::CopySeg), 256);
     const size_t o_mx = o_pk + align_up(n_pk * sizeof(double), 256);
     const size_t o_fr = o_mx + align_up(n_pk * sizeof(unsigned long long), 256);
     const size_t bytes = o_fr + (size_t)wg_frames * 128;
@@ -1626,7 +1638,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         }
         if (n_rd) memcpy(h + o_rd, rd.data(), n_rd * sizeof(trm_cuda_utterance));
         memcpy(h + o_ib, ib.data(), ib.size() * sizeof(long long));
-        if (n_mv) memcpy(h + o_mv, mv.data(), mv.size() * sizeof(long long));
+        if (n_mv) memcpy(h + o_mv, mv.data(), n_mv * sizeof(trm::CopySeg));
         for (size_t j = 0; j < n_pk; ++j) ((double *)(h + o_pk))[j] = pcm->peak[rd_entry[j]];
         if (n_pk) memset(h + o_mx, 0, n_pk * sizeof(unsigned long long));
     }
@@ -1666,9 +1678,8 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         if ((rc = K.pcm_pool(&a, ctx->sm_count * 8, st)) != 0) return fail("pool PCM launch", (cudaError_t)rc);
     }
     if (n_mv > 0) {
-        trm::PoolMoveArgs a{};
-        a.moves = (const long long *)(d + o_mv); a.buf = p->d_tube; a.esz = (int)p->esz; a.n = (int)n_mv;
-        if ((rc = trm_k_pool_move(&a, st)) != 0) return fail("pool history move launch", (cudaError_t)rc);
+        const trm::SegCopyArgs a{(const trm::CopySeg *)(d + o_mv), (int)n_mv};
+        if ((rc = trm_k_segment_copy(&a, st)) != 0) return fail("pool history move launch", (cudaError_t)rc);
     }
     if (pcm) {
         if (pcm->out && pcm->offset[n] > 0)
@@ -1720,6 +1731,192 @@ int trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const
     std::vector<int64_t> out_offset((size_t)n + 1);
     const PoolPcm pcm{peak, pcm_host, pcm_offset, max_host};
     return pool_push(p, n, slot, n_frames, frames_host, flush, nullptr, out_offset.data(), &pcm);
+}
+
+// ---- snapshots: the part of a slot that is not its voice ------------------------------------------------------------
+int trm_cuda_pool_check_state(const trm_cuda_utterance *v, const trm_cuda_pool_slot_state *c)
+{
+    const long long cp = v->controlPeriod;
+    if (cp <= 0 || v->tri == 0) return pool_err(-4, "trm_cuda_pool: voice without rates");
+    // what pool_push keeps true between pushes; every index and length a kernel uses after a restore derives from these.
+    // 2^32 frames (200 days at 250 Hz) keep the converter's position arithmetic (samples x 65536) inside 64 bits.
+    const long long fs = c->frames_seen;
+    if (fs < 0 || fs > (1ll << 32) || c->pend_frames < 0 || c->pend_first < 0 || c->pend_first + c->pend_frames != fs)
+        return pool_err(-4, "snapshot: the frame counters do not agree");
+    const long long avail = fs >= 2 ? (fs - 1) * cp : 0;
+    if (c->s_done < 0 || c->s_done % trm::TB != 0 || c->s_done > avail || c->pend_first != c->s_done / cp)
+        return pool_err(-4, "snapshot: the waveguide position does not agree with the frames");
+    if (c->fresh != (c->s_done == 0 ? 1 : 0))   // the waveguide has run exactly when it has produced samples
+        return pool_err(-4, "snapshot: the fresh flag does not agree with the waveguide position");
+    if (c->out_done < 0 || c->out_done > src_safe_outputs(c->s_done, v->tri))
+        return pool_err(-4, "snapshot: more outputs returned than the waveguide position allows");
+    if (c->in_start < 0 || c->in_start % 4 != 0 || c->in_start > c->s_done || c->in_start > pool_keep_from(c->out_done, v->tri, v->padSize))
+        return pool_err(-4, "snapshot: the kept history does not cover what the converter reads next");
+    return 0;
+}
+
+int64_t trm_cuda_pool_slot_bytes(int precision, const trm_cuda_pool_slot_state *c)
+{
+    const size_t esz = prec_esz(precision);
+    return (int64_t)c->pend_frames * 128 + (c->fresh ? 0 : (int64_t)trm::tube_state_bytes(esz)) +
+           (int64_t)(c->s_done - c->in_start) * (int64_t)esz;
+}
+
+// bytes of a snapshot's slot part that live on the device: carried state (unless fresh), then kept history
+static size_t pool_device_bytes(const trm_cuda_pool *p, const trm_cuda_pool_slot_state &c)
+{
+    return (c.fresh ? 0 : trm::tube_state_bytes(p->esz)) + (size_t)(c.s_done - c.in_start) * p->esz;
+}
+
+int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st, void *const *dst)
+{
+    if (n < 0 || n > p->cap || (n > 0 && (!slot || !st))) return pool_err(-4, "trm_cuda_pool_save: bad arguments");
+    {
+        std::vector<unsigned char> named((size_t)p->cap, 0);
+        for (int i = 0; i < n; ++i) {
+            const int s = slot[i];
+            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_save: no such slot");
+            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_save: the slot is not open");
+            if (named[s]) return pool_err(-4, "trm_cuda_pool_save: a slot is named twice");
+            named[s] = 1;
+        }
+    }
+    for (int i = 0; i < n; ++i) {
+        const trm_cuda_pool::Slot &sl = p->slots[slot[i]];
+        st[i] = trm_cuda_pool_slot_state{sl.frames_seen, sl.s_done, sl.out_done, sl.in_start, sl.pend_first, sl.pend_frames,
+                                         sl.fresh ? 1 : 0};
+    }
+    if (!dst || n == 0) return 0;
+
+    // gather every slot's device part into packed staging ([segments][entry 0][entry 1] ...; all 16-byte multiples), one
+    // copy back
+    const size_t sb = trm::tube_state_bytes(p->esz);
+    std::vector<size_t> at((size_t)n + 1, 0);
+    for (int i = 0; i < n; ++i) at[i + 1] = at[i] + pool_device_bytes(p, st[i]);
+    const size_t o_stg = align_up((size_t)2 * n * sizeof(trm::CopySeg), 256);
+    const size_t bytes = o_stg + at[n];
+    int rc;
+    CK(cudaSetDevice(p->ctx->device));
+    if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
+    if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
+    unsigned char *h = p->stage.base, *d = p->scratch.base;
+    trm::CopySeg *seg = (trm::CopySeg *)h;
+    int n_seg = 0;
+    for (int i = 0; i < n; ++i) {
+        const int s = slot[i];
+        unsigned long long to = (unsigned long long)(uintptr_t)(d + o_stg + at[i]);
+        if (!st[i].fresh) {
+            seg[n_seg++] = {(unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), to, sb};
+            to += sb;
+        }
+        const long long hist = st[i].s_done - st[i].in_start;
+        if (hist > 0) seg[n_seg++] = {p->tube_addr(p->tube_at(s, p->slots[s].cur)), to, (unsigned long long)hist * p->esz};
+    }
+    if (n_seg > 0) {
+        cudaStream_t cs = p->st;
+        CK(cudaMemcpyAsync(d, h, (size_t)n_seg * sizeof(trm::CopySeg), cudaMemcpyHostToDevice, cs));
+        const trm::SegCopyArgs a{(const trm::CopySeg *)d, n_seg};
+        if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("snapshot gather launch", (cudaError_t)rc);
+        CK(cudaMemcpyAsync(h + o_stg, d + o_stg, at[n], cudaMemcpyDeviceToHost, cs));
+        CK(cudaStreamSynchronize(cs));
+    }
+    for (int i = 0; i < n; ++i) {
+        const trm_cuda_pool::Slot &sl = p->slots[slot[i]];
+        unsigned char *o = (unsigned char *)dst[i];
+        if (sl.pend_frames) memcpy(o, sl.pending.data(), (size_t)sl.pend_frames * 128);
+        memcpy(o + (size_t)sl.pend_frames * 128, h + o_stg + at[i], at[i + 1] - at[i]);
+    }
+    return 0;
+}
+
+int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voice, const double *wavetables,
+                          const trm_cuda_pool_slot_state *st, const void *const *src, int32_t *slot_out)
+{
+    if (n < 0 || (n > 0 && (!voice || !wavetables || !st || !src || !slot_out)))
+        return pool_err(-4, "trm_cuda_pool_restore: bad arguments");
+    if (n == 0) return 0;
+    // ---- everything is checked before the pool changes ----------------------------------------------------------------
+    long long stride = p->stride, cap_out = p->cap_out;     // the sizes after this call's reservations
+    for (int i = 0; i < n; ++i) {
+        int rc = trm_cuda_pool_check_state(&voice[i], &st[i]);
+        if (rc != 0) return rc;
+        long long s, c;
+        pool_sizes(p, &voice[i], &s, &c);
+        stride = std::max(stride, s);
+        cap_out = std::max(cap_out, c);
+    }
+    for (int i = 0; i < n; ++i) {
+        // pool_push appends the pending frames before its capacity check: the next push of the restored slot, with as many
+        // frames as this pool takes and a flush, must stay inside one history row and one slot's outputs
+        const trm_cuda_utterance &v = voice[i];
+        const long long fs = st[i].frames_seen + p->max_m;
+        const long long avail = fs >= 2 ? (fs - 1) * v.controlPeriod : 0;
+        const long long out_flush = (long long)(((unsigned long long)(avail + 2 * v.padSize) * 65536ull + v.tri - 1) / v.tri);
+        const long long out = std::max(out_flush, src_safe_outputs(avail / trm::TB * trm::TB, v.tri));
+        if (avail - st[i].in_start > stride || out - st[i].out_done > cap_out)
+            return pool_err(-4, "trm_cuda_pool_restore: a snapshot's history and pending frames do not fit this pool's next push");
+    }
+    std::vector<int> free_slot;
+    for (int s = 0; s < p->cap && (int)free_slot.size() < n; ++s)
+        if (!p->slots[s].open) free_slot.push_back(s);
+    if ((int)free_slot.size() < n) return pool_err(-7, "trm_cuda_pool_restore: fewer free slots than snapshots");
+
+    int rc;
+    for (int i = 0; i < n; ++i)
+        if ((rc = trm_cuda_pool_reserve(p, &voice[i])) != 0) return rc;
+    // ---- one upload ([segments][wavetables][entry 0's state and history] ...), one scatter -----------------------------
+    const size_t sb = trm::tube_state_bytes(p->esz), wt = TRM_TABLE_LENGTH * sizeof(double);
+    std::vector<size_t> at((size_t)n + 1, 0);
+    for (int i = 0; i < n; ++i) at[i + 1] = at[i] + pool_device_bytes(p, st[i]);
+    const size_t o_wt = align_up((size_t)3 * n * sizeof(trm::CopySeg), 256);
+    const size_t o_dev = o_wt + (size_t)n * wt;
+    const size_t bytes = o_dev + at[n];
+    CK(cudaSetDevice(p->ctx->device));
+    if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
+    if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
+    unsigned char *h = p->stage.base, *d = p->scratch.base;
+    trm::CopySeg *seg = (trm::CopySeg *)h;
+    int n_seg = 0;
+    memcpy(h + o_wt, wavetables, (size_t)n * wt);
+    for (int i = 0; i < n; ++i) {
+        const int s = free_slot[i];
+        seg[n_seg++] = {(unsigned long long)(uintptr_t)(d + o_wt + (size_t)i * wt),
+                        (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH), wt};
+        memcpy(h + o_dev + at[i], (const unsigned char *)src[i] + (size_t)st[i].pend_frames * 128, at[i + 1] - at[i]);
+        unsigned long long from = (unsigned long long)(uintptr_t)(d + o_dev + at[i]);
+        if (!st[i].fresh) {
+            seg[n_seg++] = {from, (unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), sb};
+            from += sb;
+        }
+        const long long hist = st[i].s_done - st[i].in_start;
+        if (hist > 0) seg[n_seg++] = {from, p->tube_addr(p->tube_at(s, 0)), (unsigned long long)hist * p->esz};
+    }
+    cudaStream_t cs = p->st;
+    CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
+    const trm::SegCopyArgs a{(const trm::CopySeg *)d, n_seg};
+    if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("snapshot scatter launch", (cudaError_t)rc);
+    CK(cudaStreamSynchronize(cs));
+    // ---- the slots open only now that the device work has finished without error -------------------------------------
+    for (int i = 0; i < n; ++i) {
+        const int s = free_slot[i];
+        trm_cuda_pool::Slot &sl = p->slots[s];
+        sl = trm_cuda_pool::Slot();
+        sl.open = true;
+        sl.fresh = st[i].fresh != 0;
+        sl.voice = voice[i];
+        sl.voice.voice = s;
+        sl.cur = 0;
+        sl.frames_seen = st[i].frames_seen;
+        sl.s_done = st[i].s_done;
+        sl.out_done = st[i].out_done;
+        sl.in_start = st[i].in_start;
+        sl.pend_first = st[i].pend_first;
+        sl.pend_frames = st[i].pend_frames;
+        sl.pending.resize((size_t)st[i].pend_frames * 16);
+        if (st[i].pend_frames) memcpy(sl.pending.data(), src[i], (size_t)st[i].pend_frames * 128);
+        slot_out[i] = s;
+    }
+    return 0;
 }
 
 int trm_cuda_resident_create(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,

@@ -1148,6 +1148,8 @@ void TRMStreamFree(TRMStream *t)
 /* ---- stream pool: independent streaming slots, each with its own voice ---- */
 struct TRMStreamPool {
     trm_cuda_pool *p;
+    int capacity, precision;
+    TRMInputParameters *voice;      /* [capacity]: the voice each open slot was opened or restored with (snapshots) */
 };
 
 /* shim codes: -4 / -7 are argument / call-order refusals (message set by the shim), anything else is CUDA */
@@ -1166,10 +1168,13 @@ TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_p
         return NULL;
     }
     TRMStreamPool *t = calloc(1, sizeof *t);
-    if (!t) { *err = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); return NULL; }
+    if (t) t->voice = calloc((size_t)capacity, sizeof *t->voice);
+    if (!t || !t->voice) { free(t); *err = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); return NULL; }
+    t->capacity = capacity;
+    t->precision = precision;
     trm_cuda_ctx *ctx;
     int lane;
-    if ((*err = acquire_ctx(device, &ctx, &lane)) != TRM_OK) { free(t); return NULL; }
+    if ((*err = acquire_ctx(device, &ctx, &lane)) != TRM_OK) { free(t->voice); free(t); return NULL; }
     int rc = trm_cuda_pool_create(ctx, precision, capacity, max_frames_per_push, &t->p);
     release_ctx(device, lane);      /* the pool owns its buffers, wavetables, stream and scratch: no lane is held */
     if (rc == 0) {
@@ -1185,6 +1190,7 @@ TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_p
     if (rc != 0) {
         *err = pool_rc(rc);
         trm_cuda_pool_destroy(t->p);
+        free(t->voice);
         free(t);
         return NULL;
     }
@@ -1203,14 +1209,25 @@ int TRMStreamPoolOpen(TRMStreamPool *t, const TRMInputParameters *voice)
     int slot = -1;
     rc = trm_cuda_pool_open(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, &slot);
     voice_set_free(&vs);
-    return rc != 0 ? pool_rc(rc) : slot;
+    if (rc != 0) return pool_rc(rc);
+    t->voice[slot] = *voice;
+    return slot;
 }
 
 int TRMStreamPoolClose(TRMStreamPool *t, int slot)
 {
     if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
     const int rc = trm_cuda_pool_close(t->p, slot);
-    return rc != 0 ? pool_rc(rc) : TRM_OK;
+    if (rc != 0) return pool_rc(rc);
+    memset(&t->voice[slot], 0, sizeof t->voice[slot]);
+    return TRM_OK;
+}
+
+/* a push succeeded: the slots it flushed are free again */
+static void pool_forget_flushed(TRMStreamPool *t, int n, const int32_t *slot, const uint8_t *flush)
+{
+    for (int i = 0; flush && i < n; i++)
+        if (flush[i]) memset(&t->voice[slot[i]], 0, sizeof t->voice[slot[i]]);
 }
 
 int64_t TRMStreamPoolSlotCapacity(const TRMStreamPool *t) { return t ? trm_cuda_pool_slot_capacity(t->p) : 0; }
@@ -1220,7 +1237,9 @@ int TRMStreamPoolPush(TRMStreamPool *t, int n, const int32_t *slot, const int32_
 {
     if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
     const int rc = trm_cuda_pool_push(t->p, n, slot, n_frames, (const double *)frames, flush, samples_out, out_offset);
-    return rc != 0 ? pool_rc(rc) : TRM_OK;
+    if (rc != 0) return pool_rc(rc);
+    pool_forget_flushed(t, n, slot, flush);
+    return TRM_OK;
 }
 
 int TRMStreamPoolPushPCM16(TRMStreamPool *t, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
@@ -1229,14 +1248,216 @@ int TRMStreamPoolPushPCM16(TRMStreamPool *t, int n, const int32_t *slot, const i
     if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
     const int rc = trm_cuda_pool_push_pcm16(t->p, n, slot, n_frames, (const double *)frames, flush, peak, pcm_out, pcm_offset,
                                             max_out);
-    return rc != 0 ? pool_rc(rc) : TRM_OK;
+    if (rc != 0) return pool_rc(rc);
+    pool_forget_flushed(t, n, slot, flush);
+    return TRM_OK;
 }
 
 void TRMStreamPoolFree(TRMStreamPool *t)
 {
     if (!t) return;
     trm_cuda_pool_destroy(t->p);
+    free(t->voice);
     free(t);
+}
+
+/* ---- stream pool snapshots (include/trm.h): header, voice and derived constants here, the slot part in the shim ---- */
+#if defined(__BYTE_ORDER__) && __BYTE_ORDER__ != __ORDER_LITTLE_ENDIAN__
+#error "snapshot data parts are copied as they lie in memory: little-endian hosts only"
+#endif
+#define SNAP_VERSION   1u
+#define SNAP_HEADER    32                 /* magic, version, precision, total bytes, checksum */
+#define SNAP_VOICE     192
+#define SNAP_DERIVED   24
+#define SNAP_COUNTERS  48
+#define SNAP_FIXED     (SNAP_HEADER + SNAP_VOICE + SNAP_DERIVED + SNAP_COUNTERS)
+static const unsigned char snap_magic[8] = {'T', 'R', 'M', 'S', 'N', 'A', 'P', 0};
+
+static uint64_t fnv1a64(const unsigned char *p, size_t n)
+{
+    uint64_t h = 0xcbf29ce484222325ull;
+    for (size_t i = 0; i < n; i++) h = (h ^ p[i]) * 0x100000001b3ull;
+    return h;
+}
+
+/* little-endian writers / readers, one field at a time */
+static unsigned char *put_u32(unsigned char *o, uint32_t v) { for (int i = 0; i < 4; i++) o[i] = (unsigned char)(v >> (8 * i)); return o + 4; }
+static unsigned char *put_u64(unsigned char *o, uint64_t v) { for (int i = 0; i < 8; i++) o[i] = (unsigned char)(v >> (8 * i)); return o + 8; }
+static unsigned char *put_f32(unsigned char *o, float v) { uint32_t b; memcpy(&b, &v, 4); return put_u32(o, b); }
+static unsigned char *put_f64(unsigned char *o, double v) { uint64_t b; memcpy(&b, &v, 8); return put_u64(o, b); }
+static uint32_t get_u32(const unsigned char **q) { uint32_t v = 0; for (int i = 0; i < 4; i++) v |= (uint32_t)(*q)[i] << (8 * i); *q += 4; return v; }
+static uint64_t get_u64(const unsigned char **q) { uint64_t v = 0; for (int i = 0; i < 8; i++) v |= (uint64_t)(*q)[i] << (8 * i); *q += 8; return v; }
+static float get_f32(const unsigned char **q) { uint32_t b = get_u32(q); float v; memcpy(&v, &b, 4); return v; }
+static double get_f64(const unsigned char **q) { uint64_t b = get_u64(q); double v; memcpy(&v, &b, 8); return v; }
+
+static unsigned char *put_voice(unsigned char *o, const TRMInputParameters *ip)
+{
+    o = put_u32(o, (uint32_t)ip->outputFileFormat); o = put_f32(o, ip->outputRate); o = put_f32(o, ip->controlRate);
+    o = put_f64(o, ip->volume); o = put_u32(o, (uint32_t)ip->channels); o = put_f64(o, ip->balance);
+    o = put_u32(o, (uint32_t)ip->waveform);
+    o = put_f64(o, ip->tp); o = put_f64(o, ip->tnMin); o = put_f64(o, ip->tnMax); o = put_f64(o, ip->breathiness);
+    o = put_f64(o, ip->length); o = put_f64(o, ip->temperature); o = put_f64(o, ip->lossFactor); o = put_f64(o, ip->apScale);
+    o = put_f64(o, ip->mouthCoef); o = put_f64(o, ip->noseCoef);
+    for (int i = 0; i < TRM_TOTAL_NASAL_SECTIONS; i++) o = put_f64(o, ip->noseRadius[i]);
+    o = put_f64(o, ip->throatCutoff); o = put_f64(o, ip->throatVol); o = put_u32(o, (uint32_t)ip->usesModulation);
+    return put_f64(o, ip->mixOffset);
+}
+
+static void get_voice(const unsigned char **q, TRMInputParameters *ip)
+{
+    memset(ip, 0, sizeof *ip);
+    ip->outputFileFormat = (int32_t)get_u32(q); ip->outputRate = get_f32(q); ip->controlRate = get_f32(q);
+    ip->volume = get_f64(q); ip->channels = (int32_t)get_u32(q); ip->balance = get_f64(q);
+    ip->waveform = (int32_t)get_u32(q);
+    ip->tp = get_f64(q); ip->tnMin = get_f64(q); ip->tnMax = get_f64(q); ip->breathiness = get_f64(q);
+    ip->length = get_f64(q); ip->temperature = get_f64(q); ip->lossFactor = get_f64(q); ip->apScale = get_f64(q);
+    ip->mouthCoef = get_f64(q); ip->noseCoef = get_f64(q);
+    for (int i = 0; i < TRM_TOTAL_NASAL_SECTIONS; i++) ip->noseRadius[i] = get_f64(q);
+    ip->throatCutoff = get_f64(q); ip->throatVol = get_f64(q); ip->usesModulation = (int32_t)get_u32(q);
+    ip->mixOffset = get_f64(q);
+}
+
+/* the derived constants a snapshot stores, from the voice's descriptor */
+static void snap_derived(const trm_cuda_utterance *d, int precision, uint32_t out[6])
+{
+    out[0] = (uint32_t)d->controlPeriod; out[1] = (uint32_t)d->sampleRate; out[2] = d->tri;
+    out[3] = (uint32_t)d->padSize; out[4] = (uint32_t)d->channels; out[5] = precision == TRM_PRECISION_FP32 ? 4u : 8u;
+}
+
+/* One snapshot, checked as far as it can be without a pool: on success *ip, *d (descriptor, n_frames = 2 as Open builds
+ * it), the glottal table row in vs (row d->voice), the counters and a pointer to the data part. */
+static int snap_parse(const unsigned char *b, int64_t bytes, voice_set *vs, int *precision, TRMInputParameters *ip,
+                      trm_cuda_utterance *d, trm_cuda_pool_slot_state *st, const unsigned char **data)
+{
+    if (!b || bytes < SNAP_HEADER) return set_err(TRM_ERR_PARAM, "snapshot: shorter than its header%s", "");
+    const unsigned char *q = b + 8;
+    if (memcmp(b, snap_magic, 8) != 0) return set_err(TRM_ERR_PARAM, "snapshot: not a stream pool snapshot%s", "");
+    if (get_u32(&q) != SNAP_VERSION) return set_err(TRM_ERR_PARAM, "snapshot: unknown format version%s", "");
+    const uint32_t prec = get_u32(&q);
+    const uint64_t total = get_u64(&q), sum = get_u64(&q);
+    if (total != (uint64_t)bytes || bytes < SNAP_FIXED) return set_err(TRM_ERR_PARAM, "snapshot: length does not match%s", "");
+    if (fnv1a64(b + SNAP_HEADER, (size_t)bytes - SNAP_HEADER) != sum) return set_err(TRM_ERR_PARAM, "snapshot: checksum mismatch%s", "");
+    if (prec > 2u || !precision_ok((int)prec)) return set_err(TRM_ERR_PARAM, "snapshot: unknown precision%s", "");
+    *precision = (int)prec;
+    get_voice(&q, ip);
+    int rc = describe(ip, 2, vs, d, NULL);
+    if (rc != TRM_OK) return rc;
+    uint32_t want[6];
+    snap_derived(d, *precision, want);
+    for (int i = 0; i < 6; i++)
+        if (get_u32(&q) != want[i])
+            return set_err(TRM_ERR_PARAM, "snapshot: derived constants differ from the voice's (another library build?)%s", "");
+    st->frames_seen = (int64_t)get_u64(&q); st->s_done = (int64_t)get_u64(&q); st->out_done = (int64_t)get_u64(&q);
+    st->in_start = (int64_t)get_u64(&q); st->pend_first = (int64_t)get_u64(&q);
+    st->pend_frames = (int32_t)get_u32(&q); st->fresh = (int32_t)get_u32(&q);
+    if (trm_cuda_pool_check_state(d, st) != 0) return set_err(TRM_ERR_PARAM, "%s", trm_cuda_last_error());
+    if (bytes != SNAP_FIXED + trm_cuda_pool_slot_bytes(*precision, st))
+        return set_err(TRM_ERR_PARAM, "snapshot: length does not match its counters%s", "");
+    *data = q;
+    return TRM_OK;
+}
+
+int TRMStreamPoolSave(TRMStreamPool *t, int n, const int32_t *slot, void *blob, int64_t blob_capacity, int64_t *offset)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    if (n < 0 || !offset || (n > 0 && !slot)) return set_err(TRM_ERR_PARAM, "bad snapshot arguments%s", "");
+    trm_cuda_pool_slot_state *st = calloc((size_t)n + 1, sizeof *st);
+    void **dst = calloc((size_t)n + 1, sizeof *dst);
+    voice_set vs;
+    memset(&vs, 0, sizeof vs);
+    int rc = TRM_OK;
+    if (!st || !dst) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
+    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, NULL)) != 0) { rc = pool_rc(rc); goto done; }   /* checks the slots */
+    offset[0] = 0;
+    for (int i = 0; i < n; i++) offset[i + 1] = offset[i] + SNAP_FIXED + trm_cuda_pool_slot_bytes(t->precision, &st[i]);
+    if (!blob) goto done;
+    if (blob_capacity < offset[n]) { rc = set_err(TRM_ERR_PARAM, "snapshot buffer too small%s", ""); goto done; }
+    unsigned char *base = blob;
+    for (int i = 0; i < n; i++) dst[i] = base + offset[i] + SNAP_FIXED;
+    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, dst)) != 0) { rc = pool_rc(rc); goto done; }
+    for (int i = 0; i < n; i++) {
+        const TRMInputParameters *ip = &t->voice[slot[i]];
+        trm_cuda_utterance d;
+        if ((rc = describe(ip, 2, &vs, &d, NULL)) != TRM_OK) goto done;
+        uint32_t dv[6];
+        snap_derived(&d, t->precision, dv);
+        unsigned char *b = base + offset[i], *o = b;
+        memcpy(o, snap_magic, 8);
+        o = put_u32(o + 8, SNAP_VERSION);
+        o = put_u32(o, (uint32_t)t->precision);
+        o = put_u64(o, (uint64_t)(offset[i + 1] - offset[i]));
+        unsigned char *sum_at = o;
+        o = put_voice(o + 8, ip);
+        for (int k = 0; k < 6; k++) o = put_u32(o, dv[k]);
+        o = put_u64(o, (uint64_t)st[i].frames_seen); o = put_u64(o, (uint64_t)st[i].s_done);
+        o = put_u64(o, (uint64_t)st[i].out_done); o = put_u64(o, (uint64_t)st[i].in_start);
+        o = put_u64(o, (uint64_t)st[i].pend_first);
+        o = put_u32(o, (uint32_t)st[i].pend_frames); o = put_u32(o, (uint32_t)st[i].fresh);
+        put_u64(sum_at, fnv1a64(b + SNAP_HEADER, (size_t)(offset[i + 1] - offset[i]) - SNAP_HEADER));
+    }
+done:
+    voice_set_free(&vs);
+    free(st);
+    free(dst);
+    return rc;
+}
+
+int TRMStreamPoolRestore(TRMStreamPool *t, int n, const void *blob, const int64_t *offset, int32_t *slot_out)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    if (n < 0 || (n > 0 && (!blob || !offset || !slot_out))) return set_err(TRM_ERR_PARAM, "bad snapshot arguments%s", "");
+    if (n == 0) return TRM_OK;
+    trm_cuda_pool_slot_state *st = calloc((size_t)n, sizeof *st);
+    trm_cuda_utterance *d = calloc((size_t)n, sizeof *d);
+    TRMInputParameters *ip = calloc((size_t)n, sizeof *ip);
+    double *tables = malloc((size_t)n * TRM_TABLE_LENGTH * sizeof *tables);
+    const void **src = calloc((size_t)n, sizeof *src);
+    voice_set vs;
+    memset(&vs, 0, sizeof vs);
+    int rc = TRM_OK;
+    if (!st || !d || !ip || !tables || !src) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
+    for (int i = 0; i < n; i++) {
+        if (offset[i] < 0 || offset[i + 1] < offset[i]) { rc = set_err(TRM_ERR_PARAM, "snapshot offsets are not ascending%s", ""); goto done; }
+        int prec;
+        const unsigned char *data;
+        if ((rc = snap_parse((const unsigned char *)blob + offset[i], offset[i + 1] - offset[i], &vs, &prec, &ip[i], &d[i], &st[i],
+                             &data)) != TRM_OK)
+            goto done;
+        if (prec != t->precision) { rc = set_err(TRM_ERR_PARAM, "snapshot of another precision%s", ""); goto done; }
+        src[i] = data;
+    }
+    /* the table rows are final only now (vs may have grown while parsing) */
+    for (int i = 0; i < n; i++)
+        memcpy(tables + (size_t)i * TRM_TABLE_LENGTH, vs.tables + (size_t)d[i].voice * TRM_TABLE_LENGTH, TRM_TABLE_LENGTH * sizeof *tables);
+    if ((rc = trm_cuda_pool_restore(t->p, n, d, tables, st, (const void *const *)src, slot_out)) != 0) { rc = pool_rc(rc); goto done; }
+    for (int i = 0; i < n; i++) t->voice[slot_out[i]] = ip[i];
+done:
+    voice_set_free(&vs);
+    free(st); free(d); free(ip); free(tables); free(src);
+    return rc;
+}
+
+int TRMStreamPoolSnapshotInfo(const void *blob, int64_t bytes, TRMStreamSnapshotInfo *info)
+{
+    if (!blob || !info) return set_err(TRM_ERR_PARAM, "null snapshot or info%s", "");
+    voice_set vs;
+    memset(&vs, 0, sizeof vs);
+    int prec;
+    TRMInputParameters ip;
+    trm_cuda_utterance d;
+    trm_cuda_pool_slot_state st;
+    const unsigned char *data;
+    const int rc = snap_parse(blob, bytes, &vs, &prec, &ip, &d, &st, &data);
+    voice_set_free(&vs);
+    if (rc != TRM_OK) return rc;
+    memset(info, 0, sizeof *info);
+    info->precision = prec;
+    info->channels = d.channels;
+    info->voice = ip;
+    info->frames_pushed = st.frames_seen;
+    info->samples_returned = st.out_done;
+    info->bytes = bytes;
+    return TRM_OK;
 }
 
 /* ---- asynchronous calls: one host thread per ticket; two tickets per device overlap (context lanes) ---- */

@@ -358,6 +358,53 @@ int TRMStreamPoolPushPCM16(TRMStreamPool *pool, int n, const int32_t *slot, cons
                            int16_t *pcm_out, int64_t *pcm_offset /* [n + 1] */, double *max_out);
 void TRMStreamPoolFree(TRMStreamPool *pool);
 
+/* Snapshots: a live slot as a self-contained byte string that continues in any pool of the same precision, on any device,
+ * in any process.  Moving streams off a GPU (save, close, restore elsewhere), growing a pool, surviving a restart and
+ * branching a stream (restore while the saved slot keeps going) all use these three calls.
+ *
+ * Continuation.  A slot restored from a snapshot behaves as the saved slot would have from that point, whatever either
+ * pool does: its later Push / PushPCM16 outputs, appended to what the saved slot had returned before the save, equal the
+ * one-shot TRMBatch synthesis bit for bit (samples, PCM at a given peak, per-push maxima).  Saving does not change the
+ * saved slot; closing it after the save is a migration, letting it continue is a fork.  The PCM peak is not part of the
+ * state: it is passed with every push, as before.
+ * What it depends on.  A snapshot holds no device pointers, slot numbers, device ordinals or pool sizes, and
+ * save(restore(b)) == b byte for byte.  It restores into a pool with another capacity, max_frames_per_push, slot index or
+ * device, but only into the same precision code (FP64 conformance and FP64 strict carry different states).
+ * Format (little-endian, written field by field; libtrm owns it):
+ *   header    8 bytes "TRMSNAP\0", u32 version (1), u32 precision, u64 total bytes, u64 FNV-1a 64 of every byte after it
+ *   voice     TRMInputParameters field by field, no padding (192 bytes)
+ *   derived   u32 controlPeriod, sampleRate, timeRegisterIncrement, padSize, channels, element size (4 or 8)
+ *   counters  i64 frames pushed, tube-rate samples synthesized, output samples returned, first tube-rate sample kept,
+ *             first pending frame; i32 pending frames, fresh (1 while the waveguide has not run)
+ *   data      pending frames [n][16] f64; the carried waveguide state (32 + 96 x element size bytes) unless fresh; the
+ *             kept tube-rate history [synthesized - first kept] of the precision's element type
+ * Restore derives the glottal table and every derived constant again from the voice, as TRMStreamPoolOpen does, and checks
+ * the counters against each other and the voice: a corrupt snapshot can give wrong audio but never an access outside
+ * the slot's own buffers. */
+typedef struct TRMStreamSnapshotInfo {
+    int32_t precision;               /* TRM_PRECISION_* the snapshot restores into                                 */
+    int32_t channels;                /* int16 elements per PCM frame of the stream                                  */
+    TRMInputParameters voice;
+    int64_t frames_pushed;           /* control frames the stream has received                                      */
+    int64_t samples_returned;        /* output-rate samples (PCM frames) it has returned                            */
+    int64_t bytes;                   /* size of the snapshot                                                        */
+} TRMStreamSnapshotInfo;
+/* Snapshots of n distinct open slots, packed: slot[i]'s bytes are blob[offset[i] .. offset[i+1]).  blob == NULL: only
+ * fills offset (sizes from host bookkeeping, no device work).  Refused before anything is written: an unopened slot
+ * (TRM_ERR_STATE), a slot named twice or blob_capacity < offset[n] (TRM_ERR_PARAM). */
+int TRMStreamPoolSave(TRMStreamPool *pool, int n, const int32_t *slot, void *blob, int64_t blob_capacity,
+                      int64_t *offset /* [n + 1] */);
+/* Opens n free slots from n snapshots (the same packing); slot_out[i] is the slot that continues snapshot i.  All n are
+ * checked before anything changes, and a refused call leaves the pool as it was: bad magic, version, length or checksum,
+ * another precision, derived constants that differ from the voice's (e.g. a snapshot from another library build), or
+ * counters that disagree (TRM_ERR_PARAM); a voice TRMBatchCreate refuses (its code); kept history and pending frames
+ * that would not fit this pool's next push of max_frames_per_push frames (TRM_ERR_PARAM); fewer than n free slots
+ * (TRM_ERR_STATE).  SlotCapacity may grow, as with Open. */
+int TRMStreamPoolRestore(TRMStreamPool *pool, int n, const void *blob, const int64_t *offset /* [n + 1] */, int32_t *slot_out);
+/* Host only (no device needed): validates one snapshot as Restore does, apart from the destination pool, and reports
+ * what it holds.  Lets a router pick a pool before restoring. */
+int TRMStreamPoolSnapshotInfo(const void *blob, int64_t bytes, TRMStreamSnapshotInfo *info);
+
 /* ---------------------------------------------------------------------------------------------
  * Sweeps (BASELINE configs[4]: 10^6 synthetic 2 s utterances): n utterances of one voice whose control tracks are the walk2
  * workload of include/trm_workload.h, generated on the device (utterance k = index first_index + k of stream `seed`) --

@@ -209,6 +209,28 @@ int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int3
  * samples entry i produced (0.0 if none).  pcm_kernel's arithmetic (TRMTubeModel.m:515-559) and include/trm.h's contract. */
 int  trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
                               const uint8_t *flush, const double *peak, int16_t *pcm_host, int64_t *pcm_offset, double *max_host);
+/* Snapshots (include/trm.h TRMStreamPoolSave): what a slot carries from one push to the next apart from its voice.  The
+ * counters are the slot's stream positions: frames received, tube-rate samples synthesized (a multiple of 16), output
+ * samples returned, first tube-rate sample still kept, first pending frame; pending frames [pend_first, frames_seen) and
+ * fresh = 1 while the waveguide has not run (no carried state exists yet). */
+typedef struct trm_cuda_pool_slot_state {
+    int64_t frames_seen, s_done, out_done, in_start, pend_first;
+    int32_t pend_frames, fresh;
+} trm_cuda_pool_slot_state;
+/* Host only: 0 if a slot with this voice can hold these counters, -4 if not.  A slot restored with counters that pass
+ * reads and writes only inside its own history row, state and pending frames. */
+int  trm_cuda_pool_check_state(const trm_cuda_utterance *voice, const trm_cuda_pool_slot_state *st);
+/* Bytes of a slot's data part: pend_frames x 16 doubles, the carried state unless fresh (trm::tube_state_bytes), then the
+ * kept history s_done - in_start elements of the precision's type. */
+int64_t trm_cuda_pool_slot_bytes(int precision, const trm_cuda_pool_slot_state *st);
+/* st[i] receives the counters of n distinct open slots; with dst (may be NULL: counters only, no device work), dst[i]
+ * receives slot[i]'s data part (trm_cuda_pool_slot_bytes).  The slots are not changed.  -7: a slot is not open. */
+int  trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st, void *const *dst);
+/* Opens n free slots continuing n saved ones: voice[i] (voice.voice ignored) with its glottal table wavetables[i][512],
+ * counters st[i] and data part src[i].  Refused before any change: counters that fail trm_cuda_pool_check_state or whose
+ * next full push would not fit this pool's rows (-4), fewer than n free slots (-7).  slot_out[i] is entry i's slot. */
+int  trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voice, const double *wavetables,
+                           const trm_cuda_pool_slot_state *st, const void *const *src, int32_t *slot_out);
 void trm_cuda_pool_destroy(trm_cuda_pool *p);
 /*
  * Control frames on the device (replaces -[EventList generateOutputInTimeRange:...], EventList.m:883-1061): uploads
