@@ -70,7 +70,7 @@ template <> struct Wide<float> {
 template <> struct Wide<double> {
     using Unit = double2;
     static constexpr int MAX_PAIRS = 14;
-    static constexpr int NF = 12;
+    static constexpr int NF = STRICT ? 12 : 10;      // conformance: the frication taps travel as two values and a mask
     static constexpr int UP = 2 * MAX_PAIRS + 1;
     static constexpr int OUT_LD = 18;
     // Register redistribution (conformance mode): the CTA is launched with one extra warpgroup, which caps every thread
@@ -93,6 +93,17 @@ constexpr int WIDE_SLOTS = 2;
 // {recurrence + 3, 4, 4, 3}.
 constexpr int WIDE_IDLE_WARP = 12;
 
+// Oscillator history (even / odd 2x-rate samples) that the 49-tap FIR of a block reads: FIR_HIST old values, then the
+// block's TB new ones.  FP64 conformance mode keeps a circular buffer of FIR_RING values whose first FIR_HIST entries are
+// repeated past its end: the window of block b starts at TB * (b % 3) and is always contiguous, and a block only writes
+// its new values (a value that lands in the repeated part is written twice).  Nothing moves, which saves a slide's
+// shared-memory traffic and a warp barrier per block.  The other modes keep the window at the start of the buffer and
+// slide it down by one block after every block (strict mode's 12-unit ring leaves no room for the larger buffer, and
+// in FP32 fast mode the circular form costs the stream-pool kernel spills).
+template <typename R> constexpr bool HIST_RING = sizeof(R) == 8 && !STRICT;
+constexpr int FIR_RING = 3 * TB;                     // a multiple of TB, >= FIR_HIST + TB
+template <typename R> constexpr int HIST_LEN = HIST_RING<R> ? FIR_RING + FIR_HIST : FIR_HIST + TB;
+
 // feed-forward state of one utterance that must be in shared memory
 template <typename R>
 struct alignas(16) FFHalf {
@@ -101,7 +112,7 @@ struct alignas(16) FFHalf {
     double CST[12];                          // per-utterance constants of the feed-forward phases (global loads of the
                                              // descriptor inside the block loop sat on the warp's critical path)
     double INC[TB];                          // oscillator increments of the block (conformance mode: every lane walks them)
-    R HE[FIR_HIST + TB], HO[FIR_HIST + TB];  // oscillator history, even / odd 2x-rate samples
+    R HE[HIST_LEN<R>], HO[HIST_LEN<R>];      // oscillator history, even / odd 2x-rate samples
     R pad[16 / sizeof(R)];                   // FP32: size = 64 mod 128 bytes, so the two utterances of a warp (adjacent
                                              // FFHalf's, 16 consecutive floats each) read disjoint bank halves
 };
@@ -118,6 +129,7 @@ struct WideSmem {
     R *out_ptr[32];
     long long n_cta;
 };
+static_assert(sizeof(WideSmem<double>) <= 227 * 1024 && sizeof(WideSmem<float>) <= 227 * 1024, "one CTA per SM: 227 kB");
 
 // Waiting on a ring barrier.  try_wait returns after a short hardware-defined time whether or not the phase completed,
 // so a bare loop around it spins: measured (ncu, round 2), the 14 feed-forward warps of a CTA waiting for the recurrence
@@ -522,7 +534,11 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
             //     e = a - b;  x = kd e;  right-going = fma(a, d, x) (+ tap fr);  left-going = fma(b, d, x)
             // which is (a + k e) d and (b + k e) d of TRMTubeModel.m:796-829 with one rounding placed differently.
             // Record of one sample (feed-forward warps, below):
-            //   {kd0,kd1} {kd2,aL d} {kd4,kd6} {kd7,kd8} {k9,kd10} {aU d,FC1} {FC2,FC3} {FC4,FC5} {FC6,FC7} {FC8,2g} {2b,in} {ff,thr}
+            //   {kd0,kd1} {kd2,aL d} {kd4,kd6} {kd7,kd8} {k9,kd10} {aU d,2g} {2b,tsel} {tE,tO} {in,ff} {thr,-}
+            // Frication tap k (FC(k+1), injected into junction k) is tE / tO for an even / odd k if bit k of tsel is set,
+            // else +0 -- the same value the reference's eight-tap array holds (at most two taps are non-zero), so every
+            // junction still adds tap * fr with the same fused multiply-add and the same bits: selects replace the loads of
+            // six zeros.
             // Per-utterance constants live in registers (the warp has 168 of them): the shared-memory pipe is this kernel's
             // bottleneck (ncu: 74 % of its wavefront rate), and 17 constant loads per sample were 11 % of the traffic.
             const double c_tb1 = D->tb1, c_gain = D->throatGain;
@@ -559,32 +575,33 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                         const int s = s0 + si;
                         // Written stage by stage ACROSS the junctions: the operations of one stage are mutually independent,
                         // so the FP64 pipe (one warp instruction per ~2.25 cycles, 8-cycle latency) always has a ready one.
-                        const double2 q9 = W.ring[slot][9][s][lane], q10 = W.ring[slot][10][s][lane], q11 = W.ring[slot][11][s][lane];
-                        const double2 q0 = W.ring[slot][0][s][lane], q1 = W.ring[slot][1][s][lane], q2 = W.ring[slot][2][s][lane];
-                        const double2 q3 = W.ring[slot][3][s][lane], q4 = W.ring[slot][4][s][lane], q5 = W.ring[slot][5][s][lane];
-                        const double2 q6 = W.ring[slot][6][s][lane], q7 = W.ring[slot][7][s][lane], q8 = W.ring[slot][8][s][lane];
+                        const double2 q5 = W.ring[slot][5][s][lane], q6 = W.ring[slot][6][s][lane], q8 = W.ring[slot][8][s][lane];
+                        const double2 q9 = W.ring[slot][9][s][lane], q0 = W.ring[slot][0][s][lane], q1 = W.ring[slot][1][s][lane];
+                        const double2 q2 = W.ring[slot][2][s][lane], q3 = W.ring[slot][3][s][lane], q4 = W.ring[slot][4][s][lane];
+                        const double2 q7 = W.ring[slot][7][s][lane];
+                        const unsigned tsel = (unsigned)__double_as_longlong(q6.y);
+                        auto tap = [&](int k) { return (tsel & (1u << k)) ? ((k & 1) ? q7.y : q7.x) : 0.0; };
                         // ---- stage 1: differences, first products ----
-                        const double fr1 = fma(q9.y, y1, q11.x);                      // band-pass (TRMFilters.m:19-29, factor 2 folded in)
-                        const double th = fma(c_tb1, thy, q11.y);                     // throat low-pass (TRMFilters.m:72-77)
+                        const double fr1 = fma(q5.y, y1, q8.y);                       // band-pass (TRMFilters.m:19-29, factor 2 folded in)
+                        const double th = fma(c_tb1, thy, q9.x);                      // throat low-pass (TRMFilters.m:72-77)
                         const double e0 = t[0] - bt[1], e1 = t[1] - bt[2], e2 = t[2] - bt[3], e4 = t[4] - bt[5];
                         const double e6 = t[6] - bt[7], e7 = t[7] - bt[8], e8 = t[8] - bt[9];
                         const double en0 = nt[0] - nb[1], en1 = nt[1] - nb[2], en2 = nt[2] - nb[3], en3 = nt[3] - nb[4], en4 = nt[4] - nb[5];
                         const double pa = q1.y * t[3];                                // velum 3-way junction (m:810-813), d folded in
                         const double mk = q4.x * t[9], nkk = c_nk4 * nt[5];           // mouth / nose (m:832-835, 846-849)
                         const double m1 = c_mb11 * m_ry, n1 = c_nb11 * n_ry;
-                        const double g0 = fma(bt[0], d, q10.y);                       // glottis end (m:792)
+                        const double g0 = fma(bt[0], d, q8.x);                        // glottis end (m:792)
                         const double h5 = bt[6] * d;                                  // S6|S7: pure delay (m:821-822)
                         // ---- stage 2: kd-products ----
-                        const double fr = fma(-q10.x, y2, fr1);
+                        const double fr = fma(-q6.x, y2, fr1);
                         const double x0 = q0.x * e0, x1 = q0.y * e1, x2 = q1.x * e2, x4 = q2.x * e4, x6 = q2.y * e6, x7 = q3.x * e7, x8 = q3.y * e8;
                         const double xn0 = q4.y * en0, xn1 = c_nk0 * en1, xn2 = c_nk1 * en2, xn3 = c_nk2 * en3, xn4 = c_nk3 * en4;
                         const double pb = fma(q1.y, bt[4], pa);
                         const double refl = fma(c_ma10, mk, -m1), refn = fma(c_na10, nkk, -n1);
                         const double mx1 = t[9] + mk, nx1 = nt[5] + nkk;
                         y2 = y1; y1 = fr; thy = th;
-                        const double q5x = q5.x, q5y = q5.y, q7y = q7.y, q9x = q9.x;
                         // ---- stage 3: waves before injection, radiation filters ----
-                        const double jp = fma(q5x, nb[0], pb);
+                        const double jp = fma(q5.x, nb[0], pb);
                         const double u1 = fma(t[0], d, x0), v0 = fma(bt[1], d, x0);
                         const double u2 = fma(t[1], d, x1), v1 = fma(bt[2], d, x1);
                         const double u3 = fma(t[2], d, x2), v2 = fma(bt[3], d, x2);
@@ -597,7 +614,7 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                         const double un3 = fma(nt[2], d, xn2), vn2 = fma(nb[3], d, xn2);
                         const double un4 = fma(nt[3], d, xn3), vn3 = fma(nb[4], d, xn3);
                         const double un5 = fma(nt[4], d, xn4), vn4 = fma(nb[5], d, xn4);
-                        const double f5 = q7y * fr;
+                        const double f5 = tap(4) * fr;
                         // radiation filter (TRMFilters.m:47-60): a21 = b21 = -a20 by construction (TRMFilters.m:34-45), so
                         // a20 x + a21 x[n-1] - b21 y[n-1] = a20 ((x - x[n-1]) + y[n-1])
                         const double ra = mx1 - m_rx, rb = nx1 - n_rx;
@@ -608,13 +625,13 @@ __device__ __forceinline__ void wide_recurrence_warp(WideSmem<R> &W, const WideA
                         const double t6n = fma(t[5], d, f5);
                         t[0] = g0;
                         t[1] = u1;                    bt[0] = v0;
-                        t[2] = fma(q5y, fr, u2);      bt[1] = v1;
-                        t[3] = fma(q6.x, fr, u3);     bt[2] = v2;
-                        t[5] = fma(q7.x, fr, u5);     bt[4] = v4;
-                        t[7] = fma(q8.x, fr, u7);     bt[6] = v6;
-                        t[8] = fma(q8.y, fr, u8);     bt[7] = v7;
-                        t[9] = fma(q9x, fr, u9);      bt[8] = v8;
-                        t[4] = fma(q6.y, fr, w4);     bt[3] = b3n;
+                        t[2] = fma(tap(0), fr, u2);   bt[1] = v1;
+                        t[3] = fma(tap(1), fr, u3);   bt[2] = v2;
+                        t[5] = fma(tap(3), fr, u5);   bt[4] = v4;
+                        t[7] = fma(tap(5), fr, u7);   bt[6] = v6;
+                        t[8] = fma(tap(6), fr, u8);   bt[7] = v7;
+                        t[9] = fma(tap(7), fr, u9);   bt[8] = v8;
+                        t[4] = fma(tap(2), fr, w4);   bt[3] = b3n;
                         t[6] = t6n;                   bt[5] = h5;
                         bt[9] = b9n;
                         nt[0] = nt0n;
@@ -736,6 +753,7 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
     const unsigned long long MASK44 = (1ull << 44) - 1ull;
     const unsigned long long pw1 = c_noise_pow[hl + 1], pwB = c_noise_pow[TB];
     R xm1 = 0, xm2 = 0;
+    int hs = 0;                                            // oscillator history: start of this block's FIR window
     const int pf = hl >> 1, pc = hl & 1;                   // parameter lane -> (unit, component) of the staged value
     if (st_h) {
         // streaming: oscillator position, noise generator, oscillator / band-pass input history of the previous call
@@ -744,7 +762,11 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
         kb = st_h[2];
         fresh = st_h[3] != 0ull;
         xm1 = st_v[STATE_XM]; xm2 = st_v[STATE_XM + 1];
-        for (int i = hl; i < FIR_HIST; i += TB) { S.HE[i] = st_v[STATE_HE + i]; S.HO[i] = st_v[STATE_HO + i]; }
+        for (int i = hl; i < FIR_HIST; i += TB) {
+            const R e = st_v[STATE_HE + i], o = st_v[STATE_HO + i];
+            S.HE[i] = e; S.HO[i] = o;
+            if (HIST_RING<R>) { S.HE[FIR_RING + i] = e; S.HO[FIR_RING + i] = o; }
+        }
     }
     // FP64 conformance mode: parameter lane p also carries function p of its parameter as a complex number (rc, rs) that
     // is multiplied by (dc, ds) every sample -- geometric for the exponentials (rs = ds = 0), a rotation for the angles:
@@ -986,14 +1008,13 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             const double sum = (2.0 * dd) * rcp_fast((r2[3] + r2[3]) + v2);
             const double aLd = sum * r2[3], aUd = sum * v2;
             const double kd10 = kd(v2, S.CST[C_NR1SQ]);
-            double tap[8];
-            {
-                const int ipos = (int)fpos;
-                const double comp = fpos - (double)ipos;
-                const double t0 = (1.0 - comp) * fa, t1 = comp * fa;
-#pragma unroll
-                for (int q = 0; q < 8; ++q) tap[q] = (q == ipos) ? t0 : ((ipos >= 0 && q == ipos + 1) ? t1 : 0.0);
-            }
+            // frication taps (m:760-773): (1 - c) amp at i = (int) position, c amp at i + 1 if that is a tap, 0 elsewhere.
+            // Sent as the even junction's value, the odd junction's value and the set of junctions that take them.
+            const int ipos = (int)fpos;
+            const double comp = fpos - (double)ipos;
+            const double t0 = (1.0 - comp) * fa, t1 = comp * fa;
+            const bool even = (ipos & 1) == 0;
+            const unsigned tsel = ((unsigned)ipos < 8u) ? (3u << ipos) & 0xFFu : 0u;
             // band-pass (TRMFilters.m:9-17): beta = (1 - tan u) / (2 (1 + tan u)) = (cos u - sin u) / (2 (cos u + sin u))
             const double cu = prm[19], su = prm[13], cosv = prm[18];
             const double beta2 = (cu - su) * rcp_fast(cu + su);
@@ -1004,12 +1025,9 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             W.ring[slot][2][hl][ucol] = make_double2(kd4, kd6);
             W.ring[slot][3][hl][ucol] = make_double2(kd7, kd8);
             W.ring[slot][4][hl][ucol] = make_double2(k9, kd10);
-            W.ring[slot][5][hl][ucol] = make_double2(aUd, tap[0]);
-            W.ring[slot][6][hl][ucol] = make_double2(tap[1], tap[2]);
-            W.ring[slot][7][hl][ucol] = make_double2(tap[3], tap[4]);
-            W.ring[slot][8][hl][ucol] = make_double2(tap[5], tap[6]);
-            W.ring[slot][9][hl][ucol] = make_double2(tap[7], gamma2);
-            reinterpret_cast<double *>(&W.ring[slot][10][hl][ucol])[0] = beta2;
+            W.ring[slot][5][hl][ucol] = make_double2(aUd, gamma2);
+            W.ring[slot][6][hl][ucol] = make_double2(beta2, __longlong_as_double((long long)tsel));
+            W.ring[slot][7][hl][ucol] = make_double2(even ? t0 : t1, even ? t1 : t0);
         } else if constexpr (FAST) {
             const float axf = amplitude_f(prm[1]);
             ax_d = (double)axf;
@@ -1217,7 +1235,9 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
 
         TPH(5);
         // ---- A2: table look-ups, FIR, source mixing (TRMWavetable.m:174-195, m:305-337) --------------------------
+        R *const he = &S.HE[hs + FIR_HIST + hl], *const ho = &S.HO[hs + FIR_HIST + hl];   // this lane's new value
         {
+            R ev, ov;
             if (!active) { p0 = 0.0; p1 = 0.0; }
             const double newDiv2 = (double)div2 - rint(ax_d * S.CST[C_TNDELTA]);
             const double Ld = newDiv2 - (double)div1;
@@ -1233,8 +1253,8 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
                 const float w01 = table_value_fast(wt_base, hi0, div1, inv_div1, newDiv2, scale, pulse_wave);
                 const float w10 = table_value_fast(wt_base, lo1, div1, inv_div1, newDiv2, scale, pulse_wave);
                 const float w11 = table_value_fast(wt_base, hi1, div1, inv_div1, newDiv2, scale, pulse_wave);
-                S.HE[FIR_HIST + hl] = w00 + ((float)(p0 - (double)lo0) * (w01 - w00));
-                S.HO[FIR_HIST + hl] = w10 + ((float)(p1 - (double)lo1) * (w11 - w10));
+                ev = w00 + ((float)(p0 - (double)lo0) * (w01 - w00));
+                ov = w10 + ((float)(p1 - (double)lo1) * (w11 - w10));
             } else {
                 const R scale = F64C ? (R)rcp_fast(Ld * Ld) : (R)(1.0 / (Ld * Ld));
                 if (F64C && pulse_wave) {
@@ -1251,23 +1271,24 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
                         return (di >= newDiv2) ? 0.0 : v;
                     };
                     const double w00 = value(lo0), w01 = value(hi0), w10 = value(lo1), w11 = value(hi1);
-                    S.HE[FIR_HIST + hl] = fma(p0 - (double)lo0, w01 - w00, w00);
-                    S.HO[FIR_HIST + hl] = fma(p1 - (double)lo1, w11 - w10, w10);
+                    ev = fma(p0 - (double)lo0, w01 - w00, w00);
+                    ov = fma(p1 - (double)lo1, w11 - w10, w10);
                 } else {
                     R w0 = table_value<R>(wt_base, lo0, div1, div2, newDiv2, scale, pulse_wave);
                     R w1 = table_value<R>(wt_base, hi0, div1, div2, newDiv2, scale, pulse_wave);
-                    S.HE[FIR_HIST + hl] = w0 + ((R)(p0 - (double)lo0) * (w1 - w0));
+                    ev = w0 + ((R)(p0 - (double)lo0) * (w1 - w0));
                     w0 = table_value<R>(wt_base, lo1, div1, div2, newDiv2, scale, pulse_wave);
                     w1 = table_value<R>(wt_base, hi1, div1, div2, newDiv2, scale, pulse_wave);
-                    S.HO[FIR_HIST + hl] = w0 + ((R)(p1 - (double)lo1) * (w1 - w0));
+                    ov = w0 + ((R)(p1 - (double)lo1) * (w1 - w0));
                 }
             }
+            *he = ev; *ho = ov;
+            if (HIST_RING<R> && hs + FIR_HIST + hl >= FIR_RING) { he[-FIR_RING] = ev; ho[-FIR_RING] = ov; }
         }
         __syncwarp(FULL);
         TPH(6);
         R sig;
         {
-            const R *ho = &S.HO[FIR_HIST + hl], *he = &S.HE[FIR_HIST + hl];
             R pulse0;
             // (Measured and not kept: two outputs per lane from 13 + 13 aligned 128-bit loads -- 52 shared-memory wavefronts
             //  per block instead of 98, but half the lanes idle and twice the FP64 instructions: 10.85 -> 11.19 ms.)
@@ -1315,6 +1336,9 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             xm1 = l1;
             if constexpr (FAST) {
                 W.ring[slot][10][hl][ucol] = make_float4(tube_in, bp_ff, thr_in, 0.0f);
+            } else if constexpr (F64C) {
+                W.ring[slot][8][hl][ucol] = make_double2(tube_in, bp_ff);
+                reinterpret_cast<double *>(&W.ring[slot][9][hl][ucol])[0] = thr_in;
             } else {
                 reinterpret_cast<double *>(&W.ring[slot][10][hl][ucol])[1] = tube_in;
                 W.ring[slot][11][hl][ucol] = make_double2(bp_ff, thr_in);
@@ -1323,7 +1347,9 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
         __syncwarp(FULL);
         TPH(7);
         if (lane == 0) mbar_arrive(&W.full[slot]);
-        {
+        if constexpr (HIST_RING<R>) {
+            hs = (hs + TB == FIR_RING) ? 0 : hs + TB;
+        } else {
             // slide the oscillator history down by one block (rows TB.. -> 0..)
             const R e0 = S.HE[TB + hl], o0 = S.HO[TB + hl];
             const R e1 = (hl < FIR_HIST - TB) ? S.HE[2 * TB + hl] : (R)0;
@@ -1331,8 +1357,8 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             __syncwarp(FULL);
             S.HE[hl] = e0; S.HO[hl] = o0;
             if (hl < FIR_HIST - TB) { S.HE[TB + hl] = e1; S.HO[TB + hl] = o1; }
+            __syncwarp(FULL);
         }
-        __syncwarp(FULL);
         if (PER_UTT && st_h && ends_in_block(n_tube, blk)) {
             // the utterance's last sample is in this block (a whole block except at the end of a stream): the state after it
             if (hl == 0) {
@@ -1342,7 +1368,7 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
                 st_h[3] = 0ull;
                 st_v[STATE_XM] = xm1; st_v[STATE_XM + 1] = xm2;
             }
-            for (int i = hl; i < FIR_HIST; i += TB) { st_v[STATE_HE + i] = S.HE[i]; st_v[STATE_HO + i] = S.HO[i]; }
+            for (int i = hl; i < FIR_HIST; i += TB) { st_v[STATE_HE + i] = S.HE[hs + i]; st_v[STATE_HO + i] = S.HO[hs + i]; }
         }
         TPH(8);
     }
@@ -1362,7 +1388,7 @@ __device__ __forceinline__ void wide_feed_forward_warp(WideSmem<R> &W, const Wid
             st_h[3] = 0ull;
             st_v[STATE_XM] = xm1; st_v[STATE_XM + 1] = xm2;
         }
-        for (int i = hl; i < FIR_HIST; i += TB) { st_v[STATE_HE + i] = S.HE[i]; st_v[STATE_HO + i] = S.HO[i]; }
+        for (int i = hl; i < FIR_HIST; i += TB) { st_v[STATE_HE + i] = S.HE[hs + i]; st_v[STATE_HO + i] = S.HO[hs + i]; }
     }
 }
 
@@ -1383,7 +1409,7 @@ __global__ void __launch_bounds__(Wide<R>::THREADS, 1) tube_wide_kernel(WideArgs
         constexpr int NW = (int)(sizeof(W.ring) / 4);
         for (int i = threadIdx.x; i < NW; i += blockDim.x) w[i] = 0u;
         for (int h = warp; h < 2 * Wide<R>::MAX_PAIRS; h += blockDim.x >> 5) {
-            for (int i = lane; i < FIR_HIST + TB; i += 32) { W.ff[h].HE[i] = (R)0; W.ff[h].HO[i] = (R)0; }
+            for (int i = lane; i < HIST_LEN<R>; i += 32) { W.ff[h].HE[i] = (R)0; W.ff[h].HO[i] = (R)0; }
             if (lane < TB) W.ff[h].INC[lane] = 0.0;
         }
         if (threadIdx.x == 0) {
