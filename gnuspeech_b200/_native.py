@@ -142,6 +142,7 @@ def lib():
     sig("TRMStreamFree", None, vp)
     sig("TRMStreamPoolCreate", vp, C.c_int, C.c_int, C.c_int, C.c_int, P(C.c_int))
     sig("TRMStreamPoolOpen", C.c_int, vp, vp)
+    sig("TRMStreamPoolOpenEvents", C.c_int, vp, vp, vp, i64, vp, P(i64))
     sig("TRMStreamPoolClose", C.c_int, vp, C.c_int)
     sig("TRMStreamPoolSlotCapacity", i64, vp)
     sig("TRMStreamPoolPush", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp)

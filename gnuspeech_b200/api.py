@@ -539,7 +539,8 @@ class TRMStreamPool(object):
     """Streaming slots that open, advance and end independently, each with its own voice (TRMStreamPoolCreate / Open /
     Push / Close): a server's requests arrive at different times with different voices, and one push advances any subset
     of them, each by its own number of frames, with one waveguide and one resampler launch.  Each slot's pushes,
-    concatenated, equal the one-shot synthesis of its utterance bit for bit.  Used by one thread at a time."""
+    concatenated, equal the one-shot synthesis of its utterance bit for bit.  A slot opened with open_events generates
+    its frames on the device from a Monet event list as it advances.  Used by one thread at a time."""
 
     def __init__(self, capacity, precision=N.TRM_PRECISION_FP64, max_frames_per_push=64, device=0):
         err = C.c_int(0)
@@ -557,6 +558,18 @@ class TRMStreamPool(object):
             check(slot, "TRMStreamPoolOpen")
         return slot
 
+    def open_events(self, ip, events, fg=None):
+        """Opens a free slot with voice `ip` whose frames are generated on the device from `events` (a TRMEvent array)
+        with settings `fg` (None: TRMFrameGeneration() defaults) as the slot advances (TRMStreamPoolOpenEvents).  Push
+        it with an int: the number of frames to generate.  Returns (slot, frames the list expands to)."""
+        events = np.ascontiguousarray(events, dtype=EVENT_DTYPE)
+        fg = TRMFrameGeneration() if fg is None else fg
+        nf = C.c_int64(0)
+        slot = N.lib().TRMStreamPoolOpenEvents(self._h, C.byref(ip), _ptr(events), len(events), C.byref(fg), C.byref(nf))
+        if slot < 0:
+            check(slot, "TRMStreamPoolOpenEvents")
+        return slot, int(nf.value)
+
     def close(self, slot):
         """Abandons an open slot without its tail; the slot becomes free."""
         check(N.lib().TRMStreamPoolClose(self._h, slot), "TRMStreamPoolClose")
@@ -566,19 +579,22 @@ class TRMStreamPool(object):
 
     @staticmethod
     def _entries(frames, flush):
-        """The push's entries as the C call takes them: slots, frame counts, frames back to back, flush flags."""
+        """The push's entries as the C call takes them: slots, frame counts, frames back to back, flush flags.  An int
+        value is the number of frames an event slot generates; it adds no frames."""
         slots = list(frames.keys()) + [s for s in flush if s not in frames]
-        parts = [np.ascontiguousarray(frames.get(s, np.zeros((0, 16))), dtype=np.float64).reshape(-1, 16) for s in slots]
+        gen = {s: int(frames[s]) for s in slots if isinstance(frames.get(s), (int, np.integer))}
+        parts = [np.zeros((0, 16)) if s in gen else
+                 np.ascontiguousarray(frames.get(s, np.zeros((0, 16))), dtype=np.float64).reshape(-1, 16) for s in slots]
         slot_a = np.array(slots, dtype=np.int32)
-        nf_a = np.array([p.shape[0] for p in parts], dtype=np.int32)
+        nf_a = np.array([gen[s] if s in gen else p.shape[0] for s, p in zip(slots, parts)], dtype=np.int32)
         fl = set(flush)
         flush_a = np.array([1 if s in fl else 0 for s in slots], dtype=np.uint8)
         allf = np.concatenate(parts) if parts else np.zeros((0, 16))
         return slots, slot_a, nf_a, (allf if allf.shape[0] else None), flush_a
 
     def push(self, frames, flush=()):
-        """frames: {slot: (m, 16) float64} (m may be 0); flush: slots that end with this push.  Returns {slot: samples}
-        for every slot named in `frames` or `flush`."""
+        """frames: {slot: (m, 16) float64} (m may be 0), or {slot: m} for a slot opened with open_events; flush: slots
+        that end with this push.  Returns {slot: samples} for every slot named in `frames` or `flush`."""
         slots, slot_a, nf_a, fr, flush_a = self._entries(frames, flush)
         n = len(slots)
         out = np.zeros(max(1, n * self.slot_capacity()), self.dtype)

@@ -146,6 +146,31 @@ struct FrameGenArgs {
     float *seed_out;                      // [n_utt] drift seed at exit, may be null
 };
 
+// A stream pool slot's generator between pushes (framegen_pool_kernel): the whole FrameGen of its warp -- cv / cd of all
+// 32 lanes, the rest as every lane holds it -- and the slot's settings, written when the slot opens.
+struct FrameGenPoolState {
+    double cv[32], cd[32];
+    double cv32, cd32, cd33, cd34, cd35;
+    long long i;
+    unsigned long long now, next;
+    float seed, prev, pitchDeviation, pitchOffset, a0, b1;
+    trm_cuda_framegen fg;
+};
+struct FrameGenPoolEntry {
+    unsigned long long events;            // device address of the slot's event list
+    long long count;                      // its events
+    unsigned long long out;               // device address of the first new frame (rows of 16 doubles)
+    int slot;                             // index into FrameGenPoolArgs::state
+    int m;                                // frames to generate (the list has at least that many left)
+    int setup;                            // != 0: the slot's first frames, the state is set up from fg instead of loaded
+    int reserved;
+};
+struct FrameGenPoolArgs {
+    const FrameGenPoolEntry *ent;         // [n]
+    int n;
+    FrameGenPoolState *state;             // [capacity]
+};
+
 struct KernelInfo {
     // resampler shapes (src_kernel.cuh SrcCfg): [0] handles every converter signature, [1] (if n_src_shapes == 2) is
     // the faster shape for up-sampling signatures whose work-item window fits its smaller staging buffer

@@ -10,6 +10,14 @@ extern "C" int trm_k_framegen(const trm::FrameGenArgs *a, cudaStream_t s)
     return (int)cudaGetLastError();
 }
 
+extern "C" int trm_k_framegen_pool(const trm::FrameGenPoolArgs *a, cudaStream_t s)
+{
+    if (a->n <= 0) return 0;
+    const int warps = 4;
+    trm::framegen_pool_kernel<<<(a->n + warps - 1) / warps, warps * 32, 0, s>>>(*a);
+    return (int)cudaGetLastError();
+}
+
 // ---- config 5: control tracks generated on the device (include/trm_workload.h TRMWorkloadWalk2, bit-identical) -----------
 __device__ __forceinline__ unsigned long long w2_splitmix(unsigned long long &s)
 {

@@ -33,6 +33,7 @@ TRM_DECLARE_LAUNCHERS(f64)
 TRM_DECLARE_LAUNCHERS(f32)
 TRM_DECLARE_LAUNCHERS(f64s)
 int trm_k_framegen(const trm::FrameGenArgs *, cudaStream_t);
+int trm_k_framegen_pool(const trm::FrameGenPoolArgs *, cudaStream_t);
 int trm_k_workload_walk2(unsigned long long, unsigned long long, long long, int, double *, cudaStream_t);
 int trm_k_pcm_checksum(const trm_cuda_utterance *, int, const int16_t *, unsigned long long *, cudaStream_t);
 int trm_k_pool_prepare(const trm::PoolPrepArgs *, cudaStream_t);
@@ -1340,6 +1341,11 @@ struct trm_cuda_pool {
         std::vector<double> pending;    // [pend_frames][16]: frames from the control interval in progress on
         long long pend_first = 0;
         int pend_frames = 0;
+        // event-fed slots (trm_cuda_pool_open_events): frames are generated on the device, and the pending ones live in
+        // row pcur of the slot's two pending-frame rows instead of `pending`
+        bool events = false;
+        long long ev_count = 0, ev_frames = 0;   // events of the list, frames it expands to
+        int pcur = 0;
     };
     trm_cuda_ctx *ctx = nullptr;
     int precision = 0, cap = 0, max_m = 0;
@@ -1354,11 +1360,22 @@ struct trm_cuda_pool {
     unsigned char *d_state = nullptr;   // [cap] carried waveguide states
     trm_cuda_utterance *d_desc = nullptr;   // [cap] waveguide descriptors, indexed by slot like the states
     double *d_wavetables = nullptr;     // [cap][512]: row s is slot s's glottal table
+    // event-fed slots, allocated by the first trm_cuda_pool_open_events
+    std::vector<trm_cuda_event *> d_events;   // [cap] slot s's event list (grow-only, reused by later opens)
+    std::vector<long long> events_cap;
+    trm::FrameGenPoolState *d_gen = nullptr;  // [cap] generator states
+    double *d_pend = nullptr;           // [2][cap][pend_rows][16] pending frames, two rows per slot
+    int pend_rows = 0;
     Arena scratch;                      // per-push tables and frames (one upload)
     HostStage stage;
     cudaStream_t st = nullptr;
     long long tube_at(int slot, int buf) const { return ((long long)buf * cap + slot) * stride; }
     unsigned long long tube_addr(long long elem) const { return (unsigned long long)(uintptr_t)(d_tube + (size_t)elem * esz); }
+    // device address of pending frame k of row `buf` of a slot
+    unsigned long long pend_addr(int slot, int buf, long long k) const
+    {
+        return (unsigned long long)(uintptr_t)(d_pend + (((size_t)buf * cap + slot) * pend_rows + (size_t)k) * 16);
+    }
 };
 
 static int pool_err(int code, const char *what)
@@ -1376,6 +1393,8 @@ int trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max
     p->ctx = ctx; p->precision = precision; p->cap = capacity; p->max_m = max_frames_per_push;
     p->esz = prec_esz(precision);
     p->slots.resize(capacity);
+    p->d_events.assign(capacity, nullptr);
+    p->events_cap.assign(capacity, 0);
     cudaError_t e = cudaMalloc((void **)&p->d_state, (size_t)capacity * trm::tube_state_bytes(p->esz));
     if (e == cudaSuccess) e = cudaMalloc((void **)&p->d_desc, (size_t)capacity * sizeof(trm_cuda_utterance));
     if (e == cudaSuccess) e = cudaMalloc((void **)&p->d_wavetables, (size_t)capacity * TRM_TABLE_LENGTH * sizeof(double));
@@ -1449,6 +1468,56 @@ int trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const 
     return 0;
 }
 
+int trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable,
+                              const trm_cuda_event *events, int64_t n_events, int64_t n_frames, const trm_cuda_framegen *fg,
+                              int *slot)
+{
+    *slot = -1;
+    int s = 0;
+    while (s < p->cap && p->slots[s].open) ++s;
+    if (s == p->cap) return pool_err(-7, "trm_cuda_pool_open_events: every slot is open");
+    int rc = trm_cuda_pool_reserve(p, voice);
+    if (rc != 0) return rc;
+    if (!p->d_gen) {
+        // Between pushes a slot keeps the frames from the control interval its waveguide position s_done lies in:
+        // s_done is the last whole 16-sample block before the last frame, so at most 1 + ceil(15 / controlPeriod) <= TB
+        // frames.  A push appends at most max_m more.
+        const int rows = p->max_m + trm::TB;
+        trm::FrameGenPoolState *gen = nullptr;
+        double *pend = nullptr;
+        cudaError_t e = cudaMalloc((void **)&gen, (size_t)p->cap * sizeof(trm::FrameGenPoolState));
+        if (e == cudaSuccess) e = cudaMalloc((void **)&pend, (size_t)2 * p->cap * rows * 128);
+        if (e != cudaSuccess) {
+            if (gen) cudaFree(gen);
+            return fail("trm_cuda_pool_open_events", e);
+        }
+        p->d_gen = gen;
+        p->d_pend = pend;
+        p->pend_rows = rows;
+    }
+    if (n_events > p->events_cap[s]) {
+        if (p->d_events[s]) cudaFree(p->d_events[s]);
+        p->d_events[s] = nullptr;
+        p->events_cap[s] = 0;
+        CK(cudaMalloc((void **)&p->d_events[s], (size_t)n_events * sizeof(trm_cuda_event)));
+        p->events_cap[s] = n_events;
+    }
+    if (n_events > 0) CK(cudaMemcpy(p->d_events[s], events, (size_t)n_events * sizeof(trm_cuda_event), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(&p->d_gen[s].fg, fg, sizeof(trm_cuda_framegen), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH, wavetable, TRM_TABLE_LENGTH * sizeof(double), cudaMemcpyHostToDevice));
+    trm_cuda_pool::Slot &sl = p->slots[s];
+    sl = trm_cuda_pool::Slot();
+    sl.open = true;
+    sl.fresh = true;
+    sl.voice = *voice;
+    sl.voice.voice = s;
+    sl.events = true;
+    sl.ev_count = n_events;
+    sl.ev_frames = n_frames;
+    *slot = s;
+    return 0;
+}
+
 int trm_cuda_pool_close(trm_cuda_pool *p, int slot)
 {
     if (slot < 0 || slot >= p->cap) return pool_err(-4, "trm_cuda_pool_close: no such slot");
@@ -1470,6 +1539,10 @@ void trm_cuda_pool_destroy(trm_cuda_pool *p)
     if (p->d_state) cudaFree(p->d_state);
     if (p->d_desc) cudaFree(p->d_desc);
     if (p->d_wavetables) cudaFree(p->d_wavetables);
+    for (trm_cuda_event *ev : p->d_events)
+        if (ev) cudaFree(ev);
+    if (p->d_gen) cudaFree(p->d_gen);
+    if (p->d_pend) cudaFree(p->d_pend);
     p->scratch.release();
     p->stage.release();
     delete p;
@@ -1503,7 +1576,13 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             named[s] = 1;
             if (n_frames[i] < 0 || n_frames[i] > p->max_m) return pool_err(-4, "trm_cuda_pool_push: more frames than the pool was created for");
             if (pcm && !(std::isfinite(pcm->peak[i]) && pcm->peak[i] > 0.0)) return pool_err(-4, "trm_cuda_pool_push_pcm16: a peak is not finite and > 0");
-            total_in += n_frames[i];
+            const trm_cuda_pool::Slot &sl = p->slots[s];
+            if (!sl.events) {
+                total_in += n_frames[i];
+                continue;
+            }
+            if (sl.frames_seen + n_frames[i] > sl.ev_frames) return pool_err(-4, "trm_cuda_pool_push: more frames than the slot's event list has left");
+            if (sl.pend_frames + n_frames[i] > p->pend_rows) return fail_msg("trm_cuda_pool_push: internal capacity (pending frames)");
         }
     }
     if (total_in > 0 && !frames_host) return pool_err(-4, "trm_cuda_pool_push: null frames");
@@ -1526,6 +1605,8 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         bool flush = false, run = false;
         long long target = 0, n_new = 0, out_total = 0, next_in = 0;
         int skip = 0, nf_call = 0;
+        int gen_at = 0;             // event-fed: pending-row index of the first frame this push generates
+        bool setup = false;         // event-fed: these are the slot's first frames
     };
     std::vector<Entry> E((size_t)n);
     const double *fp = frames_host;
@@ -1538,8 +1619,13 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         trm_cuda_pool::Slot &sl = p->slots[e.slot];
         const int m = n_frames[i];
         if (m) {
-            sl.pending.insert(sl.pending.end(), fp, fp + (size_t)m * 16);
-            fp += (size_t)m * 16;
+            if (sl.events) {
+                e.gen_at = sl.pend_frames;
+                e.setup = sl.frames_seen == 0;
+            } else {
+                sl.pending.insert(sl.pending.end(), fp, fp + (size_t)m * 16);
+                fp += (size_t)m * 16;
+            }
             sl.pend_frames += m;
             sl.frames_seen += m;
         }
@@ -1574,11 +1660,28 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     std::vector<long long> ib(1, 0);                      // work-item prefix
     std::vector<trm::CopySeg> mv;                         // history moves
     std::vector<int> rd_entry;                            // entry of each resampler view
+    std::vector<trm::FrameGenPoolEntry> ge;               // event-fed entries that generate frames
+    std::vector<trm::CopySeg> fs;                         // event-fed pending frames kept for the next push (other row)
+    size_t n_fb = 0;                                      // event-fed entries whose frames the waveguide reads
+    long long fed_frames = 0;                             // frames the waveguide reads from frame-fed entries (uploaded)
     for (int i = 0; i < n; ++i) {
         const Entry &e = E[i];
-        if (!e.run) continue;
         const trm_cuda_pool::Slot &sl = p->slots[e.slot];
-        if (e.n_new > 0) wg.push_back(i);
+        if (sl.events && n_frames[i] > 0)
+            ge.push_back({(unsigned long long)(uintptr_t)p->d_events[e.slot], sl.ev_count, p->pend_addr(e.slot, sl.pcur, e.gen_at),
+                          e.slot, n_frames[i], e.setup ? 1 : 0, 0});
+        if (!e.run) continue;
+        if (e.n_new > 0) {
+            wg.push_back(i);
+            if (sl.events) ++n_fb;
+            else fed_frames += e.nf_call;
+        }
+        if (sl.events && !e.flush) {
+            // the frames before the interval the next push starts in are dropped (bookkeeping below)
+            const int drop = (int)(e.target / sl.voice.controlPeriod - sl.pend_first), kept = sl.pend_frames - drop;
+            if (drop > 0 && kept > 0)
+                fs.push_back({p->pend_addr(e.slot, sl.pcur, drop), p->pend_addr(e.slot, sl.pcur ^ 1, 0), (unsigned long long)kept * 128});
+        }
         const long long n_ret = e.out_total - sl.out_done;
         if (n_ret > 0) {
             trm_cuda_utterance r = sl.voice;              // global sample indices of the stream
@@ -1609,8 +1712,12 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     const size_t n_pk = pcm ? n_rd : 0;                   // PCM: peak and max |y| of each resampler view
     const size_t o_pk = o_mv + align_up(n_mv * sizeof(trm::CopySeg), 256);
     const size_t o_mx = o_pk + align_up(n_pk * sizeof(double), 256);
-    const size_t o_fr = o_mx + align_up(n_pk * sizeof(unsigned long long), 256);
-    const size_t bytes = o_fr + (size_t)wg_frames * 128;
+    const size_t n_ge = ge.size(), n_fs = fs.size() + n_fb;
+    const size_t o_ge = o_mx + align_up(n_pk * sizeof(unsigned long long), 256);
+    const size_t o_fs = o_ge + align_up(n_ge * sizeof(trm::FrameGenPoolEntry), 256);
+    const size_t o_fr = o_fs + align_up(n_fs * sizeof(trm::CopySeg), 256);
+    // the frame region holds the frame-fed entries' frames (uploaded), then the event-fed ones' (copied on the device)
+    const size_t bytes = o_fr + (size_t)wg_frames * 128, up = o_fr + (size_t)fed_frames * 128;
     int rc;
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
     if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
@@ -1619,12 +1726,13 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         trm_cuda_utterance *dt = (trm_cuda_utterance *)(h + o_dt);
         int *ord = (int *)(h + o_ord), *rst = (int *)(h + o_rst);
         double *fr = (double *)(h + o_fr);
-        long long f_at = 0;
+        trm::CopySeg *fb = (trm::CopySeg *)(h + o_fs) + fs.size();
+        long long f_at = 0, ev_at = fed_frames;
         for (size_t k = 0; k < wg.size(); ++k) {
             const Entry &e = E[wg[k]];
             const trm_cuda_pool::Slot &sl = p->slots[e.slot];
             trm_cuda_utterance d = sl.voice;
-            d.frame_offset = f_at;
+            d.frame_offset = sl.events ? ev_at : f_at;
             d.n_frames = e.nf_call;
             d.n_tube = e.n_new;
             d.tube_offset = p->tube_at(e.slot, sl.cur) + (sl.s_done - sl.in_start);
@@ -1633,9 +1741,17 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             dt[k] = d;
             ord[k] = e.slot;
             rst[k] = sl.fresh ? 1 : 0;
-            memcpy(fr + (size_t)f_at * 16, &sl.pending[(size_t)e.skip * 16], (size_t)e.nf_call * 128);
-            f_at += e.nf_call;
+            if (sl.events) {
+                *fb++ = {p->pend_addr(e.slot, sl.pcur, e.skip), (unsigned long long)(uintptr_t)(p->scratch.base + o_fr + (size_t)ev_at * 128),
+                         (unsigned long long)e.nf_call * 128};
+                ev_at += e.nf_call;
+            } else {
+                memcpy(fr + (size_t)f_at * 16, &sl.pending[(size_t)e.skip * 16], (size_t)e.nf_call * 128);
+                f_at += e.nf_call;
+            }
         }
+        if (n_ge) memcpy(h + o_ge, ge.data(), n_ge * sizeof(trm::FrameGenPoolEntry));
+        if (!fs.empty()) memcpy(h + o_fs, fs.data(), fs.size() * sizeof(trm::CopySeg));
         if (n_rd) memcpy(h + o_rd, rd.data(), n_rd * sizeof(trm_cuda_utterance));
         memcpy(h + o_ib, ib.data(), ib.size() * sizeof(long long));
         if (n_mv) memcpy(h + o_mv, mv.data(), n_mv * sizeof(trm::CopySeg));
@@ -1644,7 +1760,17 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     }
     unsigned char *d = p->scratch.base;
     cudaStream_t st = p->st;
-    CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d, h, up, cudaMemcpyHostToDevice, st));
+    if (n_ge > 0) {
+        // event-fed slots: new frames appended to the pending row, then that row's frames copied where the waveguide
+        // reads them and the kept ones to the slot's other row
+        const trm::FrameGenPoolArgs a{(const trm::FrameGenPoolEntry *)(d + o_ge), (int)n_ge, p->d_gen};
+        if ((rc = trm_k_framegen_pool(&a, st)) != 0) return fail("pool frame generator launch", (cudaError_t)rc);
+    }
+    if (n_fs > 0) {
+        const trm::SegCopyArgs a{(const trm::CopySeg *)(d + o_fs), (int)n_fs};
+        if ((rc = trm_k_segment_copy(&a, st)) != 0) return fail("pool frame move launch", (cudaError_t)rc);
+    }
     const KernelSet &K = g_kernels[p->precision];
     const trm::KernelInfo &ki = ctx->ki(p->precision);
     const int n_w = (int)wg.size();
@@ -1710,7 +1836,8 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         const long long nf0 = sl.s_done / sl.voice.controlPeriod;
         const int drop = (int)(nf0 - sl.pend_first);
         if (drop > 0) {
-            sl.pending.erase(sl.pending.begin(), sl.pending.begin() + (size_t)drop * 16);
+            if (!sl.events) sl.pending.erase(sl.pending.begin(), sl.pending.begin() + (size_t)drop * 16);
+            else if (sl.pend_frames > drop) sl.pcur ^= 1;      // the kept frames were copied to the other row
             sl.pend_frames -= drop;
             sl.pend_first = nf0;
         }
@@ -1778,6 +1905,7 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
             if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_save: no such slot");
             if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_save: the slot is not open");
             if (named[s]) return pool_err(-4, "trm_cuda_pool_save: a slot is named twice");
+            if (p->slots[s].events) return pool_err(-7, "trm_cuda_pool_save: a slot fed from an event list has no snapshot");
             named[s] = 1;
         }
     }

@@ -1033,21 +1033,28 @@ int64_t TRMEventListFrameCount(const TRMEvent *ev, int64_t count)
     return emitted;
 }
 
+/* One event list the generator runs on: n_frames must be its TRMEventListFrameCount. */
+static int check_event_list(const TRMEvent *ev, int64_t n_events, int64_t n_frames)
+{
+    const int64_t want = n_events >= 0 ? TRMEventListFrameCount(ev, n_events) : -1;
+    if (want != n_frames)
+        return set_err(TRM_ERR_PARAM, "utterance frame count differs from TRMEventListFrameCount of its event list%s", "");
+    /* every TRM parameter track needs a value after the first event: the reference's set-up loop (EventList.m:919-930)
+     * scans forward for one without a bound and reads past the array otherwise */
+    for (int j = 0; j < 16 && n_events >= 2; j++) {
+        int found = 0;
+        for (int64_t k = 1; k < n_events && !found; k++) found = !isnan(ev[k].value[j]);
+        if (!found) return set_err(TRM_ERR_PARAM, "event list: a parameter track has no value after the first event%s", "");
+    }
+    return TRM_OK;
+}
+
 static int check_event_lists(const TRMBatch *b, const TRMEvent *events, const int64_t *event_offset, const int32_t *n_events)
 {
     if (!events || !event_offset || !n_events) return set_err(TRM_ERR_PARAM, "null event arguments%s", "");
     for (int u = 0; u < b->n; u++) {
-        const int64_t want = n_events[u] >= 0 ? TRMEventListFrameCount(events + event_offset[u], n_events[u]) : -1;
-        if (want != b->desc[u].n_frames)
-            return set_err(TRM_ERR_PARAM, "utterance frame count differs from TRMEventListFrameCount of its event list%s", "");
-        /* every TRM parameter track needs a value after the first event: the reference's set-up loop (EventList.m:919-930)
-         * scans forward for one without a bound and reads past the array otherwise */
-        const TRMEvent *ev = events + event_offset[u];
-        for (int j = 0; j < 16 && n_events[u] >= 2; j++) {
-            int found = 0;
-            for (int32_t k = 1; k < n_events[u] && !found; k++) found = !isnan(ev[k].value[j]);
-            if (!found) return set_err(TRM_ERR_PARAM, "event list: a parameter track has no value after the first event%s", "");
-        }
+        const int rc = check_event_list(events + event_offset[u], n_events[u], b->desc[u].n_frames);
+        if (rc != TRM_OK) return rc;
     }
     return TRM_OK;
 }
@@ -1211,6 +1218,28 @@ int TRMStreamPoolOpen(TRMStreamPool *t, const TRMInputParameters *voice)
     voice_set_free(&vs);
     if (rc != 0) return pool_rc(rc);
     t->voice[slot] = *voice;
+    return slot;
+}
+
+int TRMStreamPoolOpenEvents(TRMStreamPool *t, const TRMInputParameters *voice, const TRMEvent *events, int64_t n_events,
+                            const TRMFrameGeneration *fg, int64_t *n_frames_out)
+{
+    if (!t || !voice) return set_err(TRM_ERR_PARAM, "null stream pool or voice%s", "");
+    voice_set vs;
+    trm_cuda_utterance d;
+    memset(&vs, 0, sizeof vs);
+    int rc = describe(voice, 2, &vs, &d, NULL);
+    if (rc != TRM_OK) { voice_set_free(&vs); return rc; }
+    if (!events || !fg) { voice_set_free(&vs); return set_err(TRM_ERR_PARAM, "null event arguments%s", ""); }
+    const int64_t n_frames = n_events >= 0 ? TRMEventListFrameCount(events, n_events) : 0;
+    if ((rc = check_event_list(events, n_events, n_frames)) != TRM_OK) { voice_set_free(&vs); return rc; }
+    int slot = -1;
+    rc = trm_cuda_pool_open_events(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, (const trm_cuda_event *)events,
+                                   n_events, n_frames, (const trm_cuda_framegen *)fg, &slot);
+    voice_set_free(&vs);
+    if (rc != 0) return pool_rc(rc);
+    t->voice[slot] = *voice;
+    if (n_frames_out) *n_frames_out = n_frames;
     return slot;
 }
 

@@ -328,6 +328,27 @@ TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_p
 /* Opens a free slot with this voice (validated exactly as TRMBatchCreate validates a voice); returns the slot >= 0 or a
  * negative TRM_ERR_*.  Pool full: TRM_ERR_STATE. */
 int TRMStreamPoolOpen(TRMStreamPool *pool, const TRMInputParameters *voice);
+/* Opens a free slot with `voice` whose control frames come from an event list (TRMEvent, as TRMBatchGenerateFrames
+ * takes it) and frame-generation settings `fg`.  The list is validated as check_event_lists validates a batch's lists
+ * and copied to the device; *n_frames_out (may be NULL) = TRMEventListFrameCount(events, n_events).
+ * The voice is validated as TRMStreamPoolOpen validates it; a list the batch path refuses is refused with the same code
+ * (TRM_ERR_PARAM); pool full: TRM_ERR_STATE.  Returns the slot >= 0 or a negative TRM_ERR_*.
+ * Such a slot is an event slot until it ends:
+ *   Push.  In TRMStreamPoolPush / TRMStreamPoolPushPCM16, n_frames[i] of an event slot's entry is the number of frames to
+ *     generate for it, continuing where its previous push stopped; it takes nothing from `frames`, which frame-fed entries
+ *     consume back to back as always (one push may mix both; `frames` may be NULL when no frame-fed entry has frames).
+ *     An entry that would take the slot past its list's frame count is refused (TRM_ERR_PARAM) with the push's other
+ *     refusals, before any device work.
+ *   Continuation.  Advanced to the end of its list and flushed, a slot's pushes, concatenated, equal what
+ *     TRMBatchSynthesizeEvents returns for a one-utterance batch with the same voice, events and fg, bit for bit: samples
+ *     in every precision; PCM16 and the per-push maxima when the peak given is that utterance's maximumSampleValue --
+ *     for any split of the frames over pushes, whatever the other slots do.
+ *   Early end.  A flush before the end of the list ends the slot as a frame-fed flush does: its output equals the
+ *     one-shot synthesis of the k frames generated so far (the first k of TRMBatchGenerateFrames' frames for the list).
+ *   Close and flush free the slot as for any slot; it may be reopened either way.  TRMStreamPoolSave refuses event slots
+ *     (TRM_ERR_STATE). */
+int TRMStreamPoolOpenEvents(TRMStreamPool *pool, const TRMInputParameters *voice, const TRMEvent *events,
+                            int64_t n_events, const TRMFrameGeneration *fg, int64_t *n_frames_out);
 /* Abandons an open slot without its tail (client went away); the slot becomes free. */
 int TRMStreamPoolClose(TRMStreamPool *pool, int slot);
 /* Samples one slot can return from one push (row bound for samples_out).  Sized at creation for the default voice; it
@@ -390,8 +411,9 @@ typedef struct TRMStreamSnapshotInfo {
     int64_t bytes;                   /* size of the snapshot                                                        */
 } TRMStreamSnapshotInfo;
 /* Snapshots of n distinct open slots, packed: slot[i]'s bytes are blob[offset[i] .. offset[i+1]).  blob == NULL: only
- * fills offset (sizes from host bookkeeping, no device work).  Refused before anything is written: an unopened slot
- * (TRM_ERR_STATE), a slot named twice or blob_capacity < offset[n] (TRM_ERR_PARAM). */
+ * fills offset (sizes from host bookkeeping, no device work).  Refused before anything is written: an unopened slot or a
+ * slot opened with TRMStreamPoolOpenEvents (TRM_ERR_STATE), a slot named twice or blob_capacity < offset[n]
+ * (TRM_ERR_PARAM). */
 int TRMStreamPoolSave(TRMStreamPool *pool, int n, const int32_t *slot, void *blob, int64_t blob_capacity,
                       int64_t *offset /* [n + 1] */);
 /* Opens n free slots from n snapshots (the same packing); slot_out[i] is the slot that continues snapshot i.  All n are

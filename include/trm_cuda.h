@@ -198,9 +198,17 @@ int  trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int ma
 int  trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *voice);
 /* voice.voice is ignored: `wavetable` (512 doubles) becomes the slot's own glottal table.  *slot receives the slot. */
 int  trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, int *slot);
+/* The same, for a slot whose frames are generated on the device from an event list (libtrm has checked it: n_frames =
+ * its frame count, every parameter track has a value after the first event) with settings fg, as
+ * trm_cuda_generate_frames generates them.  The list is copied to the slot's device storage (grow-only, kept for later
+ * opens of the slot). */
+int  trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable,
+                               const trm_cuda_event *events, int64_t n_events, int64_t n_frames, const trm_cuda_framegen *fg,
+                               int *slot);
 int  trm_cuda_pool_close(trm_cuda_pool *p, int slot);
 int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one slot can return from one push */
-/* entry i: slot[i] gets n_frames[i] frames (taken back to back from frames_host, rows of 16 doubles); flush[i] != 0 ends
+/* entry i: slot[i] gets n_frames[i] frames (taken back to back from frames_host, rows of 16 doubles; for a slot opened
+ * with trm_cuda_pool_open_events, generated from its list instead -- -4 past the list's end); flush[i] != 0 ends
  * the slot and frees it.  samples_host receives the samples packed (entry i: [out_offset[i], out_offset[i+1])). */
 int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
                         const uint8_t *flush, void *samples_host, int64_t *out_offset);
@@ -224,7 +232,8 @@ int  trm_cuda_pool_check_state(const trm_cuda_utterance *voice, const trm_cuda_p
  * kept history s_done - in_start elements of the precision's type. */
 int64_t trm_cuda_pool_slot_bytes(int precision, const trm_cuda_pool_slot_state *st);
 /* st[i] receives the counters of n distinct open slots; with dst (may be NULL: counters only, no device work), dst[i]
- * receives slot[i]'s data part (trm_cuda_pool_slot_bytes).  The slots are not changed.  -7: a slot is not open. */
+ * receives slot[i]'s data part (trm_cuda_pool_slot_bytes).  The slots are not changed.  -7: a slot is not open, or was
+ * opened with trm_cuda_pool_open_events. */
 int  trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st, void *const *dst);
 /* Opens n free slots continuing n saved ones: voice[i] (voice.voice ignored) with its glottal table wavetables[i][512],
  * counters st[i] and data part src[i].  Refused before any change: counters that fail trm_cuda_pool_check_state or whose
