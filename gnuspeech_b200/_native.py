@@ -63,6 +63,11 @@ class TRMStreamSnapshotInfoStruct(C.Structure):
                 ("frames_pushed", C.c_int64), ("samples_returned", C.c_int64), ("bytes", C.c_int64)]
 
 
+class TRMStreamSnapshotEventInfoStruct(C.Structure):
+    _fields_ = [("from_events", C.c_int32), ("n_events", C.c_int64), ("list_frames", C.c_int64),
+                ("frames_generated", C.c_int64), ("fg", TRMFrameGenerationStruct)]
+
+
 _lib = None
 
 
@@ -151,6 +156,8 @@ def lib():
     sig("TRMStreamPoolSave", C.c_int, vp, C.c_int, vp, vp, i64, vp)
     sig("TRMStreamPoolRestore", C.c_int, vp, C.c_int, vp, vp, vp)
     sig("TRMStreamPoolSnapshotInfo", C.c_int, vp, i64, P(TRMStreamSnapshotInfoStruct))
+    sig("TRMStreamPoolSaveAny", C.c_int, vp, C.c_int, vp, vp, i64, vp)
+    sig("TRMStreamPoolSnapshotEventInfo", C.c_int, vp, i64, P(TRMStreamSnapshotEventInfoStruct))
     sig("TRMBatchSynthesizeAsync", vp, vp, vp, vp, vp, vp, C.c_int, vp)
     sig("TRMBatchWait", C.c_int, vp)
     sig("TRMBatchMakeResident", vp, vp, vp, C.c_int, P(C.c_int))

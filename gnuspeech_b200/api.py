@@ -618,21 +618,24 @@ class TRMStreamPool(object):
                                              _ptr(pcm), _ptr(off), _ptr(mx)), "TRMStreamPoolPushPCM16")
         return {s: (pcm[off[i]:off[i + 1]].copy(), float(mx[i])) for i, s in enumerate(slots)}
 
-    def save(self, slots):
+    def save(self, slots, event_slots=False):
         """Snapshots of open slots (TRMStreamPoolSave): {slot: bytes}.  Each restores into any pool of this precision
-        and continues the stream bit for bit; the saved slots are not changed."""
+        and continues the stream bit for bit; the saved slots are not changed.  Slots opened with open_events are
+        refused unless event_slots is True (TRMStreamPoolSaveAny): they are then saved as format version 2, with their
+        event list and generator state; frame-fed slots give the same bytes either way."""
+        fn = "TRMStreamPoolSaveAny" if event_slots else "TRMStreamPoolSave"
+        save = getattr(N.lib(), fn)
         slots = [int(s) for s in slots]
         slot_a = np.array(slots, dtype=np.int32)
         off = np.zeros(len(slots) + 1, np.int64)
-        check(N.lib().TRMStreamPoolSave(self._h, len(slots), _ptr(slot_a), None, 0, _ptr(off)), "TRMStreamPoolSave")
+        check(save(self._h, len(slots), _ptr(slot_a), None, 0, _ptr(off)), fn)
         blob = np.zeros(max(1, int(off[-1])), np.uint8)
-        check(N.lib().TRMStreamPoolSave(self._h, len(slots), _ptr(slot_a), _ptr(blob), blob.size, _ptr(off)),
-              "TRMStreamPoolSave")
+        check(save(self._h, len(slots), _ptr(slot_a), _ptr(blob), blob.size, _ptr(off)), fn)
         return {s: blob[off[i]:off[i + 1]].tobytes() for i, s in enumerate(slots)}
 
     def restore(self, snapshots):
-        """Opens one free slot per snapshot (bytes from save, in this or any other pool of the same precision); returns
-        the slots in order.  All or nothing (TRMStreamPoolRestore)."""
+        """Opens one free slot per snapshot (bytes from save, in this or any other pool of the same precision; an event
+        slot's snapshot restores as an event slot); returns the slots in order.  All or nothing (TRMStreamPoolRestore)."""
         snapshots = [bytes(b) for b in snapshots]
         off = np.zeros(len(snapshots) + 1, np.int64)
         off[1:] = np.cumsum([len(b) for b in snapshots])
@@ -653,15 +656,24 @@ class TRMStreamPool(object):
 def snapshot_info(snapshot):
     """What a stream pool snapshot holds, after the checks a restore makes apart from the destination pool
     (TRMStreamPoolSnapshotInfo; needs no device): {precision, channels, voice (TRMInputParameters), frames_pushed,
-    samples_returned, bytes}.  Raises TRMError for a snapshot a restore would refuse on its own."""
+    samples_returned, bytes, events}.  events is None for a frame-fed slot's snapshot, or for an event slot's
+    (TRMStreamPoolSnapshotEventInfo) {n_events, list_frames, frames_generated, fg (TRMFrameGeneration)}.  Raises
+    TRMError for a snapshot a restore would refuse on its own."""
     b = bytes(snapshot)
     buf = C.create_string_buffer(b, max(1, len(b)))
     info = N.TRMStreamSnapshotInfoStruct()
     check(N.lib().TRMStreamPoolSnapshotInfo(buf, len(b), C.byref(info)), "TRMStreamPoolSnapshotInfo")
+    ev = N.TRMStreamSnapshotEventInfoStruct()
+    check(N.lib().TRMStreamPoolSnapshotEventInfo(buf, len(b), C.byref(ev)), "TRMStreamPoolSnapshotEventInfo")
     voice = TRMInputParameters()
     C.memmove(C.byref(voice), C.byref(info.voice), C.sizeof(voice))
+    events = None
+    if ev.from_events:
+        fg = TRMFrameGeneration()
+        C.memmove(C.byref(fg), C.byref(ev.fg), C.sizeof(fg))
+        events = {"n_events": ev.n_events, "list_frames": ev.list_frames, "frames_generated": ev.frames_generated, "fg": fg}
     return {"precision": info.precision, "channels": info.channels, "voice": voice, "frames_pushed": info.frames_pushed,
-            "samples_returned": info.samples_returned, "bytes": info.bytes}
+            "samples_returned": info.samples_returned, "bytes": info.bytes, "events": events}
 
 
 class TRMBatchTicket(object):

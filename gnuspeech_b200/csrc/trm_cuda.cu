@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -1345,6 +1346,7 @@ struct trm_cuda_pool {
         // row pcur of the slot's two pending-frame rows instead of `pending`
         bool events = false;
         long long ev_count = 0, ev_frames = 0;   // events of the list, frames it expands to
+        trm_cuda_framegen fg{};                  // its settings (the device copy is in d_gen[slot].fg)
         int pcur = 0;
     };
     trm_cuda_ctx *ctx = nullptr;
@@ -1468,6 +1470,45 @@ int trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const 
     return 0;
 }
 
+// Between pushes a slot keeps the frames from the control interval its waveguide position s_done lies in: s_done is the
+// last whole 16-sample block before the last frame, so at most 1 + ceil(15 / controlPeriod) <= TB frames.  A push
+// appends at most max_m more.
+static int pool_pend_rows(const trm_cuda_pool *p) { return p->max_m + trm::TB; }
+
+// the event-fed slots' generator states and pending-frame rows, allocated for every slot by the first event-fed open or
+// restore
+static int pool_event_storage(trm_cuda_pool *p)
+{
+    if (p->d_gen) return 0;
+    const int rows = pool_pend_rows(p);
+    trm::FrameGenPoolState *gen = nullptr;
+    double *pend = nullptr;
+    CK(cudaSetDevice(p->ctx->device));
+    cudaError_t e = cudaMalloc((void **)&gen, (size_t)p->cap * sizeof(trm::FrameGenPoolState));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&pend, (size_t)2 * p->cap * rows * 128);
+    if (e != cudaSuccess) {
+        if (gen) cudaFree(gen);
+        return fail("pool event storage", e);
+    }
+    p->d_gen = gen;
+    p->d_pend = pend;
+    p->pend_rows = rows;
+    return 0;
+}
+
+// slot s's event list storage, grown to n_events (grow-only: kept for later event-fed opens of the slot)
+static int pool_event_list(trm_cuda_pool *p, int s, int64_t n_events)
+{
+    if (n_events <= p->events_cap[s]) return 0;
+    CK(cudaSetDevice(p->ctx->device));
+    if (p->d_events[s]) cudaFree(p->d_events[s]);
+    p->d_events[s] = nullptr;
+    p->events_cap[s] = 0;
+    CK(cudaMalloc((void **)&p->d_events[s], (size_t)n_events * sizeof(trm_cuda_event)));
+    p->events_cap[s] = n_events;
+    return 0;
+}
+
 int trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable,
                               const trm_cuda_event *events, int64_t n_events, int64_t n_frames, const trm_cuda_framegen *fg,
                               int *slot)
@@ -1477,31 +1518,9 @@ int trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice,
     while (s < p->cap && p->slots[s].open) ++s;
     if (s == p->cap) return pool_err(-7, "trm_cuda_pool_open_events: every slot is open");
     int rc = trm_cuda_pool_reserve(p, voice);
+    if (rc == 0) rc = pool_event_storage(p);
+    if (rc == 0) rc = pool_event_list(p, s, n_events);
     if (rc != 0) return rc;
-    if (!p->d_gen) {
-        // Between pushes a slot keeps the frames from the control interval its waveguide position s_done lies in:
-        // s_done is the last whole 16-sample block before the last frame, so at most 1 + ceil(15 / controlPeriod) <= TB
-        // frames.  A push appends at most max_m more.
-        const int rows = p->max_m + trm::TB;
-        trm::FrameGenPoolState *gen = nullptr;
-        double *pend = nullptr;
-        cudaError_t e = cudaMalloc((void **)&gen, (size_t)p->cap * sizeof(trm::FrameGenPoolState));
-        if (e == cudaSuccess) e = cudaMalloc((void **)&pend, (size_t)2 * p->cap * rows * 128);
-        if (e != cudaSuccess) {
-            if (gen) cudaFree(gen);
-            return fail("trm_cuda_pool_open_events", e);
-        }
-        p->d_gen = gen;
-        p->d_pend = pend;
-        p->pend_rows = rows;
-    }
-    if (n_events > p->events_cap[s]) {
-        if (p->d_events[s]) cudaFree(p->d_events[s]);
-        p->d_events[s] = nullptr;
-        p->events_cap[s] = 0;
-        CK(cudaMalloc((void **)&p->d_events[s], (size_t)n_events * sizeof(trm_cuda_event)));
-        p->events_cap[s] = n_events;
-    }
     if (n_events > 0) CK(cudaMemcpy(p->d_events[s], events, (size_t)n_events * sizeof(trm_cuda_event), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(&p->d_gen[s].fg, fg, sizeof(trm_cuda_framegen), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH, wavetable, TRM_TABLE_LENGTH * sizeof(double), cudaMemcpyHostToDevice));
@@ -1514,6 +1533,8 @@ int trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice,
     sl.events = true;
     sl.ev_count = n_events;
     sl.ev_frames = n_frames;
+    sl.fg = *fg;
+    sl.fg.reserved = 0;                 // a snapshot stores 0 there, whatever the caller left in it
     *slot = s;
     return 0;
 }
@@ -1895,7 +1916,39 @@ static size_t pool_device_bytes(const trm_cuda_pool *p, const trm_cuda_pool_slot
     return (c.fresh ? 0 : trm::tube_state_bytes(p->esz)) + (size_t)(c.s_done - c.in_start) * p->esz;
 }
 
-int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st, void *const *dst)
+// the generator part of the device state is the FrameGen fields, in the snapshot's order, ahead of the settings
+static_assert(offsetof(trm::FrameGenPoolState, fg) == TRM_FRAMEGEN_STATE_BYTES, "generator state layout");
+static_assert(sizeof(trm_cuda_event) == 296, "event layout");
+
+static size_t pool_gen_bytes(const trm_cuda_pool_slot_state &c) { return c.frames_seen > 0 ? TRM_FRAMEGEN_STATE_BYTES : 0; }
+
+int64_t trm_cuda_pool_event_bytes(const trm_cuda_pool_slot_state *st, const trm_cuda_pool_event_state *ev)
+{
+    return ev->events ? (int64_t)pool_gen_bytes(*st) + ev->n_events * (int64_t)sizeof(trm_cuda_event) : 0;
+}
+
+// A slot's part of the snapshot staging, packed slot after slot from 16-byte boundaries: [pending frames (event-fed
+// slots: they are on the device)][carried state][kept history][event list][generator state].  The list precedes the
+// generator so that both the list and everything before it start on 16 bytes; the data part orders them the other way.
+struct SnapStage {
+    size_t pend = 0, dev = 0, list = 0, gen = 0;
+    size_t bytes() const { return align_up(pend + dev + list + gen, 16); }
+};
+
+static SnapStage snap_stage(const trm_cuda_pool *p, const trm_cuda_pool_slot_state &c, const trm_cuda_pool_event_state *ev)
+{
+    SnapStage g;
+    g.dev = pool_device_bytes(p, c);
+    if (ev && ev->events) {
+        g.pend = (size_t)c.pend_frames * 128;
+        g.list = (size_t)ev->n_events * sizeof(trm_cuda_event);
+        g.gen = pool_gen_bytes(c);
+    }
+    return g;
+}
+
+int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st,
+                       trm_cuda_pool_event_state *ev, void *const *dst)
 {
     if (n < 0 || n > p->cap || (n > 0 && (!slot || !st))) return pool_err(-4, "trm_cuda_pool_save: bad arguments");
     {
@@ -1905,7 +1958,7 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
             if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_save: no such slot");
             if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_save: the slot is not open");
             if (named[s]) return pool_err(-4, "trm_cuda_pool_save: a slot is named twice");
-            if (p->slots[s].events) return pool_err(-7, "trm_cuda_pool_save: a slot fed from an event list has no snapshot");
+            if (p->slots[s].events && !ev) return pool_err(-7, "trm_cuda_pool_save: a slot fed from an event list has no version 1 snapshot");
             named[s] = 1;
         }
     }
@@ -1913,15 +1966,27 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
         const trm_cuda_pool::Slot &sl = p->slots[slot[i]];
         st[i] = trm_cuda_pool_slot_state{sl.frames_seen, sl.s_done, sl.out_done, sl.in_start, sl.pend_first, sl.pend_frames,
                                          sl.fresh ? 1 : 0};
+        if (ev) {
+            ev[i] = trm_cuda_pool_event_state{};
+            if (sl.events) {
+                ev[i].events = 1;
+                ev[i].n_events = sl.ev_count;
+                ev[i].ev_frames = sl.ev_frames;
+                ev[i].fg = sl.fg;
+            }
+        }
     }
     if (!dst || n == 0) return 0;
 
-    // gather every slot's device part into packed staging ([segments][entry 0][entry 1] ...; all 16-byte multiples), one
-    // copy back
+    // gather every slot's device part into packed staging ([segments][slot 0][slot 1] ..., SnapStage), one copy back
     const size_t sb = trm::tube_state_bytes(p->esz);
+    std::vector<SnapStage> sg((size_t)n);
     std::vector<size_t> at((size_t)n + 1, 0);
-    for (int i = 0; i < n; ++i) at[i + 1] = at[i] + pool_device_bytes(p, st[i]);
-    const size_t o_stg = align_up((size_t)2 * n * sizeof(trm::CopySeg), 256);
+    for (int i = 0; i < n; ++i) {
+        sg[i] = snap_stage(p, st[i], ev ? &ev[i] : nullptr);
+        at[i + 1] = at[i] + sg[i].bytes();
+    }
+    const size_t o_stg = align_up((size_t)5 * n * sizeof(trm::CopySeg), 256);
     const size_t bytes = o_stg + at[n];
     int rc;
     CK(cudaSetDevice(p->ctx->device));
@@ -1932,13 +1997,26 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
     int n_seg = 0;
     for (int i = 0; i < n; ++i) {
         const int s = slot[i];
+        const trm_cuda_pool::Slot &sl = p->slots[s];
         unsigned long long to = (unsigned long long)(uintptr_t)(d + o_stg + at[i]);
+        if (sg[i].pend) {
+            seg[n_seg++] = {p->pend_addr(s, sl.pcur, 0), to, sg[i].pend};
+            to += sg[i].pend;
+        }
         if (!st[i].fresh) {
             seg[n_seg++] = {(unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), to, sb};
             to += sb;
         }
         const long long hist = st[i].s_done - st[i].in_start;
-        if (hist > 0) seg[n_seg++] = {p->tube_addr(p->tube_at(s, p->slots[s].cur)), to, (unsigned long long)hist * p->esz};
+        if (hist > 0) {
+            seg[n_seg++] = {p->tube_addr(p->tube_at(s, sl.cur)), to, (unsigned long long)hist * p->esz};
+            to += (unsigned long long)hist * p->esz;
+        }
+        if (sg[i].list) {
+            seg[n_seg++] = {(unsigned long long)(uintptr_t)p->d_events[s], to, sg[i].list};
+            to += sg[i].list;
+        }
+        if (sg[i].gen) seg[n_seg++] = {(unsigned long long)(uintptr_t)(p->d_gen + s), to, sg[i].gen};
     }
     if (n_seg > 0) {
         cudaStream_t cs = p->st;
@@ -1948,23 +2026,33 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
         CK(cudaMemcpyAsync(h + o_stg, d + o_stg, at[n], cudaMemcpyDeviceToHost, cs));
         CK(cudaStreamSynchronize(cs));
     }
+    // data part: [pending frames][state][history] then, event-fed, [generator][list]
     for (int i = 0; i < n; ++i) {
         const trm_cuda_pool::Slot &sl = p->slots[slot[i]];
+        const SnapStage &g = sg[i];
+        const unsigned char *from = h + o_stg + at[i];
         unsigned char *o = (unsigned char *)dst[i];
-        if (sl.pend_frames) memcpy(o, sl.pending.data(), (size_t)sl.pend_frames * 128);
-        memcpy(o + (size_t)sl.pend_frames * 128, h + o_stg + at[i], at[i + 1] - at[i]);
+        const size_t host_pend = sl.events ? 0 : (size_t)sl.pend_frames * 128;
+        if (host_pend) memcpy(o, sl.pending.data(), host_pend);
+        o += host_pend;
+        memcpy(o, from, g.pend + g.dev);
+        o += g.pend + g.dev;
+        if (g.gen) memcpy(o, from + g.pend + g.dev + g.list, g.gen);
+        if (g.list) memcpy(o + g.gen, from + g.pend + g.dev, g.list);
     }
     return 0;
 }
 
 int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voice, const double *wavetables,
-                          const trm_cuda_pool_slot_state *st, const void *const *src, int32_t *slot_out)
+                          const trm_cuda_pool_slot_state *st, const trm_cuda_pool_event_state *ev, const void *const *src,
+                          int32_t *slot_out)
 {
     if (n < 0 || (n > 0 && (!voice || !wavetables || !st || !src || !slot_out)))
         return pool_err(-4, "trm_cuda_pool_restore: bad arguments");
     if (n == 0) return 0;
     // ---- everything is checked before the pool changes ----------------------------------------------------------------
     long long stride = p->stride, cap_out = p->cap_out;     // the sizes after this call's reservations
+    bool any_events = false;
     for (int i = 0; i < n; ++i) {
         int rc = trm_cuda_pool_check_state(&voice[i], &st[i]);
         if (rc != 0) return rc;
@@ -1972,6 +2060,14 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
         pool_sizes(p, &voice[i], &s, &c);
         stride = std::max(stride, s);
         cap_out = std::max(cap_out, c);
+        if (ev && ev[i].events) {
+            if (ev[i].n_events < 0 || st[i].frames_seen > ev[i].ev_frames)
+                return pool_err(-4, "trm_cuda_pool_restore: the event part does not agree with the counters");
+            // pool_push appends a push's frames to the pending row before it checks the row's capacity
+            if (st[i].pend_frames + p->max_m > pool_pend_rows(p))
+                return pool_err(-4, "trm_cuda_pool_restore: a snapshot's pending frames and this pool's next push do not fit its pending-frame rows");
+            any_events = true;
+        }
     }
     for (int i = 0; i < n; ++i) {
         // pool_push appends the pending frames before its capacity check: the next push of the restored slot, with as many
@@ -1992,11 +2088,23 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
     int rc;
     for (int i = 0; i < n; ++i)
         if ((rc = trm_cuda_pool_reserve(p, &voice[i])) != 0) return rc;
-    // ---- one upload ([segments][wavetables][entry 0's state and history] ...), one scatter -----------------------------
+    if (any_events) {
+        if ((rc = pool_event_storage(p)) != 0) return rc;
+        for (int i = 0; i < n; ++i)
+            if (ev[i].events && (rc = pool_event_list(p, free_slot[i], ev[i].n_events)) != 0) return rc;
+    }
+    // ---- one upload ([segments][wavetables][entry 0's SnapStage, generator with settings] ...), one scatter -----------
     const size_t sb = trm::tube_state_bytes(p->esz), wt = TRM_TABLE_LENGTH * sizeof(double);
+    const size_t gs = sizeof(trm::FrameGenPoolState);   // event-fed: the whole generator state, settings included
+    std::vector<SnapStage> sg((size_t)n);
     std::vector<size_t> at((size_t)n + 1, 0);
-    for (int i = 0; i < n; ++i) at[i + 1] = at[i] + pool_device_bytes(p, st[i]);
-    const size_t o_wt = align_up((size_t)3 * n * sizeof(trm::CopySeg), 256);
+    for (int i = 0; i < n; ++i) {
+        const trm_cuda_pool_event_state *e = ev ? &ev[i] : nullptr;
+        sg[i] = snap_stage(p, st[i], e);
+        if (e && e->events) sg[i].gen = gs;
+        at[i + 1] = at[i] + sg[i].bytes();
+    }
+    const size_t o_wt = align_up((size_t)6 * n * sizeof(trm::CopySeg), 256);
     const size_t o_dev = o_wt + (size_t)n * wt;
     const size_t bytes = o_dev + at[n];
     CK(cudaSetDevice(p->ctx->device));
@@ -2008,16 +2116,40 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
     memcpy(h + o_wt, wavetables, (size_t)n * wt);
     for (int i = 0; i < n; ++i) {
         const int s = free_slot[i];
+        const SnapStage &g = sg[i];
         seg[n_seg++] = {(unsigned long long)(uintptr_t)(d + o_wt + (size_t)i * wt),
                         (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH), wt};
-        memcpy(h + o_dev + at[i], (const unsigned char *)src[i] + (size_t)st[i].pend_frames * 128, at[i + 1] - at[i]);
+        // the data part: [pending frames][state][history] then, event-fed, [generator (frames_seen > 0)][list]
+        const unsigned char *in = (const unsigned char *)src[i] + (g.pend ? 0 : (size_t)st[i].pend_frames * 128);
+        unsigned char *stg = h + o_dev + at[i];
+        memcpy(stg, in, g.pend + g.dev);
         unsigned long long from = (unsigned long long)(uintptr_t)(d + o_dev + at[i]);
+        if (g.pend) {
+            seg[n_seg++] = {from, p->pend_addr(s, 0, 0), g.pend};
+            from += g.pend;
+        }
         if (!st[i].fresh) {
             seg[n_seg++] = {from, (unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), sb};
             from += sb;
         }
         const long long hist = st[i].s_done - st[i].in_start;
-        if (hist > 0) seg[n_seg++] = {from, p->tube_addr(p->tube_at(s, 0)), (unsigned long long)hist * p->esz};
+        if (hist > 0) {
+            seg[n_seg++] = {from, p->tube_addr(p->tube_at(s, 0)), (unsigned long long)hist * p->esz};
+            from += (unsigned long long)hist * p->esz;
+        }
+        if (!g.gen) continue;
+        const size_t gen_in = pool_gen_bytes(st[i]);
+        memcpy(stg + g.pend + g.dev, in + g.pend + g.dev + gen_in, g.list);
+        if (g.list) {
+            seg[n_seg++] = {from, (unsigned long long)(uintptr_t)p->d_events[s], g.list};
+            from += g.list;
+        }
+        // a slot with no frames yet sets its generator up on its first push: only the settings matter
+        trm::FrameGenPoolState gen{};
+        if (gen_in) memcpy(&gen, in + g.pend + g.dev, gen_in);
+        gen.fg = ev[i].fg;
+        memcpy(stg + g.pend + g.dev + g.list, &gen, gs);
+        seg[n_seg++] = {from, (unsigned long long)(uintptr_t)(p->d_gen + s), gs};
     }
     cudaStream_t cs = p->st;
     CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
@@ -2040,8 +2172,16 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
         sl.in_start = st[i].in_start;
         sl.pend_first = st[i].pend_first;
         sl.pend_frames = st[i].pend_frames;
-        sl.pending.resize((size_t)st[i].pend_frames * 16);
-        if (st[i].pend_frames) memcpy(sl.pending.data(), src[i], (size_t)st[i].pend_frames * 128);
+        if (ev && ev[i].events) {
+            sl.events = true;
+            sl.ev_count = ev[i].n_events;
+            sl.ev_frames = ev[i].ev_frames;
+            sl.fg = ev[i].fg;
+            sl.pcur = 0;
+        } else {
+            sl.pending.resize((size_t)st[i].pend_frames * 16);
+            if (st[i].pend_frames) memcpy(sl.pending.data(), src[i], (size_t)st[i].pend_frames * 128);
+        }
         slot_out[i] = s;
     }
     return 0;

@@ -1294,12 +1294,14 @@ void TRMStreamPoolFree(TRMStreamPool *t)
 #if defined(__BYTE_ORDER__) && __BYTE_ORDER__ != __ORDER_LITTLE_ENDIAN__
 #error "snapshot data parts are copied as they lie in memory: little-endian hosts only"
 #endif
-#define SNAP_VERSION   1u
+#define SNAP_VERSION   1u                 /* frame-fed slots */
+#define SNAP_VERSION_EVENTS 2u            /* event-fed slots: the event header, generator state and list follow */
 #define SNAP_HEADER    32                 /* magic, version, precision, total bytes, checksum */
 #define SNAP_VOICE     192
 #define SNAP_DERIVED   24
 #define SNAP_COUNTERS  48
 #define SNAP_FIXED     (SNAP_HEADER + SNAP_VOICE + SNAP_DERIVED + SNAP_COUNTERS)
+#define SNAP_EVHEADER  72                 /* n_events, list_frames, fg (48 bytes), generator flag, reserved */
 static const unsigned char snap_magic[8] = {'T', 'R', 'M', 'S', 'N', 'A', 'P', 0};
 
 static uint64_t fnv1a64(const unsigned char *p, size_t n)
@@ -1346,6 +1348,18 @@ static void get_voice(const unsigned char **q, TRMInputParameters *ip)
     ip->mixOffset = get_f64(q);
 }
 
+/* the event header of a version-2 snapshot (the generator flag is 1 exactly when frames were generated) */
+static unsigned char *put_event_header(unsigned char *o, const trm_cuda_pool_event_state *ev, int64_t frames_generated)
+{
+    o = put_u64(o, (uint64_t)ev->n_events); o = put_u64(o, (uint64_t)ev->ev_frames);
+    o = put_u32(o, (uint32_t)ev->fg.useMacroIntonation); o = put_u32(o, (uint32_t)ev->fg.useMicroIntonation);
+    o = put_u32(o, (uint32_t)ev->fg.useSmoothIntonation); o = put_u32(o, (uint32_t)ev->fg.useDrift);
+    o = put_f64(o, ev->fg.driftDeviation); o = put_f64(o, ev->fg.driftCutoff); o = put_f64(o, ev->fg.pitch);
+    o = put_f32(o, ev->fg.driftSeed); o = put_u32(o, 0u);   /* reserved */
+    o = put_u32(o, frames_generated > 0 ? 1u : 0u);
+    return put_u32(o, 0u);
+}
+
 /* the derived constants a snapshot stores, from the voice's descriptor */
 static void snap_derived(const trm_cuda_utterance *d, int precision, uint32_t out[6])
 {
@@ -1353,18 +1367,85 @@ static void snap_derived(const trm_cuda_utterance *d, int precision, uint32_t ou
     out[3] = (uint32_t)d->padSize; out[4] = (uint32_t)d->channels; out[5] = precision == TRM_PRECISION_FP32 ? 4u : 8u;
 }
 
-/* One snapshot, checked as far as it can be without a pool: on success *ip, *d (descriptor, n_frames = 2 as Open builds
- * it), the glottal table row in vs (row d->voice), the counters and a pointer to the data part. */
-static int snap_parse(const unsigned char *b, int64_t bytes, voice_set *vs, int *precision, TRMInputParameters *ip,
-                      trm_cuda_utterance *d, trm_cuda_pool_slot_state *st, const unsigned char **data)
+/* framegen_step's current event, clock and time of the current event after k frames of a list that expands to at least
+ * k (k >= 1): the walk of TRMEventListFrameCount stopped after k steps.  (framegen_step leaves `next` as it is once the
+ * last event is passed.) */
+static void framegen_position(const TRMEvent *ev, int64_t count, int64_t k, int64_t *i, uint64_t *now, uint64_t *next)
 {
+    int64_t j = 1;
+    uint64_t t = 0, nx = (uint64_t)ev[1].time;
+    while (k > 0) {
+        const uint64_t steps = nx > t ? (nx - t + 3) / 4 : 1;
+        if ((uint64_t)k < steps) { t += 4 * (uint64_t)k; break; }
+        t += 4 * steps;
+        k -= (int64_t)steps;
+        if (++j == count) break;
+        nx = (uint64_t)ev[j].time;
+    }
+    *i = j; *now = t; *next = nx;
+}
+
+/* A version-2 snapshot's event header at *q (moved past it), checked with the rest of the snapshot up to `end` against
+ * the counters: the length, the generator flag, the list as TRMStreamPoolOpenEvents checks it, its frame count and the
+ * generator's position.  The track values, deltas and drift state are not checked: they only ever reach the audio. */
+static int snap_parse_events(const unsigned char **q, const unsigned char *end, const trm_cuda_pool_slot_state *st,
+                             int precision, trm_cuda_pool_event_state *ev)
+{
+    const unsigned char *h = *q;
+    ev->events = 1;
+    ev->n_events = (int64_t)get_u64(&h); ev->ev_frames = (int64_t)get_u64(&h);
+    ev->fg.useMacroIntonation = (int32_t)get_u32(&h); ev->fg.useMicroIntonation = (int32_t)get_u32(&h);
+    ev->fg.useSmoothIntonation = (int32_t)get_u32(&h); ev->fg.useDrift = (int32_t)get_u32(&h);
+    ev->fg.driftDeviation = get_f64(&h); ev->fg.driftCutoff = get_f64(&h); ev->fg.pitch = get_f64(&h);
+    ev->fg.driftSeed = get_f32(&h); ev->fg.reserved = (int32_t)get_u32(&h);
+    const uint32_t generator = get_u32(&h), reserved = get_u32(&h);
+    if (ev->fg.reserved != 0 || reserved != 0) return set_err(TRM_ERR_PARAM, "snapshot: reserved event header fields are not 0%s", "");
+    if (generator != (st->frames_seen > 0 ? 1u : 0u))
+        return set_err(TRM_ERR_PARAM, "snapshot: the generator flag does not agree with the frames generated%s", "");
+    const int64_t fixed = trm_cuda_pool_slot_bytes(precision, st), gen = generator ? TRM_FRAMEGEN_STATE_BYTES : 0;
+    const int64_t list_bytes = (int64_t)(end - h) - fixed - gen;
+    if (ev->n_events < 0 || list_bytes < 0 || list_bytes % (int64_t)sizeof(TRMEvent) != 0 ||
+        list_bytes / (int64_t)sizeof(TRMEvent) != ev->n_events)
+        return set_err(TRM_ERR_PARAM, "snapshot: length does not match its counters and events%s", "");
+    if (ev->ev_frames < 0 || st->frames_seen > ev->ev_frames)
+        return set_err(TRM_ERR_PARAM, "snapshot: more frames generated than the event list has%s", "");
+    /* the list, aligned for reading (the blob may sit at any offset) */
+    TRMEvent *list = malloc((size_t)ev->n_events * sizeof *list + 1);
+    if (!list) return set_err(TRM_ERR_NOMEM, "out of memory%s", "");
+    memcpy(list, h + fixed + gen, (size_t)ev->n_events * sizeof *list);
+    int rc = check_event_list(list, ev->n_events, ev->ev_frames);
+    if (rc == TRM_OK && generator) {
+        const unsigned char *g = h + fixed + 552;          /* i, now, next after cv[32], cd[32] and tracks 32..35 */
+        const int64_t gi = (int64_t)get_u64(&g);
+        const uint64_t gnow = get_u64(&g), gnext = get_u64(&g);
+        int64_t wi;
+        uint64_t wnow, wnext;
+        framegen_position(list, ev->n_events, st->frames_seen, &wi, &wnow, &wnext);
+        if (gi != wi || gnow != wnow || gnext != wnext)
+            rc = set_err(TRM_ERR_PARAM, "snapshot: the generator's position does not agree with the frames generated%s", "");
+    }
+    free(list);
+    *q = h;
+    return rc;
+}
+
+/* One snapshot, checked as far as it can be without a pool: on success *ip, *d (descriptor, n_frames = 2 as Open builds
+ * it), the glottal table row in vs (row d->voice), the counters, the event part (ev->events = 0 for version 1) and a
+ * pointer to the data part. */
+static int snap_parse(const unsigned char *b, int64_t bytes, voice_set *vs, int *precision, TRMInputParameters *ip,
+                      trm_cuda_utterance *d, trm_cuda_pool_slot_state *st, trm_cuda_pool_event_state *ev,
+                      const unsigned char **data)
+{
+    memset(ev, 0, sizeof *ev);
     if (!b || bytes < SNAP_HEADER) return set_err(TRM_ERR_PARAM, "snapshot: shorter than its header%s", "");
     const unsigned char *q = b + 8;
     if (memcmp(b, snap_magic, 8) != 0) return set_err(TRM_ERR_PARAM, "snapshot: not a stream pool snapshot%s", "");
-    if (get_u32(&q) != SNAP_VERSION) return set_err(TRM_ERR_PARAM, "snapshot: unknown format version%s", "");
+    const uint32_t version = get_u32(&q);
+    if (version != SNAP_VERSION && version != SNAP_VERSION_EVENTS) return set_err(TRM_ERR_PARAM, "snapshot: unknown format version%s", "");
+    const int64_t fixed = SNAP_FIXED + (version == SNAP_VERSION_EVENTS ? SNAP_EVHEADER : 0);
     const uint32_t prec = get_u32(&q);
     const uint64_t total = get_u64(&q), sum = get_u64(&q);
-    if (total != (uint64_t)bytes || bytes < SNAP_FIXED) return set_err(TRM_ERR_PARAM, "snapshot: length does not match%s", "");
+    if (total != (uint64_t)bytes || bytes < fixed) return set_err(TRM_ERR_PARAM, "snapshot: length does not match%s", "");
     if (fnv1a64(b + SNAP_HEADER, (size_t)bytes - SNAP_HEADER) != sum) return set_err(TRM_ERR_PARAM, "snapshot: checksum mismatch%s", "");
     if (prec > 2u || !precision_ok((int)prec)) return set_err(TRM_ERR_PARAM, "snapshot: unknown precision%s", "");
     *precision = (int)prec;
@@ -1380,39 +1461,49 @@ static int snap_parse(const unsigned char *b, int64_t bytes, voice_set *vs, int 
     st->in_start = (int64_t)get_u64(&q); st->pend_first = (int64_t)get_u64(&q);
     st->pend_frames = (int32_t)get_u32(&q); st->fresh = (int32_t)get_u32(&q);
     if (trm_cuda_pool_check_state(d, st) != 0) return set_err(TRM_ERR_PARAM, "%s", trm_cuda_last_error());
-    if (bytes != SNAP_FIXED + trm_cuda_pool_slot_bytes(*precision, st))
+    if (version == SNAP_VERSION_EVENTS) {
+        if ((rc = snap_parse_events(&q, b + bytes, st, *precision, ev)) != TRM_OK) return rc;
+    } else if (bytes != SNAP_FIXED + trm_cuda_pool_slot_bytes(*precision, st)) {
         return set_err(TRM_ERR_PARAM, "snapshot: length does not match its counters%s", "");
+    }
     *data = q;
     return TRM_OK;
 }
 
-int TRMStreamPoolSave(TRMStreamPool *t, int n, const int32_t *slot, void *blob, int64_t blob_capacity, int64_t *offset)
+/* TRMStreamPoolSave (any_kind = 0: event slots refused) and TRMStreamPoolSaveAny (= 1: they are saved as version 2) */
+static int pool_save(TRMStreamPool *t, int n, const int32_t *slot, void *blob, int64_t blob_capacity, int64_t *offset,
+                     int any_kind)
 {
     if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
     if (n < 0 || !offset || (n > 0 && !slot)) return set_err(TRM_ERR_PARAM, "bad snapshot arguments%s", "");
     trm_cuda_pool_slot_state *st = calloc((size_t)n + 1, sizeof *st);
+    trm_cuda_pool_event_state *ev = any_kind ? calloc((size_t)n + 1, sizeof *ev) : NULL;
     void **dst = calloc((size_t)n + 1, sizeof *dst);
     voice_set vs;
     memset(&vs, 0, sizeof vs);
     int rc = TRM_OK;
-    if (!st || !dst) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
-    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, NULL)) != 0) { rc = pool_rc(rc); goto done; }   /* checks the slots */
+    if (!st || !dst || (any_kind && !ev)) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
+    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, ev, NULL)) != 0) { rc = pool_rc(rc); goto done; }   /* checks the slots */
     offset[0] = 0;
-    for (int i = 0; i < n; i++) offset[i + 1] = offset[i] + SNAP_FIXED + trm_cuda_pool_slot_bytes(t->precision, &st[i]);
+    for (int i = 0; i < n; i++) {
+        const int64_t head = SNAP_FIXED + (ev && ev[i].events ? SNAP_EVHEADER + trm_cuda_pool_event_bytes(&st[i], &ev[i]) : 0);
+        offset[i + 1] = offset[i] + head + trm_cuda_pool_slot_bytes(t->precision, &st[i]);
+    }
     if (!blob) goto done;
     if (blob_capacity < offset[n]) { rc = set_err(TRM_ERR_PARAM, "snapshot buffer too small%s", ""); goto done; }
     unsigned char *base = blob;
-    for (int i = 0; i < n; i++) dst[i] = base + offset[i] + SNAP_FIXED;
-    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, dst)) != 0) { rc = pool_rc(rc); goto done; }
+    for (int i = 0; i < n; i++) dst[i] = base + offset[i] + SNAP_FIXED + (ev && ev[i].events ? SNAP_EVHEADER : 0);
+    if ((rc = trm_cuda_pool_save(t->p, n, slot, st, ev, dst)) != 0) { rc = pool_rc(rc); goto done; }
     for (int i = 0; i < n; i++) {
         const TRMInputParameters *ip = &t->voice[slot[i]];
         trm_cuda_utterance d;
         if ((rc = describe(ip, 2, &vs, &d, NULL)) != TRM_OK) goto done;
         uint32_t dv[6];
         snap_derived(&d, t->precision, dv);
+        const int events = ev && ev[i].events;
         unsigned char *b = base + offset[i], *o = b;
         memcpy(o, snap_magic, 8);
-        o = put_u32(o + 8, SNAP_VERSION);
+        o = put_u32(o + 8, events ? SNAP_VERSION_EVENTS : SNAP_VERSION);
         o = put_u32(o, (uint32_t)t->precision);
         o = put_u64(o, (uint64_t)(offset[i + 1] - offset[i]));
         unsigned char *sum_at = o;
@@ -1422,13 +1513,25 @@ int TRMStreamPoolSave(TRMStreamPool *t, int n, const int32_t *slot, void *blob, 
         o = put_u64(o, (uint64_t)st[i].out_done); o = put_u64(o, (uint64_t)st[i].in_start);
         o = put_u64(o, (uint64_t)st[i].pend_first);
         o = put_u32(o, (uint32_t)st[i].pend_frames); o = put_u32(o, (uint32_t)st[i].fresh);
+        if (events) put_event_header(o, &ev[i], st[i].frames_seen);
         put_u64(sum_at, fnv1a64(b + SNAP_HEADER, (size_t)(offset[i + 1] - offset[i]) - SNAP_HEADER));
     }
 done:
     voice_set_free(&vs);
     free(st);
+    free(ev);
     free(dst);
     return rc;
+}
+
+int TRMStreamPoolSave(TRMStreamPool *t, int n, const int32_t *slot, void *blob, int64_t blob_capacity, int64_t *offset)
+{
+    return pool_save(t, n, slot, blob, blob_capacity, offset, 0);
+}
+
+int TRMStreamPoolSaveAny(TRMStreamPool *t, int n, const int32_t *slot, void *blob, int64_t blob_capacity, int64_t *offset)
+{
+    return pool_save(t, n, slot, blob, blob_capacity, offset, 1);
 }
 
 int TRMStreamPoolRestore(TRMStreamPool *t, int n, const void *blob, const int64_t *offset, int32_t *slot_out)
@@ -1437,6 +1540,7 @@ int TRMStreamPoolRestore(TRMStreamPool *t, int n, const void *blob, const int64_
     if (n < 0 || (n > 0 && (!blob || !offset || !slot_out))) return set_err(TRM_ERR_PARAM, "bad snapshot arguments%s", "");
     if (n == 0) return TRM_OK;
     trm_cuda_pool_slot_state *st = calloc((size_t)n, sizeof *st);
+    trm_cuda_pool_event_state *ev = calloc((size_t)n, sizeof *ev);
     trm_cuda_utterance *d = calloc((size_t)n, sizeof *d);
     TRMInputParameters *ip = calloc((size_t)n, sizeof *ip);
     double *tables = malloc((size_t)n * TRM_TABLE_LENGTH * sizeof *tables);
@@ -1444,13 +1548,13 @@ int TRMStreamPoolRestore(TRMStreamPool *t, int n, const void *blob, const int64_
     voice_set vs;
     memset(&vs, 0, sizeof vs);
     int rc = TRM_OK;
-    if (!st || !d || !ip || !tables || !src) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
+    if (!st || !ev || !d || !ip || !tables || !src) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
     for (int i = 0; i < n; i++) {
         if (offset[i] < 0 || offset[i + 1] < offset[i]) { rc = set_err(TRM_ERR_PARAM, "snapshot offsets are not ascending%s", ""); goto done; }
         int prec;
         const unsigned char *data;
         if ((rc = snap_parse((const unsigned char *)blob + offset[i], offset[i + 1] - offset[i], &vs, &prec, &ip[i], &d[i], &st[i],
-                             &data)) != TRM_OK)
+                             &ev[i], &data)) != TRM_OK)
             goto done;
         if (prec != t->precision) { rc = set_err(TRM_ERR_PARAM, "snapshot of another precision%s", ""); goto done; }
         src[i] = data;
@@ -1458,26 +1562,35 @@ int TRMStreamPoolRestore(TRMStreamPool *t, int n, const void *blob, const int64_
     /* the table rows are final only now (vs may have grown while parsing) */
     for (int i = 0; i < n; i++)
         memcpy(tables + (size_t)i * TRM_TABLE_LENGTH, vs.tables + (size_t)d[i].voice * TRM_TABLE_LENGTH, TRM_TABLE_LENGTH * sizeof *tables);
-    if ((rc = trm_cuda_pool_restore(t->p, n, d, tables, st, (const void *const *)src, slot_out)) != 0) { rc = pool_rc(rc); goto done; }
+    if ((rc = trm_cuda_pool_restore(t->p, n, d, tables, st, ev, (const void *const *)src, slot_out)) != 0) { rc = pool_rc(rc); goto done; }
     for (int i = 0; i < n; i++) t->voice[slot_out[i]] = ip[i];
 done:
     voice_set_free(&vs);
-    free(st); free(d); free(ip); free(tables); free(src);
+    free(st); free(ev); free(d); free(ip); free(tables); free(src);
+    return rc;
+}
+
+/* a snapshot parsed as Restore parses it, no pool needed */
+static int snap_read(const void *blob, int64_t bytes, int *prec, TRMInputParameters *ip, trm_cuda_utterance *d,
+                     trm_cuda_pool_slot_state *st, trm_cuda_pool_event_state *ev)
+{
+    voice_set vs;
+    memset(&vs, 0, sizeof vs);
+    const unsigned char *data;
+    const int rc = snap_parse(blob, bytes, &vs, prec, ip, d, st, ev, &data);
+    voice_set_free(&vs);
     return rc;
 }
 
 int TRMStreamPoolSnapshotInfo(const void *blob, int64_t bytes, TRMStreamSnapshotInfo *info)
 {
     if (!blob || !info) return set_err(TRM_ERR_PARAM, "null snapshot or info%s", "");
-    voice_set vs;
-    memset(&vs, 0, sizeof vs);
     int prec;
     TRMInputParameters ip;
     trm_cuda_utterance d;
     trm_cuda_pool_slot_state st;
-    const unsigned char *data;
-    const int rc = snap_parse(blob, bytes, &vs, &prec, &ip, &d, &st, &data);
-    voice_set_free(&vs);
+    trm_cuda_pool_event_state ev;
+    const int rc = snap_read(blob, bytes, &prec, &ip, &d, &st, &ev);
     if (rc != TRM_OK) return rc;
     memset(info, 0, sizeof *info);
     info->precision = prec;
@@ -1486,6 +1599,26 @@ int TRMStreamPoolSnapshotInfo(const void *blob, int64_t bytes, TRMStreamSnapshot
     info->frames_pushed = st.frames_seen;
     info->samples_returned = st.out_done;
     info->bytes = bytes;
+    return TRM_OK;
+}
+
+int TRMStreamPoolSnapshotEventInfo(const void *blob, int64_t bytes, TRMStreamSnapshotEventInfo *info)
+{
+    if (!blob || !info) return set_err(TRM_ERR_PARAM, "null snapshot or info%s", "");
+    int prec;
+    TRMInputParameters ip;
+    trm_cuda_utterance d;
+    trm_cuda_pool_slot_state st;
+    trm_cuda_pool_event_state ev;
+    const int rc = snap_read(blob, bytes, &prec, &ip, &d, &st, &ev);
+    if (rc != TRM_OK) return rc;
+    memset(info, 0, sizeof *info);
+    if (!ev.events) return TRM_OK;
+    info->from_events = 1;
+    info->n_events = ev.n_events;
+    info->list_frames = ev.ev_frames;
+    info->frames_generated = st.frames_seen;
+    memcpy(&info->fg, &ev.fg, sizeof info->fg);
     return TRM_OK;
 }
 

@@ -346,7 +346,7 @@ int TRMStreamPoolOpen(TRMStreamPool *pool, const TRMInputParameters *voice);
  *   Early end.  A flush before the end of the list ends the slot as a frame-fed flush does: its output equals the
  *     one-shot synthesis of the k frames generated so far (the first k of TRMBatchGenerateFrames' frames for the list).
  *   Close and flush free the slot as for any slot; it may be reopened either way.  TRMStreamPoolSave refuses event slots
- *     (TRM_ERR_STATE). */
+ *     (TRM_ERR_STATE); TRMStreamPoolSaveAny saves them (format version 2, below). */
 int TRMStreamPoolOpenEvents(TRMStreamPool *pool, const TRMInputParameters *voice, const TRMEvent *events,
                             int64_t n_events, const TRMFrameGeneration *fg, int64_t *n_frames_out);
 /* Abandons an open slot without its tail (client went away); the slot becomes free. */
@@ -401,7 +401,28 @@ void TRMStreamPoolFree(TRMStreamPool *pool);
  *             kept tube-rate history [synthesized - first kept] of the precision's element type
  * Restore derives the glottal table and every derived constant again from the voice, as TRMStreamPoolOpen does, and checks
  * the counters against each other and the voice: a corrupt snapshot can give wrong audio but never an access outside
- * the slot's own buffers. */
+ * the slot's own buffers.
+ *
+ * Event slots (TRMStreamPoolOpenEvents) are saved by TRMStreamPoolSaveAny as format version 2, which carries the event list
+ * and the frame generator's state with the stream.  A restored version-2 slot is an event slot: pushes give it frame
+ * counts, it may flush early and it may be saved again.  Its continuation contract is the event slot's: advanced to the
+ * end of its list and flushed, its outputs, appended to what the saved slot returned before the save, equal
+ * TRMBatchSynthesizeEvents for that voice, list and fg bit for bit (samples; PCM16 and per-push maxima at the utterance's
+ * peak); flushed earlier, they equal the one-shot synthesis of the frames generated so far.  Saving does not change the
+ * slot, migration and fork both work, and save(restore(b)) == b.
+ * Format version 2: header (version 2), voice, derived and counters as version 1 (frames pushed = frames generated), then
+ *   events    (at byte 296, 72 bytes) i64 n_events, list_frames (TRMEventListFrameCount of the list); fg field by field:
+ *             i32 useMacroIntonation, useMicroIntonation, useSmoothIntonation, useDrift, f64 driftDeviation, driftCutoff,
+ *             pitch, f32 driftSeed, i32 reserved (0); u32 generator (1 exactly when frames generated > 0), u32 reserved (0)
+ *   data      the version-1 data part (the pending frames are the generated ones the slot still needs); then, if generator
+ *             is 1, the generator state: f64 cv[32], cd[32], cv32, cd32, cd33, cd34, cd35; i64 i; u64 now, next; f32 seed,
+ *             prev, pitchDeviation, pitchOffset, a0, b1 (600 bytes); then the whole list, n_events x (i64 time, 36 f64)
+ * Restore checks a version-2 snapshot as a version-1 one and further: the length against n_events and generator, the list
+ * as TRMStreamPoolOpenEvents checks it, list_frames against the list, frames generated <= list_frames, the generator flag,
+ * the generator's event index and clock (i, now, next) against the frames generated, and that the pending frames plus a
+ * push of max_frames_per_push fit the destination's pending-frame rows (TRM_ERR_PARAM).  The tracks' values and deltas and
+ * the drift state are not checked: they can give wrong audio, never an access outside the slot (only i and n_events index
+ * the list, and the checks pin i to [1, n_events]). */
 typedef struct TRMStreamSnapshotInfo {
     int32_t precision;               /* TRM_PRECISION_* the snapshot restores into                                 */
     int32_t channels;                /* int16 elements per PCM frame of the stream                                  */
@@ -413,19 +434,36 @@ typedef struct TRMStreamSnapshotInfo {
 /* Snapshots of n distinct open slots, packed: slot[i]'s bytes are blob[offset[i] .. offset[i+1]).  blob == NULL: only
  * fills offset (sizes from host bookkeeping, no device work).  Refused before anything is written: an unopened slot or a
  * slot opened with TRMStreamPoolOpenEvents (TRM_ERR_STATE), a slot named twice or blob_capacity < offset[n]
- * (TRM_ERR_PARAM). */
+ * (TRM_ERR_PARAM).  Writes version 1 only, so a caller that stores snapshots for a version-1 reader never gets another. */
 int TRMStreamPoolSave(TRMStreamPool *pool, int n, const int32_t *slot, void *blob, int64_t blob_capacity,
                       int64_t *offset /* [n + 1] */);
-/* Opens n free slots from n snapshots (the same packing); slot_out[i] is the slot that continues snapshot i.  All n are
- * checked before anything changes, and a refused call leaves the pool as it was: bad magic, version, length or checksum,
- * another precision, derived constants that differ from the voice's (e.g. a snapshot from another library build), or
- * counters that disagree (TRM_ERR_PARAM); a voice TRMBatchCreate refuses (its code); kept history and pending frames
- * that would not fit this pool's next push of max_frames_per_push frames (TRM_ERR_PARAM); fewer than n free slots
- * (TRM_ERR_STATE).  SlotCapacity may grow, as with Open. */
+/* TRMStreamPoolSave for slots of either kind: an event slot is saved as version 2 instead of being refused; a frame-fed
+ * slot's snapshot is byte for byte what TRMStreamPoolSave writes.  One call may mix both kinds (draining a GPU is one
+ * save).  Arguments, packing, blob == NULL sizing and the other refusals are TRMStreamPoolSave's. */
+int TRMStreamPoolSaveAny(TRMStreamPool *pool, int n, const int32_t *slot, void *blob, int64_t blob_capacity,
+                         int64_t *offset /* [n + 1] */);
+/* Opens n free slots from n snapshots of version 1 or 2 (the same packing); slot_out[i] is the slot that continues
+ * snapshot i.  All n are checked before anything changes, and a refused call leaves the pool as it was: bad magic,
+ * version, length or checksum, another precision, derived constants that differ from the voice's (e.g. a snapshot from
+ * another library build), counters that disagree, or a version-2 event part that fails its checks (TRM_ERR_PARAM); a
+ * voice TRMBatchCreate refuses (its code); kept history and pending frames that would not fit this pool's next push of
+ * max_frames_per_push frames (TRM_ERR_PARAM); fewer than n free slots (TRM_ERR_STATE).  SlotCapacity may grow, as with
+ * Open. */
 int TRMStreamPoolRestore(TRMStreamPool *pool, int n, const void *blob, const int64_t *offset /* [n + 1] */, int32_t *slot_out);
 /* Host only (no device needed): validates one snapshot as Restore does, apart from the destination pool, and reports
  * what it holds.  Lets a router pick a pool before restoring. */
 int TRMStreamPoolSnapshotInfo(const void *blob, int64_t bytes, TRMStreamSnapshotInfo *info);
+/* What a version-2 snapshot holds about its event list.  A router schedules a restored event slot's pushes with
+ * list_frames - frames_generated: a push past the end of the list is refused. */
+typedef struct TRMStreamSnapshotEventInfo {
+    int32_t from_events;             /* 1 for version 2 (an event slot); 0 for version 1, every other field 0           */
+    int64_t n_events;                /* events of the list                                                          */
+    int64_t list_frames;             /* TRMEventListFrameCount of the list                                          */
+    int64_t frames_generated;        /* frames generated (and pushed) so far                                        */
+    TRMFrameGeneration fg;
+} TRMStreamSnapshotEventInfo;
+/* Host only: checks the snapshot as TRMStreamPoolSnapshotInfo does and reports its event part. */
+int TRMStreamPoolSnapshotEventInfo(const void *blob, int64_t bytes, TRMStreamSnapshotEventInfo *info);
 
 /* ---------------------------------------------------------------------------------------------
  * Sweeps (BASELINE configs[4]: 10^6 synthetic 2 s utterances): n utterances of one voice whose control tracks are the walk2

@@ -231,15 +231,34 @@ int  trm_cuda_pool_check_state(const trm_cuda_utterance *voice, const trm_cuda_p
 /* Bytes of a slot's data part: pend_frames x 16 doubles, the carried state unless fresh (trm::tube_state_bytes), then the
  * kept history s_done - in_start elements of the precision's type. */
 int64_t trm_cuda_pool_slot_bytes(int precision, const trm_cuda_pool_slot_state *st);
+/* What an event-fed slot (trm_cuda_pool_open_events) carries besides the counters.  Its data part is the frame-fed one
+ * (its pending frames come from the slot's device row) followed by the generator state after frames_seen frames --
+ * TRM_FRAMEGEN_STATE_BYTES, only when frames_seen > 0: f64 cv[32], cd[32], cv32, cd32, cd33, cd34, cd35; i64 i;
+ * u64 now, next; f32 seed, prev, pitchDeviation, pitchOffset, a0, b1 -- then the whole list, n_events trm_cuda_event. */
+#define TRM_FRAMEGEN_STATE_BYTES 600
+typedef struct trm_cuda_pool_event_state {
+    int32_t events;             /* 1: the slot is event-fed; 0: frame-fed, every other field 0 */
+    int32_t reserved;
+    int64_t n_events;           /* events of its list */
+    int64_t ev_frames;          /* frames the list expands to (TRMEventListFrameCount) */
+    trm_cuda_framegen fg;
+} trm_cuda_pool_event_state;
+/* Bytes of the event part that follows trm_cuda_pool_slot_bytes in an event-fed slot's data part (0 for frame-fed). */
+int64_t trm_cuda_pool_event_bytes(const trm_cuda_pool_slot_state *st, const trm_cuda_pool_event_state *ev);
 /* st[i] receives the counters of n distinct open slots; with dst (may be NULL: counters only, no device work), dst[i]
- * receives slot[i]'s data part (trm_cuda_pool_slot_bytes).  The slots are not changed.  -7: a slot is not open, or was
- * opened with trm_cuda_pool_open_events. */
-int  trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st, void *const *dst);
+ * receives slot[i]'s data part (trm_cuda_pool_slot_bytes, plus trm_cuda_pool_event_bytes for an event-fed slot).  The
+ * slots are not changed.  ev == NULL: a slot opened with trm_cuda_pool_open_events is refused (-7); otherwise ev[i]
+ * describes slot[i].  -7: a slot is not open. */
+int  trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_pool_slot_state *st,
+                        trm_cuda_pool_event_state *ev, void *const *dst);
 /* Opens n free slots continuing n saved ones: voice[i] (voice.voice ignored) with its glottal table wavetables[i][512],
- * counters st[i] and data part src[i].  Refused before any change: counters that fail trm_cuda_pool_check_state or whose
- * next full push would not fit this pool's rows (-4), fewer than n free slots (-7).  slot_out[i] is entry i's slot. */
+ * counters st[i], event part ev[i] (ev may be NULL: all frame-fed) and data part src[i].  libtrm has checked an event
+ * part's list and generator position against the counters.  Refused before any change: counters that fail
+ * trm_cuda_pool_check_state or whose next full push would not fit this pool's rows or pending-frame rows (-4), fewer
+ * than n free slots (-7).  Every allocation precedes the first slot opened.  slot_out[i] is entry i's slot. */
 int  trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voice, const double *wavetables,
-                           const trm_cuda_pool_slot_state *st, const void *const *src, int32_t *slot_out);
+                           const trm_cuda_pool_slot_state *st, const trm_cuda_pool_event_state *ev, const void *const *src,
+                           int32_t *slot_out);
 void trm_cuda_pool_destroy(trm_cuda_pool *p);
 /*
  * Control frames on the device (replaces -[EventList generateOutputInTimeRange:...], EventList.m:883-1061): uploads
