@@ -191,7 +191,7 @@ struct ChunkPlan {
     struct Group { int u_begin, u_end; long long item_begin, item_end, max_n_out, pcm_lo, pcm_hi; };
     // Time split: when every utterance of the chunk has the same number of frames, the waveguide runs as two launches
     // (tube samples before / from control frame `split_frame`, recurrence state carried in `state` exactly as
-    // trm_cuda_stream_push does), so that the upload of the later frames overlaps the first launch.  0 = one launch.
+    // a stream pool push does), so that the upload of the later frames overlaps the first launch.  0 = one launch.
     int split_frame = 0, uniform_frames = 0;
     std::vector<trm_cuda_utterance> desc_t[2];
     std::vector<Group> groups;
@@ -415,7 +415,7 @@ int plan_chunk(const trm_cuda_utterance *desc, int u0, int u1, const trm::Kernel
 
 // Arms the time split of a planned chunk: launch 0 covers the tube samples before control frame f1 (rounded down to a
 // whole 16-sample block per utterance), launch 1 the rest, continuing from the saved state in the middle of a control
-// interval (jc0) exactly like a streaming push.
+// interval (jc0) exactly like a stream pool push.
 void arm_time_split(ChunkPlan &p, int f1)
 {
     const size_t n = p.desc.size();
@@ -1072,33 +1072,9 @@ int trm_cuda_generate_frames(trm_cuda_ctx *ctx, int n, const trm_cuda_utterance 
 }
 
 /* ------------------------------------------------------------------------------------------------------------
- * streaming
+ * stream pool: slots at independent positions, each with its own voice (TRMStream is its lockstep use: n slots of one
+ * voice, advanced by the same frames, flushed together)
  * ---------------------------------------------------------------------------------------------------------- */
-struct trm_cuda_stream {
-    trm_cuda_ctx *ctx = nullptr;
-    int precision = 0, n = 0, max_m = 0;
-    size_t esz = 8;
-    trm_cuda_utterance voice{};
-    int cp = 0;
-    long long frames_seen = 0;     // control frames pushed so far (per stream)
-    long long s_done = 0;          // tube-rate samples produced so far (multiple of 16 until the flush)
-    long long out_done = 0;        // output-rate samples returned so far
-    long long in_start = 0;        // first tube-rate sample still in the device buffer (multiple of 4)
-    bool flushed = false;
-    std::vector<double> pending;   // [stream][pend_frames][16]: frames from the control interval in progress on
-    long long pend_first = 0;      // index of the first pending frame
-    int pend_frames = 0;
-    long long cap_tube = 0, cap_out = 0;     // elements per stream
-    unsigned char *d_tube[2] = {nullptr, nullptr};
-    int cur = 0;
-    unsigned char *d_out = nullptr, *d_state = nullptr;
-    double *d_frames = nullptr;
-    double *d_wavetables = nullptr;    // own copy: the stream does not hold a context lane between pushes
-    Arena scratch;                 // descriptors + resampler plan of a push
-    HostStage stage;
-    cudaStream_t st = nullptr;
-};
-
 static long long src_safe_outputs(long long n_in, unsigned tri)
 {
     // outputs whose right filter wing lies inside the first n_in input samples: P(n) = (n*tri)>>16 <= n_in-1
@@ -1106,239 +1082,16 @@ static long long src_safe_outputs(long long n_in, unsigned tri)
     return (long long)(((unsigned long long)n_in * 65536ull + tri - 1) / tri);
 }
 
-int trm_cuda_stream_create(trm_cuda_ctx *ctx, int precision, int n_streams, const trm_cuda_utterance *voice,
-                           int max_frames_per_push, trm_cuda_stream **out)
-{
-    *out = nullptr;
-    if (n_streams <= 0 || max_frames_per_push <= 0) return fail_msg("trm_cuda_stream_create: bad sizes");
-    CK(cudaSetDevice(ctx->device));
-    trm_cuda_stream *s = new trm_cuda_stream();
-    s->ctx = ctx; s->precision = precision; s->n = n_streams; s->max_m = max_frames_per_push;
-    if (precision < 0 || precision > 2) return fail_msg("unknown precision code");
-    s->esz = prec_esz(precision);
-    s->voice = *voice;
-    s->cp = voice->controlPeriod;
-    const long long max_new = (long long)(max_frames_per_push + 1) * s->cp + 32;
-    s->cap_tube = (long long)align_up((size_t)(max_new + 128), 32);
-    s->cap_out = (long long)align_up((size_t)(src_safe_outputs(max_new + 64, voice->tri) + 64), 32);
-    const size_t st_bytes = trm::tube_state_bytes(s->esz);
-    cudaError_t e = cudaSuccess;
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = cudaMalloc((void **)&s->d_tube[k], (size_t)n_streams * s->cap_tube * s->esz);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&s->d_out, (size_t)n_streams * s->cap_out * s->esz);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&s->d_state, (size_t)n_streams * st_bytes);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&s->d_frames, (size_t)n_streams * (max_frames_per_push + 3) * 128);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->st, cudaStreamNonBlocking);
-    if (e == cudaSuccess && !ctx->wt_host.empty()) {
-        e = cudaMalloc((void **)&s->d_wavetables, ctx->wt_host.size() * sizeof(double));
-        if (e == cudaSuccess) e = cudaMemcpy(s->d_wavetables, ctx->wt_host.data(), ctx->wt_host.size() * sizeof(double), cudaMemcpyHostToDevice);
-    }
-    if (e == cudaSuccess) {
-        // fresh state: everything zero, "no sample yet" flag set, noise generator at its start
-        std::vector<unsigned char> init((size_t)n_streams * st_bytes, 0);
-        for (int u = 0; u < n_streams; ++u) {
-            unsigned long long *h = (unsigned long long *)(init.data() + (size_t)u * st_bytes);
-            h[2] = ctx->noise_k0;
-            h[3] = 1ull;
-        }
-        e = cudaMemcpy(s->d_state, init.data(), init.size(), cudaMemcpyHostToDevice);
-    }
-    if (e != cudaSuccess) { trm_cuda_stream_destroy(s); return fail("trm_cuda_stream_create", e); }
-    *out = s;
-    return 0;
-}
-
-int64_t trm_cuda_stream_capacity(const trm_cuda_stream *s) { return s->cap_out; }
-
-void trm_cuda_stream_destroy(trm_cuda_stream *s)
-{
-    if (!s) return;
-    cudaSetDevice(s->ctx->device);
-    if (s->st) { cudaStreamSynchronize(s->st); cudaStreamDestroy(s->st); }
-    for (auto &p : s->d_tube) if (p) cudaFree(p);
-    if (s->d_out) cudaFree(s->d_out);
-    if (s->d_state) cudaFree(s->d_state);
-    if (s->d_frames) cudaFree(s->d_frames);
-    if (s->d_wavetables) cudaFree(s->d_wavetables);
-    s->scratch.release();
-    s->stage.release();
-    delete s;
-}
-
-int trm_cuda_stream_push(trm_cuda_stream *s, const double *frames_host, int m, int flush, void *samples_host, int64_t *n_samples)
-{
-    if (n_samples) *n_samples = 0;
-    if (s->flushed) return fail_msg("trm_cuda_stream_push: the streams were flushed");
-    if (m < 0 || m > s->max_m) return fail_msg("trm_cuda_stream_push: more frames than the stream was created for");
-    trm_cuda_ctx *ctx = s->ctx;
-    CK(cudaSetDevice(ctx->device));
-    const int n = s->n, cp = s->cp;
-    // ---- frames: keep everything from the control interval in progress on ------------------------------------
-    {
-        const int keep = s->pend_frames;
-        std::vector<double> next((size_t)n * (keep + m) * 16);
-        for (int u = 0; u < n; ++u) {
-            if (keep) memcpy(&next[(size_t)u * (keep + m) * 16], &s->pending[(size_t)u * keep * 16], (size_t)keep * 128);
-            if (m) memcpy(&next[((size_t)u * (keep + m) + keep) * 16], frames_host + (size_t)u * m * 16, (size_t)m * 128);
-        }
-        s->pending.swap(next);
-        s->pend_frames = keep + m;
-        s->frames_seen += m;
-    }
-    const long long avail = s->frames_seen >= 2 ? (s->frames_seen - 1) * cp : 0;      // tube samples the frames define
-    const long long target = flush ? avail : avail / trm::TB * trm::TB;               // whole blocks until the end
-    const long long n_new = target - s->s_done;
-    const unsigned tri = s->voice.tri;
-    const int pad = s->voice.padSize;
-    const long long out_total = flush ? (long long)(((unsigned long long)(target + 2 * pad) * 65536ull + tri - 1) / tri)
-                                      : src_safe_outputs(target, tri);
-    if (flush && s->frames_seen < 1) { s->flushed = true; return 0; }
-    if (n_new <= 0 && !(flush && out_total > s->out_done)) { if (flush) s->flushed = true; return 0; }
-    cudaStream_t st = s->st;
-    const bool f64 = prec_is_f64(s->precision);
-    const KernelSet &K = g_kernels[s->precision];
-    const trm::KernelInfo &ki = ctx->ki(s->precision);
-    // ---- waveguide: samples [s_done, target) -----------------------------------------------------------------
-    const long long f0 = s->s_done / cp;                          // control interval the call starts in
-    const int jc0 = (int)(s->s_done % cp);
-    const int skip = (int)(f0 - s->pend_first);                   // pending frames before it are no longer needed
-    const int nf_call = s->pend_frames - skip;
-    std::vector<trm_cuda_utterance> dt(n), ds(n);
-    for (int u = 0; u < n; ++u) {
-        trm_cuda_utterance d = s->voice;
-        d.frame_offset = (long long)u * nf_call;
-        d.n_frames = nf_call;
-        d.n_tube = n_new > 0 ? n_new : 0;
-        d.tube_offset = (long long)u * s->cap_tube + (s->s_done - s->in_start);
-        d.jc0 = jc0;
-        d.out_start = 0; d.in_start = 0;
-        dt[u] = d;
-        trm_cuda_utterance r = s->voice;                          // resampler view: global sample indices
-        r.n_tube = target;
-        r.tube_offset = (long long)u * s->cap_tube - s->in_start;
-        r.n_out = out_total;
-        r.out_start = s->out_done;
-        r.in_start = s->in_start;
-        r.out_offset = (long long)u * s->cap_out - (s->out_done / 4 * 4);
-        r.pcm_offset = 0;
-        ds[u] = r;
-    }
-    if (target - s->in_start > s->cap_tube || out_total - s->out_done / 4 * 4 > s->cap_out) return fail_msg("trm_cuda_stream_push: internal capacity");
-    ChunkPlan plan;
-    if (plan_chunk(ds.data(), 0, n, ki, plan) != 0) return -1;
-    // plan_chunk rebases offsets to the chunk's span: streaming keeps its own (virtual) offsets
-    for (int u = 0; u < n; ++u) { plan.desc[u].tube_offset = ds[u].tube_offset; plan.desc[u].out_offset = ds[u].out_offset; plan.desc[u].frame_offset = 0; }
-    size_t bytes = plan.stage_bytes() + align_up((size_t)n * sizeof(trm_cuda_utterance), 256) + 1024;
-    int rc;
-    if ((rc = s->scratch.reserve(bytes + 4096)) != 0) return rc;
-    if ((rc = s->stage.reserve(bytes + (size_t)n * nf_call * 128 + 4096)) != 0) return rc;
-    s->scratch.reset();
-    DeviceChunk dc;
-    dc.n = n;
-    dc.desc = (trm_cuda_utterance *)s->scratch.take((size_t)n * sizeof(trm_cuda_utterance));
-    dc.order = nullptr;
-    dc.tile_utt = (int *)s->scratch.take(plan.tile_utt.size() * sizeof(int));
-    dc.tile_nt = (int *)s->scratch.take(plan.tile_nt.size() * sizeof(int));
-    dc.tile_max_out = (long long *)s->scratch.take(plan.tile_max_out.size() * sizeof(long long));
-    dc.tile_first_out = (long long *)s->scratch.take(plan.tile_first_out.size() * sizeof(long long));
-    dc.item_base = (long long *)s->scratch.take(plan.item_base.size() * sizeof(long long));
-    dc.maxbits = (unsigned long long *)s->scratch.take((size_t)n * sizeof(unsigned long long));
-    auto *d_dt = (trm_cuda_utterance *)s->scratch.take((size_t)n * sizeof(trm_cuda_utterance));
-    dc.total_items = plan.total_items; dc.n_tiles = (int)plan.n_tiles(); dc.max_n_out = plan.max_n_out; dc.src_shape = plan.src_shape;
-    {
-        unsigned char *q = s->stage.base;
-        auto put = [&](void *dst, const void *src, size_t b) -> int {
-            if (!b) return 0;
-            memcpy(q, src, b);
-            CK(cudaMemcpyAsync(dst, q, b, cudaMemcpyHostToDevice, st));
-            q += align_up(b, 256);
-            return 0;
-        };
-        if ((rc = put(dc.desc, plan.desc.data(), (size_t)n * sizeof(trm_cuda_utterance))) != 0) return rc;
-        if ((rc = put(dc.tile_utt, plan.tile_utt.data(), plan.tile_utt.size() * sizeof(int))) != 0) return rc;
-        if ((rc = put(dc.tile_nt, plan.tile_nt.data(), plan.tile_nt.size() * sizeof(int))) != 0) return rc;
-        if ((rc = put(dc.tile_max_out, plan.tile_max_out.data(), plan.tile_max_out.size() * sizeof(long long))) != 0) return rc;
-        if ((rc = put(dc.tile_first_out, plan.tile_first_out.data(), plan.tile_first_out.size() * sizeof(long long))) != 0) return rc;
-        if ((rc = put(dc.item_base, plan.item_base.data(), plan.item_base.size() * sizeof(long long))) != 0) return rc;
-        if ((rc = put(d_dt, dt.data(), (size_t)n * sizeof(trm_cuda_utterance))) != 0) return rc;
-        if (n_new > 0) {
-            // frames of this call: pending[skip ..) of every stream, back to back
-            double *fq = (double *)q;
-            for (int u = 0; u < n; ++u)
-                memcpy(fq + (size_t)u * nf_call * 16, &s->pending[((size_t)u * s->pend_frames + skip) * 16], (size_t)nf_call * 128);
-            CK(cudaMemcpyAsync(s->d_frames, fq, (size_t)n * nf_call * 128, cudaMemcpyHostToDevice, st));
-        }
-    }
-    if (n_new > 0) {
-        trm::TubeArgs a{};
-        a.state = s->d_state; a.desc = d_dt; a.order = nullptr; a.n_utt = n; a.frames = s->d_frames; a.tube = s->d_tube[s->cur];
-        a.wavetables = s->d_wavetables ? s->d_wavetables : ctx->d_wavetables; a.noise_k0 = ctx->noise_k0;
-        const int gmax = ki.wide_max_utt;
-        const int groups = std::max(1, std::min(ctx->sm_count, (n + 1) / 2));
-        const int g2 = (n + groups - 1) / groups > gmax ? (n + gmax - 1) / gmax : groups;
-        rc = K.tube_wide(&a, g2, st);
-        if (rc != 0) return fail("stream waveguide launch", (cudaError_t)rc);
-    }
-    // ---- resampler: outputs [out_done, out_total) ------------------------------------------------------------
-    const long long n_ret = out_total - s->out_done;
-    if (n_ret > 0) {
-        trm::SrcArgs a{};
-        a.desc = dc.desc; a.n_utt = n; a.tube = s->d_tube[s->cur]; a.out = s->d_out; a.maxbits = dc.maxbits;
-        a.table = f64 ? ctx->d_tab_f64 : ctx->d_tab_f32;
-        a.ctab = f64 ? ctx->d_ctab_f64 : ctx->d_ctab_f32;
-        a.tile_utt = dc.tile_utt; a.tile_nt = dc.tile_nt; a.tile_max_out = dc.tile_max_out; a.tile_first_out = dc.tile_first_out;
-        a.item_base = dc.item_base; a.n_tiles = dc.n_tiles; a.total_items = dc.total_items;
-        const int grid = ctx->sm_count * std::max(1, ki.src[dc.src_shape].ctas_per_sm);
-        rc = K.src(&a, grid, dc.src_shape, st);
-        if (rc != 0) return fail("stream resampler launch", (cudaError_t)rc);
-        if (samples_host)
-            CK(cudaMemcpy2DAsync(samples_host, (size_t)s->cap_out * s->esz, s->d_out + (size_t)(s->out_done % 4) * s->esz,
-                                 (size_t)s->cap_out * s->esz, (size_t)n_ret * s->esz, (size_t)n, cudaMemcpyDeviceToHost, st));
-    }
-    // ---- keep what the next call's filter wings reach back to: x[P(next) - 2*pad - 1 ..] -----------------------
-    long long next_in = flush ? target : (long long)(((unsigned long long)out_total * tri) >> 16) - 2 * pad - 4;
-    if (next_in < 0) next_in = 0;
-    next_in = next_in / 4 * 4;
-    if (next_in < s->in_start) next_in = s->in_start;
-    if (!flush) {
-        const long long keep = target - next_in;
-        CK(cudaMemcpy2DAsync(s->d_tube[s->cur ^ 1], (size_t)s->cap_tube * s->esz,
-                             s->d_tube[s->cur] + (size_t)(next_in - s->in_start) * s->esz, (size_t)s->cap_tube * s->esz,
-                             (size_t)keep * s->esz, (size_t)n, cudaMemcpyDeviceToDevice, st));
-        s->cur ^= 1;
-    }
-    CK(cudaStreamSynchronize(st));
-    s->in_start = next_in;
-    s->s_done = target;
-    s->out_done = out_total;
-    // frames before the interval the next call starts in are done with
-    {
-        const long long nf0 = s->s_done / cp;
-        const int drop = (int)(nf0 - s->pend_first);
-        if (drop > 0) {
-            const int keep = s->pend_frames - drop;
-            std::vector<double> next((size_t)n * keep * 16);
-            for (int u = 0; u < n; ++u)
-                memcpy(&next[(size_t)u * keep * 16], &s->pending[((size_t)u * s->pend_frames + drop) * 16], (size_t)keep * 128);
-            s->pending.swap(next);
-            s->pend_frames = keep;
-            s->pend_first = nf0;
-        }
-    }
-    if (flush) s->flushed = true;
-    if (n_samples) *n_samples = n_ret > 0 ? n_ret : 0;
-    return 0;
-}
-
-/* ------------------------------------------------------------------------------------------------------------
- * stream pool: slots at independent positions, each with its own voice (the per-slot form of trm_cuda_stream_push)
- * ---------------------------------------------------------------------------------------------------------- */
 struct trm_cuda_pool {
     struct Slot {
         bool open = false;
         bool fresh = false;             // opened since its last waveguide launch: the carried state starts from zero there
         trm_cuda_utterance voice{};     // descriptor template (voice = the slot's wavetable row)
         int cur = 0;                    // history buffer that holds the slot's tube-rate samples
-        long long frames_seen = 0, s_done = 0, out_done = 0, in_start = 0;   // as trm_cuda_stream, per slot
+        long long frames_seen = 0;      // control frames pushed so far
+        long long s_done = 0;           // tube-rate samples produced so far (multiple of 16 until the flush)
+        long long out_done = 0;         // output-rate samples returned so far
+        long long in_start = 0;         // first tube-rate sample still in the history buffer (multiple of 4)
         std::vector<double> pending;    // [pend_frames][16]: frames from the control interval in progress on
         long long pend_first = 0;
         int pend_frames = 0;
@@ -1406,7 +1159,7 @@ int trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max
     return 0;
 }
 
-// the sizes trm_cuda_stream_create gives one stream of this voice: history elements per slot and buffer, samples per push
+// what one slot of this voice needs: history elements per slot and buffer, samples per push
 static void pool_sizes(const trm_cuda_pool *p, const trm_cuda_utterance *v, long long *stride, long long *cap_out)
 {
     const long long max_new = (long long)(p->max_m + 1) * v->controlPeriod + 32;
@@ -1578,12 +1331,13 @@ struct PoolPcm {
 };
 
 // One push: samples (pcm == nullptr) into samples_host, or PCM16 as `pcm` says.  out_offset receives the packed sample
-// offsets either way (the layout of d_out).
+// offsets either way; d_out holds the samples packed, or in rows of cap_out when out_stride > 0 (samples only).
 static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
-                     const uint8_t *flush, void *samples_host, int64_t *out_offset, const PoolPcm *pcm)
+                     const uint8_t *flush, void *samples_host, int64_t out_stride, int64_t *out_offset, const PoolPcm *pcm)
 {
     // ---- arguments: everything is checked before the pool changes -----------------------------------------------
     if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_push: bad entry count");
+    if (out_stride < 0 || (out_stride > 0 && out_stride < p->cap_out)) return pool_err(-4, "trm_cuda_pool_push: row stride below the slot capacity");
     if (!out_offset || (n > 0 && (!slot || !n_frames))) return pool_err(-4, "trm_cuda_pool_push: null argument");
     if (pcm && (!pcm->offset || (n > 0 && !pcm->peak))) return pool_err(-4, "trm_cuda_pool_push_pcm16: null argument");
     long long total_in = 0;
@@ -1620,7 +1374,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         p->pcm_cap = 2 * (long long)p->cap * p->cap_out;
     }
 
-    // ---- per entry: what trm_cuda_stream_push computes for one stream ------------------------------------------------
+    // ---- per entry: the samples its frames make computable, the outputs they make safe, the history still needed ------
     struct Entry {
         int slot = 0;
         bool flush = false, run = false;
@@ -1631,7 +1385,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     };
     std::vector<Entry> E((size_t)n);
     const double *fp = frames_host;
-    long long wg_frames = 0, total_out = 0;
+    long long wg_frames = 0, total_out = 0, max_ret = 0;
     int n_wg = 0;
     for (int i = 0; i < n; ++i) {
         Entry &e = E[i];
@@ -1671,6 +1425,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             if (e.target - sl.in_start > p->stride || n_ret > p->cap_out) return fail_msg("trm_cuda_pool_push: internal capacity");
         }
         total_out += n_ret > 0 ? n_ret : 0;
+        max_ret = std::max(max_ret, n_ret);
         out_offset[i + 1] = total_out;
         if (pcm) pcm->offset[i + 1] = pcm->offset[i] + (n_ret > 0 ? n_ret * sl.voice.channels : 0);
     }
@@ -1711,7 +1466,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             r.n_out = e.out_total;
             r.out_start = sl.out_done;
             r.in_start = sl.in_start;
-            r.out_offset = out_offset[i];
+            r.out_offset = out_stride > 0 ? i * p->cap_out : out_offset[i];
             r.pcm_offset = pcm ? pcm->offset[i] : 0;
             rd.push_back(r);
             rd_entry.push_back(i);
@@ -1834,7 +1589,11 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         // the maxima come back into the staging buffer (its upload precedes this copy on the stream)
         if (pcm->max && n_pk) CK(cudaMemcpyAsync(h + o_mx, d + o_mx, n_pk * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     } else if (samples_host && total_out > 0) {
-        CK(cudaMemcpyAsync(samples_host, p->d_out, (size_t)total_out * p->esz, cudaMemcpyDeviceToHost, st));
+        if (out_stride > 0)
+            CK(cudaMemcpy2DAsync(samples_host, (size_t)out_stride * p->esz, p->d_out, (size_t)p->cap_out * p->esz,
+                                 (size_t)max_ret * p->esz, (size_t)n, cudaMemcpyDeviceToHost, st));
+        else
+            CK(cudaMemcpyAsync(samples_host, p->d_out, (size_t)total_out * p->esz, cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
     if (pcm && pcm->max) {
@@ -1867,9 +1626,9 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
 }
 
 int trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
-                       const uint8_t *flush, void *samples_host, int64_t *out_offset)
+                       const uint8_t *flush, void *samples_host, int64_t out_stride, int64_t *out_offset)
 {
-    return pool_push(p, n, slot, n_frames, frames_host, flush, samples_host, out_offset, nullptr);
+    return pool_push(p, n, slot, n_frames, frames_host, flush, samples_host, out_stride, out_offset, nullptr);
 }
 
 int trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
@@ -1878,7 +1637,7 @@ int trm_cuda_pool_push_pcm16(trm_cuda_pool *p, int n, const int32_t *slot, const
     if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_push: bad entry count");
     std::vector<int64_t> out_offset((size_t)n + 1);
     const PoolPcm pcm{peak, pcm_host, pcm_offset, max_host};
-    return pool_push(p, n, slot, n_frames, frames_host, flush, nullptr, out_offset.data(), &pcm);
+    return pool_push(p, n, slot, n_frames, frames_host, flush, nullptr, 0, out_offset.data(), &pcm);
 }
 
 // ---- snapshots: the part of a slot that is not its voice ------------------------------------------------------------

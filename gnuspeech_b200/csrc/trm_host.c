@@ -1099,10 +1099,13 @@ int TRMBatchSynthesizeEvents(TRMBatch *b, const TRMEvent *events, const int64_t 
 }
 
 /* ---- streaming (TRAcT-style): many voices advanced together, state carried on the device ---- */
+/* The lockstep use of the stream pool: slot i is stream i, every push advances all of them by the same frames. */
 struct TRMStream {
-    trm_cuda_stream *s;
-    voice_set voices;
-    int device, lane;
+    trm_cuda_pool *p;
+    int n, max_m, flushed;
+    int32_t *slot, *n_frames;       /* [n] the entries of every push: stream i's slot, m frames each */
+    uint8_t *flush;                 /* [n] */
+    int64_t *offset;                /* [n+1] packed offsets the pool returns (every stream gets the same count) */
 };
 
 TRMStream *TRMStreamCreate(int n_streams, const TRMInputParameters *voice, int precision, int max_frames_per_push,
@@ -1115,40 +1118,72 @@ TRMStream *TRMStreamCreate(int n_streams, const TRMInputParameters *voice, int p
         return NULL;
     }
     TRMStream *t = calloc(1, sizeof *t);
-    if (!t) { *err = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); return NULL; }
-    trm_cuda_utterance d;
-    rates_t r;
-    if ((*err = describe(voice, 2, &t->voices, &d, &r)) != TRM_OK) { free(t); return NULL; }
-    trm_cuda_ctx *ctx;
-    if ((*err = acquire_ctx(device, &ctx, &t->lane)) != TRM_OK) { voice_set_free(&t->voices); free(t); return NULL; }
-    t->device = device;
-    if (trm_cuda_set_wavetables(ctx, t->voices.tables, t->voices.n) != 0 ||
-        trm_cuda_stream_create(ctx, precision, n_streams, &d, max_frames_per_push, &t->s) != 0) {
-        *err = cuda_err();
-        release_ctx(device, t->lane);
-        voice_set_free(&t->voices);
-        free(t);
+    if (t) {
+        t->slot = calloc((size_t)n_streams, sizeof *t->slot);
+        t->n_frames = calloc((size_t)n_streams, sizeof *t->n_frames);
+        t->flush = calloc((size_t)n_streams, sizeof *t->flush);
+        t->offset = calloc((size_t)n_streams + 1, sizeof *t->offset);
+    }
+    if (!t || !t->slot || !t->n_frames || !t->flush || !t->offset) {
+        TRMStreamFree(t);
+        *err = set_err(TRM_ERR_NOMEM, "out of memory%s", "");
         return NULL;
     }
-    release_ctx(device, t->lane);      /* the stream owns its wavetable copy, streams and scratch: no lane is held */
+    t->n = n_streams;
+    t->max_m = max_frames_per_push;
+    voice_set vs;
+    trm_cuda_utterance d;
+    memset(&vs, 0, sizeof vs);
+    if ((*err = describe(voice, 2, &vs, &d, NULL)) != TRM_OK) { voice_set_free(&vs); TRMStreamFree(t); return NULL; }
+    trm_cuda_ctx *ctx;
+    int lane;
+    if ((*err = acquire_ctx(device, &ctx, &lane)) != TRM_OK) { voice_set_free(&vs); TRMStreamFree(t); return NULL; }
+    int rc = trm_cuda_pool_create(ctx, precision, n_streams, max_frames_per_push, &t->p);
+    release_ctx(device, lane);      /* the pool owns its buffers, wavetables, stream and scratch: no lane is held */
+    /* sized for this voice alone, so that the capacity is what one stream of it needs */
+    if (rc == 0) rc = trm_cuda_pool_reserve(t->p, &d);
+    for (int i = 0; i < n_streams && rc == 0; i++)
+        rc = trm_cuda_pool_open(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, &t->slot[i]);
+    voice_set_free(&vs);
+    if (rc != 0) {
+        *err = cuda_err();
+        TRMStreamFree(t);
+        return NULL;
+    }
     *err = TRM_OK;
     return t;
 }
 
-int64_t TRMStreamCapacity(const TRMStream *t) { return t ? trm_cuda_stream_capacity(t->s) : 0; }
+int64_t TRMStreamCapacity(const TRMStream *t) { return t ? trm_cuda_pool_slot_capacity(t->p) : 0; }
 
 int TRMStreamPush(TRMStream *t, const TRMParameters *frames, int m, int flush, void *samples_out, int64_t *n_samples)
 {
     if (!t) return set_err(TRM_ERR_PARAM, "null stream%s", "");
-    if (trm_cuda_stream_push(t->s, (const double *)frames, m, flush, samples_out, n_samples) != 0) return cuda_err();
+    if (n_samples) *n_samples = 0;
+    if (t->flushed) return set_err(TRM_ERR_CUDA, "CUDA: %s", "trm_cuda_stream_push: the streams were flushed");
+    if (m < 0 || m > t->max_m)
+        return set_err(TRM_ERR_CUDA, "CUDA: %s", "trm_cuda_stream_push: more frames than the stream was created for");
+    for (int i = 0; i < t->n; i++) {
+        t->n_frames[i] = m;
+        t->flush[i] = flush ? 1 : 0;
+    }
+    /* [stream][m][16] is the pool's back-to-back frame layout; samples come back in rows of the capacity */
+    if (trm_cuda_pool_push(t->p, t->n, t->slot, t->n_frames, (const double *)frames, t->flush, samples_out,
+                           trm_cuda_pool_slot_capacity(t->p), t->offset) != 0)
+        return cuda_err();
+    if (flush) t->flushed = 1;      /* the pool has freed the slots */
+    if (n_samples) *n_samples = t->offset[1] - t->offset[0];
     return TRM_OK;
 }
 
 void TRMStreamFree(TRMStream *t)
 {
     if (!t) return;
-    trm_cuda_stream_destroy(t->s);
-    voice_set_free(&t->voices);
+    trm_cuda_pool_destroy(t->p);
+    free(t->slot);
+    free(t->n_frames);
+    free(t->flush);
+    free(t->offset);
     free(t);
 }
 
@@ -1265,7 +1300,7 @@ int TRMStreamPoolPush(TRMStreamPool *t, int n, const int32_t *slot, const int32_
                       const uint8_t *flush, void *samples_out, int64_t *out_offset)
 {
     if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
-    const int rc = trm_cuda_pool_push(t->p, n, slot, n_frames, (const double *)frames, flush, samples_out, out_offset);
+    const int rc = trm_cuda_pool_push(t->p, n, slot, n_frames, (const double *)frames, flush, samples_out, 0, out_offset);
     if (rc != 0) return pool_rc(rc);
     pool_forget_flushed(t, n, slot, flush);
     return TRM_OK;

@@ -186,8 +186,8 @@ template <typename R> __device__ __forceinline__ R *state_vals(void *state, int 
     return reinterpret_cast<R *>(state_hdr<R>(state, u) + STATE_HDR);
 }
 
-// Streaming state capture.  PER_UTT = false (batch, time split, TRMStream: every utterance of a CTA gets the same number
-// of samples, or there is no state): the state is stored when the CTA's loop ends.  PER_UTT = true (stream pool,
+// Streaming state capture.  PER_UTT = false (batch and time split: every utterance of a CTA gets the same number of
+// samples, or there is no state): the state is stored when the CTA's loop ends.  PER_UTT = true (stream pool,
 // trm_cuda_pool_push: the utterances of one CTA may have different sample counts, and the warps keep running past an
 // utterance's end until the longest one of the CTA is done): each utterance's state is stored at the end of the block
 // that holds its last sample.  Two instantiations, so that the paths without per-utterance capture keep their code.

@@ -69,7 +69,7 @@ typedef struct trm_cuda_utterance {
     double   throatGain;
     double   volumeAmp;         /* amplitude(volume)                                                   */
     double   leftGain, rightGain; /* stereo factors applied on top of scale (TRMTubeModel.m:532-533)   */
-    /* streaming (trm_cuda_stream_*): a call continues an utterance.  All zero for whole utterances.              */
+    /* stream pool (trm_cuda_pool_*), time split: a call continues an utterance.  All zero for whole utterances.   */
     int64_t  out_start;         /* first output-rate sample this call produces (earlier ones exist already)       */
     int64_t  in_start;          /* first tube-rate sample still in memory (multiple of 4; earlier ones are gone)  */
     int32_t  jc0;               /* tube samples already produced inside the first control interval of `frames`    */
@@ -168,23 +168,6 @@ int  trm_cuda_copy_probe(int device, const void *host_in, size_t h2d_bytes, void
                          double *ms);
 
 /*
- * Streaming synthesis (TRAcT-style, Applications/TRAcT/tube.c:1096-1191: output as it is produced, no normalisation):
- * n_streams voices with the SAME rates (one trm_cuda_utterance template: controlPeriod, converter signature ...) are
- * advanced together.  Every push appends `m` control frames per stream (frames_host: [stream][m][16] doubles) and
- * returns the un-normalised output-rate samples that became computable (samples_host: [stream][*n_samples], row
- * stride = capacity given at creation; double or float by precision).  Calls cover whole 16-sample blocks of the
- * waveguide, the state of every recurrence is carried on the device: the concatenation of all pushes plus the flush
- * is bit-identical to synthesizing the whole utterance at once.  flush != 0 ends the streams (converter tail, as
- * -synthesize does at the end of an utterance); the object can then be destroyed.
- */
-typedef struct trm_cuda_stream trm_cuda_stream;
-int  trm_cuda_stream_create(trm_cuda_ctx *ctx, int precision, int n_streams, const trm_cuda_utterance *voice,
-                            int max_frames_per_push, trm_cuda_stream **out);
-int64_t trm_cuda_stream_capacity(const trm_cuda_stream *s);          /* samples per stream a push can return */
-int  trm_cuda_stream_push(trm_cuda_stream *s, const double *frames_host, int m, int flush, void *samples_host,
-                          int64_t *n_samples);
-void trm_cuda_stream_destroy(trm_cuda_stream *s);
-/*
  * Stream pool: `capacity` streaming slots that open, advance and end independently, each with its own voice (its own
  * template: control period, converter signature, glottal table).  A push advances any subset of open slots, each by its
  * own number of frames; all of them are synthesized by one waveguide launch and one resampler launch.  Each slot's pushes,
@@ -209,9 +192,11 @@ int  trm_cuda_pool_close(trm_cuda_pool *p, int slot);
 int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one slot can return from one push */
 /* entry i: slot[i] gets n_frames[i] frames (taken back to back from frames_host, rows of 16 doubles; for a slot opened
  * with trm_cuda_pool_open_events, generated from its list instead -- -4 past the list's end); flush[i] != 0 ends
- * the slot and frees it.  samples_host receives the samples packed (entry i: [out_offset[i], out_offset[i+1])). */
+ * the slot and frees it.  out_offset[i+1] - out_offset[i] samples are entry i's.  out_stride == 0: samples_host receives
+ * them packed (entry i: [out_offset[i], out_offset[i+1])); out_stride >= SlotCapacity (else -4): in rows, entry i's
+ * from samples_host[i * out_stride] on (what follows them in the row is undefined). */
 int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
-                        const uint8_t *flush, void *samples_host, int64_t *out_offset);
+                        const uint8_t *flush, void *samples_host, int64_t out_stride, int64_t *out_offset);
 /* the same push, returning PCM16 scaled against peak[i] (finite, > 0), saturated: entry i's int16 elements are
  * pcm_host[pcm_offset[i], pcm_offset[i+1]), channels interleaved; max_host[i] (may be NULL) receives max |y| over the
  * samples entry i produced (0.0 if none).  pcm_kernel's arithmetic (TRMTubeModel.m:515-559) and include/trm.h's contract. */
