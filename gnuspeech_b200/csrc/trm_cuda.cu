@@ -1175,6 +1175,27 @@ static long long pool_keep_from(long long out_total, unsigned tri, int pad)
     return next_in / 4 * 4;
 }
 
+// What a push that takes slot sl on to frames_seen frames, flushing it or not, makes of it: the tube-rate samples it has
+// then (target), the outputs it has returned (out_total), the first tube-rate sample the converter still needs (next_in),
+// and whether that push stays inside one history row of `stride` elements and `cap_out` outputs of one push.
+struct PoolAdvance {
+    long long target = 0, out_total = 0, next_in = 0;
+    bool fits = false;
+};
+
+static PoolAdvance pool_advance(const trm_cuda_pool::Slot &sl, long long frames_seen, bool flush, long long stride, long long cap_out)
+{
+    const unsigned tri = sl.voice.tri;
+    const int pad = sl.voice.padSize;
+    const long long avail = frames_seen >= 2 ? (frames_seen - 1) * sl.voice.controlPeriod : 0;
+    PoolAdvance a;
+    a.target = flush ? avail : avail / trm::TB * trm::TB;
+    a.out_total = flush ? (long long)(((unsigned long long)(a.target + 2 * pad) * 65536ull + tri - 1) / tri) : src_safe_outputs(a.target, tri);
+    a.next_in = std::max(flush ? a.target / 4 * 4 : pool_keep_from(a.out_total, tri, pad), sl.in_start);
+    a.fits = a.target - sl.in_start <= stride && a.out_total - sl.out_done <= cap_out;
+    return a;
+}
+
 int trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *v)
 {
     if (v->controlPeriod <= 0 || v->tri == 0) return pool_err(-4, "trm_cuda_pool: voice without rates");
@@ -1204,21 +1225,51 @@ int trm_cuda_pool_reserve(trm_cuda_pool *p, const trm_cuda_utterance *v)
     return 0;
 }
 
-int trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, int *slot)
+// the first slot from `from` on that is not open (p->cap if there is none)
+static int pool_free_slot(const trm_cuda_pool *p, int from)
 {
-    *slot = -1;
-    int s = 0;
-    while (s < p->cap && p->slots[s].open) ++s;
-    if (s == p->cap) return pool_err(-7, "trm_cuda_pool_open: every slot is open");
+    while (from < p->cap && p->slots[from].open) ++from;
+    return from;
+}
+
+// slot s opened with this voice (its wavetable row is row s), fresh or not; event-fed when ev says so
+static trm_cuda_pool::Slot pool_slot(int s, const trm_cuda_utterance &voice, bool fresh, const trm_cuda_pool_event_state *ev)
+{
+    trm_cuda_pool::Slot sl;
+    sl.open = true;
+    sl.fresh = fresh;
+    sl.voice = voice;
+    sl.voice.voice = s;
+    if (ev && ev->events) {
+        sl.events = true;
+        sl.ev_count = ev->n_events;
+        sl.ev_frames = ev->ev_frames;
+        sl.fg = ev->fg;
+        sl.fg.reserved = 0;             // a snapshot stores 0 there, whatever the caller left in it
+    }
+    return sl;
+}
+
+// a free slot for this voice, with the pool's rows reserved for the voice and the slot's wavetable row written; it opens
+// when the caller sets its Slot
+static int pool_claim(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, const char *full, int *slot)
+{
+    const int s = pool_free_slot(p, 0);
+    if (s == p->cap) return pool_err(-7, full);
     int rc = trm_cuda_pool_reserve(p, voice);
     if (rc != 0) return rc;
     CK(cudaMemcpy(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH, wavetable, TRM_TABLE_LENGTH * sizeof(double), cudaMemcpyHostToDevice));
-    trm_cuda_pool::Slot &sl = p->slots[s];
-    sl = trm_cuda_pool::Slot();
-    sl.open = true;
-    sl.fresh = true;
-    sl.voice = *voice;
-    sl.voice.voice = s;
+    *slot = s;
+    return 0;
+}
+
+int trm_cuda_pool_open(trm_cuda_pool *p, const trm_cuda_utterance *voice, const double *wavetable, int *slot)
+{
+    *slot = -1;
+    int s;
+    const int rc = pool_claim(p, voice, wavetable, "trm_cuda_pool_open: every slot is open", &s);
+    if (rc != 0) return rc;
+    p->slots[s] = pool_slot(s, *voice, true, nullptr);
     *slot = s;
     return 0;
 }
@@ -1267,27 +1318,15 @@ int trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice,
                               int *slot)
 {
     *slot = -1;
-    int s = 0;
-    while (s < p->cap && p->slots[s].open) ++s;
-    if (s == p->cap) return pool_err(-7, "trm_cuda_pool_open_events: every slot is open");
-    int rc = trm_cuda_pool_reserve(p, voice);
+    int s;
+    int rc = pool_claim(p, voice, wavetable, "trm_cuda_pool_open_events: every slot is open", &s);
     if (rc == 0) rc = pool_event_storage(p);
     if (rc == 0) rc = pool_event_list(p, s, n_events);
     if (rc != 0) return rc;
     if (n_events > 0) CK(cudaMemcpy(p->d_events[s], events, (size_t)n_events * sizeof(trm_cuda_event), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(&p->d_gen[s].fg, fg, sizeof(trm_cuda_framegen), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH, wavetable, TRM_TABLE_LENGTH * sizeof(double), cudaMemcpyHostToDevice));
-    trm_cuda_pool::Slot &sl = p->slots[s];
-    sl = trm_cuda_pool::Slot();
-    sl.open = true;
-    sl.fresh = true;
-    sl.voice = *voice;
-    sl.voice.voice = s;
-    sl.events = true;
-    sl.ev_count = n_events;
-    sl.ev_frames = n_frames;
-    sl.fg = *fg;
-    sl.fg.reserved = 0;                 // a snapshot stores 0 there, whatever the caller left in it
+    const trm_cuda_pool_event_state ev{1, 0, n_events, n_frames, *fg};
+    p->slots[s] = pool_slot(s, *voice, true, &ev);
     *slot = s;
     return 0;
 }
@@ -1366,63 +1405,40 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     if (n == 0) return 0;
     trm_cuda_ctx *ctx = p->ctx;
     CK(cudaSetDevice(ctx->device));
-    if (pcm && p->pcm_cap < 2 * p->cap * p->cap_out) {   // stereo: two int16 per sample
-        if (p->d_pcm) cudaFree(p->d_pcm);
-        p->d_pcm = nullptr;
-        p->pcm_cap = 0;
-        CK(cudaMalloc((void **)&p->d_pcm, (size_t)2 * p->cap * p->cap_out * sizeof(int16_t)));
-        p->pcm_cap = 2 * (long long)p->cap * p->cap_out;
-    }
 
-    // ---- per entry: the samples its frames make computable, the outputs they make safe, the history still needed ------
+    // ---- per entry, what the push makes of its slot: the samples its frames make computable, the outputs they make
+    // safe, the history still needed.  The slots change only in the bookkeeping, once the device work has succeeded. ----
     struct Entry {
         int slot = 0;
         bool flush = false, run = false;
-        long long target = 0, n_new = 0, out_total = 0, next_in = 0;
-        int skip = 0, nf_call = 0;
-        int gen_at = 0;             // event-fed: pending-row index of the first frame this push generates
-        bool setup = false;         // event-fed: these are the slot's first frames
+        long long frames_seen = 0;          // the slot's frames after the push
+        int pend_frames = 0;                // its pending frames after the push, the waveguide's frames when it runs
+        const double *frames = nullptr;     // frame-fed: the push's new frames, in frames_host
+        PoolAdvance a;
+        long long n_new = 0;
     };
     std::vector<Entry> E((size_t)n);
     const double *fp = frames_host;
     long long wg_frames = 0, total_out = 0, max_ret = 0;
-    int n_wg = 0;
     for (int i = 0; i < n; ++i) {
         Entry &e = E[i];
         e.slot = slot[i];
         e.flush = flush && flush[i];
-        trm_cuda_pool::Slot &sl = p->slots[e.slot];
-        const int m = n_frames[i];
-        if (m) {
-            if (sl.events) {
-                e.gen_at = sl.pend_frames;
-                e.setup = sl.frames_seen == 0;
-            } else {
-                sl.pending.insert(sl.pending.end(), fp, fp + (size_t)m * 16);
-                fp += (size_t)m * 16;
-            }
-            sl.pend_frames += m;
-            sl.frames_seen += m;
+        const trm_cuda_pool::Slot &sl = p->slots[e.slot];
+        e.frames_seen = sl.frames_seen + n_frames[i];
+        e.pend_frames = sl.pend_frames + n_frames[i];
+        if (!sl.events) {
+            e.frames = fp;
+            fp += (size_t)n_frames[i] * 16;
         }
-        const long long cp = sl.voice.controlPeriod;
-        const unsigned tri = sl.voice.tri;
-        const int pad = sl.voice.padSize;
-        const long long avail = sl.frames_seen >= 2 ? (sl.frames_seen - 1) * cp : 0;
-        e.target = e.flush ? avail : avail / trm::TB * trm::TB;
-        e.n_new = e.target - sl.s_done;
-        e.out_total = e.flush ? (long long)(((unsigned long long)(e.target + 2 * pad) * 65536ull + tri - 1) / tri) : src_safe_outputs(e.target, tri);
-        e.run = !(e.flush && sl.frames_seen < 1) && (e.n_new > 0 || (e.flush && e.out_total > sl.out_done));
+        e.a = pool_advance(sl, e.frames_seen, e.flush, p->stride, p->cap_out);
+        e.n_new = e.a.target - sl.s_done;
+        e.run = !(e.flush && e.frames_seen < 1) && (e.n_new > 0 || (e.flush && e.a.out_total > sl.out_done));
         long long n_ret = 0;
         if (e.run) {
-            const long long f0 = sl.s_done / cp;
-            e.skip = (int)(f0 - sl.pend_first);
-            e.nf_call = sl.pend_frames - e.skip;
-            if (e.n_new > 0) { ++n_wg; wg_frames += e.nf_call; }
-            n_ret = e.out_total - sl.out_done;
-            long long next_in = e.flush ? e.target / 4 * 4 : pool_keep_from(e.out_total, tri, pad);
-            if (next_in < sl.in_start) next_in = sl.in_start;
-            e.next_in = next_in;
-            if (e.target - sl.in_start > p->stride || n_ret > p->cap_out) return fail_msg("trm_cuda_pool_push: internal capacity");
+            if (e.n_new > 0) wg_frames += e.pend_frames;
+            n_ret = e.a.out_total - sl.out_done;
+            if (!e.a.fits) return fail_msg("trm_cuda_pool_push: internal capacity");
         }
         total_out += n_ret > 0 ? n_ret : 0;
         max_ret = std::max(max_ret, n_ret);
@@ -1443,27 +1459,27 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     for (int i = 0; i < n; ++i) {
         const Entry &e = E[i];
         const trm_cuda_pool::Slot &sl = p->slots[e.slot];
-        if (sl.events && n_frames[i] > 0)
-            ge.push_back({(unsigned long long)(uintptr_t)p->d_events[e.slot], sl.ev_count, p->pend_addr(e.slot, sl.pcur, e.gen_at),
-                          e.slot, n_frames[i], e.setup ? 1 : 0, 0});
+        if (sl.events && n_frames[i] > 0)   // appended after the slot's pending frames; set-up on its first frames
+            ge.push_back({(unsigned long long)(uintptr_t)p->d_events[e.slot], sl.ev_count, p->pend_addr(e.slot, sl.pcur, sl.pend_frames),
+                          e.slot, n_frames[i], sl.frames_seen == 0 ? 1 : 0, 0});
         if (!e.run) continue;
         if (e.n_new > 0) {
             wg.push_back(i);
             if (sl.events) ++n_fb;
-            else fed_frames += e.nf_call;
+            else fed_frames += e.pend_frames;
         }
         if (sl.events && !e.flush) {
             // the frames before the interval the next push starts in are dropped (bookkeeping below)
-            const int drop = (int)(e.target / sl.voice.controlPeriod - sl.pend_first), kept = sl.pend_frames - drop;
+            const int drop = (int)(e.a.target / sl.voice.controlPeriod - sl.pend_first), kept = e.pend_frames - drop;
             if (drop > 0 && kept > 0)
                 fs.push_back({p->pend_addr(e.slot, sl.pcur, drop), p->pend_addr(e.slot, sl.pcur ^ 1, 0), (unsigned long long)kept * 128});
         }
-        const long long n_ret = e.out_total - sl.out_done;
+        const long long n_ret = e.a.out_total - sl.out_done;
         if (n_ret > 0) {
             trm_cuda_utterance r = sl.voice;              // global sample indices of the stream
-            r.n_tube = e.target;
+            r.n_tube = e.a.target;
             r.tube_offset = p->tube_at(e.slot, sl.cur) - sl.in_start;
-            r.n_out = e.out_total;
+            r.n_out = e.a.out_total;
             r.out_start = sl.out_done;
             r.in_start = sl.in_start;
             r.out_offset = out_stride > 0 ? i * p->cap_out : out_offset[i];
@@ -1472,9 +1488,9 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             rd_entry.push_back(i);
             ib.push_back(ib.back() + (n_ret + 31) / 32);
         }
-        const long long keep = e.target - e.next_in;
+        const long long keep = e.a.target - e.a.next_in;
         if (!e.flush && keep > 0)
-            mv.push_back({p->tube_addr(p->tube_at(e.slot, sl.cur) + (e.next_in - sl.in_start)), p->tube_addr(p->tube_at(e.slot, sl.cur ^ 1)),
+            mv.push_back({p->tube_addr(p->tube_at(e.slot, sl.cur) + (e.a.next_in - sl.in_start)), p->tube_addr(p->tube_at(e.slot, sl.cur ^ 1)),
                           (unsigned long long)keep * p->esz});
     }
     std::stable_sort(wg.begin(), wg.end(), [&](int a, int b) { return E[a].n_new > E[b].n_new; });
@@ -1494,6 +1510,13 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     const size_t o_fr = o_fs + align_up(n_fs * sizeof(trm::CopySeg), 256);
     // the frame region holds the frame-fed entries' frames (uploaded), then the event-fed ones' (copied on the device)
     const size_t bytes = o_fr + (size_t)wg_frames * 128, up = o_fr + (size_t)fed_frames * 128;
+    if (pcm && p->pcm_cap < 2 * p->cap * p->cap_out) {   // stereo: two int16 per sample
+        if (p->d_pcm) cudaFree(p->d_pcm);
+        p->d_pcm = nullptr;
+        p->pcm_cap = 0;
+        CK(cudaMalloc((void **)&p->d_pcm, (size_t)2 * p->cap * p->cap_out * sizeof(int16_t)));
+        p->pcm_cap = 2 * (long long)p->cap * p->cap_out;
+    }
     int rc;
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
     if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
@@ -1509,7 +1532,7 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             const trm_cuda_pool::Slot &sl = p->slots[e.slot];
             trm_cuda_utterance d = sl.voice;
             d.frame_offset = sl.events ? ev_at : f_at;
-            d.n_frames = e.nf_call;
+            d.n_frames = e.pend_frames;
             d.n_tube = e.n_new;
             d.tube_offset = p->tube_at(e.slot, sl.cur) + (sl.s_done - sl.in_start);
             d.jc0 = (int)(sl.s_done % sl.voice.controlPeriod);
@@ -1517,13 +1540,16 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
             dt[k] = d;
             ord[k] = e.slot;
             rst[k] = sl.fresh ? 1 : 0;
+            // the waveguide reads every pending frame: the slot's first pending frame is the one its position s_done lies in
             if (sl.events) {
-                *fb++ = {p->pend_addr(e.slot, sl.pcur, e.skip), (unsigned long long)(uintptr_t)(p->scratch.base + o_fr + (size_t)ev_at * 128),
-                         (unsigned long long)e.nf_call * 128};
-                ev_at += e.nf_call;
+                *fb++ = {p->pend_addr(e.slot, sl.pcur, 0), (unsigned long long)(uintptr_t)(p->scratch.base + o_fr + (size_t)ev_at * 128),
+                         (unsigned long long)e.pend_frames * 128};
+                ev_at += e.pend_frames;
             } else {
-                memcpy(fr + (size_t)f_at * 16, &sl.pending[(size_t)e.skip * 16], (size_t)e.nf_call * 128);
-                f_at += e.nf_call;
+                // the slot's pending frames, then the push's new ones
+                if (sl.pend_frames) memcpy(fr + (size_t)f_at * 16, sl.pending.data(), (size_t)sl.pend_frames * 128);
+                if (n_frames[wg[k]]) memcpy(fr + (size_t)(f_at + sl.pend_frames) * 16, e.frames, (size_t)n_frames[wg[k]] * 128);
+                f_at += e.pend_frames;
             }
         }
         if (n_ge) memcpy(h + o_ge, ge.data(), n_ge * sizeof(trm::FrameGenPoolEntry));
@@ -1601,26 +1627,31 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         for (size_t j = 0; j < n_pk; ++j) memcpy(&pcm->max[rd_entry[j]], h + o_mx + j * sizeof(unsigned long long), sizeof(double));
     }
 
-    // ---- bookkeeping -------------------------------------------------------------------------------------------
+    // ---- bookkeeping: the only place a push changes its slots ------------------------------------------------------
     for (int i = 0; i < n; ++i) {
         const Entry &e = E[i];
         trm_cuda_pool::Slot &sl = p->slots[e.slot];
         if (e.flush) { sl = trm_cuda_pool::Slot(); continue; }     // ended: the slot is free again
-        if (!e.run) continue;
-        if (e.n_new > 0) sl.fresh = false;
-        sl.in_start = e.next_in;
-        sl.s_done = e.target;
-        sl.out_done = e.out_total;
-        sl.cur ^= 1;
-        // frames before the interval the next push starts in are done with
-        const long long nf0 = sl.s_done / sl.voice.controlPeriod;
-        const int drop = (int)(nf0 - sl.pend_first);
-        if (drop > 0) {
-            if (!sl.events) sl.pending.erase(sl.pending.begin(), sl.pending.begin() + (size_t)drop * 16);
-            else if (sl.pend_frames > drop) sl.pcur ^= 1;      // the kept frames were copied to the other row
-            sl.pend_frames -= drop;
-            sl.pend_first = nf0;
+        sl.frames_seen = e.frames_seen;
+        sl.pend_frames = e.pend_frames;
+        int drop = 0;
+        if (e.run) {
+            if (e.n_new > 0) sl.fresh = false;
+            sl.in_start = e.a.next_in;
+            sl.s_done = e.a.target;
+            sl.out_done = e.a.out_total;
+            sl.cur ^= 1;
+            // frames before the interval the next push starts in are done with
+            drop = (int)(sl.s_done / sl.voice.controlPeriod - sl.pend_first);
         }
+        if (!sl.events) {
+            sl.pending.insert(sl.pending.end(), e.frames, e.frames + (size_t)n_frames[i] * 16);
+            sl.pending.erase(sl.pending.begin(), sl.pending.begin() + (size_t)drop * 16);
+        } else if (drop > 0 && sl.pend_frames > drop) {
+            sl.pcur ^= 1;                                          // the kept frames were copied to the other row
+        }
+        sl.pend_frames -= drop;
+        sl.pend_first += drop;
     }
     return 0;
 }
@@ -1669,12 +1700,6 @@ int64_t trm_cuda_pool_slot_bytes(int precision, const trm_cuda_pool_slot_state *
            (int64_t)(c->s_done - c->in_start) * (int64_t)esz;
 }
 
-// bytes of a snapshot's slot part that live on the device: carried state (unless fresh), then kept history
-static size_t pool_device_bytes(const trm_cuda_pool *p, const trm_cuda_pool_slot_state &c)
-{
-    return (c.fresh ? 0 : trm::tube_state_bytes(p->esz)) + (size_t)(c.s_done - c.in_start) * p->esz;
-}
-
 // the generator part of the device state is the FrameGen fields, in the snapshot's order, ahead of the settings
 static_assert(offsetof(trm::FrameGenPoolState, fg) == TRM_FRAMEGEN_STATE_BYTES, "generator state layout");
 static_assert(sizeof(trm_cuda_event) == 296, "event layout");
@@ -1686,22 +1711,31 @@ int64_t trm_cuda_pool_event_bytes(const trm_cuda_pool_slot_state *st, const trm_
     return ev->events ? (int64_t)pool_gen_bytes(*st) + ev->n_events * (int64_t)sizeof(trm_cuda_event) : 0;
 }
 
-// A slot's part of the snapshot staging, packed slot after slot from 16-byte boundaries: [pending frames (event-fed
-// slots: they are on the device)][carried state][kept history][event list][generator state].  The list precedes the
-// generator so that both the list and everything before it start on 16 bytes; the data part orders them the other way.
+// A slot's parts on the device, in the order of its part of the snapshot staging (packed slot after slot from 16-byte
+// boundaries): pending frames (event-fed slots: they are on the device), carried state (unless fresh), kept history,
+// event list, generator state.  The list precedes the generator so that both the list and everything before it start
+// on 16 bytes; the data part orders them the other way.
 struct SnapStage {
-    size_t pend = 0, dev = 0, list = 0, gen = 0;
-    size_t bytes() const { return align_up(pend + dev + list + gen, 16); }
+    enum { PEND, STATE, HIST, LIST, GEN, N_PARTS };
+    unsigned long long at[N_PARTS] = {};    // device address
+    size_t size[N_PARTS] = {};              // bytes, 0 for a part the slot does not have
+    size_t head() const { return size[PEND] + size[STATE] + size[HIST]; }     // the bytes before the list
+    size_t bytes() const { return align_up(head() + size[LIST] + size[GEN], 16); }
 };
 
-static SnapStage snap_stage(const trm_cuda_pool *p, const trm_cuda_pool_slot_state &c, const trm_cuda_pool_event_state *ev)
+// the parts of slot s, whose history is in buffer sl.cur and pending frames in row sl.pcur, with gen_bytes of its
+// generator state
+static SnapStage snap_stage(const trm_cuda_pool *p, int s, const trm_cuda_pool::Slot &sl, size_t gen_bytes)
 {
     SnapStage g;
-    g.dev = pool_device_bytes(p, c);
-    if (ev && ev->events) {
-        g.pend = (size_t)c.pend_frames * 128;
-        g.list = (size_t)ev->n_events * sizeof(trm_cuda_event);
-        g.gen = pool_gen_bytes(c);
+    auto part = [&](int k, unsigned long long at, size_t size) { g.at[k] = at; g.size[k] = size; };
+    const size_t sb = trm::tube_state_bytes(p->esz);
+    if (sl.events) part(SnapStage::PEND, p->pend_addr(s, sl.pcur, 0), (size_t)sl.pend_frames * 128);
+    if (!sl.fresh) part(SnapStage::STATE, (unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), sb);
+    part(SnapStage::HIST, p->tube_addr(p->tube_at(s, sl.cur)), (size_t)(sl.s_done - sl.in_start) * p->esz);
+    if (sl.events) {
+        part(SnapStage::LIST, (unsigned long long)(uintptr_t)p->d_events[s], (size_t)sl.ev_count * sizeof(trm_cuda_event));
+        part(SnapStage::GEN, (unsigned long long)(uintptr_t)(p->d_gen + s), gen_bytes);
     }
     return g;
 }
@@ -1738,14 +1772,13 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
     if (!dst || n == 0) return 0;
 
     // gather every slot's device part into packed staging ([segments][slot 0][slot 1] ..., SnapStage), one copy back
-    const size_t sb = trm::tube_state_bytes(p->esz);
     std::vector<SnapStage> sg((size_t)n);
     std::vector<size_t> at((size_t)n + 1, 0);
     for (int i = 0; i < n; ++i) {
-        sg[i] = snap_stage(p, st[i], ev ? &ev[i] : nullptr);
+        sg[i] = snap_stage(p, slot[i], p->slots[slot[i]], pool_gen_bytes(st[i]));
         at[i + 1] = at[i] + sg[i].bytes();
     }
-    const size_t o_stg = align_up((size_t)5 * n * sizeof(trm::CopySeg), 256);
+    const size_t o_stg = align_up((size_t)SnapStage::N_PARTS * n * sizeof(trm::CopySeg), 256);
     const size_t bytes = o_stg + at[n];
     int rc;
     CK(cudaSetDevice(p->ctx->device));
@@ -1755,27 +1788,12 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
     trm::CopySeg *seg = (trm::CopySeg *)h;
     int n_seg = 0;
     for (int i = 0; i < n; ++i) {
-        const int s = slot[i];
-        const trm_cuda_pool::Slot &sl = p->slots[s];
         unsigned long long to = (unsigned long long)(uintptr_t)(d + o_stg + at[i]);
-        if (sg[i].pend) {
-            seg[n_seg++] = {p->pend_addr(s, sl.pcur, 0), to, sg[i].pend};
-            to += sg[i].pend;
-        }
-        if (!st[i].fresh) {
-            seg[n_seg++] = {(unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), to, sb};
-            to += sb;
-        }
-        const long long hist = st[i].s_done - st[i].in_start;
-        if (hist > 0) {
-            seg[n_seg++] = {p->tube_addr(p->tube_at(s, sl.cur)), to, (unsigned long long)hist * p->esz};
-            to += (unsigned long long)hist * p->esz;
-        }
-        if (sg[i].list) {
-            seg[n_seg++] = {(unsigned long long)(uintptr_t)p->d_events[s], to, sg[i].list};
-            to += sg[i].list;
-        }
-        if (sg[i].gen) seg[n_seg++] = {(unsigned long long)(uintptr_t)(p->d_gen + s), to, sg[i].gen};
+        for (int k = 0; k < SnapStage::N_PARTS; ++k)
+            if (sg[i].size[k]) {
+                seg[n_seg++] = {sg[i].at[k], to, sg[i].size[k]};
+                to += sg[i].size[k];
+            }
     }
     if (n_seg > 0) {
         cudaStream_t cs = p->st;
@@ -1789,15 +1807,16 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
     for (int i = 0; i < n; ++i) {
         const trm_cuda_pool::Slot &sl = p->slots[slot[i]];
         const SnapStage &g = sg[i];
+        const size_t list = g.size[SnapStage::LIST], gen = g.size[SnapStage::GEN];
         const unsigned char *from = h + o_stg + at[i];
         unsigned char *o = (unsigned char *)dst[i];
         const size_t host_pend = sl.events ? 0 : (size_t)sl.pend_frames * 128;
         if (host_pend) memcpy(o, sl.pending.data(), host_pend);
         o += host_pend;
-        memcpy(o, from, g.pend + g.dev);
-        o += g.pend + g.dev;
-        if (g.gen) memcpy(o, from + g.pend + g.dev + g.list, g.gen);
-        if (g.list) memcpy(o + g.gen, from + g.pend + g.dev, g.list);
+        memcpy(o, from, g.head());
+        o += g.head();
+        if (gen) memcpy(o, from + g.head() + list, gen);
+        if (list) memcpy(o + gen, from + g.head(), list);
     }
     return 0;
 }
@@ -1822,27 +1841,31 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
         if (ev && ev[i].events) {
             if (ev[i].n_events < 0 || st[i].frames_seen > ev[i].ev_frames)
                 return pool_err(-4, "trm_cuda_pool_restore: the event part does not agree with the counters");
-            // pool_push appends a push's frames to the pending row before it checks the row's capacity
+            // so that pool_push's pending-row capacity check never refuses the restored slot's next push
             if (st[i].pend_frames + p->max_m > pool_pend_rows(p))
                 return pool_err(-4, "trm_cuda_pool_restore: a snapshot's pending frames and this pool's next push do not fit its pending-frame rows");
             any_events = true;
         }
     }
-    for (int i = 0; i < n; ++i) {
-        // pool_push appends the pending frames before its capacity check: the next push of the restored slot, with as many
-        // frames as this pool takes and a flush, must stay inside one history row and one slot's outputs
-        const trm_cuda_utterance &v = voice[i];
-        const long long fs = st[i].frames_seen + p->max_m;
-        const long long avail = fs >= 2 ? (fs - 1) * v.controlPeriod : 0;
-        const long long out_flush = (long long)(((unsigned long long)(avail + 2 * v.padSize) * 65536ull + v.tri - 1) / v.tri);
-        const long long out = std::max(out_flush, src_safe_outputs(avail / trm::TB * trm::TB, v.tri));
-        if (avail - st[i].in_start > stride || out - st[i].out_done > cap_out)
-            return pool_err(-4, "trm_cuda_pool_restore: a snapshot's history and pending frames do not fit this pool's next push");
+    // the slots as they open, in the first n free slots (slot p->cap once there are none left).  The next push of each,
+    // with as many frames as this pool takes, flushing or not, must stay inside one history row and one slot's outputs,
+    // so that pool_push's capacity check never refuses it.
+    std::vector<int> free_slot((size_t)n);
+    std::vector<trm_cuda_pool::Slot> made((size_t)n);
+    for (int i = 0, s = -1; i < n; ++i) {
+        s = free_slot[i] = pool_free_slot(p, std::min(s + 1, p->cap));
+        trm_cuda_pool::Slot &sl = made[i] = pool_slot(s, voice[i], st[i].fresh != 0, ev ? &ev[i] : nullptr);
+        sl.frames_seen = st[i].frames_seen;
+        sl.s_done = st[i].s_done;
+        sl.out_done = st[i].out_done;
+        sl.in_start = st[i].in_start;
+        sl.pend_first = st[i].pend_first;
+        sl.pend_frames = st[i].pend_frames;
+        for (const bool fl : {false, true})
+            if (!pool_advance(sl, sl.frames_seen + p->max_m, fl, stride, cap_out).fits)
+                return pool_err(-4, "trm_cuda_pool_restore: a snapshot's history and pending frames do not fit this pool's next push");
     }
-    std::vector<int> free_slot;
-    for (int s = 0; s < p->cap && (int)free_slot.size() < n; ++s)
-        if (!p->slots[s].open) free_slot.push_back(s);
-    if ((int)free_slot.size() < n) return pool_err(-7, "trm_cuda_pool_restore: fewer free slots than snapshots");
+    if (free_slot[n - 1] == p->cap) return pool_err(-7, "trm_cuda_pool_restore: fewer free slots than snapshots");
 
     int rc;
     for (int i = 0; i < n; ++i)
@@ -1853,17 +1876,15 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
             if (ev[i].events && (rc = pool_event_list(p, free_slot[i], ev[i].n_events)) != 0) return rc;
     }
     // ---- one upload ([segments][wavetables][entry 0's SnapStage, generator with settings] ...), one scatter -----------
-    const size_t sb = trm::tube_state_bytes(p->esz), wt = TRM_TABLE_LENGTH * sizeof(double);
+    const size_t wt = TRM_TABLE_LENGTH * sizeof(double);
     const size_t gs = sizeof(trm::FrameGenPoolState);   // event-fed: the whole generator state, settings included
     std::vector<SnapStage> sg((size_t)n);
     std::vector<size_t> at((size_t)n + 1, 0);
     for (int i = 0; i < n; ++i) {
-        const trm_cuda_pool_event_state *e = ev ? &ev[i] : nullptr;
-        sg[i] = snap_stage(p, st[i], e);
-        if (e && e->events) sg[i].gen = gs;
+        sg[i] = snap_stage(p, free_slot[i], made[i], gs);
         at[i + 1] = at[i] + sg[i].bytes();
     }
-    const size_t o_wt = align_up((size_t)6 * n * sizeof(trm::CopySeg), 256);
+    const size_t o_wt = align_up((size_t)(1 + SnapStage::N_PARTS) * n * sizeof(trm::CopySeg), 256);
     const size_t o_dev = o_wt + (size_t)n * wt;
     const size_t bytes = o_dev + at[n];
     CK(cudaSetDevice(p->ctx->device));
@@ -1874,41 +1895,28 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
     int n_seg = 0;
     memcpy(h + o_wt, wavetables, (size_t)n * wt);
     for (int i = 0; i < n; ++i) {
-        const int s = free_slot[i];
         const SnapStage &g = sg[i];
         seg[n_seg++] = {(unsigned long long)(uintptr_t)(d + o_wt + (size_t)i * wt),
-                        (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)s * TRM_TABLE_LENGTH), wt};
-        // the data part: [pending frames][state][history] then, event-fed, [generator (frames_seen > 0)][list]
-        const unsigned char *in = (const unsigned char *)src[i] + (g.pend ? 0 : (size_t)st[i].pend_frames * 128);
-        unsigned char *stg = h + o_dev + at[i];
-        memcpy(stg, in, g.pend + g.dev);
+                        (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)free_slot[i] * TRM_TABLE_LENGTH), wt};
         unsigned long long from = (unsigned long long)(uintptr_t)(d + o_dev + at[i]);
-        if (g.pend) {
-            seg[n_seg++] = {from, p->pend_addr(s, 0, 0), g.pend};
-            from += g.pend;
-        }
-        if (!st[i].fresh) {
-            seg[n_seg++] = {from, (unsigned long long)(uintptr_t)(p->d_state + (size_t)s * sb), sb};
-            from += sb;
-        }
-        const long long hist = st[i].s_done - st[i].in_start;
-        if (hist > 0) {
-            seg[n_seg++] = {from, p->tube_addr(p->tube_at(s, 0)), (unsigned long long)hist * p->esz};
-            from += (unsigned long long)hist * p->esz;
-        }
-        if (!g.gen) continue;
-        const size_t gen_in = pool_gen_bytes(st[i]);
-        memcpy(stg + g.pend + g.dev, in + g.pend + g.dev + gen_in, g.list);
-        if (g.list) {
-            seg[n_seg++] = {from, (unsigned long long)(uintptr_t)p->d_events[s], g.list};
-            from += g.list;
-        }
+        for (int k = 0; k < SnapStage::N_PARTS; ++k)
+            if (g.size[k]) {
+                seg[n_seg++] = {from, g.at[k], g.size[k]};
+                from += g.size[k];
+            }
+        // the data part: [pending frames (frame-fed: they stay on the host)][state][history] then, event-fed, [generator
+        // (frames_seen > 0)][list]
+        const unsigned char *in = (const unsigned char *)src[i] + (made[i].events ? 0 : (size_t)st[i].pend_frames * 128);
+        unsigned char *stg = h + o_dev + at[i];
+        memcpy(stg, in, g.head());
+        if (!made[i].events) continue;
+        const size_t gen_in = pool_gen_bytes(st[i]), list = g.size[SnapStage::LIST];
+        memcpy(stg + g.head(), in + g.head() + gen_in, list);
         // a slot with no frames yet sets its generator up on its first push: only the settings matter
         trm::FrameGenPoolState gen{};
-        if (gen_in) memcpy(&gen, in + g.pend + g.dev, gen_in);
+        if (gen_in) memcpy(&gen, in + g.head(), gen_in);
         gen.fg = ev[i].fg;
-        memcpy(stg + g.pend + g.dev + g.list, &gen, gs);
-        seg[n_seg++] = {from, (unsigned long long)(uintptr_t)(p->d_gen + s), gs};
+        memcpy(stg + g.head() + list, &gen, gs);
     }
     cudaStream_t cs = p->st;
     CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
@@ -1917,31 +1925,10 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
     CK(cudaStreamSynchronize(cs));
     // ---- the slots open only now that the device work has finished without error -------------------------------------
     for (int i = 0; i < n; ++i) {
-        const int s = free_slot[i];
-        trm_cuda_pool::Slot &sl = p->slots[s];
-        sl = trm_cuda_pool::Slot();
-        sl.open = true;
-        sl.fresh = st[i].fresh != 0;
-        sl.voice = voice[i];
-        sl.voice.voice = s;
-        sl.cur = 0;
-        sl.frames_seen = st[i].frames_seen;
-        sl.s_done = st[i].s_done;
-        sl.out_done = st[i].out_done;
-        sl.in_start = st[i].in_start;
-        sl.pend_first = st[i].pend_first;
-        sl.pend_frames = st[i].pend_frames;
-        if (ev && ev[i].events) {
-            sl.events = true;
-            sl.ev_count = ev[i].n_events;
-            sl.ev_frames = ev[i].ev_frames;
-            sl.fg = ev[i].fg;
-            sl.pcur = 0;
-        } else {
-            sl.pending.resize((size_t)st[i].pend_frames * 16);
-            if (st[i].pend_frames) memcpy(sl.pending.data(), src[i], (size_t)st[i].pend_frames * 128);
-        }
-        slot_out[i] = s;
+        trm_cuda_pool::Slot &sl = made[i];
+        if (!sl.events) sl.pending.assign((const double *)src[i], (const double *)src[i] + (size_t)st[i].pend_frames * 16);
+        p->slots[free_slot[i]] = std::move(sl);
+        slot_out[i] = free_slot[i];
     }
     return 0;
 }

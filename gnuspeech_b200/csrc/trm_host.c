@@ -1240,41 +1240,47 @@ TRMStreamPool *TRMStreamPoolCreate(int capacity, int precision, int max_frames_p
     return t;
 }
 
-int TRMStreamPoolOpen(TRMStreamPool *t, const TRMInputParameters *voice)
+/* Opens a free slot with this voice, fed with frames or, when event_fed, from an event list (*n_frames receives its frame
+ * count).  Returns the slot or a TRM_ERR_*. */
+static int pool_open(TRMStreamPool *t, const TRMInputParameters *voice, int event_fed, const TRMEvent *events, int64_t n_events,
+                     const TRMFrameGeneration *fg, int64_t *n_frames)
 {
     if (!t || !voice) return set_err(TRM_ERR_PARAM, "null stream pool or voice%s", "");
     voice_set vs;
     trm_cuda_utterance d;
     memset(&vs, 0, sizeof vs);
     int rc = describe(voice, 2, &vs, &d, NULL);
+    if (rc == TRM_OK && event_fed) {
+        if (!events || !fg) {
+            rc = set_err(TRM_ERR_PARAM, "null event arguments%s", "");
+        } else {
+            *n_frames = n_events >= 0 ? TRMEventListFrameCount(events, n_events) : 0;
+            rc = check_event_list(events, n_events, *n_frames);
+        }
+    }
     if (rc != TRM_OK) { voice_set_free(&vs); return rc; }
+    const double *wavetable = vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH;
     int slot = -1;
-    rc = trm_cuda_pool_open(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, &slot);
+    rc = event_fed ? trm_cuda_pool_open_events(t->p, &d, wavetable, (const trm_cuda_event *)events, n_events, *n_frames,
+                                               (const trm_cuda_framegen *)fg, &slot)
+                   : trm_cuda_pool_open(t->p, &d, wavetable, &slot);
     voice_set_free(&vs);
     if (rc != 0) return pool_rc(rc);
     t->voice[slot] = *voice;
     return slot;
 }
 
+int TRMStreamPoolOpen(TRMStreamPool *t, const TRMInputParameters *voice)
+{
+    return pool_open(t, voice, 0, NULL, 0, NULL, NULL);
+}
+
 int TRMStreamPoolOpenEvents(TRMStreamPool *t, const TRMInputParameters *voice, const TRMEvent *events, int64_t n_events,
                             const TRMFrameGeneration *fg, int64_t *n_frames_out)
 {
-    if (!t || !voice) return set_err(TRM_ERR_PARAM, "null stream pool or voice%s", "");
-    voice_set vs;
-    trm_cuda_utterance d;
-    memset(&vs, 0, sizeof vs);
-    int rc = describe(voice, 2, &vs, &d, NULL);
-    if (rc != TRM_OK) { voice_set_free(&vs); return rc; }
-    if (!events || !fg) { voice_set_free(&vs); return set_err(TRM_ERR_PARAM, "null event arguments%s", ""); }
-    const int64_t n_frames = n_events >= 0 ? TRMEventListFrameCount(events, n_events) : 0;
-    if ((rc = check_event_list(events, n_events, n_frames)) != TRM_OK) { voice_set_free(&vs); return rc; }
-    int slot = -1;
-    rc = trm_cuda_pool_open_events(t->p, &d, vs.tables + (size_t)d.voice * TRM_TABLE_LENGTH, (const trm_cuda_event *)events,
-                                   n_events, n_frames, (const trm_cuda_framegen *)fg, &slot);
-    voice_set_free(&vs);
-    if (rc != 0) return pool_rc(rc);
-    t->voice[slot] = *voice;
-    if (n_frames_out) *n_frames_out = n_frames;
+    int64_t n_frames = 0;
+    const int slot = pool_open(t, voice, 1, events, n_events, fg, &n_frames);
+    if (slot >= 0 && n_frames_out) *n_frames_out = n_frames;
     return slot;
 }
 

@@ -359,7 +359,9 @@ int64_t TRMStreamPoolSlotCapacity(const TRMStreamPool *pool);
  * (flush may be NULL: no flush) ends slot[i] (converter tail, as at the end of -synthesize) and frees it.  Samples (double,
  * or float in FP32 mode) are packed: entry i's are samples_out[out_offset[i] .. out_offset[i+1]); samples_out holds
  * n * SlotCapacity elements.  An unopened slot (TRM_ERR_STATE), a slot named twice or too many frames (TRM_ERR_PARAM)
- * fail the whole push before any work: the pool is left exactly as it was. */
+ * fail the whole push before any work: the pool is left exactly as it was.  So does any other error returned before the
+ * push's first launch (out of device memory, say): every slot is as it was.  After a CUDA error during the push's device
+ * work (TRM_ERR_CUDA) the pool's contents are undefined: free it. */
 int TRMStreamPoolPush(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames, const TRMParameters *frames,
                       const uint8_t *flush, void *samples_out, int64_t *out_offset /* [n + 1] */);
 /* As TRMStreamPoolPush, but entry i's new output comes back as 16-bit PCM, host endian, channels interleaved as the
@@ -373,7 +375,8 @@ int TRMStreamPoolPush(TRMStreamPool *pool, int n, const int32_t *slot, const int
  * the samples entry i produced in this push, 0.0 if none (NaN never wins, as in maximumSampleValue); the maximum over a
  * slot's pushes equals TRMBatch's maximumSampleValue.  peak[i] must be finite and > 0 (TRM_ERR_PARAM).  All refusals of
  * TRMStreamPoolPush apply, and are checked, with peak, before any device work: a refused push leaves the pool unchanged.
- * A slot may be advanced by TRMStreamPoolPush and TRMStreamPoolPushPCM16 in any order. */
+ * Other errors leave the pool as they do for TRMStreamPoolPush.  A slot may be advanced by TRMStreamPoolPush and
+ * TRMStreamPoolPushPCM16 in any order. */
 int TRMStreamPoolPushPCM16(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames,
                            const TRMParameters *frames, const uint8_t *flush, const double *peak,
                            int16_t *pcm_out, int64_t *pcm_offset /* [n + 1] */, double *max_out);

@@ -194,7 +194,10 @@ int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one 
  * with trm_cuda_pool_open_events, generated from its list instead -- -4 past the list's end); flush[i] != 0 ends
  * the slot and frees it.  out_offset[i+1] - out_offset[i] samples are entry i's.  out_stride == 0: samples_host receives
  * them packed (entry i: [out_offset[i], out_offset[i+1])); out_stride >= SlotCapacity (else -4): in rows, entry i's
- * from samples_host[i * out_stride] on (what follows them in the row is undefined). */
+ * from samples_host[i * out_stride] on (what follows them in the row is undefined).  A push changes its slots only once
+ * its device work has finished: an error returned before its first launch (a refusal, an internal capacity failure, an
+ * allocation or the upload failing) leaves every slot as it was; after a CUDA error during its device work the pool's
+ * contents are undefined and the pool is to be destroyed. */
 int  trm_cuda_pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t *n_frames, const double *frames_host,
                         const uint8_t *flush, void *samples_host, int64_t out_stride, int64_t *out_offset);
 /* the same push, returning PCM16 scaled against peak[i] (finite, > 0), saturated: entry i's int16 elements are
