@@ -144,6 +144,7 @@ def lib():
     sig("TRMStreamCreate", vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, vp)
     sig("TRMStreamCapacity", i64, vp)
     sig("TRMStreamPush", C.c_int, vp, vp, C.c_int, C.c_int, vp, vp)
+    sig("TRMStreamSetVoice", C.c_int, vp, vp, vp, vp)
     sig("TRMStreamFree", None, vp)
     sig("TRMStreamPoolCreate", vp, C.c_int, C.c_int, C.c_int, C.c_int, P(C.c_int))
     sig("TRMStreamPoolOpen", C.c_int, vp, vp)
@@ -152,6 +153,7 @@ def lib():
     sig("TRMStreamPoolSlotCapacity", i64, vp)
     sig("TRMStreamPoolPush", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp)
     sig("TRMStreamPoolPushPCM16", C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp)
+    sig("TRMStreamPoolSetVoice", C.c_int, vp, C.c_int, vp, vp, vp, vp)
     sig("TRMStreamPoolFree", None, vp)
     sig("TRMStreamPoolSave", C.c_int, vp, C.c_int, vp, vp, i64, vp)
     sig("TRMStreamPoolRestore", C.c_int, vp, C.c_int, vp, vp, vp)

@@ -526,6 +526,14 @@ class TRMStream(object):
               "TRMStreamPush")
         return self._buf[:, :k.value].copy()
 
+    def set_voice(self, ip):
+        """Every stream continues with voice `ip` from the next push, its state kept (TRMStreamSetVoice; the rules of
+        TRMStreamPool.set_voice).  Returns (tube_sample, output_sample), the same for every stream."""
+        ts, os_ = C.c_int64(0), C.c_int64(0)
+        check(N.lib().TRMStreamSetVoice(self._h, C.byref(ip), C.byref(ts), C.byref(os_)), "TRMStreamSetVoice")
+        self._ip = ip
+        return int(ts.value), int(os_.value)
+
     def free(self):
         if self._h:
             N.lib().TRMStreamFree(self._h)
@@ -617,6 +625,23 @@ class TRMStreamPool(object):
         check(N.lib().TRMStreamPoolPushPCM16(self._h, n, _ptr(slot_a), _ptr(nf_a), _ptr(fr), _ptr(flush_a), _ptr(peak_a),
                                              _ptr(pcm), _ptr(off), _ptr(mx)), "TRMStreamPoolPushPCM16")
         return {s: (pcm[off[i]:off[i + 1]].copy(), float(mx[i])) for i, s in enumerate(slots)}
+
+    def set_voice(self, voices):
+        """voices: {slot: TRMInputParameters}.  Each open slot continues with its new voice from the next push, every
+        piece of its state kept (TRMStreamPoolSetVoice): any field may change as long as the control period, tube rate,
+        converter and channels stay.  Returns {slot: (tube_sample, output_sample)}: the tube-rate sample from which the
+        new voice is synthesized, and the output sample from which PCM pushes use its volume and balance.  All or
+        nothing: a refused call changes no slot."""
+        slots = [int(s) for s in voices]
+        n = len(slots)
+        slot_a = np.array(slots, dtype=np.int32)
+        arr = (N.TRMInputParametersStruct * max(1, n))()
+        for i, s in enumerate(slots):
+            C.memmove(C.byref(arr[i]), C.byref(voices[s]), C.sizeof(N.TRMInputParametersStruct))
+        ts = np.zeros(max(1, n), np.int64)
+        os_ = np.zeros(max(1, n), np.int64)
+        check(N.lib().TRMStreamPoolSetVoice(self._h, n, _ptr(slot_a), arr, _ptr(ts), _ptr(os_)), "TRMStreamPoolSetVoice")
+        return {s: (int(ts[i]), int(os_[i])) for i, s in enumerate(slots)}
 
     def save(self, slots, event_slots=False):
         """Snapshots of open slots (TRMStreamPoolSave): {slot: bytes}.  Each restores into any pool of this precision

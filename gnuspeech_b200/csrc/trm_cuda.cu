@@ -1339,6 +1339,57 @@ int trm_cuda_pool_close(trm_cuda_pool *p, int slot)
     return 0;
 }
 
+int trm_cuda_pool_set_voice(trm_cuda_pool *p, int n, const int32_t *slot, const trm_cuda_utterance *voice,
+                            const double *wavetables, int64_t *tube_sample, int64_t *output_sample)
+{
+    // ---- everything is checked before the pool changes -----------------------------------------------------------------
+    if (n < 0 || n > p->cap) return pool_err(-4, "trm_cuda_pool_set_voice: bad entry count");
+    if (n > 0 && (!slot || !voice || !wavetables)) return pool_err(-4, "trm_cuda_pool_set_voice: null argument");
+    {
+        std::vector<unsigned char> named((size_t)p->cap, 0);
+        for (int i = 0; i < n; ++i) {
+            const int s = slot[i];
+            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_set_voice: no such slot");
+            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_set_voice: the slot is not open");
+            if (named[s]) return pool_err(-4, "trm_cuda_pool_set_voice: a slot is named twice");
+            named[s] = 1;
+            const trm_cuda_utterance &v = voice[i], &c = p->slots[s].voice;
+            if (v.controlPeriod != c.controlPeriod || v.sampleRate != c.sampleRate || v.tri != c.tri || v.padSize != c.padSize ||
+                v.channels != c.channels)
+                return pool_err(-4, "trm_cuda_pool_set_voice: the new voice's rate constants differ from the slot's");
+        }
+    }
+    if (n == 0) return 0;
+    // ---- one upload ([segments][rows]), one scatter to the slots' wavetable rows ----------------------------------------
+    const size_t wt = TRM_TABLE_LENGTH * sizeof(double);
+    const size_t o_wt = align_up((size_t)n * sizeof(trm::CopySeg), 256);
+    const size_t bytes = o_wt + (size_t)n * wt;
+    CK(cudaSetDevice(p->ctx->device));
+    int rc;
+    if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
+    if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
+    unsigned char *h = p->stage.base, *d = p->scratch.base;
+    trm::CopySeg *seg = (trm::CopySeg *)h;
+    memcpy(h + o_wt, wavetables, (size_t)n * wt);
+    for (int i = 0; i < n; ++i)
+        seg[i] = {(unsigned long long)(uintptr_t)(d + o_wt + (size_t)i * wt),
+                  (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)slot[i] * TRM_TABLE_LENGTH), wt};
+    cudaStream_t cs = p->st;
+    CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
+    const trm::SegCopyArgs a{(const trm::CopySeg *)d, n};
+    if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("voice change scatter launch", (cudaError_t)rc);
+    CK(cudaStreamSynchronize(cs));
+    // ---- the slots change only now that the rows are in place -----------------------------------------------------------
+    for (int i = 0; i < n; ++i) {
+        trm_cuda_pool::Slot &sl = p->slots[slot[i]];
+        sl.voice = voice[i];
+        sl.voice.voice = slot[i];
+        if (tube_sample) tube_sample[i] = sl.s_done;
+        if (output_sample) output_sample[i] = sl.out_done;
+    }
+    return 0;
+}
+
 int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p) { return p->cap_out; }
 
 void trm_cuda_pool_destroy(trm_cuda_pool *p)

@@ -1103,6 +1103,7 @@ int TRMBatchSynthesizeEvents(TRMBatch *b, const TRMEvent *events, const int64_t 
 struct TRMStream {
     trm_cuda_pool *p;
     int n, max_m, flushed;
+    TRMInputParameters voice;       /* every stream's voice (TRMStreamSetVoice changes it) */
     int32_t *slot, *n_frames;       /* [n] the entries of every push: stream i's slot, m frames each */
     uint8_t *flush;                 /* [n] */
     int64_t *offset;                /* [n+1] packed offsets the pool returns (every stream gets the same count) */
@@ -1131,6 +1132,7 @@ TRMStream *TRMStreamCreate(int n_streams, const TRMInputParameters *voice, int p
     }
     t->n = n_streams;
     t->max_m = max_frames_per_push;
+    t->voice = *voice;
     voice_set vs;
     trm_cuda_utterance d;
     memset(&vs, 0, sizeof vs);
@@ -1661,6 +1663,76 @@ int TRMStreamPoolSnapshotEventInfo(const void *blob, int64_t bytes, TRMStreamSna
     info->frames_generated = st.frames_seen;
     memcpy(&info->fg, &ev.fg, sizeof info->fg);
     return TRM_OK;
+}
+
+/* ---- voice changes (TRMStreamPoolSetVoice, TRMStreamSetVoice) ---- */
+/* Entry i moves slot[i] of pool p from the voice *cur[i] to voice[shared ? 0 : i].  cur[i] is NULL for a slot number
+ * outside the pool (the shim refuses it).  Only on success does *cur[i] become the new voice. */
+static int pool_set_voice(trm_cuda_pool *p, int n, const int32_t *slot, TRMInputParameters *const *cur,
+                          const TRMInputParameters *voice, int shared, int64_t *tube_sample, int64_t *output_sample)
+{
+    trm_cuda_utterance *d = calloc((size_t)n + 1, sizeof *d);
+    double *tables = malloc(((size_t)n + 1) * TRM_TABLE_LENGTH * sizeof *tables);
+    voice_set vs;
+    memset(&vs, 0, sizeof vs);
+    int rc = TRM_OK;
+    if (!d || !tables) { rc = set_err(TRM_ERR_NOMEM, "out of memory%s", ""); goto done; }
+    for (int i = 0; i < n; i++) {
+        if ((rc = describe(&voice[shared ? 0 : i], 2, &vs, &d[i], NULL)) != TRM_OK) goto done;
+        /* an open slot's voice always describes (it was checked when the slot opened); an unopened slot's does not, and
+         * the shim refuses the slot */
+        trm_cuda_utterance now;
+        if (cur[i] && describe(cur[i], 2, &vs, &now, NULL) == TRM_OK) {
+            uint32_t want[6], got[6];
+            snap_derived(&now, TRM_PRECISION_FP64, want);
+            snap_derived(&d[i], TRM_PRECISION_FP64, got);
+            if (memcmp(want, got, sizeof want) != 0) {
+                rc = set_err(TRM_ERR_PARAM, "the new voice's rate constants (control period, sample rate, converter, channels) "
+                                            "differ from the stream's: a new tract length, temperature or rate is a new stream%s", "");
+                goto done;
+            }
+        }
+    }
+    /* the table rows are final only now (vs may have grown while describing) */
+    for (int i = 0; i < n; i++)
+        memcpy(tables + (size_t)i * TRM_TABLE_LENGTH, vs.tables + (size_t)d[i].voice * TRM_TABLE_LENGTH, TRM_TABLE_LENGTH * sizeof *tables);
+    if ((rc = trm_cuda_pool_set_voice(p, n, slot, d, tables, tube_sample, output_sample)) != 0) { rc = pool_rc(rc); goto done; }
+    for (int i = 0; i < n; i++) *cur[i] = voice[shared ? 0 : i];
+done:
+    voice_set_free(&vs);
+    free(d);
+    free(tables);
+    return rc;
+}
+
+int TRMStreamPoolSetVoice(TRMStreamPool *t, int n, const int32_t *slot, const TRMInputParameters *voice, int64_t *tube_sample,
+                          int64_t *output_sample)
+{
+    if (!t) return set_err(TRM_ERR_PARAM, "null stream pool%s", "");
+    if (n < 0 || n > t->capacity || (n > 0 && (!slot || !voice))) return set_err(TRM_ERR_PARAM, "bad voice change arguments%s", "");
+    TRMInputParameters **cur = calloc((size_t)n + 1, sizeof *cur);
+    if (!cur) return set_err(TRM_ERR_NOMEM, "out of memory%s", "");
+    for (int i = 0; i < n; i++) cur[i] = slot[i] >= 0 && slot[i] < t->capacity ? &t->voice[slot[i]] : NULL;
+    const int rc = pool_set_voice(t->p, n, slot, cur, voice, 0, tube_sample, output_sample);
+    free(cur);
+    return rc;
+}
+
+int TRMStreamSetVoice(TRMStream *t, const TRMInputParameters *voice, int64_t *tube_sample, int64_t *output_sample)
+{
+    if (!t || !voice) return set_err(TRM_ERR_PARAM, "null stream or voice%s", "");
+    if (t->flushed) return set_err(TRM_ERR_STATE, "the streams were flushed%s", "");
+    TRMInputParameters **cur = calloc((size_t)t->n, sizeof *cur);
+    int64_t *ts = calloc((size_t)t->n, sizeof *ts), *os = calloc((size_t)t->n, sizeof *os);
+    int rc = TRM_OK;
+    if (!cur || !ts || !os) rc = set_err(TRM_ERR_NOMEM, "out of memory%s", "");
+    for (int i = 0; rc == TRM_OK && i < t->n; i++) cur[i] = &t->voice;
+    if (rc == TRM_OK) rc = pool_set_voice(t->p, t->n, t->slot, cur, voice, 1, ts, os);
+    /* the streams advance in lockstep: every one is at the same sample */
+    if (rc == TRM_OK && tube_sample) *tube_sample = ts[0];
+    if (rc == TRM_OK && output_sample) *output_sample = os[0];
+    free(cur); free(ts); free(os);
+    return rc;
 }
 
 /* ---- asynchronous calls: one host thread per ticket; two tickets per device overlap (context lanes) ---- */

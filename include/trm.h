@@ -309,6 +309,10 @@ int64_t TRMStreamCapacity(const TRMStream *stream);
 /* frames: [stream][m] TRMParameters; samples_out: [stream][TRMStreamCapacity()] ; *n_samples = samples returned per
  * stream by this push.  flush != 0 ends the streams (the converter's tail, as at the end of -synthesize). */
 int TRMStreamPush(TRMStream *stream, const TRMParameters *frames, int m, int flush, void *samples_out, int64_t *n_samples);
+/* TRMStreamPoolSetVoice (below) for all n streams at once: every stream continues with `voice`.  The streams are in
+ * lockstep, so one *tube_sample / *output_sample (either may be NULL) holds for all of them.  After the flush:
+ * TRM_ERR_STATE. */
+int TRMStreamSetVoice(TRMStream *stream, const TRMInputParameters *voice, int64_t *tube_sample, int64_t *output_sample);
 void TRMStreamFree(TRMStream *stream);
 
 /* ---------------------------------------------------------------------------------------------
@@ -380,6 +384,35 @@ int TRMStreamPoolPush(TRMStreamPool *pool, int n, const int32_t *slot, const int
 int TRMStreamPoolPushPCM16(TRMStreamPool *pool, int n, const int32_t *slot, const int32_t *n_frames,
                            const TRMParameters *frames, const uint8_t *flush, const double *peak,
                            int16_t *pcm_out, int64_t *pcm_offset /* [n + 1] */, double *max_out);
+/* Changes the voice of n distinct open slots (frame-fed or event-fed), effective from the next push: TRAcT's sliders on
+ * a stream that keeps playing.  Slot slot[i] continues with voice[i]; every piece of carried state (oscillator, noise,
+ * filter memories, tube waves, converter, pending frames) is kept, so the stream does not restart from silence.
+ *   What may change.  Any field, as long as the new voice derives the same rate constants as the slot's current voice:
+ *     control period, tube sample rate, converter increment and pad, channels (what a snapshot stores as "derived").  So
+ *     outputRate, controlRate, temperature, channels and the tract length stay (a length or temperature that rounds to
+ *     the same control period is accepted); changing the tract length is a new stream.  Everything else may change:
+ *     volume, balance, waveform, tp / tnMin / tnMax, breathiness, lossFactor, apScale, mouthCoef, noseCoef,
+ *     noseRadius[1..5], throatCutoff, throatVol, usesModulation, mixOffset.
+ *   Where it takes effect.  The tube model uses the new voice from tube-rate sample tube_sample[i] on: the first sample
+ *     the slot has not synthesized, floor16((frames pushed - 1) * controlPeriod) after two frames or more, else 0.  Frames
+ *     already pushed whose samples lie at or after it are synthesized with the new voice.  volume and balance apply to the
+ *     PCM16 of every output a later TRMStreamPoolPushPCM16 returns, from output sample output_sample[i] on; float samples
+ *     are unscaled, so they do not depend on them.  tube_sample and output_sample may be NULL.
+ *   Continuation.  A slot's pushes, concatenated, equal the synthesis of its frames with the voice schedule "opening voice
+ *     from sample 0, each new voice from its tube_sample", within the tolerance of the slot's TRM_PRECISION_* mode, and
+ *     the pushes after a change are bit-identical for any split of the frames over pushes.  One exception in FP32: that
+ *     mode carries the mouth and nose reflection memories multiplied by the damping factor, so across a change of
+ *     lossFactor they continue for one sample with the previous factor.  Measured against the exact schedule: about
+ *     80 dB SNR for 0.5 -> 5 % alone on 0.4 s at control period 63, 71-75 dB for random changes that include it, down
+ *     to 44-49 dB for a short stream (800 samples) at control period 8.  The FP64 modes have no such exception.
+ *     TRMStreamPoolSave / SaveAny store the current voice (TRMStreamPoolSnapshotInfo reports it) and a restore continues
+ *     with it, bit for bit; the snapshot format does not change.
+ *   Refusals.  All n entries are checked before anything changes, and a refused call leaves the pool exactly as it was:
+ *     an unopened slot (TRM_ERR_STATE); a slot named twice or a voice whose rate constants differ (TRM_ERR_PARAM); a voice
+ *     TRMBatchCreate refuses (its code).  A CUDA error while the glottal table rows go up (TRM_ERR_CUDA) leaves the pool's
+ *     contents undefined, as for a push. */
+int TRMStreamPoolSetVoice(TRMStreamPool *pool, int n, const int32_t *slot, const TRMInputParameters *voice /* [n] */,
+                          int64_t *tube_sample /* [n] or NULL */, int64_t *output_sample /* [n] or NULL */);
 void TRMStreamPoolFree(TRMStreamPool *pool);
 
 /* Snapshots: a live slot as a self-contained byte string that continues in any pool of the same precision, on any device,

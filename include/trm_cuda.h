@@ -189,6 +189,15 @@ int  trm_cuda_pool_open_events(trm_cuda_pool *p, const trm_cuda_utterance *voice
                                const trm_cuda_event *events, int64_t n_events, int64_t n_frames, const trm_cuda_framegen *fg,
                                int *slot);
 int  trm_cuda_pool_close(trm_cuda_pool *p, int slot);
+/* New voices for n distinct open slots (frame-fed or event-fed), effective from the next push: voice[i] replaces slot[i]'s
+ * descriptor template (voice[i].voice is ignored) and wavetables[i] (512 doubles) its glottal table row; the carried
+ * state, counters and pending frames are kept.  voice[i] must have the slot's rate constants (controlPeriod, sampleRate,
+ * tri, padSize, channels; else -4: the slot's buffers and counters are laid out for them).  tube_sample[i] /
+ * output_sample[i] (either may be NULL) receive the slot's first tube-rate sample and first output sample not yet
+ * synthesized: where the new voice starts.  The rows go up in one copy and are scattered on the device; the slots change
+ * only once that has finished. */
+int  trm_cuda_pool_set_voice(trm_cuda_pool *p, int n, const int32_t *slot, const trm_cuda_utterance *voice,
+                             const double *wavetables, int64_t *tube_sample, int64_t *output_sample);
 int64_t trm_cuda_pool_slot_capacity(const trm_cuda_pool *p);     /* samples one slot can return from one push */
 /* entry i: slot[i] gets n_frames[i] frames (taken back to back from frames_host, rows of 16 doubles; for a slot opened
  * with trm_cuda_pool_open_events, generated from its list instead -- -4 past the list's end); flush[i] != 0 ends
