@@ -106,7 +106,7 @@ extern "C" int trm_k_pcm_checksum(const trm_cuda_utterance *desc, int n_utt, con
 // ---- stream pool bookkeeping (trm_cuda_pool_push) ---------------------------------------------------------------------
 // One CTA per entry: its waveguide descriptor goes to the slot's place in the array the waveguide kernel indexes, and a
 // slot opened since its last launch gets a fresh carried state -- everything zero, the noise generator at its start, the
-// "no sample yet" flag set (what upload_plan writes on the host for a time split).
+// "no sample yet" flag set (the state a time-split batch chunk uploads with its tables).
 __global__ void pool_prepare_kernel(trm::PoolPrepArgs a)
 {
     const int e = blockIdx.x, slot = a.slot[e];

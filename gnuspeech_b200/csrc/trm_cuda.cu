@@ -94,14 +94,17 @@ int fail_msg(const char *what)
         if (_e != cudaSuccess) return fail(#call, _e);                                             \
     } while (0)
 
-constexpr int MAX_SLOTS = 16;  // upper bound of chunks in flight (each on its own stream and arena)
+constexpr int MAX_SLOTS = 16;  // upper bound of chunks in flight (each with its own arena, staging and events)
 constexpr int MAX_OUT_GROUPS = 4;   // output groups of a chunk (ChunkPlan::groups)
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// Parts of one packed buffer, each from a 256-byte boundary: the same offsets address the device scratch and its host image.
+struct Pack { size_t bytes = 0; size_t part(size_t n) { const size_t at = align_up(bytes, 256); bytes = at + n; return at; } };
+
 struct Arena {
     unsigned char *base = nullptr;
-    size_t cap = 0, used = 0;
+    size_t cap = 0;
     int reserve(size_t bytes)
     {
         if (bytes <= cap) return 0;
@@ -113,18 +116,11 @@ struct Arena {
         cap = bytes;
         return 0;
     }
-    void reset() { used = 0; }
-    void *take(size_t bytes)
-    {
-        size_t off = align_up(used, 256);
-        used = off + bytes;
-        return base + off;
-    }
     void release()
     {
         if (base) cudaFree(base);
         base = nullptr;
-        cap = used = 0;
+        cap = 0;
     }
 };
 
@@ -150,29 +146,8 @@ struct HostStage {
     }
 };
 
-// Everything one chunk needs on the device, carved from an arena.
-struct DeviceChunk {
-    int n = 0;
-    trm_cuda_utterance *desc = nullptr;
-    int *order = nullptr;
-    int *tile_utt = nullptr, *tile_nt = nullptr;
-    long long *tile_max_out = nullptr, *tile_first_out = nullptr, *item_base = nullptr;
-    unsigned long long *maxbits = nullptr;
-    double *frames = nullptr;               // (holds float32 rows when the plan says f32_frames: the kernels widen on read)
-    bool f32_frames = false;
-    void *tube = nullptr, *out = nullptr;
-    int16_t *pcm = nullptr;
-    long long total_items = 0, max_n_out = 0;
-    int n_tiles = 0;
-    int src_shape = 0;                      // resampler shape the tiles were built for (KernelInfo::src[])
-    // time split (ChunkPlan::split_frame > 0): descriptors of the two waveguide launches and the state carried between them
-    trm_cuda_utterance *desc_t[2] = {nullptr, nullptr};
-    void *state = nullptr;
-    size_t tube_elems = 0, out_elems = 0, pcm_elems = 0, frame_rows = 0;
-    const double *wavetables = nullptr;     // own copy of the glottal tables (device-resident batches); null = the context's
-};
-
-// Host-side plan of one chunk: rebased descriptors + where its spans live in the caller's arrays.
+// Host-side plan of one chunk: rebased descriptors, where its spans live in the caller's arrays, and where its parts live
+// in its device scratch.
 struct ChunkPlan {
     int u0 = 0, u1 = 0;
     std::vector<trm_cuda_utterance> desc;   // rebased to chunk-local offsets
@@ -184,8 +159,9 @@ struct ChunkPlan {
     long long frames_lo = 0;                // host frame index of the span start (dense case)
     size_t frame_rows = 0;
     long long tube_lo = 0, out_lo = 0, pcm_lo = 0;   // host element offsets of the spans
+    long long tube_n = 0, out_n = 0, pcm_n = 0;      // their lengths (what the copy-outs move)
     size_t tube_elems = 0, out_elems = 0, pcm_elems = 0;
-    int src_shape = 0;
+    int src_shape = 0;                      // resampler shape the tiles were built for (KernelInfo::src[])
     // Output groups: contiguous utterance ranges whose resampling + scaling is launched separately, so that the PCM of
     // one group can leave for the host while the next group is still being resampled (tiles never span groups).
     struct Group { int u_begin, u_end; long long item_begin, item_end, max_n_out, pcm_lo, pcm_hi; };
@@ -198,35 +174,15 @@ struct ChunkPlan {
     long long total_items = 0, max_n_out = 0;
     size_t n_tiles() const { return tile_nt.size(); }
     bool f32_frames = false;                // the caller's frames are float32 rows (64 bytes)
-    size_t arena_bytes(size_t esz, bool want_pcm) const
-    {
-        size_t n = desc.size(), b = 0;
-        auto add = [&](size_t x) { b = align_up(b, 256) + x; };
-        add(n * sizeof(trm_cuda_utterance));
-        add(n * sizeof(int));
-        add(tile_utt.size() * sizeof(int));
-        add(tile_nt.size() * sizeof(int));
-        add(tile_max_out.size() * sizeof(long long));
-        add(tile_first_out.size() * sizeof(long long));
-        add(item_base.size() * sizeof(long long));
-        add(n * sizeof(unsigned long long));
-        add(frame_rows * 128);
-        add(tube_elems * esz);
-        add(out_elems * esz);
-        if (want_pcm) add(pcm_elems * sizeof(int16_t));
-        if (split_frame > 0) { add(n * sizeof(trm_cuda_utterance)); add(n * sizeof(trm_cuda_utterance)); add(n * trm::tube_state_bytes(esz)); }
-        return b + 256;
-    }
-    size_t stage_bytes() const
-    {
-        size_t n = desc.size();
-        return align_up(n * sizeof(trm_cuda_utterance), 256) + align_up(n * sizeof(int), 256) +
-               align_up(tile_utt.size() * sizeof(int), 256) + align_up(tile_nt.size() * sizeof(int), 256) +
-               align_up(tile_max_out.size() * sizeof(long long), 256) + align_up(tile_first_out.size() * sizeof(long long), 256) +
-               align_up(item_base.size() * sizeof(long long), 256) +
-               (split_frame > 0 ? 2 * align_up(n * sizeof(trm_cuda_utterance), 256) + align_up(n * trm::tube_state_bytes(8), 256) : 0) +
-               align_up(n * sizeof(unsigned long long), 256);     // (last: the maxima come back here)
-    }
+    // Byte offsets of the parts in the chunk's device scratch (chunk_layout).  The uploaded tables come first, [0, up):
+    // the pinned staging holds them at the same offsets and receives the maxima back at theirs.  The frame part holds
+    // float32 rows when f32_frames (the kernels widen on read); the PCM part exists when want_pcm.
+    struct Offsets {
+        size_t desc, order, tile_utt, tile_nt, tile_max_out, tile_first_out, item_base, desc_t[2], state;
+        size_t maxbits, frames, tube, out, pcm;
+    } at{};
+    size_t up = 0, arena = 0, stage = 0;
+    bool want_pcm = false;
 };
 
 }  // namespace
@@ -254,7 +210,7 @@ struct trm_cuda_ctx {
     uint64_t noise_k0 = 0;
     trm::KernelInfo info[3]{};        // by precision code
     const trm::KernelInfo &ki(int precision) const { return info[precision]; }
-    cudaStream_t streams[MAX_SLOTS]{};
+    cudaStream_t s_out = nullptr;     // copy-out of the chunk pipeline; also wavetable, frame generator and sweep work
     Arena arenas[MAX_SLOTS];
     HostStage stages[MAX_SLOTS];
     int n_slots = 3;              // chunks in flight: one uploading, one computing, one downloading
@@ -268,7 +224,6 @@ struct trm_cuda_resident {
     int precision = 0;
     ChunkPlan plan;
     Arena arena;
-    DeviceChunk dc;
     double *d_wavetables = nullptr;     // the batch's glottal tables: the context's set may be replaced by later calls
 };
 
@@ -309,6 +264,7 @@ int plan_chunk(const trm_cuda_utterance *desc, int u0, int u1, const trm::Kernel
     p.frames_dense = (f_hi - f_lo) <= f_sum + f_sum / 2 + 64;
     p.frames_lo = f_lo;
     p.tube_lo = t_lo; p.out_lo = o_lo; p.pcm_lo = c_lo;
+    p.tube_n = t_hi - t_lo; p.out_n = o_hi - o_lo; p.pcm_n = c_hi - c_lo;
     p.tube_elems = (size_t)align_up((size_t)(t_hi - t_lo), TRM_ALIGN_ELEMS);
     p.out_elems = (size_t)align_up((size_t)(o_hi - o_lo), TRM_ALIGN_ELEMS);
     p.pcm_elems = (size_t)align_up((size_t)(c_hi - c_lo), TRM_ALIGN_ELEMS);
@@ -438,86 +394,76 @@ void arm_time_split(ChunkPlan &p, int f1)
     }
 }
 
-void carve(Arena &a, const ChunkPlan &p, size_t esz, bool want_pcm, DeviceChunk &dc)
+// Lays out the chunk's device scratch (ChunkPlan::at), once the plan and its time split are final.
+void chunk_layout(ChunkPlan &p, size_t esz, bool want_pcm)
 {
     const size_t n = p.desc.size();
-    a.reset();
-    dc.n = (int)n;
-    dc.desc = (trm_cuda_utterance *)a.take(n * sizeof(trm_cuda_utterance));
-    dc.order = (int *)a.take(n * sizeof(int));
-    dc.tile_utt = (int *)a.take(p.tile_utt.size() * sizeof(int));
-    dc.tile_nt = (int *)a.take(p.tile_nt.size() * sizeof(int));
-    dc.tile_max_out = (long long *)a.take(p.tile_max_out.size() * sizeof(long long));
-    dc.tile_first_out = (long long *)a.take(p.tile_first_out.size() * sizeof(long long));
-    dc.item_base = (long long *)a.take(p.item_base.size() * sizeof(long long));
-    dc.maxbits = (unsigned long long *)a.take(n * sizeof(unsigned long long));
-    dc.frames = (double *)a.take(p.frame_rows * 128);
-    dc.f32_frames = p.f32_frames;
-    dc.tube = a.take(p.tube_elems * esz);
-    dc.out = a.take(p.out_elems * esz);
-    dc.pcm = want_pcm ? (int16_t *)a.take(p.pcm_elems * sizeof(int16_t)) : nullptr;
+    ChunkPlan::Offsets &o = p.at;
+    o = {};
+    Pack pk;
+    o.desc = pk.part(n * sizeof(trm_cuda_utterance));
+    o.order = pk.part(n * sizeof(int));
+    o.tile_utt = pk.part(p.tile_utt.size() * sizeof(int));
+    o.tile_nt = pk.part(p.tile_nt.size() * sizeof(int));
+    o.tile_max_out = pk.part(p.tile_max_out.size() * sizeof(long long));
+    o.tile_first_out = pk.part(p.tile_first_out.size() * sizeof(long long));
+    o.item_base = pk.part(p.item_base.size() * sizeof(long long));
     if (p.split_frame > 0) {
-        dc.desc_t[0] = (trm_cuda_utterance *)a.take(n * sizeof(trm_cuda_utterance));
-        dc.desc_t[1] = (trm_cuda_utterance *)a.take(n * sizeof(trm_cuda_utterance));
-        dc.state = a.take(n * trm::tube_state_bytes(esz));
-    } else {
-        dc.desc_t[0] = dc.desc_t[1] = nullptr;
-        dc.state = nullptr;
+        o.desc_t[0] = pk.part(n * sizeof(trm_cuda_utterance));
+        o.desc_t[1] = pk.part(n * sizeof(trm_cuda_utterance));
+        o.state = pk.part(n * trm::tube_state_bytes(esz));
     }
-    dc.total_items = p.total_items;
-    dc.n_tiles = (int)p.n_tiles();
-    dc.src_shape = p.src_shape;
-    dc.max_n_out = p.max_n_out;
-    dc.tube_elems = p.tube_elems; dc.out_elems = p.out_elems; dc.pcm_elems = p.pcm_elems; dc.frame_rows = p.frame_rows;
+    p.up = pk.bytes;
+    o.maxbits = pk.part(n * sizeof(unsigned long long));
+    p.stage = pk.bytes;
+    o.frames = pk.part(p.frame_rows * 128);
+    o.tube = pk.part(p.tube_elems * esz);
+    o.out = pk.part(p.out_elems * esz);
+    if (want_pcm) o.pcm = pk.part(p.pcm_elems * sizeof(int16_t));
+    p.arena = pk.bytes;
+    p.want_pcm = want_pcm;
 }
 
-// small tables (descriptors, order, tile prefix) -> device, through pinned staging when given
-int upload_plan(const ChunkPlan &p, const DeviceChunk &dc, unsigned char *stage, cudaStream_t s, size_t esz = 8, unsigned long long noise_k0 = 0)
+// The chunk's tables ([0, up) of its layout) -> device in one copy: through the pinned staging `stage` (the pipeline's:
+// the copy stays asynchronous), or through a pageable image when there is none.
+int upload_plan(const ChunkPlan &p, unsigned char *base, unsigned char *stage, cudaStream_t s, size_t esz = 8, unsigned long long noise_k0 = 0)
 {
     const size_t n = p.desc.size();
     if (n == 0) return 0;
-    unsigned char *q = stage;
-    auto put = [&](void *dst, const void *src, size_t bytes) -> int {
-        if (bytes == 0) return 0;
-        const void *from = src;
-        if (stage) {                       // pinned staging keeps the copy asynchronous
-            memcpy(q, src, bytes);
-            from = q;
-            q += align_up(bytes, 256);
-        }
-        CK(cudaMemcpyAsync(dst, from, bytes, cudaMemcpyHostToDevice, s));
-        return 0;
-    };
-    int rc;
-    if ((rc = put(dc.desc, p.desc.data(), n * sizeof(trm_cuda_utterance))) != 0) return rc;
-    if ((rc = put(dc.order, p.order.data(), n * sizeof(int))) != 0) return rc;
-    if ((rc = put(dc.tile_utt, p.tile_utt.data(), p.tile_utt.size() * sizeof(int))) != 0) return rc;
-    if ((rc = put(dc.tile_nt, p.tile_nt.data(), p.tile_nt.size() * sizeof(int))) != 0) return rc;
-    if ((rc = put(dc.tile_max_out, p.tile_max_out.data(), p.tile_max_out.size() * sizeof(long long))) != 0) return rc;
-    if ((rc = put(dc.tile_first_out, p.tile_first_out.data(), p.tile_first_out.size() * sizeof(long long))) != 0) return rc;
-    if ((rc = put(dc.item_base, p.item_base.data(), p.item_base.size() * sizeof(long long))) != 0) return rc;
-    if (p.split_frame > 0 && dc.state) {
-        if ((rc = put(dc.desc_t[0], p.desc_t[0].data(), n * sizeof(trm_cuda_utterance))) != 0) return rc;
-        if ((rc = put(dc.desc_t[1], p.desc_t[1].data(), n * sizeof(trm_cuda_utterance))) != 0) return rc;
+    std::vector<unsigned char> image;
+    if (!stage) {
+        image.resize(p.up);
+        stage = image.data();
+    }
+    auto put = [&](size_t at, const void *src, size_t bytes) { if (bytes) memcpy(stage + at, src, bytes); };
+    put(p.at.desc, p.desc.data(), n * sizeof(trm_cuda_utterance));
+    put(p.at.order, p.order.data(), n * sizeof(int));
+    put(p.at.tile_utt, p.tile_utt.data(), p.tile_utt.size() * sizeof(int));
+    put(p.at.tile_nt, p.tile_nt.data(), p.tile_nt.size() * sizeof(int));
+    put(p.at.tile_max_out, p.tile_max_out.data(), p.tile_max_out.size() * sizeof(long long));
+    put(p.at.tile_first_out, p.tile_first_out.data(), p.tile_first_out.size() * sizeof(long long));
+    put(p.at.item_base, p.item_base.data(), p.item_base.size() * sizeof(long long));
+    if (p.split_frame > 0) {
+        put(p.at.desc_t[0], p.desc_t[0].data(), n * sizeof(trm_cuda_utterance));
+        put(p.at.desc_t[1], p.desc_t[1].data(), n * sizeof(trm_cuda_utterance));
         // fresh recurrence state: everything zero, noise generator at its start, "no sample yet" flag set
         const size_t sb = trm::tube_state_bytes(esz);
-        std::vector<unsigned char> init(n * sb, 0);
+        memset(stage + p.at.state, 0, n * sb);
         for (size_t u = 0; u < n; ++u) {
-            unsigned long long *h = (unsigned long long *)(init.data() + u * sb);
+            unsigned long long *h = (unsigned long long *)(stage + p.at.state + u * sb);
             h[2] = noise_k0;
             h[3] = 1ull;
         }
-        if ((rc = put(dc.state, init.data(), init.size())) != 0) return rc;
     }
+    CK(cudaMemcpyAsync(base, stage, p.up, cudaMemcpyHostToDevice, s));
     return 0;
 }
 
-int upload_frames(const ChunkPlan &p, const DeviceChunk &dc, const trm_cuda_utterance *desc_global,
-                  const void *frames_host, cudaStream_t s)
+int upload_frames(const ChunkPlan &p, unsigned char *base, const trm_cuda_utterance *desc_global, const void *frames_host, cudaStream_t s)
 {
     if (p.frame_rows == 0) return 0;
     const size_t row = p.f32_frames ? 64 : 128;                     // bytes per frame in the caller's array and on the device
-    unsigned char *dst = (unsigned char *)dc.frames;
+    unsigned char *dst = base + p.at.frames;
     const unsigned char *src = (const unsigned char *)frames_host;
     if (p.frames_dense) {
         CK(cudaMemcpyAsync(dst, src + (size_t)p.frames_lo * row, p.frame_rows * row, cudaMemcpyDefault, s));
@@ -542,40 +488,48 @@ int wide_groups(const trm_cuda_ctx *ctx, const trm::KernelInfo &ki, int n)
     return waves * sm;
 }
 
-int launch_stage(trm_cuda_ctx *ctx, int precision, int stage, const DeviceChunk &dc, cudaStream_t s, const ChunkPlan::Group *grp = nullptr,
-                 int time_part = -1)
+// One kernel stage of a planned chunk whose scratch starts at `base`; `wavetables` overrides the context's glottal tables
+// (device-resident batches keep their own copy), null = the context's.
+int launch_stage(trm_cuda_ctx *ctx, int precision, int stage, const ChunkPlan &p, unsigned char *base, const double *wavetables,
+                 cudaStream_t s, const ChunkPlan::Group *grp = nullptr, int time_part = -1)
 {
     const bool f64 = prec_is_f64(precision);
     const KernelSet &K = g_kernels[precision];
+    const int n = (int)p.desc.size();
+    const auto *desc = (const trm_cuda_utterance *)(base + p.at.desc);
+    auto *maxbits = (unsigned long long *)(base + p.at.maxbits);
     int rc = 0;
     if (stage == TRM_STAGE_TUBE) {
         trm::TubeArgs a{};
-        a.desc = dc.desc; a.order = dc.order; a.n_utt = dc.n; a.frames = dc.frames; a.frames_f32 = dc.f32_frames ? 1 : 0; a.tube = dc.tube;
-        a.wavetables = dc.wavetables ? dc.wavetables : ctx->d_wavetables; a.noise_k0 = ctx->noise_k0;
-        if (time_part >= 0) { a.desc = dc.desc_t[time_part]; a.state = dc.state; }     // (lane-per-utterance mapping only)
+        a.desc = desc; a.order = (const int *)(base + p.at.order); a.n_utt = n; a.frames = base + p.at.frames;
+        a.frames_f32 = p.f32_frames ? 1 : 0; a.tube = base + p.at.tube;
+        a.wavetables = wavetables ? wavetables : ctx->d_wavetables; a.noise_k0 = ctx->noise_k0;
+        // time split: launch time_part's descriptors, the recurrence state carried from launch 0 to launch 1
+        if (time_part >= 0) { a.desc = (const trm_cuda_utterance *)(base + p.at.desc_t[time_part]); a.state = base + p.at.state; }
         const trm::KernelInfo &ki = ctx->ki(precision);
-        const int groups = wide_groups(ctx, ki, dc.n);
+        const int groups = wide_groups(ctx, ki, n);
         if (groups > 0) rc = K.tube_wide(&a, groups, s);
     } else if (stage == TRM_STAGE_SRC) {
         // (the running maxima are cleared once per chunk: by the ungrouped launch, or by the first group's)
-        if (!grp || grp->u_begin == 0) CK(cudaMemsetAsync(dc.maxbits, 0, (size_t)dc.n * sizeof(unsigned long long), s));
+        if (!grp || grp->u_begin == 0) CK(cudaMemsetAsync(maxbits, 0, (size_t)n * sizeof(unsigned long long), s));
         trm::SrcArgs a{};
-        a.desc = dc.desc; a.n_utt = dc.n; a.tube = dc.tube; a.out = dc.out; a.maxbits = dc.maxbits;
+        a.desc = desc; a.n_utt = n; a.tube = base + p.at.tube; a.out = base + p.at.out; a.maxbits = maxbits;
         a.table = f64 ? ctx->d_tab_f64 : ctx->d_tab_f32;
         a.ctab = f64 ? ctx->d_ctab_f64 : ctx->d_ctab_f32;
-        a.tile_utt = dc.tile_utt; a.tile_nt = dc.tile_nt; a.tile_max_out = dc.tile_max_out; a.tile_first_out = dc.tile_first_out;
-        a.item_base = dc.item_base;
-        a.n_tiles = dc.n_tiles; a.total_items = dc.total_items;
+        a.tile_utt = (const int *)(base + p.at.tile_utt); a.tile_nt = (const int *)(base + p.at.tile_nt);
+        a.tile_max_out = (const long long *)(base + p.at.tile_max_out); a.tile_first_out = (const long long *)(base + p.at.tile_first_out);
+        a.item_base = (const long long *)(base + p.at.item_base);
+        a.n_tiles = (int)p.n_tiles(); a.total_items = p.total_items;
         if (grp) { a.item_begin = grp->item_begin; a.item_end = grp->item_end; if (a.item_end <= a.item_begin) return 0; }
         const trm::KernelInfo &ki = ctx->ki(precision);
-        const int grid = ctx->sm_count * std::max(1, ki.src[dc.src_shape].ctas_per_sm);
-        rc = K.src(&a, grid, dc.src_shape, s);
+        const int grid = ctx->sm_count * std::max(1, ki.src[p.src_shape].ctas_per_sm);
+        rc = K.src(&a, grid, p.src_shape, s);
     } else if (stage == TRM_STAGE_PCM) {
-        if (!dc.pcm) return 0;
+        if (!p.want_pcm) return 0;
         trm::PcmArgs a{};
-        a.desc = dc.desc; a.n_utt = grp ? grp->u_end : dc.n; a.u_begin = grp ? grp->u_begin : 0;
-        a.out = dc.out; a.maxbits = dc.maxbits; a.pcm = dc.pcm;
-        const long long longest = grp ? grp->max_n_out : dc.max_n_out;
+        a.desc = desc; a.n_utt = grp ? grp->u_end : n; a.u_begin = grp ? grp->u_begin : 0;
+        a.out = base + p.at.out; a.maxbits = maxbits; a.pcm = (int16_t *)(base + p.at.pcm);
+        const long long longest = grp ? grp->max_n_out : p.max_n_out;
         rc = K.pcm(&a, longest, s);
     }
     if (rc != 0) return fail("kernel launch", (cudaError_t)rc);
@@ -619,10 +573,11 @@ extern "C" {
 
 const char *trm_cuda_last_error(void) { return g_err.c_str(); }
 
-// The pipeline keeps up to MAX_SLOTS streams busy; with the default of 8 hardware work queues, streams alias
-// onto the same queue and one chunk's kernels wait behind another chunk's copies.  Must be set before the
-// CUDA context exists, so it is done on the first entry into the library (no effect if the host application
-// already initialised CUDA: such callers set CUDA_DEVICE_MAX_CONNECTIONS=32 themselves).
+// A device's copy-in and compute queues, the copy-out stream of each of its contexts and each stream pool's stream are
+// busy at once; with the default of 8 hardware work queues, streams alias onto the same queue and one chunk's kernels
+// wait behind another chunk's copies.  Must be set before the CUDA context exists, so it is done on the first entry
+// into the library (no effect if the host application already initialised CUDA: such callers set
+// CUDA_DEVICE_MAX_CONNECTIONS=32 themselves).
 static void want_many_connections() { setenv("CUDA_DEVICE_MAX_CONNECTIONS", "32", 0); }
 
 int trm_cuda_device_count(void)
@@ -676,8 +631,6 @@ int trm_cuda_fp_peak(int device, int precision, int reps, double *tflops)
     return 0;
 }
 
-int trm_cuda_stage_launches(int stage) { return (stage >= 0 && stage < TRM_STAGE_COUNT) ? 1 : 0; }
-
 int trm_cuda_ctx_create(int device, const trm_cuda_tables *t, trm_cuda_ctx **out)
 {
     *out = nullptr;
@@ -728,7 +681,7 @@ int trm_cuda_ctx_create(int device, const trm_cuda_tables *t, trm_cuda_ctx **out
         CK(cudaDeviceSynchronize());
     }
     {
-        // streams[2] = copy-out of the chunk pipeline (trm_cuda_synthesize_host); frames and kernels go to the device's
+        // s_out = copy-out of the chunk pipeline (trm_cuda_synthesize_host); frames and kernels go to the device's
         // shared copy-in and compute queues
         {
             std::lock_guard<std::mutex> lk(g_run_mu[device]);
@@ -737,11 +690,10 @@ int trm_cuda_ctx_create(int device, const trm_cuda_tables *t, trm_cuda_ctx **out
         }
         int lo = 0, hi = 0;
         CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));          // lo = least (numerically largest)
+        CK(cudaStreamCreateWithPriority(&c->s_out, cudaStreamNonBlocking, std::min(lo, hi + 2)));
         const char *env = getenv("TRM_SLOTS");
         if (env && atoi(env) > 0) c->n_slots = std::min(MAX_SLOTS, atoi(env));
         for (int i = 0; i < MAX_SLOTS; ++i) {
-            const int prio = std::min(lo, hi + i);
-            CK(cudaStreamCreateWithPriority(&c->streams[i], cudaStreamNonBlocking, prio));
             CK(cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&c->ev_run[i], cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&c->ev_out[i], cudaEventDisableTiming));
@@ -761,7 +713,7 @@ int trm_cuda_set_wavetables(trm_cuda_ctx *c, const double *tables, int n_voices)
     // no synchronisation that would serialise this call behind another lane's work on the same device
     if (c->wt_host.size() == n && memcmp(c->wt_host.data(), tables, n * sizeof(double)) == 0) return 0;
     CK(cudaSetDevice(c->device));
-    for (int i = 0; i < 3; ++i) CK(cudaStreamSynchronize(c->streams[i]));   // this context's own work only
+    CK(cudaStreamSynchronize(c->s_out));   // this context's own work only
     if (n_voices > c->wt_capacity) {
         if (c->d_wavetables) cudaFree(c->d_wavetables);
         c->d_wavetables = nullptr;
@@ -779,7 +731,7 @@ void trm_cuda_ctx_destroy(trm_cuda_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    for (auto &s : c->streams) if (s) cudaStreamDestroy(s);
+    if (c->s_out) cudaStreamDestroy(c->s_out);
     for (int i = 0; i < MAX_SLOTS; ++i) {
         if (c->ev_in[i]) cudaEventDestroy(c->ev_in[i]);
         if (c->ev_run[i]) cudaEventDestroy(c->ev_run[i]);
@@ -798,25 +750,9 @@ void trm_cuda_ctx_destroy(trm_cuda_ctx *c)
     delete c;
 }
 
-int trm_cuda_synthesize_host(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,
-                             const double *frames_host, int16_t *pcm_host, void *samples_host, double *max_host,
-                             void *tube_host, int64_t *launches)
-{
-    return trm_cuda_synthesize_host_ex(ctx, precision, n, desc, frames_host, pcm_host, samples_host, max_host, tube_host, launches,
-                                       nullptr, nullptr);
-}
-
-int trm_cuda_synthesize_host_ex(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,
-                                const double *frames_host, int16_t *pcm_host, void *samples_host, double *max_host,
-                                void *tube_host, int64_t *launches, void (*enqueued)(void *), void *enqueued_arg)
-{
-    return trm_cuda_synthesize_host_fmt(ctx, precision, 0, n, desc, frames_host, pcm_host, samples_host, max_host, tube_host, launches,
-                                        enqueued, enqueued_arg);
-}
-
-int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_format, int n, const trm_cuda_utterance *desc,
-                                 const void *frames_host, int16_t *pcm_host, void *samples_host, double *max_host,
-                                 void *tube_host, int64_t *launches, void (*enqueued)(void *), void *enqueued_arg)
+int trm_cuda_synthesize_host(trm_cuda_ctx *ctx, int precision, int frame_format, int n, const trm_cuda_utterance *desc,
+                             const void *frames_host, int16_t *pcm_host, void *samples_host, double *max_host,
+                             void *tube_host, int64_t *launches, void (*enqueued)(void *), void *enqueued_arg)
 {
     if (frame_format != 0 && frame_format != 1) return fail_msg("unknown frame format");
     const bool f32_frames = frame_format == 1;
@@ -832,7 +768,7 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
     // Three-stage pipeline over chunks: frames go up on the copy-in stream, the three kernels of a chunk run on the
     // compute stream (one chunk at a time: a waveguide launch fills every SM), PCM / samples come back on the copy-out
     // stream.  H2D of chunk k+1 and D2H of chunk k-1 overlap the kernels of chunk k (full-duplex PCIe).
-    cudaStream_t s_in = g_in_stream[ctx->device], s_run = g_run_stream[ctx->device], s_out = ctx->streams[2];
+    cudaStream_t s_in = g_in_stream[ctx->device], s_run = g_run_stream[ctx->device], s_out = ctx->s_out;
     // TRM_TRACE=1: per-chunk timeline of the pipeline stages (CUDA events), printed to stderr
     const bool trace = getenv("TRM_TRACE") != nullptr;
     std::vector<cudaEvent_t> tev;
@@ -862,8 +798,7 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
         const int ci = slot_chunk[slot];
         if (ci >= 0 && max_host) {
             const ChunkPlan &p = plans[slot];
-            const unsigned long long *mb =
-                (const unsigned long long *)(ctx->stages[slot].base + p.stage_bytes() - align_up(p.desc.size() * sizeof(unsigned long long), 256));
+            const unsigned long long *mb = (const unsigned long long *)(ctx->stages[slot].base + p.at.maxbits);
             for (size_t i = 0; i < p.desc.size(); ++i) {
                 double v;
                 memcpy(&v, &mb[i], sizeof v);
@@ -908,24 +843,24 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
             wide_groups(ctx, ctx->ki(precision), u1 - u0) > 0)
             arm_time_split(p, std::max(64, (int)(0.28 * p.uniform_frames)));
         const bool split = p.split_frame > 0;
-        RCD(ctx->arenas[slot].reserve(p.arena_bytes(esz, want_pcm)));
-        RCD(ctx->stages[slot].reserve(p.stage_bytes()));
-        DeviceChunk dc;
-        carve(ctx->arenas[slot], p, esz, want_pcm, dc);
+        chunk_layout(p, esz, want_pcm);
+        RCD(ctx->arenas[slot].reserve(p.arena));
+        RCD(ctx->stages[slot].reserve(p.stage));
+        unsigned char *base = ctx->arenas[slot].base;
         // ---- copy-in -----------------------------------------------------------------------------------------
         {
             std::lock_guard<std::mutex> lk(g_in_mu[ctx->device]);
             mark(s_in);
-            RCD(upload_plan(p, dc, ctx->stages[slot].base, s_in, esz, ctx->noise_k0));
+            RCD(upload_plan(p, base, ctx->stages[slot].base, s_in, esz, ctx->noise_k0));
             if (!split) {
-                RCD(upload_frames(p, dc, desc, frames_host, s_in));
+                RCD(upload_frames(p, base, desc, frames_host, s_in));
                 CKD(cudaEventRecord(ctx->ev_in[slot], s_in));
             } else {
                 // frames [0, f1] of every utterance, then the rest: two strided copies
                 const size_t row = f32_frames ? 64 : 128;
                 const size_t pitch = (size_t)p.uniform_frames * row, first = (size_t)(p.split_frame + 1) * row;
                 const unsigned char *src = (const unsigned char *)frames_host + (size_t)p.frames_lo * row;
-                unsigned char *dst = (unsigned char *)dc.frames;
+                unsigned char *dst = base + p.at.frames;
                 CKD(cudaMemcpy2DAsync(dst, pitch, src, pitch, first, (size_t)(u1 - u0), cudaMemcpyDefault, s_in));
                 CKD(cudaEventRecord(ctx->ev_in[slot], s_in));
                 CKD(cudaMemcpy2DAsync(dst + first, pitch, src + first, pitch, pitch - first, (size_t)(u1 - u0), cudaMemcpyDefault, s_in));
@@ -938,18 +873,18 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
             std::lock_guard<std::mutex> lk(g_run_mu[ctx->device]);
             CKD(cudaStreamWaitEvent(s_run, ctx->ev_in[slot], 0));
             auto waveguide = [&]() -> int {
-                if (!split) { ++n_launch; return launch_stage(ctx, precision, TRM_STAGE_TUBE, dc, s_run); }
-                int r = launch_stage(ctx, precision, TRM_STAGE_TUBE, dc, s_run, nullptr, 0);
+                if (!split) { ++n_launch; return launch_stage(ctx, precision, TRM_STAGE_TUBE, p, base, nullptr, s_run); }
+                int r = launch_stage(ctx, precision, TRM_STAGE_TUBE, p, base, nullptr, s_run, nullptr, 0);
                 if (r != 0) return r;
                 CKD(cudaStreamWaitEvent(s_run, ctx->ev_in2[slot], 0));
                 n_launch += 2;
-                return launch_stage(ctx, precision, TRM_STAGE_TUBE, dc, s_run, nullptr, 1);
+                return launch_stage(ctx, precision, TRM_STAGE_TUBE, p, base, nullptr, s_run, nullptr, 1);
             };
             if (!grouped) {
                 for (int st = 0; st < TRM_STAGE_COUNT; ++st) {
                     if (st == TRM_STAGE_PCM && !want_pcm) { mark(s_run); continue; }
                     if (st == TRM_STAGE_TUBE) rc = waveguide();
-                    else { rc = launch_stage(ctx, precision, st, dc, s_run); ++n_launch; }
+                    else { rc = launch_stage(ctx, precision, st, p, base, nullptr, s_run); ++n_launch; }
                     if (rc != 0) { drain(); return rc; }
                     mark(s_run);
                 }
@@ -959,9 +894,9 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
                 RCD(waveguide());
                 mark(s_run);
                 for (size_t g = 0; g < p.groups.size(); ++g) {
-                    RCD(launch_stage(ctx, precision, TRM_STAGE_SRC, dc, s_run, &p.groups[g]));
+                    RCD(launch_stage(ctx, precision, TRM_STAGE_SRC, p, base, nullptr, s_run, &p.groups[g]));
                     if (g + 1 == p.groups.size()) mark(s_run);
-                    RCD(launch_stage(ctx, precision, TRM_STAGE_PCM, dc, s_run, &p.groups[g]));
+                    RCD(launch_stage(ctx, precision, TRM_STAGE_PCM, p, base, nullptr, s_run, &p.groups[g]));
                     CKD(cudaEventRecord(ctx->ev_grp[slot][g], s_run));
                     n_launch += 2;
                 }
@@ -970,35 +905,29 @@ int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_for
             CKD(cudaEventRecord(ctx->ev_run[slot], s_run));
         }
         // ---- copy-out ----------------------------------------------------------------------------------------
+        const int16_t *d_pcm = (const int16_t *)(base + p.at.pcm);
         if (grouped) {
             for (size_t g = 0; g < p.groups.size(); ++g) {
                 const ChunkPlan::Group &grp = p.groups[g];
                 CKD(cudaStreamWaitEvent(s_out, ctx->ev_grp[slot][g], 0));
                 if (grp.pcm_hi > grp.pcm_lo)
-                    CKD(cudaMemcpyAsync(pcm_host + p.pcm_lo + grp.pcm_lo, dc.pcm + grp.pcm_lo, (size_t)(grp.pcm_hi - grp.pcm_lo) * sizeof(int16_t),
+                    CKD(cudaMemcpyAsync(pcm_host + p.pcm_lo + grp.pcm_lo, d_pcm + grp.pcm_lo, (size_t)(grp.pcm_hi - grp.pcm_lo) * sizeof(int16_t),
                                        cudaMemcpyDeviceToHost, s_out));
             }
         }
         CKD(cudaStreamWaitEvent(s_out, ctx->ev_run[slot], 0));
-        if (!grouped && want_pcm && p.pcm_elems) {
-            long long c_hi = 0;
-            for (const auto &d : p.desc) c_hi = std::max<long long>(c_hi, d.pcm_offset + d.n_out * d.channels);
-            CKD(cudaMemcpyAsync(pcm_host + p.pcm_lo, dc.pcm, (size_t)c_hi * sizeof(int16_t), cudaMemcpyDeviceToHost, s_out));
-        }
-        if (samples_host && p.out_elems) {
-            long long o_hi = 0;
-            for (const auto &d : p.desc) o_hi = std::max<long long>(o_hi, d.out_offset + d.n_out);
-            CKD(cudaMemcpyAsync((unsigned char *)samples_host + (size_t)p.out_lo * esz, dc.out, (size_t)o_hi * esz, cudaMemcpyDeviceToHost, s_out));
-        }
-        if (tube_host && p.tube_elems) {
-            long long t_hi = 0;
-            for (const auto &d : p.desc) t_hi = std::max<long long>(t_hi, d.tube_offset + d.n_tube);
-            CKD(cudaMemcpyAsync((unsigned char *)tube_host + (size_t)p.tube_lo * esz, dc.tube, (size_t)t_hi * esz, cudaMemcpyDeviceToHost, s_out));
-        }
-        if (max_host) {
-            unsigned char *mb = ctx->stages[slot].base + p.stage_bytes() - align_up(p.desc.size() * sizeof(unsigned long long), 256);
-            CKD(cudaMemcpyAsync(mb, dc.maxbits, p.desc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s_out));
-        }
+        if (!grouped && want_pcm && p.pcm_n)
+            CKD(cudaMemcpyAsync(pcm_host + p.pcm_lo, d_pcm, (size_t)p.pcm_n * sizeof(int16_t), cudaMemcpyDeviceToHost, s_out));
+        if (samples_host && p.out_n)
+            CKD(cudaMemcpyAsync((unsigned char *)samples_host + (size_t)p.out_lo * esz, base + p.at.out, (size_t)p.out_n * esz,
+                                cudaMemcpyDeviceToHost, s_out));
+        if (tube_host && p.tube_n)
+            CKD(cudaMemcpyAsync((unsigned char *)tube_host + (size_t)p.tube_lo * esz, base + p.at.tube, (size_t)p.tube_n * esz,
+                                cudaMemcpyDeviceToHost, s_out));
+        // the maxima come back into the staging at their device offset
+        if (max_host)
+            CKD(cudaMemcpyAsync(ctx->stages[slot].base + p.at.maxbits, base + p.at.maxbits, p.desc.size() * sizeof(unsigned long long),
+                                cudaMemcpyDeviceToHost, s_out));
         CKD(cudaEventRecord(ctx->ev_out[slot], s_out));
         mark(s_out);
         slot_chunk[slot] = ci;
@@ -1040,22 +969,23 @@ int trm_cuda_generate_frames(trm_cuda_ctx *ctx, int n, const trm_cuda_utterance 
     }
     const size_t n_fg = shared_fg ? 1 : (size_t)n;
     std::vector<long long> off(ev_offset, ev_offset + n);
-    size_t bytes = 0;
-    auto add = [&](size_t x) { bytes = align_up(bytes, 256) + x; };
-    add((size_t)n * sizeof(trm_cuda_utterance)); add((size_t)n_events * sizeof(trm_cuda_event)); add((size_t)n * sizeof(long long));
-    add((size_t)n * sizeof(int)); add(n_fg * sizeof(trm_cuda_framegen)); add((size_t)n * sizeof(float)); add((size_t)frames_hi * 128);
+    Pack pk;
+    const size_t o_desc = pk.part((size_t)n * sizeof(trm_cuda_utterance)), o_ev = pk.part((size_t)n_events * sizeof(trm_cuda_event)),
+                 o_off = pk.part((size_t)n * sizeof(long long)), o_cnt = pk.part((size_t)n * sizeof(int)),
+                 o_fg = pk.part(n_fg * sizeof(trm_cuda_framegen)), o_seed = pk.part((size_t)n * sizeof(float)),
+                 o_frames = pk.part((size_t)frames_hi * 128);
     int rc;
-    if ((rc = ctx->gen.reserve(bytes + 256)) != 0) return rc;
-    ctx->gen.reset();
+    if ((rc = ctx->gen.reserve(pk.bytes + 256)) != 0) return rc;
     trm::FrameGenArgs a{};
-    auto *d_desc = (trm_cuda_utterance *)ctx->gen.take((size_t)n * sizeof(trm_cuda_utterance));
-    auto *d_ev = (trm_cuda_event *)ctx->gen.take((size_t)n_events * sizeof(trm_cuda_event));
-    auto *d_off = (long long *)ctx->gen.take((size_t)n * sizeof(long long));
-    auto *d_cnt = (int *)ctx->gen.take((size_t)n * sizeof(int));
-    auto *d_fg = (trm_cuda_framegen *)ctx->gen.take(n_fg * sizeof(trm_cuda_framegen));
-    auto *d_seed = (float *)ctx->gen.take((size_t)n * sizeof(float));
-    auto *d_frames = (double *)ctx->gen.take((size_t)frames_hi * 128);
-    cudaStream_t s = ctx->streams[2];
+    unsigned char *d = ctx->gen.base;
+    auto *d_desc = (trm_cuda_utterance *)(d + o_desc);
+    auto *d_ev = (trm_cuda_event *)(d + o_ev);
+    auto *d_off = (long long *)(d + o_off);
+    auto *d_cnt = (int *)(d + o_cnt);
+    auto *d_fg = (trm_cuda_framegen *)(d + o_fg);
+    auto *d_seed = (float *)(d + o_seed);
+    auto *d_frames = (double *)(d + o_frames);
+    cudaStream_t s = ctx->s_out;
     CK(cudaMemcpyAsync(d_desc, desc, (size_t)n * sizeof(trm_cuda_utterance), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(d_ev, events, (size_t)n_events * sizeof(trm_cuda_event), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(d_off, off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, s));
@@ -1137,6 +1067,17 @@ static int pool_err(int code, const char *what)
 {
     g_err = what;
     return code;
+}
+
+// one entry of a call that names slots: slot s exists, is open and was not named by an earlier entry (named[], one flag
+// per slot, records it); `who` names the call in the messages
+static int pool_check_slot(const trm_cuda_pool *p, int s, std::vector<unsigned char> &named, const char *who)
+{
+    if (s < 0 || s >= p->cap) return pool_err(-4, (std::string(who) + ": no such slot").c_str());
+    if (!p->slots[s].open) return pool_err(-7, (std::string(who) + ": the slot is not open").c_str());
+    if (named[s]) return pool_err(-4, (std::string(who) + ": a slot is named twice").c_str());
+    named[s] = 1;
+    return 0;
 }
 
 int trm_cuda_pool_create(trm_cuda_ctx *ctx, int precision, int capacity, int max_frames_per_push, trm_cuda_pool **out)
@@ -1349,10 +1290,8 @@ int trm_cuda_pool_set_voice(trm_cuda_pool *p, int n, const int32_t *slot, const 
         std::vector<unsigned char> named((size_t)p->cap, 0);
         for (int i = 0; i < n; ++i) {
             const int s = slot[i];
-            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_set_voice: no such slot");
-            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_set_voice: the slot is not open");
-            if (named[s]) return pool_err(-4, "trm_cuda_pool_set_voice: a slot is named twice");
-            named[s] = 1;
+            const int rc = pool_check_slot(p, s, named, "trm_cuda_pool_set_voice");
+            if (rc != 0) return rc;
             const trm_cuda_utterance &v = voice[i], &c = p->slots[s].voice;
             if (v.controlPeriod != c.controlPeriod || v.sampleRate != c.sampleRate || v.tri != c.tri || v.padSize != c.padSize ||
                 v.channels != c.channels)
@@ -1362,21 +1301,21 @@ int trm_cuda_pool_set_voice(trm_cuda_pool *p, int n, const int32_t *slot, const 
     if (n == 0) return 0;
     // ---- one upload ([segments][rows]), one scatter to the slots' wavetable rows ----------------------------------------
     const size_t wt = TRM_TABLE_LENGTH * sizeof(double);
-    const size_t o_wt = align_up((size_t)n * sizeof(trm::CopySeg), 256);
-    const size_t bytes = o_wt + (size_t)n * wt;
+    Pack pk;
+    const size_t o_seg = pk.part((size_t)n * sizeof(trm::CopySeg)), o_wt = pk.part((size_t)n * wt), bytes = pk.bytes;
     CK(cudaSetDevice(p->ctx->device));
     int rc;
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
     if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
     unsigned char *h = p->stage.base, *d = p->scratch.base;
-    trm::CopySeg *seg = (trm::CopySeg *)h;
+    trm::CopySeg *seg = (trm::CopySeg *)(h + o_seg);
     memcpy(h + o_wt, wavetables, (size_t)n * wt);
     for (int i = 0; i < n; ++i)
         seg[i] = {(unsigned long long)(uintptr_t)(d + o_wt + (size_t)i * wt),
                   (unsigned long long)(uintptr_t)(p->d_wavetables + (size_t)slot[i] * TRM_TABLE_LENGTH), wt};
     cudaStream_t cs = p->st;
     CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
-    const trm::SegCopyArgs a{(const trm::CopySeg *)d, n};
+    const trm::SegCopyArgs a{(const trm::CopySeg *)(d + o_seg), n};
     if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("voice change scatter launch", (cudaError_t)rc);
     CK(cudaStreamSynchronize(cs));
     // ---- the slots change only now that the rows are in place -----------------------------------------------------------
@@ -1435,10 +1374,8 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
         std::vector<unsigned char> named((size_t)p->cap, 0);
         for (int i = 0; i < n; ++i) {
             const int s = slot[i];
-            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_push: no such slot");
-            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_push: the slot is not open");
-            if (named[s]) return pool_err(-4, "trm_cuda_pool_push: a slot is named twice");
-            named[s] = 1;
+            const int rc = pool_check_slot(p, s, named, "trm_cuda_pool_push");
+            if (rc != 0) return rc;
             if (n_frames[i] < 0 || n_frames[i] > p->max_m) return pool_err(-4, "trm_cuda_pool_push: more frames than the pool was created for");
             if (pcm && !(std::isfinite(pcm->peak[i]) && pcm->peak[i] > 0.0)) return pool_err(-4, "trm_cuda_pool_push_pcm16: a peak is not finite and > 0");
             const trm_cuda_pool::Slot &sl = p->slots[s];
@@ -1546,21 +1483,16 @@ static int pool_push(trm_cuda_pool *p, int n, const int32_t *slot, const int32_t
     }
     std::stable_sort(wg.begin(), wg.end(), [&](int a, int b) { return E[a].n_new > E[b].n_new; });
     const size_t n_rd = rd.size(), n_mv = mv.size();
-    const size_t o_dt = 0;
-    const size_t o_ord = o_dt + align_up(wg.size() * sizeof(trm_cuda_utterance), 256);
-    const size_t o_rst = o_ord + align_up(wg.size() * sizeof(int), 256);
-    const size_t o_rd = o_rst + align_up(wg.size() * sizeof(int), 256);
-    const size_t o_ib = o_rd + align_up(n_rd * sizeof(trm_cuda_utterance), 256);
-    const size_t o_mv = o_ib + align_up(ib.size() * sizeof(long long), 256);
     const size_t n_pk = pcm ? n_rd : 0;                   // PCM: peak and max |y| of each resampler view
-    const size_t o_pk = o_mv + align_up(n_mv * sizeof(trm::CopySeg), 256);
-    const size_t o_mx = o_pk + align_up(n_pk * sizeof(double), 256);
     const size_t n_ge = ge.size(), n_fs = fs.size() + n_fb;
-    const size_t o_ge = o_mx + align_up(n_pk * sizeof(unsigned long long), 256);
-    const size_t o_fs = o_ge + align_up(n_ge * sizeof(trm::FrameGenPoolEntry), 256);
-    const size_t o_fr = o_fs + align_up(n_fs * sizeof(trm::CopySeg), 256);
+    Pack pk;
+    const size_t o_dt = pk.part(wg.size() * sizeof(trm_cuda_utterance)), o_ord = pk.part(wg.size() * sizeof(int)),
+                 o_rst = pk.part(wg.size() * sizeof(int)), o_rd = pk.part(n_rd * sizeof(trm_cuda_utterance)),
+                 o_ib = pk.part(ib.size() * sizeof(long long)), o_mv = pk.part(n_mv * sizeof(trm::CopySeg)),
+                 o_pk = pk.part(n_pk * sizeof(double)), o_mx = pk.part(n_pk * sizeof(unsigned long long)),
+                 o_ge = pk.part(n_ge * sizeof(trm::FrameGenPoolEntry)), o_fs = pk.part(n_fs * sizeof(trm::CopySeg));
     // the frame region holds the frame-fed entries' frames (uploaded), then the event-fed ones' (copied on the device)
-    const size_t bytes = o_fr + (size_t)wg_frames * 128, up = o_fr + (size_t)fed_frames * 128;
+    const size_t o_fr = pk.part((size_t)wg_frames * 128), bytes = pk.bytes, up = o_fr + (size_t)fed_frames * 128;
     if (pcm && p->pcm_cap < 2 * p->cap * p->cap_out) {   // stereo: two int16 per sample
         if (p->d_pcm) cudaFree(p->d_pcm);
         p->d_pcm = nullptr;
@@ -1799,11 +1731,9 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
         std::vector<unsigned char> named((size_t)p->cap, 0);
         for (int i = 0; i < n; ++i) {
             const int s = slot[i];
-            if (s < 0 || s >= p->cap) return pool_err(-4, "trm_cuda_pool_save: no such slot");
-            if (!p->slots[s].open) return pool_err(-7, "trm_cuda_pool_save: the slot is not open");
-            if (named[s]) return pool_err(-4, "trm_cuda_pool_save: a slot is named twice");
+            const int rc = pool_check_slot(p, s, named, "trm_cuda_pool_save");
+            if (rc != 0) return rc;
             if (p->slots[s].events && !ev) return pool_err(-7, "trm_cuda_pool_save: a slot fed from an event list has no version 1 snapshot");
-            named[s] = 1;
         }
     }
     for (int i = 0; i < n; ++i) {
@@ -1829,14 +1759,14 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
         sg[i] = snap_stage(p, slot[i], p->slots[slot[i]], pool_gen_bytes(st[i]));
         at[i + 1] = at[i] + sg[i].bytes();
     }
-    const size_t o_stg = align_up((size_t)SnapStage::N_PARTS * n * sizeof(trm::CopySeg), 256);
-    const size_t bytes = o_stg + at[n];
+    Pack pk;
+    const size_t o_seg = pk.part((size_t)SnapStage::N_PARTS * n * sizeof(trm::CopySeg)), o_stg = pk.part(at[n]), bytes = pk.bytes;
     int rc;
     CK(cudaSetDevice(p->ctx->device));
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
     if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
     unsigned char *h = p->stage.base, *d = p->scratch.base;
-    trm::CopySeg *seg = (trm::CopySeg *)h;
+    trm::CopySeg *seg = (trm::CopySeg *)(h + o_seg);
     int n_seg = 0;
     for (int i = 0; i < n; ++i) {
         unsigned long long to = (unsigned long long)(uintptr_t)(d + o_stg + at[i]);
@@ -1848,8 +1778,8 @@ int trm_cuda_pool_save(trm_cuda_pool *p, int n, const int32_t *slot, trm_cuda_po
     }
     if (n_seg > 0) {
         cudaStream_t cs = p->st;
-        CK(cudaMemcpyAsync(d, h, (size_t)n_seg * sizeof(trm::CopySeg), cudaMemcpyHostToDevice, cs));
-        const trm::SegCopyArgs a{(const trm::CopySeg *)d, n_seg};
+        CK(cudaMemcpyAsync(d + o_seg, h + o_seg, (size_t)n_seg * sizeof(trm::CopySeg), cudaMemcpyHostToDevice, cs));
+        const trm::SegCopyArgs a{(const trm::CopySeg *)(d + o_seg), n_seg};
         if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("snapshot gather launch", (cudaError_t)rc);
         CK(cudaMemcpyAsync(h + o_stg, d + o_stg, at[n], cudaMemcpyDeviceToHost, cs));
         CK(cudaStreamSynchronize(cs));
@@ -1935,14 +1865,14 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
         sg[i] = snap_stage(p, free_slot[i], made[i], gs);
         at[i + 1] = at[i] + sg[i].bytes();
     }
-    const size_t o_wt = align_up((size_t)(1 + SnapStage::N_PARTS) * n * sizeof(trm::CopySeg), 256);
-    const size_t o_dev = o_wt + (size_t)n * wt;
-    const size_t bytes = o_dev + at[n];
+    Pack pk;
+    const size_t o_seg = pk.part((size_t)(1 + SnapStage::N_PARTS) * n * sizeof(trm::CopySeg)), o_wt = pk.part((size_t)n * wt),
+                 o_dev = pk.part(at[n]), bytes = pk.bytes;
     CK(cudaSetDevice(p->ctx->device));
     if ((rc = p->scratch.reserve(bytes + 256)) != 0) return rc;
     if ((rc = p->stage.reserve(bytes + 256)) != 0) return rc;
     unsigned char *h = p->stage.base, *d = p->scratch.base;
-    trm::CopySeg *seg = (trm::CopySeg *)h;
+    trm::CopySeg *seg = (trm::CopySeg *)(h + o_seg);
     int n_seg = 0;
     memcpy(h + o_wt, wavetables, (size_t)n * wt);
     for (int i = 0; i < n; ++i) {
@@ -1971,7 +1901,7 @@ int trm_cuda_pool_restore(trm_cuda_pool *p, int n, const trm_cuda_utterance *voi
     }
     cudaStream_t cs = p->st;
     CK(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, cs));
-    const trm::SegCopyArgs a{(const trm::CopySeg *)d, n_seg};
+    const trm::SegCopyArgs a{(const trm::CopySeg *)(d + o_seg), n_seg};
     if ((rc = trm_k_segment_copy(&a, cs)) != 0) return fail("snapshot scatter launch", (cudaError_t)rc);
     CK(cudaStreamSynchronize(cs));
     // ---- the slots open only now that the device work has finished without error -------------------------------------
@@ -1996,14 +1926,14 @@ int trm_cuda_resident_create(trm_cuda_ctx *ctx, int precision, int n, const trm_
     r->precision = precision;
     int rc;
     if ((rc = plan_chunk(desc, 0, n, ctx->ki(precision), r->plan)) != 0) { delete r; return rc; }
-    if ((rc = r->arena.reserve(r->plan.arena_bytes(esz, true))) != 0) { delete r; return rc; }
-    carve(r->arena, r->plan, esz, true, r->dc);
-    if ((rc = upload_plan(r->plan, r->dc, nullptr, 0)) != 0 || (rc = upload_frames(r->plan, r->dc, desc, frames_host, 0)) != 0) {
+    chunk_layout(r->plan, esz, true);
+    if ((rc = r->arena.reserve(r->plan.arena)) != 0) { delete r; return rc; }
+    if ((rc = upload_plan(r->plan, r->arena.base, nullptr, 0)) != 0 || (rc = upload_frames(r->plan, r->arena.base, desc, frames_host, 0)) != 0) {
         r->arena.release();
         delete r;
         return rc;
     }
-    CK(cudaMemset(r->dc.maxbits, 0, (size_t)n * sizeof(unsigned long long)));
+    CK(cudaMemset(r->arena.base + r->plan.at.maxbits, 0, (size_t)n * sizeof(unsigned long long)));
     if (!ctx->wt_host.empty()) {
         if (cudaMalloc((void **)&r->d_wavetables, ctx->wt_host.size() * sizeof(double)) != cudaSuccess ||
             cudaMemcpy(r->d_wavetables, ctx->wt_host.data(), ctx->wt_host.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) {
@@ -2012,7 +1942,6 @@ int trm_cuda_resident_create(trm_cuda_ctx *ctx, int precision, int n, const trm_
             delete r;
             return fail("resident wavetables", cudaGetLastError());
         }
-        r->dc.wavetables = r->d_wavetables;
     }
     CK(cudaDeviceSynchronize());
     *out = r;
@@ -2032,7 +1961,7 @@ void trm_cuda_resident_destroy(trm_cuda_resident *r)
 int trm_cuda_resident_stage(trm_cuda_resident *r, int stage, void *stream)
 {
     CK(cudaSetDevice(r->ctx->device));
-    return launch_stage(r->ctx, r->precision, stage, r->dc, (cudaStream_t)stream);
+    return launch_stage(r->ctx, r->precision, stage, r->plan, r->arena.base, r->d_wavetables, (cudaStream_t)stream);
 }
 
 int trm_cuda_resident_run(trm_cuda_resident *r, void *stream)
@@ -2050,18 +1979,15 @@ int trm_cuda_resident_fetch(trm_cuda_resident *r, int16_t *pcm_host, void *sampl
     CK(cudaDeviceSynchronize());
     const size_t esz = prec_esz(r->precision);
     const ChunkPlan &p = r->plan;
-    long long c_hi = 0, o_hi = 0, t_hi = 0;
-    for (const auto &d : p.desc) {
-        c_hi = std::max<long long>(c_hi, d.pcm_offset + d.n_out * d.channels);
-        o_hi = std::max<long long>(o_hi, d.out_offset + d.n_out);
-        t_hi = std::max<long long>(t_hi, d.tube_offset + d.n_tube);
-    }
-    if (pcm_host && c_hi) CK(cudaMemcpy(pcm_host + p.pcm_lo, r->dc.pcm, (size_t)c_hi * sizeof(int16_t), cudaMemcpyDeviceToHost));
-    if (samples_host && o_hi) CK(cudaMemcpy((unsigned char *)samples_host + (size_t)p.out_lo * esz, r->dc.out, (size_t)o_hi * esz, cudaMemcpyDeviceToHost));
-    if (tube_host && t_hi) CK(cudaMemcpy((unsigned char *)tube_host + (size_t)p.tube_lo * esz, r->dc.tube, (size_t)t_hi * esz, cudaMemcpyDeviceToHost));
+    const unsigned char *base = r->arena.base;
+    if (pcm_host && p.pcm_n) CK(cudaMemcpy(pcm_host + p.pcm_lo, base + p.at.pcm, (size_t)p.pcm_n * sizeof(int16_t), cudaMemcpyDeviceToHost));
+    if (samples_host && p.out_n)
+        CK(cudaMemcpy((unsigned char *)samples_host + (size_t)p.out_lo * esz, base + p.at.out, (size_t)p.out_n * esz, cudaMemcpyDeviceToHost));
+    if (tube_host && p.tube_n)
+        CK(cudaMemcpy((unsigned char *)tube_host + (size_t)p.tube_lo * esz, base + p.at.tube, (size_t)p.tube_n * esz, cudaMemcpyDeviceToHost));
     if (max_host && !p.desc.empty()) {
         std::vector<unsigned long long> mb(p.desc.size());
-        CK(cudaMemcpy(mb.data(), r->dc.maxbits, mb.size() * sizeof(mb[0]), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(mb.data(), base + p.at.maxbits, mb.size() * sizeof(mb[0]), cudaMemcpyDeviceToHost));
         for (size_t i = 0; i < mb.size(); ++i) memcpy(&max_host[i], &mb[i], sizeof(double));
     }
     return 0;
@@ -2101,13 +2027,17 @@ int trm_cuda_sweep(trm_cuda_ctx *ctx, int precision, const trm_cuda_utterance *v
     ChunkPlan plan;
     int rc;
     if ((rc = plan_chunk(desc.data(), 0, C, ki, plan)) != 0) return rc;
+    chunk_layout(plan, esz, true);
+    Pack pk{plan.arena};
+    const size_t o_sums = pk.part((size_t)C * sizeof(unsigned long long));
     Arena &arena = ctx->arenas[0];
-    if ((rc = arena.reserve(plan.arena_bytes(esz, true) + (size_t)C * sizeof(unsigned long long) + 4096)) != 0) return rc;
-    DeviceChunk dc;
-    carve(arena, plan, esz, true, dc);
-    unsigned long long *d_sums = (unsigned long long *)arena.take((size_t)C * sizeof(unsigned long long));
-    cudaStream_t st = ctx->streams[2];
-    if ((rc = upload_plan(plan, dc, nullptr, st)) != 0) return rc;
+    if ((rc = arena.reserve(pk.bytes)) != 0) return rc;
+    unsigned char *base = arena.base;
+    auto *d_sums = (unsigned long long *)(base + o_sums);
+    const auto *d_desc = (const trm_cuda_utterance *)(base + plan.at.desc);
+    const int16_t *d_pcm = (const int16_t *)(base + plan.at.pcm);
+    cudaStream_t st = ctx->s_out;
+    if ((rc = upload_plan(plan, base, nullptr, st)) != 0) return rc;
     std::vector<unsigned long long> mb((size_t)C);
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
@@ -2118,20 +2048,20 @@ int trm_cuda_sweep(trm_cuda_ctx *ctx, int precision, const trm_cuda_utterance *v
         const int m = (int)std::min<int64_t>(C, n - at);
         // (a short last chunk runs the full plan: the utterances beyond m keep the previous chunk's frames and are ignored)
         CK(cudaEventRecord(e0, st));
-        if (trm_k_workload_walk2(seed, first_index + (uint64_t)at, m, n_frames, dc.frames, st) != 0) return fail_msg("walk2 launch");
+        if (trm_k_workload_walk2(seed, first_index + (uint64_t)at, m, n_frames, (double *)(base + plan.at.frames), st) != 0) return fail_msg("walk2 launch");
         for (int stage = 0; stage < TRM_STAGE_COUNT; ++stage)
-            if ((rc = launch_stage(ctx, precision, stage, dc, st)) != 0) return rc;
-        if (trm_k_pcm_checksum(dc.desc, m, dc.pcm, d_sums, st) != 0) return fail_msg("checksum launch");
+            if ((rc = launch_stage(ctx, precision, stage, plan, base, nullptr, st)) != 0) return rc;
+        if (trm_k_pcm_checksum(d_desc, m, d_pcm, d_sums, st) != 0) return fail_msg("checksum launch");
         CK(cudaEventRecord(e1, st));
         n_launch += 5;
         CK(cudaMemcpyAsync(checksums_host + at, d_sums, (size_t)m * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(mb.data(), dc.maxbits, (size_t)m * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(mb.data(), base + plan.at.maxbits, (size_t)m * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         while (probe_at < n_probe && probe_utt[probe_at] < at + m) {
             const int64_t k = probe_utt[probe_at] - at;
             if (k >= 0) {
                 const trm_cuda_utterance &d = plan.desc[(size_t)k];
                 const int64_t cnt = std::min<int64_t>(d.n_out * d.channels, probe_stride);
-                CK(cudaMemcpyAsync(probe_pcm + probe_at * probe_stride, dc.pcm + d.pcm_offset, (size_t)cnt * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(probe_pcm + probe_at * probe_stride, d_pcm + d.pcm_offset, (size_t)cnt * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
             }
             ++probe_at;
         }
@@ -2157,11 +2087,11 @@ int trm_cuda_resident_fetch_utterance(trm_cuda_resident *r, int u, void *samples
     if (u < 0 || u >= (int)r->plan.desc.size()) return fail_msg("trm_cuda_resident_fetch_utterance: no such utterance");
     const size_t esz = prec_esz(r->precision);
     const trm_cuda_utterance &d = r->plan.desc[u];
-    if (samples_host && d.n_out) CK(cudaMemcpy(samples_host, (unsigned char *)r->dc.out + (size_t)d.out_offset * esz, (size_t)d.n_out * esz, cudaMemcpyDeviceToHost));
-    if (pcm_host && d.n_out) CK(cudaMemcpy(pcm_host, r->dc.pcm + d.pcm_offset, (size_t)d.n_out * d.channels * sizeof(int16_t), cudaMemcpyDeviceToHost));
+    if (samples_host && d.n_out) CK(cudaMemcpy(samples_host, r->arena.base + r->plan.at.out + (size_t)d.out_offset * esz, (size_t)d.n_out * esz, cudaMemcpyDeviceToHost));
+    if (pcm_host && d.n_out) CK(cudaMemcpy(pcm_host, (const int16_t *)(r->arena.base + r->plan.at.pcm) + d.pcm_offset, (size_t)d.n_out * d.channels * sizeof(int16_t), cudaMemcpyDeviceToHost));
     if (max_host) {
         unsigned long long mb = 0;
-        CK(cudaMemcpy(&mb, r->dc.maxbits + u, sizeof mb, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(&mb, (const unsigned long long *)(r->arena.base + r->plan.at.maxbits) + u, sizeof mb, cudaMemcpyDeviceToHost));
         memcpy(max_host, &mb, sizeof(double));
     }
     return 0;

@@ -888,9 +888,9 @@ static void *shard_main(void *arg)
     j->rc = acquire_ctx(j->device, &ctx, &lane);
     if (j->rc == TRM_OK) {
         if (trm_cuda_set_wavetables(ctx, j->b->voices.tables, j->b->voices.n) != 0 ||
-            trm_cuda_synthesize_host_fmt(ctx, j->b->precision, j->b->frame_format, j->u1 - j->u0, j->b->desc + j->u0, j->frames,
-                                         j->pcm, j->samples, j->b->maxima + j->u0, j->tube, &j->launches, j->enqueued,
-                                         j->enqueued_arg) != 0)
+            trm_cuda_synthesize_host(ctx, j->b->precision, j->b->frame_format, j->u1 - j->u0, j->b->desc + j->u0, j->frames,
+                                     j->pcm, j->samples, j->b->maxima + j->u0, j->tube, &j->launches, j->enqueued,
+                                     j->enqueued_arg) != 0)
             j->rc = cuda_err();
         release_ctx(j->device, lane);
     }
@@ -1089,8 +1089,8 @@ int TRMBatchSynthesizeEvents(TRMBatch *b, const TRMEvent *events, const int64_t 
     if (trm_cuda_set_wavetables(ctx, b->voices.tables, b->voices.n) != 0 ||
         trm_cuda_generate_frames(ctx, b->n, b->desc, (const trm_cuda_event *)events, event_offset, n_events,
                                  (const trm_cuda_framegen *)fg, shared_fg, &frames_dev, NULL, NULL) != 0 ||
-        trm_cuda_synthesize_host(ctx, b->precision, b->n, b->desc, frames_dev, pcm_out, samples_out, b->maxima, NULL,
-                                 &b->launches) != 0)
+        trm_cuda_synthesize_host(ctx, b->precision, 0, b->n, b->desc, frames_dev, pcm_out, samples_out, b->maxima, NULL,
+                                 &b->launches, NULL, NULL) != 0)
         rc = cuda_err();
     else
         b->launches += 1;

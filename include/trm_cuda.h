@@ -116,29 +116,21 @@ int  trm_cuda_set_wavetables(trm_cuda_ctx *ctx, const double *tables, int n_voic
  * n utterances described by desc[] (offsets relative to the host arrays) to the device in chunks,
  * runs the three stages, copies PCM / samples / max back.  Chunks are double-buffered over CUDA
  * streams so copies overlap kernels.  Blocking.
+ *   frame_format 0 = TRMParameters rows of 16 doubles (128 bytes), 1 = rows of 16 floats (64 bytes; what Monet's
+ *                generator holds, EventList.m:968-1002), staged as they are and widened by the waveguide kernel when a
+ *                parameter lane reads its value -- half the upload, identical results
  *   pcm_host     int16 [..]  or NULL      samples_host  double/float [..] or NULL
  *   max_host     double[n]   or NULL      tube_host     double/float tube-rate signal or NULL
  *   launches     receives the number of kernel launches issued (may be NULL)
+ *   enqueued     (may be NULL) `enqueued(arg)` is invoked once, from the calling thread, as soon as the first chunk's
+ *                copies and kernels are in the device queues -- libtrm's asynchronous tickets use it to start
+ *                concurrent calls in submission order (the queues are shared per device, so the order of arrival
+ *                there is the order of execution)
  */
-int trm_cuda_synthesize_host(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,
-                             const double *frames_host, int16_t *pcm_host, void *samples_host,
-                             double *max_host, void *tube_host, int64_t *launches);
-
-/* Same call; `enqueued(arg)` (may be NULL) is invoked once, from the calling thread, as soon as the first chunk's copies
- * and kernels are in the device queues -- libtrm's asynchronous tickets use it to start concurrent calls in submission
- * order (the queues are shared per device, so the order of arrival there is the order of execution). */
-int trm_cuda_synthesize_host_ex(trm_cuda_ctx *ctx, int precision, int n, const trm_cuda_utterance *desc,
-                                const double *frames_host, int16_t *pcm_host, void *samples_host,
-                                double *max_host, void *tube_host, int64_t *launches,
-                                void (*enqueued)(void *), void *arg);
-
-/* The same call with the frame format given: 0 = TRMParameters rows of 16 doubles (128 bytes), 1 = rows of 16 floats
- * (64 bytes; what Monet's generator holds, EventList.m:968-1002), staged as they are and widened by the waveguide kernel
- * when a parameter lane reads its value -- half the upload, identical results. */
-int trm_cuda_synthesize_host_fmt(trm_cuda_ctx *ctx, int precision, int frame_format, int n, const trm_cuda_utterance *desc,
-                                 const void *frames_host, int16_t *pcm_host, void *samples_host,
-                                 double *max_host, void *tube_host, int64_t *launches,
-                                 void (*enqueued)(void *), void *arg);
+int trm_cuda_synthesize_host(trm_cuda_ctx *ctx, int precision, int frame_format, int n, const trm_cuda_utterance *desc,
+                             const void *frames_host, int16_t *pcm_host, void *samples_host,
+                             double *max_host, void *tube_host, int64_t *launches,
+                             void (*enqueued)(void *), void *arg);
 
 /*
  * Device-resident path (bench `value`, roofline timing): inputs uploaded once, stages launched on the
@@ -154,7 +146,6 @@ int  trm_cuda_resident_fetch(trm_cuda_resident *res, int16_t *pcm_host, void *sa
                              double *max_host, void *tube_host);                 /* blocking D2H          */
 int  trm_cuda_resident_fetch_utterance(trm_cuda_resident *res, int u, void *samples_host, int16_t *pcm_host,
                                        double *max_host);                        /* one utterance, blocking */
-int  trm_cuda_stage_launches(int stage);     /* kernel launches one stage issues */
 /* Sweep (BASELINE configs[4]): n utterances of one voice x n_frames frames, control tracks = the walk2 workload
  * (include/trm_workload.h) generated on the device (utterance k: index first_index + k of stream seed), synthesized in
  * chunks of one full wave; per utterance an 8-byte PCM checksum sum(pcm[i] * (2 i + 1)) mod 2^64 and the maximum come back,
